@@ -1,7 +1,7 @@
 """bench.py -- headline benchmark of the B200 segmentation hot path (see the contract in DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload predict64|batch32|train|cli]
-                    [--precision bf16|fp16]
+                    [--precision bf16|fp16] [--dump-outputs DIR]
 
 workload predict64 (default, BASELINE.json configs[1]): a "step" is one pass of the predict hot path over a batch
 of 64 synthetic raw 4096x4096x3 scans (BMP pixel arrays: BGR, bottom-up, dark bands) with --exclude_nodes:
@@ -53,7 +53,15 @@ def parse():
     ap.add_argument('--precision', default='fp16', choices=['bf16', 'fp16'],
                     help='16-bit storage format of activations / weights on the predict path (same tcgen05 kind::f16 rate); '
                          'fp16 is the shipped default (meets the parity bar), bf16 is opt-in')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 / '
+                         'float64, at most 64 MB; rank 0), to compare two builds output for output on the same seeded inputs')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
+    return args
 
 
 def peaks():
@@ -148,6 +156,65 @@ def synth_processed_cpu(seed, rows=None):
     from oracle import synth
     raw, top, bottom = synth.raw_image_u8(seed, RAW)
     return raw
+
+
+# ---------------------------------------------------------------------------------------------------- output dump
+# --dump-outputs keeps fixed, seeded samples where the whole output would not fit in DUMP_LIMIT: masks of 64 images as
+# float32 are 256 MB, the weights of a training step 132 MB.  The positions depend on nothing but the seed, so two builds
+# are compared at the same pixels and the same weights.
+DUMP_LIMIT = 64 << 20
+DUMP_PIXELS = 1 << 17       # per mask canvas of 1024 x 1024: one pixel in eight (32 MB for 64 images)
+DUMP_WEIGHTS = 1 << 20      # of the 32.9 M weights and BatchNorm statistics
+
+
+def sample_index(n, k, seed=0):
+    """k sorted positions out of n, the same from run to run."""
+    return np.sort(np.random.default_rng(seed).choice(n, size=min(k, n), replace=False))
+
+
+def mask_sample(masks, heights=None):
+    """masks: u8 class canvases [n, H, W] (device or host); heights: rows of each canvas that belong to its image (None:
+    all of them).  -> float32 [n, DUMP_PIXELS], the class at fixed canvas positions, -1 where a position lies below the
+    image (those canvas rows are not part of the result)."""
+    n, H, W = masks.shape
+    idx = torch.from_numpy(sample_index(H * W, DUMP_PIXELS)).to(masks.device)
+    out = masks.reshape(n, H * W)[:, idx].float()
+    if heights is not None:
+        out[(idx // W).view(1, -1) >= heights.to(out.device).view(-1, 1)] = -1.0
+    return out.cpu().numpy()
+
+
+def weight_sample(trainer):
+    """float32 [DUMP_WEIGHTS]: the trainer's weights and BatchNorm statistics (state_dict order) at fixed positions."""
+    flat = torch.cat([v.detach().float().flatten().cpu() for v in trainer.state_dict().values() if v.is_floating_point()])
+    return flat[torch.from_numpy(sample_index(flat.numel(), DUMP_WEIGHTS))].numpy()
+
+
+def cli_outputs(root, rows):
+    """What predict.py left for its caller: the numbers of final_stats.csv and the dual masks of results/outputs (classes
+    stored as 0 / 127 / 255), the masks on 1024-wide canvases like the engine's."""
+    from PIL import Image
+    stats = np.array([[float(v) for v in r[2:]] for r in rows[1:]], dtype=np.float64)
+    masks = torch.zeros((len(rows) - 1, RAW // 4, RAW // 4), dtype=torch.uint8)
+    heights = torch.zeros(len(rows) - 1, dtype=torch.int64)
+    for i, (name, wood) in enumerate(r[:2] for r in rows[1:]):
+        m = torch.from_numpy(np.asarray(Image.open(os.path.join(root, 'results', 'outputs', wood, name))) // 127)
+        masks[i, :m.shape[0], :m.shape[1]] = m
+        heights[i] = m.shape[0]
+    return {'stats': stats, 'heights': heights.numpy().astype(np.float64), 'mask_sample': mask_sample(masks, heights)}
+
+
+def write_dump(path, arrays):
+    """arrays: name -> float32 / float64 numpy array, written as path/<name>.npy."""
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError('--dump-outputs: %s is %s, not float32 / float64' % (name, a.dtype))
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError('--dump-outputs: %d bytes exceed the %d-byte limit' % (total, DUMP_LIMIT))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 # ---------------------------------------------------------------------------------------------------- reference arm
@@ -278,6 +345,12 @@ def main():
             ms = float(t.item())
         return ms, launches
 
+    def dump(outputs):
+        """--dump-outputs: outputs() -> what the last timed step returned; called right after the timed steps, before the
+        end-to-end pass reuses the buffers."""
+        if args.dump_outputs and rank == 0:
+            write_dump(args.dump_outputs, outputs())
+
     if args.workload == 'train':
         # BASELINE.json configs[3]: one training step (fwd + weighted CE + bwd + all-reduce + Adam), batch 8 per GPU
         from oracle import synth
@@ -297,6 +370,7 @@ def main():
         sampler.start()
         ms, launches = timed(step, args.steps, args.warmup)
         clocks = sampler.summary()
+        dump(lambda: {'loss': np.array([float(res['loss'])], dtype=np.float64), 'weights_sample': weight_sample(tr)})
         # end to end: this step's images and targets come from pinned host memory, the loss is read back every step
         imgs_d, tgt_d = torch.empty_like(imgs), torch.empty_like(tgt)
 
@@ -362,6 +436,7 @@ def main():
                 if it >= args.warmup:
                     times.append(time.perf_counter() - t0)
             n_files = sum(len(f) for _, _, f in os.walk(os.path.join(root, 'results'))) + sum(len(f) for _, _, f in os.walk(os.path.join(root, 'processed')))
+            dump(lambda: cli_outputs(root, rows))
         finally:
             shutil.rmtree(root, ignore_errors=True)
         if rank == 0:
@@ -385,14 +460,16 @@ def main():
         imgs = torch.from_numpy(np.stack([synth.texture_u8(1024, 1024, 100 * rank + i) for i in range(min(B, 4))])).to(dev)
         imgs = imgs.repeat((B + imgs.shape[0] - 1) // imgs.shape[0], 1, 1, 1)[:B].contiguous()
         from neuralbarkcalculator_b200 import ops
+        last = {}
 
         def step():
             mask = calc.model.predict_mask_u8(imgs)
-            ops.remove_small_zones_u8(mask, 150, exclude_nodes=True)
+            last['out'] = ops.remove_small_zones_u8(mask, 150, exclude_nodes=True)
         sampler = ClockSampler(local_rank)
         sampler.start()
         ms, launches = timed(step, args.steps, args.warmup)
         clocks = sampler.summary()
+        dump(lambda: {'counts': last['out'][1].cpu().numpy().astype(np.float64), 'mask_sample': mask_sample(last['out'][0])})
         n_img = B
         mean_rows, prof_n, prof_h = 1024.0, B, 1024
         # end to end: the processed u8 images come from pinned host memory, masks + counts go back to pinned host memory
@@ -426,6 +503,9 @@ def main():
         sampler.start()
         ms, launches = timed(step, args.steps, args.warmup)
         clocks = sampler.summary()
+        counts, masks, heights = last['out']
+        dump(lambda: {'counts': counts.cpu().numpy().astype(np.float64), 'heights': heights.cpu().numpy().astype(np.float64),
+                      'mask_sample': mask_sample(masks, heights)})
         n_img = B
         mean_rows = float(last['out'][2].float().mean().item())      # trimmed heights of this rank's scans
         prof_n, prof_h = eng.chunk, 624
