@@ -261,8 +261,15 @@ int nbc_train_num_segments(const nbc_train_plan* plan);
 int nbc_train_segment(const nbc_train_plan* plan, int i, int64_t* offset, int64_t* count);
 int nbc_train_wait_segment(nbc_train_plan* plan, int i, void* stream);
 /* test / debug accessors: workspace byte offset + {N,H,W,C} of an intermediate (what: 0 z of unit, 1 y of unit,
- * 2 low-res logits, 3 full-res logits, 4 dL/dfull, 5 dL/dlow); units are in state_dict order (0 = stem). */
+ * 2 low-res logits, 3 full-res logits, 4 dL/dfull, 5 dL/dlow); units are in state_dict order (0 = stem).
+ * what 6 / 7 = dy / dz of the BatchNorm backward of unit `index` (bf16 NHWC, the geometry of z): byte offsets into the
+ * CAPTURE buffer, not the workspace; they hold data only for a step run with capture on. */
 int64_t nbc_train_debug_offset(const nbc_train_plan* plan, int what, int index, int32_t* dims_out);
+/* Capture for tests: with a device buffer of >= nbc_train_capture_bytes set, every nbc_train_forward_backward copies the
+ * dy its BatchNorm backward consumes and the dz it produces, per unit, into `buf` (cudaMemcpyAsync on the step's stream).
+ * The backward reuses its gradient buffers, so these are gone otherwise.  buf = NULL turns capture off (the default). */
+size_t nbc_train_capture_bytes(const nbc_train_plan* plan);
+int nbc_train_set_capture(nbc_train_plan* plan, void* buf, size_t bytes);
 int nbc_train_num_units(const nbc_train_plan* plan);
 /* weight-gradient kernels used by the plan: 0 = tcgen05 (default), 1 = mma.sync / CUDA-core cross-check kernels */
 int nbc_train_set_wgrad_impl(nbc_train_plan* plan, int impl);

@@ -85,6 +85,8 @@ SIGNATURES = {
     'nbc_train_wait_segment': (c_int, [c_void_p, c_int, c_void_p]),
     'nbc_train_debug_offset': (c_i64, [c_void_p, c_int, c_int, C.POINTER(C.c_int32)]),
     'nbc_train_num_units': (c_int, [c_void_p]),
+    'nbc_train_capture_bytes': (c_size_t, [c_void_p]),
+    'nbc_train_set_capture': (c_int, [c_void_p, c_void_p, c_size_t]),
     'nbc_train_set_wgrad_impl': (c_int, [c_void_p, c_int]),
     'nbc_train_set_loss': (c_int, [c_void_p, c_int]),
     'nbc_train_adam': (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_i64, c_float, c_float, c_float, c_float, c_float,

@@ -25,6 +25,7 @@ struct Unit {
   int sd_index;                // index of the conv weight in the 326-tensor state_dict
   // backward schedule (bytes, workspace): where the data gradient goes and what is added to it
   size_t dgrad_out_off, dgrad_res_off;
+  size_t cap_off;              // bytes, in the capture buffer: dy, then dz (each N*Ho*Wo*Cout bf16)
   bool dgrad_has_res = false, need_dgrad = true;
   ConvTcPrepared fwd, dgrad;
 };
@@ -47,6 +48,8 @@ struct nbc_train_plan {
   size_t padded_off, pool_off, pidx_off, drop_off, low_off, full_off, dfull_off, dlow_off, upws_off, gA_off, gB_off, gskip_off, dz_off,
       d1_off, d2_off, up_off, partial_off, zeros_off, wce_off, ws_bytes;
   size_t big_bytes, small_bytes;
+  size_t capture_bytes = 0;
+  void* capture = nullptr;  // nbc_train_set_capture: per-unit copies of the BN backward's dy and dz (off when null)
   void* prepared_ws = nullptr;
   int wgrad_impl = 0;   // 0 = tcgen05 (wgrad_tc.cu), 1 = mma.sync / CUDA-core cross-check kernels
   int loss_kind = 0;    // 0 = weighted CE, 1 = Lovasz-Softmax, 2 = CE / 4 + Lovasz
@@ -77,7 +80,7 @@ static int add_unit(nbc_train_plan* p, int Cin, int Cout, int k, int stride, int
   u.b_off = p->n_params, p->n_params += Cout;
   u.rs_off = p->n_stats, p->n_stats += 2 * (size_t)Cout;
   u.sd_index = sd_index;
-  u.x_off = u.z_off = u.y_off = u.st_off = u.wf_off = u.wd_off = u.dgrad_out_off = u.dgrad_res_off = 0;
+  u.x_off = u.z_off = u.y_off = u.st_off = u.wf_off = u.wd_off = u.dgrad_out_off = u.dgrad_res_off = u.cap_off = 0;
   p->units.push_back(u);
   return (int)p->units.size() - 1;
 }
@@ -131,9 +134,10 @@ extern "C" nbc_train_plan* nbc_train_create(int N, int H, int W) {
   p->cls_b_off = p->n_params, p->n_params += 3;
 
   // ---- workspace layout -------------------------------------------------------------------------------------
-  size_t off = 0;
+  size_t off = 0, cap = 0;
   for (Unit& u : p->units) {
     const size_t bytes = al((size_t)N * u.Ho * u.Wo * u.Cout * 2);
+    u.cap_off = cap, cap += 2 * bytes;
     u.z_off = off, off += bytes;
     u.y_off = off, off += bytes;
     u.st_off = off, off += al((size_t)u.Cout * 6 * 4);
@@ -172,6 +176,7 @@ extern "C" nbc_train_plan* nbc_train_create(int N, int H, int W) {
   p->dfull2_off = off, off += al((size_t)N * 3 * H * W * 4);
   p->loss2_off = off, off += al(16);
   p->ws_bytes = off;
+  p->capture_bytes = cap;
 
   // ---- static data flow: inputs of the units, gradient ping-pong of the blocks ----------------------------------
   size_t x = p->pool_off;
@@ -345,6 +350,12 @@ static int unit_backward(const Ctx& c, Unit& u, const void* dy, int relu, void* 
   int rc = bn_backward(dy, c.ws + u.y_off, c.ws + u.z_off, M, u.Cout, c.params + u.g_off, c.st(u, 0), c.st(u, 1), relu,
                        c.partial(), c.st(u, 4), c.grads + u.g_off, c.grads + u.b_off, dz, g_out, c.stream);
   if (rc) return rc;
+  if (p->capture != nullptr) {
+    const size_t bytes = (size_t)M * u.Cout * 2;
+    char* cap = reinterpret_cast<char*>(p->capture) + u.cap_off;
+    NBC_CUDA(cudaMemcpyAsync(cap, dy, bytes, cudaMemcpyDeviceToDevice, c.stream));
+    NBC_CUDA(cudaMemcpyAsync(cap + al(bytes), dz, bytes, cudaMemcpyDeviceToDevice, c.stream));
+  }
   if (u.Cin == 3)
     return c.p->wgrad_impl == 1 ? stem_wgrad(dz, c.ws + p->padded_off, p->N, u.Ho, u.Wo, c.grads + u.w_off, c.stream)
                                 : stem_wgrad_tc(dz, c.ws + p->padded_off, p->N, u.Ho, u.Wo, c.grads + u.w_off, c.stream);
@@ -481,13 +492,16 @@ extern "C" int nbc_train_forward_backward(nbc_train_plan* p, float* params, floa
 
 // debug / test accessor: byte offset into the workspace and geometry of an intermediate tensor.
 // what: 0 = z (pre-BN, bf16 NHWC) of unit `index`, 1 = y (post BN/ReLU) of unit `index`, 2 = low-res logits (f32 planar),
-// 3 = full-res logits (f32 planar), 4 = d loss / d full logits, 5 = d loss / d low-res logits.  dims_out[4] = N,H,W,C.
+// 3 = full-res logits (f32 planar), 4 = d loss / d full logits, 5 = d loss / d low-res logits;  6 = dy, 7 = dz of the BN
+// backward of unit `index` (bf16 NHWC) -- offsets into the CAPTURE buffer (nbc_train_set_capture), not the workspace.
+// dims_out[4] = N,H,W,C.
 extern "C" int64_t nbc_train_debug_offset(const nbc_train_plan* p, int what, int index, int32_t* dims_out) {
   if (!p || !dims_out) return -1;
-  if (what == 0 || what == 1) {
+  if (what == 0 || what == 1 || what == 6 || what == 7) {
     if (index < 0 || index >= (int)p->units.size()) return -1;
     const Unit& u = p->units[index];
     dims_out[0] = p->N, dims_out[1] = u.Ho, dims_out[2] = u.Wo, dims_out[3] = u.Cout;
+    if (what >= 6) return (int64_t)(u.cap_off + (what == 7 ? al((size_t)p->N * u.Ho * u.Wo * u.Cout * 2) : 0));
     return (int64_t)(what == 0 ? u.z_off : u.y_off);
   }
   if (what == 2 || what == 5) {
@@ -499,6 +513,16 @@ extern "C" int64_t nbc_train_debug_offset(const nbc_train_plan* p, int what, int
     return (int64_t)(what == 3 ? p->full_off : p->dfull_off);
   }
   return -1;
+}
+extern "C" size_t nbc_train_capture_bytes(const nbc_train_plan* p) { return p ? p->capture_bytes : 0; }
+extern "C" int nbc_train_set_capture(nbc_train_plan* p, void* buf, size_t bytes) {
+  NBC_REQUIRE(p, "nbc_train_set_capture: null plan");
+  if (buf != nullptr && bytes < p->capture_bytes) {
+    set_error("nbc_train_set_capture: buffer %zu < %zu bytes", bytes, p->capture_bytes);
+    return NBC_ERR_WORKSPACE;
+  }
+  p->capture = buf;
+  return 0;
 }
 extern "C" int nbc_train_set_wgrad_impl(nbc_train_plan* p, int impl) {
   NBC_REQUIRE(p && (impl == 0 || impl == 1), "nbc_train_set_wgrad_impl: impl must be 0 (tcgen05) or 1 (mma.sync)");

@@ -93,6 +93,7 @@ class Trainer:
             self.class_weights = w.to(device=self.device, dtype=torch.float32).contiguous()
             self._exchange(self._device_tensors(state_dict), self.params, self.stats, 0)
         self.num_batches_tracked = {k: int(v) for k, v in state_dict.items() if k.endswith('num_batches_tracked')}
+        self.capture = None
 
     def __del__(self):
         try:
@@ -144,18 +145,29 @@ class Trainer:
             self._exchange([sd[k] for k in self.keys], self.grads, None, 1)
         return {k: v for k, v in sd.items() if 'running' not in k and 'num_batches' not in k}
 
+    def enable_capture(self):
+        """Make every following step keep the dy and dz of each unit's BatchNorm backward (tests; ``debug_tensor`` 6 / 7)."""
+        with torch.cuda.device(self.device):
+            h = C.c_void_p(self.handle)
+            self.capture = torch.empty(self.lib.nbc_train_capture_bytes(h), dtype=torch.uint8, device=self.device)
+            _lib.check(self.lib.nbc_train_set_capture(h, C.c_void_p(self.capture.data_ptr()), self.capture.numel()),
+                       'nbc_train_set_capture')
+
     def debug_tensor(self, what, index=0):
         """View of an intermediate of the last step (tests): what 0/1 = z / y of unit ``index`` (bf16 NHWC), 2/3 = low / full
-        resolution logits, 4/5 = their gradients (f32 [N,3,h,w])."""
+        resolution logits, 4/5 = their gradients (f32 [N,3,h,w]), 6/7 = dy / dz of the unit's BatchNorm backward (bf16 NHWC,
+        after ``enable_capture``)."""
+        if what in (6, 7) and self.capture is None:
+            raise RuntimeError('debug tensors 6 / 7 need enable_capture()')
         dims = (C.c_int32 * 4)()
         off = self.lib.nbc_train_debug_offset(C.c_void_p(self.handle), what, index, dims)
         if off < 0:
             raise RuntimeError('bad debug tensor request')
-        base = (-self.ws.data_ptr()) % 1024 + off
+        buf, base = (self.capture, off) if what in (6, 7) else (self.ws, (-self.ws.data_ptr()) % 1024 + off)
         n, h, w, c = [int(v) for v in dims]
-        if what in (0, 1):
-            return self.ws[base:base + n * h * w * c * 2].view(torch.bfloat16).view(n, h, w, c)
-        return self.ws[base:base + n * h * w * c * 4].view(torch.float32).view(n, c, h, w)
+        if what in (0, 1, 6, 7):
+            return buf[base:base + n * h * w * c * 2].view(torch.bfloat16).view(n, h, w, c)
+        return buf[base:base + n * h * w * c * 4].view(torch.float32).view(n, c, h, w)
 
     # -- the step ------------------------------------------------------------------------------------------------------
     def forward_backward(self, images, targets, seed=0, dropout=None, update_stats=True):

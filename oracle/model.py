@@ -151,11 +151,12 @@ def upsample_argmax(logits_lowres, size):
     return up, torch.argmax(up, dim=1)
 
 
-def bicubic_weights_f32(in_size, out_size):
+def bicubic_weights_f32(in_size, out_size, clamp=True):
     """Restated index / weight arithmetic of torch's upsample_bicubic2d (align_corners=False), all in float32.
 
     scale = in/out (f32); src = scale * (dst + 0.5) - 0.5 (f32); i0 = floor(src); t = src - i0; taps i0-1..i0+2
-    clamped to [0, in-1]; cubic convolution coefficients with A = -0.75 (SURVEY.md a7)."""
+    clamped to [0, in-1]; cubic convolution coefficients with A = -0.75 (SURVEY.md a7).  ``clamp=False`` returns the
+    unclamped tap indices (a deliberately wrong variant for negative controls)."""
     A = np.float32(-0.75)
     scale = np.float32(in_size) / np.float32(out_size)
     dst = np.arange(out_size, dtype=np.float32)
@@ -172,8 +173,8 @@ def bicubic_weights_f32(in_size, out_size):
 
     one = np.float32(1)
     w = np.stack([c2(t + one), c1(t), c1(one - t), c2((one - t) + one)], axis=1).astype(np.float32)
-    idx = np.clip(i0[:, None] + np.arange(-1, 3)[None, :], 0, in_size - 1)
-    return idx, w
+    idx = i0[:, None] + np.arange(-1, 3)[None, :]
+    return (np.clip(idx, 0, in_size - 1) if clamp else idx), w
 
 
 def upsample_bicubic_restated(low, size):

@@ -224,3 +224,94 @@ def test_augment_oracle_and_pil_arithmetic():
     # reflect padding (even difference): 44 rows -> 48, two rows mirrored on each side without repeating the edge
     oi, _ = oaug.augment([img[2:46]], [dual[2:46]], [dict(p, x0=0, y0=0, hflip=0)], crop=40, target_hw=(48, 40))
     assert np.array_equal(oi[0][:3], img[2:46][[2, 1, 0]])
+
+
+# ------------------------------------------------------------------------------------------------- training backward
+# oracle/backward.py restates each backward operation of the native training step; tests/test_gpu_train_backward.py
+# compares the kernels with these helpers, so each one is pinned here to torch autograd in float64.
+@pytest.mark.parametrize('relu', [True, False])
+def test_backward_oracle_batchnorm(relu):
+    from oracle import backward as ob
+    g = torch.Generator().manual_seed(0)
+    z = (torch.randn(3, 8, 5, 7, generator=g, dtype=torch.float64) * 2 + 0.5).requires_grad_(True)
+    gamma = (torch.rand(8, generator=g, dtype=torch.float64) + 0.5).requires_grad_(True)
+    beta = torch.randn(8, generator=g, dtype=torch.float64).requires_grad_(True)
+    y = torch.nn.functional.batch_norm(z, None, None, gamma, beta, training=True, eps=1e-5)
+    if relu:
+        y = y.relu()
+    dy = torch.randn(y.shape, generator=g, dtype=torch.float64)
+    y.backward(dy)
+    ref = ob.bn_backward(dy, y.detach(), z.detach(), gamma.detach(), relu)
+    assert torch.allclose(ref['dz'], z.grad, rtol=1e-10, atol=1e-12)
+    assert torch.allclose(ref['dgamma'], gamma.grad, rtol=1e-10, atol=1e-12)
+    assert torch.allclose(ref['dbeta'], beta.grad, rtol=1e-10, atol=1e-12)
+    assert (ref['dgamma_abs'] >= ref['dgamma'].abs() - 1e-12).all() and (ref['dbeta_abs'] >= ref['dbeta'].abs() - 1e-12).all()
+    # running statistics: torch's update (momentum 0.1, unbiased variance), and the biased variant really differs
+    rm, rv = torch.randn(8, generator=g, dtype=torch.float64), torch.rand(8, generator=g, dtype=torch.float64) + 0.5
+    m_t, v_t = rm.clone(), rv.clone()
+    torch.nn.functional.batch_norm(z.detach(), m_t, v_t, training=True, momentum=0.1)
+    m, v = ob.running_stats(z.detach(), rm, rv)
+    assert torch.allclose(m, m_t, rtol=1e-12, atol=1e-14) and torch.allclose(v, v_t, rtol=1e-12)
+    assert not torch.allclose(ob.running_stats(z.detach(), rm, rv, unbiased=False)[1], v_t, rtol=1e-3)
+
+
+@pytest.mark.parametrize('H,W', [(9, 13), (8, 12), (1, 2)])
+def test_backward_oracle_maxpool_ties(H, W):
+    """First-maximum routing on inputs full of ties (a ReLU output quantised to three levels), odd and even sizes."""
+    from oracle import backward as ob
+    g = torch.Generator().manual_seed(H * 100 + W)
+    x = torch.randint(-2, 3, (2, 4, H, W), generator=g).clamp_min(0).double().requires_grad_(True)
+    y = torch.nn.functional.max_pool2d(x, 3, 2, 1)
+    dy = torch.randn(y.shape, generator=g, dtype=torch.float64)
+    y.backward(dy)
+    # up to four windows add into one input: torch sums them in another order (last-bit differences only)
+    assert torch.allclose(ob.maxpool_backward(dy, x.detach()), x.grad, rtol=1e-12, atol=1e-14)
+    if H > 1:
+        assert not torch.allclose(ob.maxpool_backward(dy, x.detach(), last=True), x.grad)
+
+
+@pytest.mark.parametrize('h,w,H,W', [(8, 16, 58, 122), (8, 12, 64, 96), (24, 32, 192, 256), (5, 3, 9, 31)])
+def test_backward_oracle_bicubic_adjoint(h, w, H, W):
+    """The dense interpolation matrices reproduce F.interpolate(bicubic) and its autograd gradient (integer and
+    non-integer ratios), and the adjoint satisfies <up(a), b> = <a, adj(b)>."""
+    from oracle import backward as ob
+    g = torch.Generator().manual_seed(h * w)
+    low = torch.randn(2, 3, h, w, generator=g).requires_grad_(True)
+    up = torch.nn.functional.interpolate(low, size=(H, W), mode='bicubic', align_corners=False)
+    # float32 taps on both sides; torch rounds the source index differently at non-integer scales (~1e-5)
+    tol = 5e-5 if (H % h or W % w) else 2e-6
+    assert (ob.upsample_bicubic(low.detach(), (H, W)) - up.detach().double()).abs().max() < tol
+    dup = torch.randn(up.shape, generator=g)
+    up.backward(dup)
+    adj = ob.upsample_adjoint(dup, (h, w))
+    assert (adj - low.grad.double()).abs().max() < tol * dup.abs().sum((2, 3)).max() / min(h, w)
+    a, b = torch.randn(2, 3, h, w, dtype=torch.float64), torch.randn(2, 3, H, W, dtype=torch.float64)
+    lhs, rhs = float((ob.upsample_bicubic(a, (H, W)) * b).sum()), float((a * ob.upsample_adjoint(b, (h, w))).sum())
+    assert abs(lhs - rhs) < 1e-10 * (abs(lhs) + 1)
+    assert (ob.upsample_adjoint(dup, (h, w), clamp=False) - adj).abs().max() > 1e-2
+
+
+def test_backward_oracle_conv_grads():
+    """conv_dgrad / conv_wgrad = autograd of conv2d at the geometries of the network: stride 2 on an odd input,
+    dilation, 7x7 stem."""
+    from oracle import backward as ob
+    g = torch.Generator().manual_seed(0)
+    for (H, W, cin, cout, k, s, p, d) in [(15, 31, 8, 16, 3, 2, 1, 1), (15, 31, 8, 16, 1, 2, 0, 1), (8, 16, 8, 8, 3, 1, 4, 4),
+                                          (29, 61, 3, 8, 7, 2, 3, 1)]:
+        x = torch.randn(2, cin, H, W, generator=g, dtype=torch.float64).requires_grad_(True)
+        w = torch.randn(cout, cin, k, k, generator=g, dtype=torch.float64).requires_grad_(True)
+        y = torch.nn.functional.conv2d(x, w, stride=s, padding=p, dilation=d)
+        dz = torch.randn(y.shape, generator=g, dtype=torch.float64)
+        y.backward(dz)
+        assert torch.allclose(ob.conv_dgrad(dz, w.detach(), x.shape, s, p, d), x.grad, rtol=1e-10, atol=1e-10)
+        assert torch.allclose(ob.conv_wgrad(x.detach(), dz, w.shape, s, p, d), w.grad, rtol=1e-10, atol=1e-10)
+
+
+def test_backward_oracle_dropout_hash():
+    """The restated hash is splitmix64 (published outputs for state 0); the keep fraction is 1 - p and the mask depends
+    on the seed."""
+    from oracle import backward as ob
+    assert [int(v) for v in ob.splitmix64_bits(0, 4)] == [0xE220A8397B1DCDAF, 0x6E789E6AA1B965F4, 0x06C45D188009454F,
+                                                           0xF88BB8A8724C81EC]
+    k1, k2 = ob.dropout_keep(7, 200000, 0.8), ob.dropout_keep(8, 200000, 0.8)
+    assert abs(k1.mean() - 0.2) < 0.005 and (k1 != k2).mean() > 0.2
