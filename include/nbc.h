@@ -226,6 +226,29 @@ int nbc_plan_profile(nbc_plan* plan, const void* input, int input_kind, int N, i
                      int max_layers);
 /* conv implementation used by the plan: 0 auto, 1 force tcgen05 where legal, 2 force mma.sync */
 int nbc_plan_set_impl(nbc_plan* plan, int impl);
+/* Test / debug hooks.  nbc_plan_set_stop(k): the forwards that follow (nbc_plan_forward, nbc_plan_forward_ragged) run
+ * steps 0..k of the launch list and return; k < 0 runs all of them (the default).  Every launch up to step k is made as
+ * in a full forward, programmatic dependent launch included.  No input of a step (x, x2, residual, the stem's staging
+ * image) is the buffer the step writes, so a forward stopped at k leaves step k's operands and its output in the
+ * workspace.  nbc_plan_num_steps / nbc_plan_step_info describe the launch list of the most recent forward. */
+typedef struct {
+  char name[24];
+  int32_t kind;       /* 0 stem on CUDA cores, 5 stem on tensor cores (staging pass + implicit GEMM), 1 maxpool,
+                         2 conv on tcgen05, 3 conv on mma.sync, 4 head 1x1 (f32 logits) */
+  /* tcgen05 kernel variant (0 for the other kinds): CTA pairs, the 64->64 3x3 halo kernel, the stem halo kernel, a second
+     source (conv3 + downsample), output channels per tile, K per stage, output staging buffers */
+  int32_t pair, halo3, stem_halo, dual, block_n, kblk, out_bufs;
+  int32_t ragged_map; /* -1 dense batch (or no tile walk), 1 compact tile map, 0 dense tile numbering, dead tiles skipped */
+  int32_t N, H, W, Cin, Cout, k, stride, pad, dil, relu;   /* input geometry of the step */
+  int32_t H2, W2, Cin2, stride2;                         /* dual: the second source (1x1, pad 0); 0 otherwise */
+  int32_t level;      /* ragged batch: row of the level table with the valid OUTPUT rows of the step; -1 dense */
+  /* byte offsets into the workspace, -1 for none.  The stem's x is its staging image (tensor-core stem only; its
+     input is the caller's image), head1x1's y is the caller's logits. */
+  int64_t x, x2, residual, y, levels;
+} nbc_plan_step;
+int nbc_plan_set_stop(nbc_plan* plan, int k);
+int nbc_plan_num_steps(const nbc_plan* plan);
+int nbc_plan_step_info(const nbc_plan* plan, int i, nbc_plan_step* out);
 
 /* ---- training step  (__main__.py:231-269: train-mode forward, loss, backward, Adam; utils.py:151-165 as the loss) ----
  * A plan is built for a fixed (N, H, W).  All state is caller-allocated and flat:

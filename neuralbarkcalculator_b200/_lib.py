@@ -13,6 +13,15 @@ class ConvDesc(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ('N', 'H', 'W', 'Cin', 'Cout', 'kh', 'kw', 'stride', 'pad', 'dil', 'relu', 'impl', 'f16')]
 
 
+class PlanStep(C.Structure):
+    """nbc_plan_step: one launch of the plan (see include/nbc.h)."""
+    _fields_ = ([('name', C.c_char * 24)]
+                + [(n, C.c_int32) for n in ('kind', 'pair', 'halo3', 'stem_halo', 'dual', 'block_n', 'kblk', 'out_bufs',
+                                            'ragged_map', 'N', 'H', 'W', 'Cin', 'Cout', 'k', 'stride', 'pad', 'dil', 'relu',
+                                            'H2', 'W2', 'Cin2', 'stride2', 'level')]
+                + [(n, C.c_int64) for n in ('x', 'x2', 'residual', 'y', 'levels')])
+
+
 # name -> (restype, argtypes); kept in one table so tests can check it against include/nbc.h
 SIGNATURES = {
     'nbc_version': (c_int, []),
@@ -71,6 +80,9 @@ SIGNATURES = {
     'nbc_plan_profile': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p,
                                  C.POINTER(c_float), C.POINTER(C.c_double), c_int]),
     'nbc_plan_set_impl': (c_int, [c_void_p, c_int]),
+    'nbc_plan_set_stop': (c_int, [c_void_p, c_int]),
+    'nbc_plan_num_steps': (c_int, [c_void_p]),
+    'nbc_plan_step_info': (c_int, [c_void_p, c_int, C.POINTER(PlanStep)]),
     'nbc_train_create': (c_void_p, [c_int, c_int, c_int]),
     'nbc_train_destroy': (None, [c_void_p]),
     'nbc_train_param_count': (c_i64, [c_void_p]),

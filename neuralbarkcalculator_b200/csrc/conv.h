@@ -29,6 +29,12 @@ int conv_tc_prepare(const ConvGeom& g, const void* x, const void* w, const float
 int conv_tc_prepare_dual(const ConvGeom& g, const void* x, const ConvGeom& g2, const void* x2, const void* w_cat,
                          const float* bias, void* y, ConvTcPrepared* out, const int* valid_h = nullptr);
 int conv_tc_run(const ConvTcPrepared* prep, cudaStream_t stream);
+// which kernel conv_tc_run launches for a prepared convolution (nbc_plan_step_info)
+struct ConvTcVariant {
+  int pair, halo3, stem_halo, dual, block_n, kblk, out_bufs;
+  int ragged_map;   // -1 dense batch, 1 compact tile map, 0 dense tile numbering with dead tiles skipped
+};
+void conv_tc_describe(const ConvTcPrepared* prep, ConvTcVariant* v);
 // stem 7x7/2 as an implicit GEMM over the padded bf16 image (see stem.cu)
 int conv_tc_prepare_stem(int N, int Ho, int Wo, int Hp, int Wp, const void* padded, const void* w224, const float* bias,
                          void* y, ConvTcPrepared* out, const int* valid_h = nullptr, int f16 = 0, int relu = 1);

@@ -1724,6 +1724,14 @@ int conv_tc_run(const ConvTcPrepared* prep, cudaStream_t stream) {
   }
 }
 
+void conv_tc_describe(const ConvTcPrepared* prep, ConvTcVariant* v) {
+  const ConvTcLaunch* L = reinterpret_cast<const ConvTcLaunch*>(prep->storage);
+  v->pair = L->pair, v->halo3 = L->halo3, v->stem_halo = L->kblk == 32 ? L->stem_halo : 0, v->dual = L->p.cblocks2 > 0;
+  v->block_n = L->block_n, v->kblk = L->kblk, v->out_bufs = L->out_bufs;
+  // the same rule as ragged_map_setup
+  v->ragged_map = L->p.valid_h == nullptr ? -1 : (L->p.ragged_compact != 0 && L->p.N <= kMaxRaggedImages ? 1 : 0);
+}
+
 int conv_tc(const ConvGeom& g, const void* x, const void* w, const float* bias, const void* residual, void* y,
             cudaStream_t stream) {
   ConvTcPrepared prep;

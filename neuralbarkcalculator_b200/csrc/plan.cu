@@ -41,6 +41,9 @@ struct Step {  // one launch of the cached forward
   ConvTcPrepared prep;
   const char* name;
   double extra_flops = 0.0;   // fused second source
+  const void* x2 = nullptr;   // fused second source (conv3 + downsample): its input and geometry
+  ConvGeom g2{};
+  int level = -1;             // ragged batch: row of the level table with the valid output rows
 };
 
 }  // namespace nbc
@@ -63,6 +66,8 @@ struct nbc_plan {
   typedef std::tuple<int, int, int, void*, int, int> Key;   // N, H, W, workspace, impl, ragged
   std::map<Key, std::vector<nbc::Step>> cache;
   std::vector<nbc::Step>* steps_ptr = nullptr;
+  Key steps_key;   // the key of *steps_ptr
+  int stop = -1;   // nbc_plan_set_stop: last step a forward runs (< 0: all)
 };
 
 namespace nbc {
@@ -162,6 +167,7 @@ static int add_conv(nbc_plan* p, const ConvLayer& L, int N, int H, int W, const 
     return NBC_ERR_INVALID;
   }
   *Ho = s.g.Ho(), *Wo = s.g.Wo();
+  if (level != nullptr) s.level = *level;
   p->steps_ptr->push_back(s);
   return 0;
 }
@@ -197,11 +203,13 @@ static int build_steps(nbc_plan* p, int N, int H, int W, void* workspace, bool r
       if (rc) return rc;
     }
     s.w = levels;   // w slot of the stem / maxpool steps = ragged level table (or nullptr)
+    s.level = ragged ? 1 : -1;
     steps.push_back(s);
     Step m;
     memset(&m.prep, 0, sizeof(m.prep));
     m.kind = 1, m.g = ConvGeom{N, d.H2, d.W2, 64, 64, 3, 3, 2, 1, 1, 0}, m.x = bufB, m.y = bufA, m.name = "maxpool";
     m.w = levels, m.bias = nullptr, m.residual = nullptr;
+    m.level = ragged ? 2 : -1;
     steps.push_back(m);
   }
   int h = d.H4, w = d.W4;
@@ -227,6 +235,7 @@ static int build_steps(nbc_plan* p, int N, int H, int W, void* workspace, bool r
       s.extra_flops = g2.flops();
       s.x = t2, s.w = B.w_cat, s.bias = B.bias_cat, s.residual = nullptr, s.y = other, s.name = "conv3+downsample";
       s.kind = 2;
+      s.x2 = in, s.g2 = g2, s.level = levels != nullptr ? lv : -1;
       rc = conv_tc_prepare_dual(s.g, t2, g2, in, B.w_cat, B.bias_cat, other, &s.prep, levels != nullptr ? levels + (size_t)lv * N : nullptr);
       if (rc) return rc;
       h3 = s.g.Ho(), w3 = s.g.Wo();
@@ -258,6 +267,7 @@ static int build_steps(nbc_plan* p, int N, int H, int W, void* workspace, bool r
   s.kind = 4, s.g = ConvGeom{N, hh, wh, 512, 3, 1, 1, 1, 0, 1, 0}, s.x = t1, s.y = logits, s.name = "head1x1";
   s.w = p->cls_w, s.bias = p->cls_b;
   s.residual = levels != nullptr ? levels + (size_t)3 * N : nullptr;      // ragged: valid rows at 1/8 resolution
+  s.level = levels != nullptr ? 3 : -1;
   steps.push_back(s);
   return 0;
 }
@@ -304,6 +314,7 @@ static int ensure_steps(nbc_plan* p, const void* images, int input_kind, int N, 
   (void)images, (void)logits;
   nbc_plan::Key key(N, H, W, workspace, p->impl, ragged ? 1 : 0);
   auto it = p->cache.find(key);
+  p->steps_key = key;
   if (it != p->cache.end()) {
     p->steps_ptr = &it->second;
     return 0;
@@ -441,9 +452,11 @@ extern "C" int nbc_plan_forward(nbc_plan* p, const void* input, int input_kind, 
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   int rc = ensure_steps(p, input, input_kind, N, H, W, lowres_logits, workspace, workspace_bytes);
   if (rc) return rc;
-  for (const Step& s : *p->steps_ptr) {
-    rc = run_step(p, s, input, input_kind, lowres_logits, stream);
+  const std::vector<Step>& steps = *p->steps_ptr;
+  for (int i = 0; i < (int)steps.size(); ++i) {
+    rc = run_step(p, steps[i], input, input_kind, lowres_logits, stream);
     if (rc) return rc;
+    if (i == p->stop) break;
   }
   return 0;
 }
@@ -461,9 +474,11 @@ extern "C" int nbc_plan_forward_ragged(nbc_plan* p, const uint8_t* canvas, int N
   int* levels = reinterpret_cast<int*>(reinterpret_cast<char*>(workspace) + 2 * big + 2 * small);
   rc = ragged_levels(heights, first_last, N, Hc, levels, stream);
   if (rc) return rc;
-  for (const Step& s : *p->steps_ptr) {
-    rc = run_step(p, s, canvas, 0, lowres_logits, stream);
+  const std::vector<Step>& steps = *p->steps_ptr;
+  for (int i = 0; i < (int)steps.size(); ++i) {
+    rc = run_step(p, steps[i], canvas, 0, lowres_logits, stream);
     if (rc) return rc;
+    if (i == p->stop) break;
   }
   return 0;
 }
@@ -492,4 +507,51 @@ extern "C" int nbc_plan_profile(nbc_plan* p, const void* input, int input_kind, 
   }
   for (auto& e : ev) cudaEventDestroy(e);
   return n;
+}
+
+// Stopping after step k leaves its operands intact: in build_steps no step reads the buffer it writes.  The stem reads
+// the caller's image (and, on tensor cores, its staging image in t2) and writes bufB; maxpool bufB -> bufA; each
+// bottleneck conv1 in -> t1, conv2 t1 -> t2, then either the fused conv3 + downsample (t2, in) -> other, or on the
+// mma.sync path downsample in -> other and conv3 (t2, residual other) -> in, or without a downsample conv3 (t2,
+// residual in) -> other; head3x3 in -> t1 and head1x1 t1 -> the caller's logits.
+extern "C" int nbc_plan_set_stop(nbc_plan* p, int k) {
+  NBC_REQUIRE(p, "nbc_plan_set_stop: null plan");
+  p->stop = k < 0 ? -1 : k;
+  return 0;
+}
+
+extern "C" int nbc_plan_num_steps(const nbc_plan* p) {
+  NBC_REQUIRE(p, "nbc_plan_num_steps: null plan");
+  return p->steps_ptr ? (int)p->steps_ptr->size() : 0;
+}
+
+extern "C" int nbc_plan_step_info(const nbc_plan* p, int i, nbc_plan_step* out) {
+  NBC_REQUIRE(p && out, "nbc_plan_step_info: null pointer");
+  NBC_REQUIRE(p->steps_ptr && i >= 0 && i < (int)p->steps_ptr->size(), "nbc_plan_step_info: no step %d", i);
+  const Step& s = (*p->steps_ptr)[i];
+  const char* ws = reinterpret_cast<const char*>(std::get<3>(p->steps_key));
+  size_t big, small;
+  buffer_sizes(std::get<0>(p->steps_key), std::get<1>(p->steps_key), std::get<2>(p->steps_key), &big, &small);
+  auto off = [&](const void* a) -> int64_t { return a ? (int64_t)(reinterpret_cast<const char*>(a) - ws) : -1; };
+  memset(out, 0, sizeof(*out));
+  snprintf(out->name, sizeof(out->name), "%s", s.name);
+  out->kind = s.kind;
+  out->ragged_map = -1;
+  if (s.kind == 2 || s.kind == 5) {
+    ConvTcVariant v;
+    conv_tc_describe(&s.prep, &v);
+    out->pair = v.pair, out->halo3 = v.halo3, out->stem_halo = v.stem_halo, out->dual = v.dual;
+    out->block_n = v.block_n, out->kblk = v.kblk, out->out_bufs = v.out_bufs, out->ragged_map = v.ragged_map;
+  }
+  out->N = s.g.N, out->H = s.g.H, out->W = s.g.W, out->Cin = s.g.Cin, out->Cout = s.g.Cout, out->k = s.g.kh;
+  out->stride = s.g.stride, out->pad = s.g.pad, out->dil = s.g.dil, out->relu = s.g.relu;
+  if (s.x2 != nullptr) out->H2 = s.g2.H, out->W2 = s.g2.W, out->Cin2 = s.g2.Cin, out->stride2 = s.g2.stride;
+  out->level = s.level;
+  const bool stem = s.kind == 0 || s.kind == 5;
+  out->x = stem ? (s.kind == 5 ? off(s.residual) : -1) : off(s.x);
+  out->x2 = off(s.x2);
+  out->residual = (s.kind == 2 || s.kind == 3) ? off(s.residual) : -1;
+  out->y = s.kind == 4 ? -1 : off(s.y);
+  out->levels = std::get<5>(p->steps_key) ? (int64_t)(2 * big + 2 * small) : -1;
+  return 0;
 }

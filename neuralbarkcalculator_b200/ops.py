@@ -507,6 +507,21 @@ class Plan:
     def set_impl(self, impl):
         _lib.check(self._lib.nbc_plan_set_impl(C.c_void_p(self.handle), int(impl)), 'nbc_plan_set_impl')
 
+    def set_stop(self, k):
+        """Debug hook: the forwards that follow run steps 0..k of the launch list only (k < 0: all, the default)."""
+        _lib.check(self._lib.nbc_plan_set_stop(C.c_void_p(self.handle), int(k)), 'nbc_plan_set_stop')
+
+    def steps(self):
+        """The launch list of the most recent forward: one dict per step (nbc_plan_step fields; workspace byte offsets)."""
+        out = []
+        for i in range(self._lib.nbc_plan_num_steps(C.c_void_p(self.handle))):
+            s = _lib.PlanStep()
+            _lib.check(self._lib.nbc_plan_step_info(C.c_void_p(self.handle), i, C.byref(s)), 'nbc_plan_step_info')
+            d = {n: getattr(s, n) for n, _ in _lib.PlanStep._fields_}
+            d['name'] = s.name.decode()
+            out.append(d)
+        return out
+
     def _workspace(self, N, H, W):
         need = self._lib.nbc_plan_workspace_bytes(C.c_void_p(self.handle), N, H, W) + 1024
         if self._ws is None or self._ws.numel() < need:
