@@ -198,6 +198,21 @@ typedef struct {
 int nbc_augment_batch(const uint8_t* images, const uint8_t* duals, int M, int Hs, int Ws, int target_h, int target_w,
                       int crop, const nbc_augment_params* params, int B, uint8_t* out_images, uint8_t* out_classes,
                       void* stream);
+/* Ragged sources with the full pad_resize  (__main__.py:153-176; utils.py:242-247 pad_resize = reflect pad by
+ * ceil(d/2) per side, then Pillow's BILINEAR resize to the target).  Sources of different sizes in one canvas:
+ * images u8 [M,Hc,Wc,3], duals u8 [M,Hc,Wc] (or NULL), dims int32 [M][2] = (height, width) of source m, which occupies
+ * rows [0, height) and columns [0, width) of its slot.  Per source and axis, d = target - size: an even d is reflect
+ * padding alone (as nbc_augment_batch); an odd d pads to target + 1 and resizes that axis back to target with Pillow's
+ * fixed-point arithmetic (Resample.c: 22 fraction bits, horizontal pass first, the intermediate rounded to u8).
+ * resize_tables: device int32 [target_h + target_w][4], the rows of the H axis then of the W axis; row i = {first padded
+ * index read, three fixed-point weights} of Pillow's (target + 1 -> target) BILINEAR coefficients (float64, converted as
+ * trunc(0.5 + k * 2^22)); rows of an axis no source resizes are not read.  Same params and outputs as
+ * nbc_augment_batch; x0 / y0 live in the target frame.  dims is read back to the host (M x 8 bytes, which waits for the
+ * stream) and a source larger than the target, or whose reflect padding is not narrower than it, is refused with
+ * NBC_ERR_INVALID naming the source before anything is launched. */
+int nbc_augment_ragged(const uint8_t* images, const uint8_t* duals, int M, int Hc, int Wc, const int32_t* dims, int target_h,
+                       int target_w, const int32_t* resize_tables, int crop, const nbc_augment_params* params, int B,
+                       uint8_t* out_images, uint8_t* out_classes, void* stream);
 
 /* ---- the whole network  (models.py:27-43 SimpleSegmentationModel.forward, 127-139 fcn_resnet50) ------------------
  * tensors_host: host array of DEVICE pointers to the 326 f32 state_dict tensors in torchvision key order

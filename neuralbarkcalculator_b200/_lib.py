@@ -68,6 +68,8 @@ SIGNATURES = {
     'nbc_confusion_matrix': (c_int, [c_void_p, c_void_p, c_int, c_i64, c_void_p, c_void_p]),
     'nbc_augment_batch': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p,
                           c_void_p]),
+    'nbc_augment_ragged': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int,
+                           c_void_p, c_void_p, c_void_p]),
     'nbc_png_idat_bound': (c_size_t, [c_int, c_int, c_int]),
     'nbc_png_idat': (c_i64, [c_void_p, c_int, c_int, c_int, c_i64, c_void_p, c_void_p, c_size_t]),
     'nbc_compose_combined': (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p]),

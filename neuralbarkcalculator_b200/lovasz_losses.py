@@ -41,9 +41,13 @@ def iou(preds, labels, C=3, EMPTY=1.):
     """lovasz_losses.py:54-73: array of per-class IoU (in %) of argmax(preds, 1) against labels, over the whole batch."""
     if C != 3:
         raise RuntimeError('iou: the B200 path is built for the 3 classes of the reference')
-    cm = _confusion(preds, labels)
+    return iou_from_confusion(_confusion(preds, labels), EMPTY)
+
+
+def iou_from_confusion(cm, EMPTY=1.):
+    """The per-class IoU (in %) of ``iou`` from a 3x3 confusion matrix cm[label, prediction]."""
     out = []
-    for i in range(C):
+    for i in range(len(cm)):
         inter = int(cm[i, i])
         union = int(cm[i, :].sum() + cm[:, i].sum() - cm[i, i])
         out.append(EMPTY if not union else float(inter) / float(union))

@@ -81,6 +81,7 @@ class Trainer:
             if loss not in kinds:
                 raise ValueError("loss must be 'weighted_ce', 'lovasz' or 'mixed'")
             _lib.check(self.lib.nbc_train_set_loss(h, kinds[loss]), 'nbc_train_set_loss')
+            self.loss_kind = loss
             n = self.lib.nbc_train_param_count(h)
             self.params = torch.zeros(n, dtype=torch.float32, device=self.device)
             self.grads = torch.zeros(n, dtype=torch.float32, device=self.device)
@@ -168,6 +169,15 @@ class Trainer:
         if what in (0, 1, 6, 7):
             return buf[base:base + n * h * w * c * 2].view(torch.bfloat16).view(n, h, w, c)
         return buf[base:base + n * h * w * c * 4].view(torch.float32).view(n, c, h, w)
+
+    def evaluate(self, ds, indices, loss=None, class_weights=None, precision=None, chunk=8):
+        """``evaluate.evaluate`` of the current weights: eval-mode forward of whole images, as predict runs them, with
+        this trainer's loss and class weights unless given."""
+        from . import evaluate as nev
+        from .models import DEFAULT_PRECISION
+        return nev.evaluate(self.state_dict(), ds, indices, loss=self.loss_kind if loss is None else loss,
+                            class_weights=self.class_weights if class_weights is None else class_weights,
+                            precision=DEFAULT_PRECISION if precision is None else precision, chunk=chunk)
 
     # -- the step ------------------------------------------------------------------------------------------------------
     def forward_backward(self, images, targets, seed=0, dropout=None, update_stats=True):

@@ -155,14 +155,7 @@ class PixelWiseF1(nn.Module):
             raise RuntimeError('PixelWiseF1: CUDA tensors required (no CPU path in neuralbarkcalculator_b200)')
         pred = ops.argmax3_u8(outputs.float())
         ops.remove_small_zones_u8(pred, 150)
-        cm = ops.confusion_matrix(pred, labels.to(outputs.device)).cpu().numpy().astype(np.float64)
-        tp = np.diag(cm)
-        denom = cm.sum(0) + cm.sum(1)
-        scores = np.where(denom > 0, 2 * tp / np.maximum(denom, 1), 0.0)
-        targets_count, outputs_count = cm.sum(1), cm.sum(0)
-        for i, count_i in enumerate(targets_count):
-            if count_i == 0 and outputs_count[i] == 0:
-                scores[i] = np.delete(scores, i).mean()
+        scores = f1_from_confusion(ops.confusion_matrix(pred, labels.to(outputs.device)).cpu().numpy())
         if self.class_to_watch is None:
             return scores.mean()
         elif self.class_to_watch == 'loss':
@@ -171,3 +164,18 @@ class PixelWiseF1(nn.Module):
             return scores[self.class_to_watch]
         else:
             return scores
+
+
+def f1_from_confusion(cm):
+    """Per-class F1 of ``PixelWiseF1`` from a 3x3 confusion matrix cm[label, prediction]: sklearn's f1_score (0 for a class
+    with neither support nor prediction), then a class absent from both targets and outputs takes the mean of the others
+    (utils.py:224-226)."""
+    cm = np.asarray(cm, dtype=np.float64)
+    tp = np.diag(cm)
+    denom = cm.sum(0) + cm.sum(1)
+    scores = np.where(denom > 0, 2 * tp / np.maximum(denom, 1), 0.0)
+    targets_count, outputs_count = cm.sum(1), cm.sum(0)
+    for i, count_i in enumerate(targets_count):
+        if count_i == 0 and outputs_count[i] == 0:
+            scores[i] = np.delete(scores, i).mean()
+    return scores
