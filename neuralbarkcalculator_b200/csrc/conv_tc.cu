@@ -16,13 +16,19 @@
 //   * epilogue (8 warps): tcgen05.ld -> + bias (+ residual) -> ReLU -> bf16 -> 128B-swizzled staging buffer in
 //     shared memory -> TMA store.  The residual group is prefetched INTO the staging buffer by TMA and updated in
 //     place, so residual reads and output writes are full 128-byte lines issued by the copy engine, not by the LSU.
-// Persistent CTAs (one per SM), warp roles: 0 = TMA producer, 1 = MMA issuer + TMEM owner, 2..9 = epilogue,
-// 10 = output / residual TMA.
-// Two kernels share this structure: conv_tc_kernel (one CTA per tile, cta_group::1) and conv_tc_pair_kernel (clusters
-// of 2 CTAs, one M = 256 cta_group::2 MMA over both SMs, half a weight tile per CTA -- further down); want_pair() holds
-// the measured rule that picks one per launch.  Consecutive conv launches are chained by programmatic dependent launch.
-#include <stdlib.h>
-
+//
+// One skeleton, four kernels.  Every kernel is a persistent CTA (one per SM) with the same warp roles:
+//   warp 0 = operand producer, warp 1 = MMA issuer + TMEM owner, warps 2..9 = epilogue (epilogue_role),
+//   warp 10 = output / residual TMA (output_role).
+// tc_prologue / tc_teardown (shared memory layout, barriers, TMEM, programmatic dependent launch, ragged map) and the
+// two output-side roles are shared; a kernel only writes its producer and MMA issuer, and names the tile walk its
+// roles follow (CtaWalk: one CTA per tile; PairWalk: a CTA pair per two tiles).
+//   conv_tc_kernel        the general case: one shifted TMA box per (tap, channel block), cta_group::1.
+//   conv_tc_pair_kernel   clusters of 2 CTAs, one M = 256 cta_group::2 MMA over both SMs, half a weight tile per CTA;
+//                         want_pair() holds the measured rule that picks it.
+//   conv_tc_stem_kernel   the stem's 128 x 1 tiles out of 7 bulk-copied input rows, weights resident.
+//   conv_tc_halo3_kernel  layer1's 64 -> 64 3x3 out of one halo box per 128 x 1 tile, weights resident.
+// Consecutive conv launches are chained by programmatic dependent launch.
 #include "common.cuh"
 #include "conv.h"
 
@@ -50,7 +56,6 @@ struct ConvTcParams {
   // beyond it are written as zeros (at least kRaggedHalo of them: the zero padding the next layer reads); tiles
   // that start beyond the halo are skipped.
   const int* valid_h;
-  int ragged_compact;   // 1: walk the compact enumeration of live M tiles (ragged_map_setup); 0: dense numbering, dead tiles skipped
   int8_t tap_map[9];
   int16_t tap_dh[9];
   int16_t tap_dw[9];
@@ -59,9 +64,6 @@ struct ConvTcParams {
   int stem_hp, stem_wp;
 };
 
-#ifndef NBC_PDL_DEFAULT
-#define NBC_PDL_DEFAULT 1
-#endif
 constexpr int kRaggedHalo = 4;   // >= the largest padding / dilation of any consumer (layer4: dilation 4)
 constexpr int kTcThreads = 352;  // warp 0 TMA operands, warp 1 MMA, warps 2..9 epilogue, warp 10 output / residual TMA
 constexpr int kOutBufBytes = 128 * 64 * 2;  // 128 pixels x 64 channels x 16 bit: one output group of a tile
@@ -69,27 +71,47 @@ constexpr int kSmemLimit = 232448;          // 227 KB of dynamic shared memory p
 constexpr int kMaxRaggedImages = 64;
 constexpr int kMapBytes = 512;   // ragged tile map (see ragged_map_setup): behind the 256-byte barrier block
 
-// BN = output channels per tile, KBLK = K elements per pipeline stage: 64 (128-byte swizzle) for the bottleneck /
-// head convs, 32 (64-byte swizzle) for the stem, whose K block is one 7-tap row of 8 pixels x 4 channels.
-// OB = output staging buffers (16 KB each): 4 when the epilogue sets the pace (residual layers, K <= 512), 2 (and a
-// deeper operand ring) when the MMA main loop does.
-template <int BN, int KBLK, int OB>
-struct TcCfg {
-  static constexpr int kABytes = 128 * KBLK * 2;  // 128 pixels x KBLK bf16
-  static constexpr int kBBytes = BN * KBLK * 2;
-  static constexpr int kStageBytes = kABytes + kBBytes;
-  static constexpr int kStagesMax = (BN == 256) ? 4 : (BN == 128 ? 6 : 8);
-  static constexpr int kFixedBytes = OB * kOutBufBytes + 256 /*barriers*/ + kMapBytes + 1024 /*align slack*/;
-  static constexpr int kStagesFit = (kSmemLimit - kFixedBytes) / kStageBytes;
-  static constexpr int kStages = kStagesFit < kStagesMax ? kStagesFit : kStagesMax;
-  static constexpr int kTmemCols = 2 * BN < 32 ? 32 : 2 * BN;
-  static constexpr int kUsedBytes = kStages * kStageBytes + kFixedBytes;
+// Shared memory of every conv kernel, in this order from a 1024-aligned base: STAGES operand stages of STAGE_BYTES,
+// W_BYTES of resident weights (halo kernels; 0 otherwise), OB output staging buffers of 16 KB, the barrier block, the
+// ragged map.  BN = output channels per tile; PAIR = a CTA of conv_tc_pair_kernel.
+constexpr int tc_fixed_bytes(int w_bytes, int ob) { return w_bytes + ob * kOutBufBytes + 256 /*barriers*/ + kMapBytes + 1024 /*align slack*/; }
+constexpr int tc_stages(int stage_bytes, int fixed_bytes, int max_stages) {
+  return (kSmemLimit - fixed_bytes) / stage_bytes < max_stages ? (kSmemLimit - fixed_bytes) / stage_bytes : max_stages;
+}
+template <int STAGES, int STAGE_BYTES, int W_BYTES, int BN, int OB, bool PAIR>
+struct TcLayout {
+  static constexpr int kStages = STAGES;
+  static constexpr int kStageBytes = STAGE_BYTES;
+  static constexpr int kWBytes = W_BYTES;
+  static constexpr int kOB = OB;
+  static constexpr bool kPair = PAIR;
+  static constexpr int kUsedBytes = STAGES * STAGE_BYTES + tc_fixed_bytes(W_BYTES, OB);
   // > half an SM's shared memory keeps one CTA (one TMEM owner) per SM
   static constexpr int kSmemBytes = kUsedBytes < 120 * 1024 ? 120 * 1024 : kUsedBytes;
-  static constexpr uint32_t kSwizzleBytes = KBLK * 2;  // 128 or 64
+  static constexpr int kTmemCols = 2 * BN;                  // two accumulator buffers
   static constexpr int kSteps = BN / 64;                    // 64-channel output groups ("steps") per tile
   static constexpr int kWarpsPerStep = (BN == 64) ? 8 : 4;  // epilogue warps that fill one staging buffer
-  static_assert(kStages >= 2 && kUsedBytes <= kSmemLimit, "shared memory budget");
+  static_assert(STAGES >= 2 && kUsedBytes <= kSmemLimit, "shared memory budget");
+  static_assert((STAGES * STAGE_BYTES) % 1024 == 0 && W_BYTES % 1024 == 0, "staging buffers 1024-aligned");
+  static_assert((2 * STAGES + 4 + 2 * OB + 1) * 8 + 4 <= 256, "barrier block");
+};
+
+// conv_tc_kernel.  KBLK = K elements per pipeline stage: 64 (128-byte swizzle) for the bottleneck / head convs, 32
+// (64-byte swizzle) for the per-window stem, whose K block is one 7-tap row of 8 pixels x 4 channels.
+// OB = output staging buffers: 4 when the epilogue sets the pace (residual layers, K <= 512), 2 (and a deeper operand
+// ring) when the MMA main loop does.
+template <int BN, int KBLK, int OB>
+struct TcCfg : TcLayout<tc_stages(128 * KBLK * 2 + BN * KBLK * 2, tc_fixed_bytes(0, OB), BN == 256 ? 4 : (BN == 128 ? 6 : 8)),
+                        128 * KBLK * 2 + BN * KBLK * 2, 0, BN, OB, false> {
+  static constexpr int kABytes = 128 * KBLK * 2;        // 128 pixels x KBLK bf16
+  static constexpr uint32_t kSwizzleBytes = KBLK * 2;   // 128 or 64
+};
+// conv_tc_pair_kernel: each CTA stages its 128 pixels of A and HALF of the weight tile
+template <int BN, int OB>
+struct TcCfgPair : TcLayout<tc_stages(128 * 64 * 2 + (BN / 2) * 64 * 2, tc_fixed_bytes(0, OB), 8), 128 * 64 * 2 + (BN / 2) * 64 * 2,
+                            0, BN, OB, true> {
+  static constexpr int kABytes = 128 * 64 * 2;
+  static_assert(BN == 128 || BN == 256, "pair kernel: BN = 128 or 256");
 };
 
 struct TileCoord {
@@ -112,10 +134,14 @@ __device__ __forceinline__ TileCoord tile_coord(const ConvTcParams& p, int tile)
 // CTAs stays balanced.  (Walking the dense numbering and skipping dead tiles left some CTAs with up to 20 % more live
 // tiles than others: the network pass of a real chunk, mean 610 of 1024 rows, took 5.9 ms against 4.9 ms for a dense
 // batch of the same work.)  s_map[i] = enumerated M tiles of the images before i, s_map[N] = their total; a virtual M
-// index maps back to the dense m_tile the rest of the kernel works with.
+// index maps back to the dense m_tile the rest of the kernel works with.  The map holds kMaxRaggedImages images; larger
+// ragged batches walk the dense numbering and skip dead tiles.
 static_assert((kMaxRaggedImages + 1) * 4 <= kMapBytes, "ragged map");
+__host__ __device__ __forceinline__ bool ragged_mapped(const ConvTcParams& p) {
+  return p.valid_h != nullptr && p.N <= kMaxRaggedImages;
+}
 __device__ __forceinline__ bool ragged_map_setup(const ConvTcParams& p, int* s_map) {
-  const bool mapped = p.valid_h != nullptr && p.ragged_compact != 0 && p.N <= kMaxRaggedImages;   // uniform over the grid
+  const bool mapped = ragged_mapped(p);   // uniform over the grid
   if (mapped) {
     if (threadIdx.x == 0) {
       int acc = 0;
@@ -141,22 +167,172 @@ __device__ __forceinline__ int ragged_real_m(const ConvTcParams& p, const int* s
   hint = img;
   return img * p.tiles_h * p.tiles_w + (vm - s_map[img]);
 }
-// a virtual tile of the walk: coordinates + "dead" (starts at or below the last valid row of its image: no loads, no MMA)
-struct VTile {
+__device__ __forceinline__ bool mtile_dead(const ConvTcParams& p, int m_tile) {
+  if (m_tile >= p.num_m_tiles) return true;
+  if (p.valid_h == nullptr) return false;
+  const int mt = m_tile / p.tiles_w;
+  return (mt % p.tiles_h) * p.th >= __ldg(p.valid_h + mt / p.tiles_h);
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Tile walks.  Each role of a CTA visits the tiles i = first(), first() + step(), ... < total in order and asks at(i, hint)
+// for this CTA's tile: its coordinates and "dead" (starts at or below the last valid row of its image: no loads, no
+// MMA).  Every role keeps its own hint, so each does one ragged-map lookup per tile.
+// ------------------------------------------------------------------------------------------------------------
+struct Tile {
   TileCoord t;
   bool dead;
 };
-__device__ __forceinline__ VTile vtile(const ConvTcParams& p, const int* s_map, int vt, int& hint) {
-  int tile = vt;
-  if (s_map != nullptr) {
-    const int vm = vt / p.num_n_tiles;
-    tile = ragged_real_m(p, s_map, vm, hint) * p.num_n_tiles + (vt - vm * p.num_n_tiles);
+// one CTA per tile, over the (virtual, see ragged_map_setup) tiles
+struct CtaWalk {
+  const int* s_map;
+  int total;
+  __device__ __forceinline__ CtaWalk(const ConvTcParams& p, const int* map)
+      : s_map(map), total((map ? map[p.N] : p.num_m_tiles) * p.num_n_tiles) {}
+  __device__ __forceinline__ int first() const { return blockIdx.x; }
+  __device__ __forceinline__ int step() const { return gridDim.x; }
+  __device__ __forceinline__ Tile at(const ConvTcParams& p, int vt, int& hint) const {
+    int tile = vt;
+    if (s_map != nullptr) {
+      const int vm = vt / p.num_n_tiles;
+      tile = ragged_real_m(p, s_map, vm, hint) * p.num_n_tiles + (vt - vm * p.num_n_tiles);
+    }
+    Tile v;
+    v.t = tile_coord(p, tile);
+    v.dead = p.valid_h != nullptr && v.t.h0 >= __ldg(p.valid_h + v.t.img);
+    return v;
   }
-  VTile v;
-  v.t = tile_coord(p, tile);
-  v.dead = p.valid_h != nullptr && v.t.h0 >= __ldg(p.valid_h + v.t.img);
-  return v;
+  __device__ __forceinline__ static bool phantom(const ConvTcParams&, const TileCoord&) { return false; }
+  // the epilogue warps hand accumulator buffer `bar` back to the MMA warp
+  __device__ __forceinline__ static void release_acc(uint64_t* bar) { mbar_arrive(bar); }
+};
+// CTA pairs: pair tiles are numbered over (virtual) M pairs; the two M tiles of a pair need not be neighbours.  CTA
+// `rank` gets its own tile of the pair, "dead" only when BOTH tiles of the pair are.  An M tile beyond the last one
+// (odd tile count) is a phantom: its loads are zero-filled and its stores dropped by the TMA unit.
+struct PairWalk {
+  const int* s_map;
+  int cluster_id, num_clusters, total, rank;
+  __device__ __forceinline__ PairWalk(const ConvTcParams& p, const int* map)
+      : s_map(map), cluster_id(blockIdx.x >> 1), num_clusters(gridDim.x >> 1),
+        total((((map ? map[p.N] : p.num_m_tiles) + 1) >> 1) * p.num_n_tiles), rank((int)cluster_ctarank()) {}
+  __device__ __forceinline__ int first() const { return cluster_id; }
+  __device__ __forceinline__ int step() const { return num_clusters; }
+  __device__ __forceinline__ Tile at(const ConvTcParams& p, int pt, int& hint) const {
+    const int mp = pt / p.num_n_tiles, n = pt - mp * p.num_n_tiles;
+    const int m0 = ragged_real_m(p, s_map, 2 * mp, hint);
+    const int m1 = ragged_real_m(p, s_map, 2 * mp + 1, hint);
+    Tile r;
+    r.dead = mtile_dead(p, m0) && mtile_dead(p, m1);
+    r.t = tile_coord(p, (rank ? m1 : m0) * p.num_n_tiles + n);
+    return r;
+  }
+  __device__ __forceinline__ static bool phantom(const ConvTcParams& p, const TileCoord& t) { return t.img >= p.N; }
+  // "accumulator empty" lives in the leader: both CTAs' epilogue warps arrive there
+  __device__ __forceinline__ static void release_acc(uint64_t* bar) { mbar_arrive_cluster(mapa_shared(smem_u32(bar), 0)); }
+};
+
+// ------------------------------------------------------------------------------------------------------------
+// Prologue and teardown
+// ------------------------------------------------------------------------------------------------------------
+struct TcShared {
+  uint8_t* stages;         // operand ring
+  uint8_t* wres;           // resident weights
+  uint8_t* obuf;           // output staging buffers
+  uint64_t* full_bar;      // operand stage landed (pair: in the leader, both producers' bytes)
+  uint64_t* empty_bar;     // operand stage consumed by the MMAs
+  uint64_t* tfull_bar;     // accumulator buffer complete
+  uint64_t* tempty_bar;    // accumulator buffer read out by the epilogue (pair: in the leader, both epilogues)
+  uint64_t* bufready_bar;  // staging buffer may be used by the epilogue (residual landed / store drained)
+  uint64_t* outready_bar;  // staging buffer holds a finished output group
+  uint64_t* w_bar;         // resident weights landed
+  const int* s_map;        // ragged tile map, nullptr: dense numbering
+  uint32_t tmem_base;
+};
+
+// a_map: the operand map the producer prefetches (nullptr: none); res: the kernel reads a residual
+template <class Cfg>
+__device__ __forceinline__ TcShared tc_prologue(const ConvTcParams& p, int warp, const CUtensorMap* a_map, bool res) {
+  extern __shared__ uint8_t smem_raw[];
+  // in a pair the dynamic shared window starts at the same offset in both CTAs (same kernel, no static shared memory),
+  // so the aligned buffers and barriers sit at identical offsets -- which cta_group::2 MMA descriptors and multicast
+  // commits need
+  TcShared s;
+  s.stages = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  s.wres = s.stages + Cfg::kStages * Cfg::kStageBytes;
+  s.obuf = s.wres + Cfg::kWBytes;
+  s.full_bar = reinterpret_cast<uint64_t*>(s.obuf + Cfg::kOB * kOutBufBytes);
+  s.empty_bar = s.full_bar + Cfg::kStages;
+  s.tfull_bar = s.empty_bar + Cfg::kStages;
+  s.tempty_bar = s.tfull_bar + 2;
+  s.bufready_bar = s.tempty_bar + 2;
+  s.outready_bar = s.bufready_bar + Cfg::kOB;
+  s.w_bar = s.outready_bar + Cfg::kOB;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(s.w_bar + 1);
+
+  if (threadIdx.x == 0) {
+    for (int i = 0; i < Cfg::kStages; ++i) {
+      mbar_init(&s.full_bar[i], Cfg::kPair ? 2 : 1);
+      mbar_init(&s.empty_bar[i], 1);
+    }
+    for (int i = 0; i < 2; ++i) {
+      mbar_init(&s.tfull_bar[i], 1);
+      mbar_init(&s.tempty_bar[i], Cfg::kPair ? 16 : 8);
+    }
+    for (int i = 0; i < Cfg::kOB; ++i) {
+      mbar_init(&s.bufready_bar[i], 1);
+      mbar_init(&s.outready_bar[i], Cfg::kWarpsPerStep);
+    }
+    if (Cfg::kWBytes > 0) mbar_init(s.w_bar, 1);
+    fence_mbar_init();
+  }
+  if (warp == 1) {
+    if (Cfg::kPair)
+      tmem_alloc_pair(tmem_slot, Cfg::kTmemCols);
+    else
+      tmem_alloc(tmem_slot, Cfg::kTmemCols);
+  }
+  const int lane = threadIdx.x & 31;
+  if (warp == 0 && lane == 0) {
+    if (a_map != nullptr) tma_prefetch_desc(a_map);
+    tma_prefetch_desc(&p.tmB);
+  }
+  if (warp == 10 && lane == 0) {
+    tma_prefetch_desc(&p.tmOut);
+    if (res) tma_prefetch_desc(&p.tmRes);
+  }
+  tc_fence_before();
+  if (Cfg::kPair)
+    cluster_sync_all();
+  else
+    __syncthreads();
+  tc_fence_after();
+  s.tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_slot);
+  // programmatic dependent launch: everything above overlapped the tail of the previous kernel; its output (our
+  // input / residual) may only be touched from here on
+  pdl_launch_dependents();
+  pdl_wait();
+
+  int* s_map = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(s.full_bar) + 256);
+  s.s_map = ragged_map_setup(p, s_map) ? s_map : nullptr;
+  return s;
 }
+
+template <class Cfg>
+__device__ __forceinline__ void tc_teardown(int warp, uint32_t tmem_base) {
+  // neither CTA of a pair may leave while the other can still touch its shared memory / barriers / TMEM
+  tc_fence_before();
+  if (Cfg::kPair)
+    cluster_sync_all();
+  else
+    __syncthreads();
+  if (warp == 1) {
+    if (Cfg::kPair)
+      tmem_dealloc_pair(tmem_base, Cfg::kTmemCols);
+    else
+      tmem_dealloc(tmem_base, Cfg::kTmemCols);
+  }
+}
+
 // output group handled by local step j of a tile (see the epilogue): half 0 of the epilogue warps owns the even
 // steps, half 1 the odd ones; each half walks its own contiguous range of channels
 template <int STEPS>
@@ -164,63 +340,177 @@ __device__ __forceinline__ int step_group(int j) {
   return STEPS == 1 ? 0 : (j & 1) * (STEPS / 2) + (j >> 1);
 }
 
-// RES / RELU / F16 are compile-time so the epilogue inner loop carries no runtime branches: on the low-K layers the
-// epilogue, not the MMA, sets the pace.
+// ------------------------------------------------------------------------------------------------------------
+// Output / residual TMA (warp 10, each CTA its own tiles).  One thread walks the (live tile, output group) steps in
+// order.  RES: the residual group of step s + OB - 1 is fetched into its staging buffer while the epilogue warps work
+// on step s; the epilogue adds the accumulator IN PLACE and the same buffer then leaves through a TMA store (full
+// 128-byte lines, no partial-sector writes).
+// ------------------------------------------------------------------------------------------------------------
+template <int BN, int OB, bool RES, class Walk>
+__device__ __forceinline__ void output_role(const ConvTcParams& p, const TcShared& s, const Walk& walk) {
+  if (elect_one()) {
+    constexpr int kSteps = BN / 64;
+    constexpr int kAhead = RES ? OB - 1 : 0;
+    // two cursors over this CTA's live tiles: ld (residual prefetch, runs ahead) and st (output stores)
+    int ld_tile = walk.first(), st_tile = walk.first(), ld_hint = 0, st_hint = 0, ld_j = 0, st_j = 0;
+    TileCoord ld_t{}, st_t{};
+    auto seek = [&](int& i, int& hint, TileCoord& t) {
+      for (; i < walk.total; i += walk.step()) {
+        const Tile v = walk.at(p, i, hint);
+        t = v.t;
+        if (!v.dead) break;
+      }
+    };
+    if (RES) seek(ld_tile, ld_hint, ld_t);
+    seek(st_tile, st_hint, st_t);
+    uint32_t ld_s = 0, st_s = 0;
+    auto issue_load = [&]() {
+      const uint32_t b = ld_s % OB;
+      mbar_expect_tx(&s.bufready_bar[b], kOutBufBytes);
+      tma_load_4d(s.obuf + b * kOutBufBytes, &p.tmRes, &s.bufready_bar[b], ld_t.n_tile * BN + step_group<kSteps>(ld_j) * 64,
+                  ld_t.w0, ld_t.h0, ld_t.img);
+      ++ld_s;
+      if (++ld_j == kSteps) {
+        ld_j = 0;
+        ld_tile += walk.step();
+        seek(ld_tile, ld_hint, ld_t);
+      }
+    };
+    if (RES) {
+      for (int i = 0; i < kAhead && ld_tile < walk.total; ++i) issue_load();
+    }
+    while (st_tile < walk.total) {
+      if (RES && ld_tile < walk.total) {
+        tma_store_wait_read<0>();   // the buffer of step ld_s - OB (= st_s - 1) has been read by its store
+        issue_load();
+      }
+      const uint32_t b = st_s % OB;
+      mbar_wait(&s.outready_bar[b], (st_s / OB) & 1u, 500 + (int)b);
+      tma_store_4d(&p.tmOut, s.obuf + b * kOutBufBytes, st_t.n_tile * BN + step_group<kSteps>(st_j) * 64, st_t.w0, st_t.h0,
+                   st_t.img);
+      tma_store_commit();
+      if (!RES) {
+        tma_store_wait_read<0>();
+        mbar_arrive(&s.bufready_bar[b]);
+      }
+      ++st_s;
+      if (++st_j == kSteps) {
+        st_j = 0;
+        st_tile += walk.step();
+        seek(st_tile, st_hint, st_t);
+      }
+    }
+    tma_store_wait_all();
+  }
+  __syncwarp();
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Epilogue (warps 2..9, each CTA its own 128 TMEM lanes).  TMEM gives each thread one pixel row of the accumulator.  The
+// thread adds bias (+ the residual it finds in the staging buffer), applies ReLU, packs to 16 bit and writes its row
+// into the 128B-swizzled staging buffer -- the layout TMA expects -- at the very address the residual came from.
+// 16-byte unit u of row r lives at r * 128 + ((u ^ (r & 7)) << 4): the 8 lanes of a quarter-warp hit 8 different
+// units, i.e. all 32 banks.  RES / RELU / F16 are compile-time so the inner loop carries no runtime branches: on the
+// low-K layers the epilogue, not the MMA, sets the pace.
+// ------------------------------------------------------------------------------------------------------------
+template <int BN, int OB, bool RES, bool RELU, bool F16, class Walk>
+__device__ __forceinline__ void epilogue_role(const ConvTcParams& p, const TcShared& s, const Walk& walk) {
+  constexpr int kSteps = BN / 64;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int ew = warp - 2;
+  const int q = warp & 3;          // TMEM lane quarter this warp may access
+  const int half = ew >> 2;        // BN >= 128: which steps of the tile; BN == 64: which 32 of the 64 columns
+  constexpr int kUnits = (BN == 64) ? 4 : 8;            // 16-byte units (8 channels) per row this warp handles per step
+  constexpr int kMySteps = (BN == 64) ? 1 : kSteps / 2;  // steps per tile of this warp
+  const int row = q * 32 + lane;                         // pixel of the tile == TMEM lane == staging row
+  const uint32_t row_off = (uint32_t)row * 128u;
+  const uint32_t rsw = (uint32_t)(row & 7);
+  const int u0 = (BN == 64) ? half * 4 : 0;
+  uint32_t acc = 0, acc_phase = 0, live_tiles = 0;
+  int hint = 0;
+  for (int vt = walk.first(); vt < walk.total; vt += walk.step()) {
+    const Tile v = walk.at(p, vt, hint);
+    const TileCoord t = v.t;
+    const bool phantom = Walk::phantom(p, t);
+    const int vh = phantom ? 0 : (p.valid_h != nullptr ? __ldg(p.valid_h + t.img) : INT_MAX);
+    const int h = t.h0 + (row >> p.tw_log2), w = t.w0 + (row & (p.tw - 1));
+    if (v.dead) {
+      // dead tile: no MMA was issued for it; only the zero halo is written (plain stores, rare)
+      if (!phantom && t.h0 < vh + kRaggedHalo && w < p.Wo && h < p.Ho && h < vh + kRaggedHalo) {
+        constexpr int kColsZ = BN / 2;
+        __nv_bfloat16* o = p.out + (((int64_t)t.img * p.Ho + h) * p.Wo + w) * p.Cout + t.n_tile * BN + half * kColsZ;
+        for (int c = 0; c < kColsZ; c += 8) *reinterpret_cast<uint4*>(o + c) = make_uint4(0u, 0u, 0u, 0u);
+      }
+      continue;
+    }
+    const bool live = h < vh;
+    mbar_wait(&s.tfull_bar[acc], acc_phase, 400 + (int)acc);
+    tc_fence_after();
+#pragma unroll
+    for (int i = 0; i < kMySteps; ++i) {
+      const int j = (BN == 64) ? 0 : half + 2 * i;
+      const int grp = step_group<kSteps>(j);
+      const uint32_t st = live_tiles * kSteps + j;
+      const uint32_t b = st % OB;
+      const int col0 = grp * 64 + u0 * 8;    // first column (within the BN tile) of this warp's units
+      uint32_t a[kUnits * 8];
+      const uint32_t t_addr = s.tmem_base + ((uint32_t)(q * 32) << 16) + acc * BN + col0;
+#pragma unroll
+      for (int k = 0; k < kUnits / 4; ++k) tmem_ld32(t_addr + 32 * k, reinterpret_cast<uint32_t(&)[32]>(a[32 * k]));
+      const float* bptr = p.bias + t.n_tile * BN + col0;
+      mbar_wait(&s.bufready_bar[b], RES ? ((st / OB) & 1u) : (((st / OB) & 1u) ^ 1u), 600 + (int)b);
+      tmem_ld_wait();
+      if (i == kMySteps - 1) {
+        // the accumulator is in registers: hand the TMEM buffer back to the MMA warp
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) Walk::release_acc(&s.tempty_bar[acc]);
+      }
+      uint8_t* rowp = s.obuf + b * kOutBufBytes + row_off;
+#pragma unroll
+      for (int u = 0; u < kUnits; ++u) {
+        const float4 b0 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8));
+        const float4 b1 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8 + 4));
+        uint4* sp = reinterpret_cast<uint4*>(rowp + ((((uint32_t)(u0 + u)) ^ rsw) << 4));
+        float v8[8] = {__uint_as_float(a[u * 8 + 0]) + b0.x, __uint_as_float(a[u * 8 + 1]) + b0.y,
+                       __uint_as_float(a[u * 8 + 2]) + b0.z, __uint_as_float(a[u * 8 + 3]) + b0.w,
+                       __uint_as_float(a[u * 8 + 4]) + b1.x, __uint_as_float(a[u * 8 + 5]) + b1.y,
+                       __uint_as_float(a[u * 8 + 6]) + b1.z, __uint_as_float(a[u * 8 + 7]) + b1.w};
+        if (RES) {
+          const uint4 r4 = *sp;
+          const uint32_t rv[4] = {r4.x, r4.y, r4.z, r4.w};
+#pragma unroll
+          for (int k = 0; k < 4; ++k) v8[2 * k] += lo16(rv[k], F16), v8[2 * k + 1] += hi16(rv[k], F16);
+        }
+        if (RELU) {
+#pragma unroll
+          for (int k = 0; k < 8; ++k) v8[k] = fmaxf(v8[k], 0.f);
+        }
+        uint4 o = make_uint4(pack16x2(v8[0], v8[1], F16), pack16x2(v8[2], v8[3], F16), pack16x2(v8[4], v8[5], F16),
+                             pack16x2(v8[6], v8[7], F16));
+        if (!live) o = make_uint4(0u, 0u, 0u, 0u);   // rows below the image in a ragged batch: the next layer's zero padding
+        *sp = o;
+      }
+      fence_proxy_async();   // make this thread's staging writes visible to the TMA (async proxy) store
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&s.outready_bar[b]);
+    }
+    ++live_tiles;
+    acc ^= 1u;
+    if (acc == 0) acc_phase ^= 1u;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// conv_tc_kernel: one CTA per tile, cta_group::1
+// ------------------------------------------------------------------------------------------------------------
 template <int BN, int KBLK, int OB, bool RES, bool RELU, bool F16>
 __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel(const __grid_constant__ ConvTcParams p) {
   using Cfg = TcCfg<BN, KBLK, OB>;
   constexpr int kABytes = Cfg::kABytes;
-  constexpr int kSteps = Cfg::kSteps;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* obuf = smem + Cfg::kStages * Cfg::kStageBytes;   // OB staging buffers, 1024-aligned (stage sizes are)
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(obuf + OB * kOutBufBytes);
-  uint64_t* empty_bar = full_bar + Cfg::kStages;
-  uint64_t* tfull_bar = empty_bar + Cfg::kStages;
-  uint64_t* tempty_bar = tfull_bar + 2;
-  uint64_t* bufready_bar = tempty_bar + 2;    // staging buffer may be used by the epilogue (residual landed / store drained)
-  uint64_t* outready_bar = bufready_bar + OB; // staging buffer holds a finished output group
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(outready_bar + OB);
-
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-  const int lane = threadIdx.x & 31;
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < Cfg::kStages; ++i) {
-      mbar_init(&full_bar[i], 1);
-      mbar_init(&empty_bar[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tfull_bar[i], 1);
-      mbar_init(&tempty_bar[i], 8);
-    }
-    for (int i = 0; i < OB; ++i) {
-      mbar_init(&bufready_bar[i], 1);
-      mbar_init(&outready_bar[i], Cfg::kWarpsPerStep);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 1) tmem_alloc(tmem_slot, Cfg::kTmemCols);
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&p.tmA[0]);
-    tma_prefetch_desc(&p.tmB);
-  }
-  if (warp == 10 && lane == 0) {
-    tma_prefetch_desc(&p.tmOut);
-    if (RES) tma_prefetch_desc(&p.tmRes);
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_slot);
-  // programmatic dependent launch: everything above overlapped the tail of the previous kernel; its output (our
-  // input / residual) may only be touched from here on
-  pdl_launch_dependents();
-  pdl_wait();
-
-  int* s_map_mem = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(full_bar) + 256);
-  const int* s_map = ragged_map_setup(p, s_map_mem) ? s_map_mem : nullptr;
-  const int total_tiles = (s_map ? s_map[p.N] : p.num_m_tiles) * p.num_n_tiles;   // VIRTUAL tiles when ragged
+  const TcShared s = tc_prologue<Cfg>(p, warp, &p.tmA[0], RES);
+  const CtaWalk walk(p, s.s_map);
   const int kblocks = p.n_taps * p.cblocks + p.cblocks2;
 
   if (warp == 0) {
@@ -228,8 +518,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel(const __grid_con
     if (elect_one()) {
       uint32_t stage = 0, phase = 0;
       int hint = 0;
-      for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-        const VTile v = vtile(p, s_map, vt, hint);
+      for (int vt = walk.first(); vt < walk.total; vt += walk.step()) {
+        const Tile v = walk.at(p, vt, hint);
         if (v.dead) continue;
         const TileCoord t = v.t;
         const int n0 = t.n_tile * BN;
@@ -237,11 +527,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel(const __grid_con
           const CUtensorMap* mA = &p.tmA[p.tap_map[tap]];
           const int cw = t.w0 + p.tap_dw[tap], ch = t.h0 + p.tap_dh[tap];
           for (int cb = 0; cb < p.cblocks; ++cb) {
-            mbar_wait(&empty_bar[stage], phase ^ 1u, 100 + (int)stage);
-            uint8_t* sA = smem + stage * Cfg::kStageBytes;
-            mbar_expect_tx(&full_bar[stage], Cfg::kStageBytes);
-            tma_load_4d(sA, mA, &full_bar[stage], cb * KBLK, cw, ch, t.img);
-            tma_load_2d(sA + kABytes, &p.tmB, &full_bar[stage], (tap * p.cblocks + cb) * KBLK, n0);
+            mbar_wait(&s.empty_bar[stage], phase ^ 1u, 100 + (int)stage);
+            uint8_t* sA = s.stages + stage * Cfg::kStageBytes;
+            mbar_expect_tx(&s.full_bar[stage], Cfg::kStageBytes);
+            tma_load_4d(sA, mA, &s.full_bar[stage], cb * KBLK, cw, ch, t.img);
+            tma_load_2d(sA + kABytes, &p.tmB, &s.full_bar[stage], (tap * p.cblocks + cb) * KBLK, n0);
             if (++stage == Cfg::kStages) {
               stage = 0;
               phase ^= 1u;
@@ -249,11 +539,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel(const __grid_con
           }
         }
         for (int cb = 0; cb < p.cblocks2; ++cb) {   // second source (fused downsample branch)
-          mbar_wait(&empty_bar[stage], phase ^ 1u, 100 + (int)stage);
-          uint8_t* sA = smem + stage * Cfg::kStageBytes;
-          mbar_expect_tx(&full_bar[stage], Cfg::kStageBytes);
-          tma_load_4d(sA, &p.tmA[p.map2], &full_bar[stage], cb * KBLK, t.w0, t.h0, t.img);
-          tma_load_2d(sA + kABytes, &p.tmB, &full_bar[stage], (p.n_taps * p.cblocks + cb) * KBLK, n0);
+          mbar_wait(&s.empty_bar[stage], phase ^ 1u, 100 + (int)stage);
+          uint8_t* sA = s.stages + stage * Cfg::kStageBytes;
+          mbar_expect_tx(&s.full_bar[stage], Cfg::kStageBytes);
+          tma_load_4d(sA, &p.tmA[p.map2], &s.full_bar[stage], cb * KBLK, t.w0, t.h0, t.img);
+          tma_load_2d(sA + kABytes, &p.tmB, &s.full_bar[stage], (p.n_taps * p.cblocks + cb) * KBLK, n0);
           if (++stage == Cfg::kStages) {
             stage = 0;
             phase ^= 1u;
@@ -268,189 +558,39 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel(const __grid_con
       constexpr uint32_t idesc = F16 ? umma_idesc_f16(128, BN) : umma_idesc_bf16(128, BN);
       uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
       int hint = 0;
-      for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-        if (vtile(p, s_map, vt, hint).dead) continue;
-        mbar_wait(&tempty_bar[acc], acc_phase ^ 1u, 300 + (int)acc);
+      for (int vt = walk.first(); vt < walk.total; vt += walk.step()) {
+        if (walk.at(p, vt, hint).dead) continue;
+        mbar_wait(&s.tempty_bar[acc], acc_phase ^ 1u, 300 + (int)acc);
         tc_fence_after();
-        const uint32_t d_tmem = tmem_base + acc * BN;
+        const uint32_t d_tmem = s.tmem_base + acc * BN;
         for (int kb = 0; kb < kblocks; ++kb) {
-          mbar_wait(&full_bar[stage], phase, 200 + (int)stage);
+          mbar_wait(&s.full_bar[stage], phase, 200 + (int)stage);
           tc_fence_after();
-          const uint32_t a_addr = smem_u32(smem + stage * Cfg::kStageBytes);
+          const uint32_t a_addr = smem_u32(s.stages + stage * Cfg::kStageBytes);
           const uint32_t b_addr = a_addr + kABytes;
 #pragma unroll
           for (int k = 0; k < KBLK / 16; ++k) {
             umma_bf16(d_tmem, umma_desc_kmajor<Cfg::kSwizzleBytes>(a_addr + k * 32),
                       umma_desc_kmajor<Cfg::kSwizzleBytes>(b_addr + k * 32), idesc, (uint32_t)((kb | k) != 0));
           }
-          umma_commit(&empty_bar[stage]);
+          umma_commit(&s.empty_bar[stage]);
           if (++stage == Cfg::kStages) {
             stage = 0;
             phase ^= 1u;
           }
         }
-        umma_commit(&tfull_bar[acc]);
+        umma_commit(&s.tfull_bar[acc]);
         acc ^= 1u;
         if (acc == 0) acc_phase ^= 1u;
       }
     }
     __syncwarp();
   } else if (warp == 10) {
-    // ================================ output / residual TMA ================================
-    // One thread walks the (live tile, output group) steps in order.  RES: the residual group of step s + OB - 1 is
-    // fetched into its staging buffer while the epilogue warps work on step s; the epilogue adds the accumulator IN
-    // PLACE and the same buffer then leaves through a TMA store (full 128-byte lines, no partial-sector writes).
-    if (elect_one()) {
-      constexpr int kAhead = RES ? OB - 1 : 0;
-      // two cursors over this CTA's live tiles: ld (residual prefetch, runs ahead) and st (output stores)
-      int ld_tile = blockIdx.x, st_tile = blockIdx.x, ld_hint = 0, st_hint = 0, ld_j = 0, st_j = 0;
-      TileCoord ld_t{}, st_t{};
-      auto ld_seek = [&]() {
-        for (; ld_tile < total_tiles; ld_tile += gridDim.x) {
-          const VTile v = vtile(p, s_map, ld_tile, ld_hint);
-          ld_t = v.t;
-          if (!v.dead) break;
-        }
-      };
-      auto st_seek = [&]() {
-        for (; st_tile < total_tiles; st_tile += gridDim.x) {
-          const VTile v = vtile(p, s_map, st_tile, st_hint);
-          st_t = v.t;
-          if (!v.dead) break;
-        }
-      };
-      ld_seek();
-      st_seek();
-      uint32_t ld_s = 0, st_s = 0;
-      auto issue_load = [&]() {
-        const uint32_t b = ld_s % OB;
-        mbar_expect_tx(&bufready_bar[b], kOutBufBytes);
-        tma_load_4d(obuf + b * kOutBufBytes, &p.tmRes, &bufready_bar[b], ld_t.n_tile * BN + step_group<kSteps>(ld_j) * 64, ld_t.w0,
-                    ld_t.h0, ld_t.img);
-        ++ld_s;
-        if (++ld_j == kSteps) {
-          ld_j = 0;
-          ld_tile += gridDim.x;
-          ld_seek();
-        }
-      };
-      if (RES) {
-        for (int i = 0; i < kAhead && ld_tile < total_tiles; ++i) issue_load();
-      }
-      while (st_tile < total_tiles) {
-        if (RES && ld_tile < total_tiles) {
-          tma_store_wait_read<0>();   // the buffer of step ld_s - OB (= st_s - 1) has been read by its store
-          issue_load();
-        }
-        const uint32_t b = st_s % OB;
-        mbar_wait(&outready_bar[b], (st_s / OB) & 1u, 500 + (int)b);
-        tma_store_4d(&p.tmOut, obuf + b * kOutBufBytes, st_t.n_tile * BN + step_group<kSteps>(st_j) * 64, st_t.w0, st_t.h0, st_t.img);
-        tma_store_commit();
-        if (!RES) {
-          tma_store_wait_read<0>();
-          mbar_arrive(&bufready_bar[b]);
-        }
-        ++st_s;
-        if (++st_j == kSteps) {
-          st_j = 0;
-          st_tile += gridDim.x;
-          st_seek();
-        }
-      }
-      tma_store_wait_all();
-    }
-    __syncwarp();
+    output_role<BN, OB, RES>(p, s, walk);
   } else {
-    // ================================ epilogue (warps 2..9) ================================
-    // TMEM gives each thread one pixel row of the accumulator.  The thread adds bias (+ the residual it finds in the
-    // staging buffer), applies ReLU, packs to 16 bit and writes its row into the 128B-swizzled staging buffer -- the
-    // layout TMA expects -- at the very address the residual came from.  16-byte unit u of row r lives at
-    // r * 128 + ((u ^ (r & 7)) << 4): the 8 lanes of a quarter-warp hit 8 different units, i.e. all 32 banks.
-    const int ew = warp - 2;
-    const int q = warp & 3;          // TMEM lane quarter this warp may access
-    const int half = ew >> 2;        // BN >= 128: which steps of the tile; BN == 64: which 32 of the 64 columns
-    constexpr int kUnits = (BN == 64) ? 4 : 8;            // 16-byte units (8 channels) per row this warp handles per step
-    constexpr int kMySteps = (BN == 64) ? 1 : kSteps / 2;  // steps per tile of this warp
-    const int row = q * 32 + lane;                         // pixel of the tile == TMEM lane == staging row
-    const uint32_t row_off = (uint32_t)row * 128u;
-    const uint32_t rsw = (uint32_t)(row & 7);
-    const int u0 = (BN == 64) ? half * 4 : 0;
-    uint32_t acc = 0, acc_phase = 0, live_tiles = 0;
-    int hint = 0;
-    for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-      const TileCoord t = vtile(p, s_map, vt, hint).t;
-      const int vh = p.valid_h != nullptr ? __ldg(p.valid_h + t.img) : INT_MAX;
-      const int h = t.h0 + (row >> p.tw_log2), w = t.w0 + (row & (p.tw - 1));
-      if (t.h0 >= vh) {
-        // dead tile: no MMA was issued for it; only the zero halo is written (plain stores, rare)
-        if (t.h0 < vh + kRaggedHalo && w < p.Wo && h < p.Ho && h < vh + kRaggedHalo) {
-          constexpr int kColsZ = BN / 2;
-          __nv_bfloat16* o = p.out + (((int64_t)t.img * p.Ho + h) * p.Wo + w) * p.Cout + t.n_tile * BN + half * kColsZ;
-          for (int c = 0; c < kColsZ; c += 8) *reinterpret_cast<uint4*>(o + c) = make_uint4(0u, 0u, 0u, 0u);
-        }
-        continue;
-      }
-      const bool live = h < vh;
-      mbar_wait(&tfull_bar[acc], acc_phase, 400 + (int)acc);
-      tc_fence_after();
-#pragma unroll
-      for (int i = 0; i < kMySteps; ++i) {
-        const int j = (BN == 64) ? 0 : half + 2 * i;
-        const int grp = step_group<kSteps>(j);
-        const uint32_t s = live_tiles * kSteps + j;
-        const uint32_t b = s % OB;
-        const int col0 = grp * 64 + u0 * 8;    // first column (within the BN tile) of this warp's units
-        uint32_t a[kUnits * 8];
-        const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * BN + col0;
-#pragma unroll
-        for (int k = 0; k < kUnits / 4; ++k) tmem_ld32(t_addr + 32 * k, reinterpret_cast<uint32_t(&)[32]>(a[32 * k]));
-        const float* bptr = p.bias + t.n_tile * BN + col0;
-        mbar_wait(&bufready_bar[b], RES ? ((s / OB) & 1u) : (((s / OB) & 1u) ^ 1u), 600 + (int)b);
-        tmem_ld_wait();
-        if (i == kMySteps - 1) {
-          // the accumulator is in registers: hand the TMEM buffer back to the MMA warp
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&tempty_bar[acc]);
-        }
-        uint8_t* rowp = obuf + b * kOutBufBytes + row_off;
-#pragma unroll
-        for (int u = 0; u < kUnits; ++u) {
-          const float4 b0 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8));
-          const float4 b1 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8 + 4));
-          uint4* sp = reinterpret_cast<uint4*>(rowp + ((((uint32_t)(u0 + u)) ^ rsw) << 4));
-          float v[8] = {__uint_as_float(a[u * 8 + 0]) + b0.x, __uint_as_float(a[u * 8 + 1]) + b0.y,
-                        __uint_as_float(a[u * 8 + 2]) + b0.z, __uint_as_float(a[u * 8 + 3]) + b0.w,
-                        __uint_as_float(a[u * 8 + 4]) + b1.x, __uint_as_float(a[u * 8 + 5]) + b1.y,
-                        __uint_as_float(a[u * 8 + 6]) + b1.z, __uint_as_float(a[u * 8 + 7]) + b1.w};
-          if (RES) {
-            const uint4 r4 = *sp;
-            const uint32_t rv[4] = {r4.x, r4.y, r4.z, r4.w};
-#pragma unroll
-            for (int k = 0; k < 4; ++k) v[2 * k] += lo16(rv[k], F16), v[2 * k + 1] += hi16(rv[k], F16);
-          }
-          if (RELU) {
-#pragma unroll
-            for (int k = 0; k < 8; ++k) v[k] = fmaxf(v[k], 0.f);
-          }
-          uint4 o = make_uint4(pack16x2(v[0], v[1], F16), pack16x2(v[2], v[3], F16), pack16x2(v[4], v[5], F16),
-                               pack16x2(v[6], v[7], F16));
-          if (!live) o = make_uint4(0u, 0u, 0u, 0u);   // rows below the image in a ragged batch: the next layer's zero padding
-          *sp = o;
-        }
-        fence_proxy_async();   // make this thread's staging writes visible to the TMA (async proxy) store
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&outready_bar[b]);
-      }
-      ++live_tiles;
-      acc ^= 1u;
-      if (acc == 0) acc_phase ^= 1u;
-    }
+    epilogue_role<BN, OB, RES, RELU, F16>(p, s, walk);
   }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, Cfg::kTmemCols);
+  tc_teardown<Cfg>(warp, s.tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -460,120 +600,31 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel(const __grid_con
 // at BN = 256, so the same shared memory holds 6 operand stages instead of 4.  The leader (rank 0) issues every MMA;
 // "stage full" barriers live in the leader (both CTAs' TMA loads count their bytes there), "stage empty" and
 // "accumulator full" are multicast by tcgen05.commit to both CTAs, "accumulator empty" is arrived remotely by the
-// peer's epilogue warps.  A pair is skipped in a ragged batch only when BOTH of its tiles are dead; an M tile beyond
-// the last one (odd tile count) is a phantom: its loads are zero-filled and its stores dropped by the TMA unit.
+// peer's epilogue warps (PairWalk::release_acc).  A pair is skipped in a ragged batch only when BOTH of its tiles are
+// dead (see PairWalk).
 // ------------------------------------------------------------------------------------------------------------
-template <int BN, int OB>
-struct TcCfgPair {
-  static constexpr int kABytes = 128 * 64 * 2;
-  static constexpr int kBBytes = (BN / 2) * 64 * 2;
-  static constexpr int kStageBytes = kABytes + kBBytes;
-  static constexpr int kFixedBytes = OB * kOutBufBytes + 256 /*barriers*/ + kMapBytes + 1024 /*align slack*/;
-  static constexpr int kStagesFit = (kSmemLimit - kFixedBytes) / kStageBytes;
-  static constexpr int kStages = kStagesFit < 8 ? kStagesFit : 8;
-  static constexpr int kTmemCols = 2 * BN;
-  static constexpr int kSmemBytes = kStages * kStageBytes + kFixedBytes;
-  static constexpr int kSteps = BN / 64;
-  static constexpr int kWarpsPerStep = 4;
-  static_assert(BN == 128 || BN == 256, "pair kernel: BN = 128 or 256");
-  static_assert(kStages >= 2 && kSmemBytes <= kSmemLimit && kSmemBytes > 120 * 1024, "shared memory budget");
-  static_assert((2 * kStages + 4 + 2 * OB) * 8 + 4 <= 256, "barrier block");
-};
-
-__device__ __forceinline__ bool mtile_dead(const ConvTcParams& p, int m_tile) {
-  if (m_tile >= p.num_m_tiles) return true;
-  if (p.valid_h == nullptr) return false;
-  const int mt = m_tile / p.tiles_w;
-  return (mt % p.tiles_h) * p.th >= __ldg(p.valid_h + mt / p.tiles_h);
-}
-// pair tiles are numbered over (virtual, see ragged_map_setup) M pairs; the two M tiles of a pair need not be neighbours.
-// PairTile = this CTA's own tile of pair tile pt (dense single-CTA coordinates) + "both tiles of the pair are dead".
-struct PairTile {
-  TileCoord t;
-  bool dead;
-};
-__device__ __forceinline__ PairTile pair_tile(const ConvTcParams& p, const int* s_map, int pt, int rank, int& hint) {
-  const int mp = pt / p.num_n_tiles, n = pt - mp * p.num_n_tiles;
-  const int m0 = ragged_real_m(p, s_map, 2 * mp, hint);
-  const int m1 = ragged_real_m(p, s_map, 2 * mp + 1, hint);
-  PairTile r;
-  r.dead = mtile_dead(p, m0) && mtile_dead(p, m1);
-  r.t = tile_coord(p, (rank ? m1 : m0) * p.num_n_tiles + n);
-  return r;
-}
-
 template <int BN, int OB, bool RES, bool RELU, bool F16>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kTcThreads, 1)
     conv_tc_pair_kernel(const __grid_constant__ ConvTcParams p) {
   using Cfg = TcCfgPair<BN, OB>;
   constexpr int kABytes = Cfg::kABytes;
-  constexpr int kSteps = Cfg::kSteps;
-  extern __shared__ uint8_t smem_raw[];
-  // the dynamic shared window starts at the same offset in both CTAs (same kernel, no static shared memory), so the
-  // aligned buffers and barriers sit at identical offsets -- which cta_group::2 MMA descriptors and multicast commits need
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* obuf = smem + Cfg::kStages * Cfg::kStageBytes;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(obuf + OB * kOutBufBytes);
-  uint64_t* empty_bar = full_bar + Cfg::kStages;
-  uint64_t* tfull_bar = empty_bar + Cfg::kStages;
-  uint64_t* tempty_bar = tfull_bar + 2;
-  uint64_t* bufready_bar = tempty_bar + 2;
-  uint64_t* outready_bar = bufready_bar + OB;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(outready_bar + OB);
-
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-  const int lane = threadIdx.x & 31;
-  const int rank = (int)cluster_ctarank();
-  const bool leader = rank == 0;
-  const int cluster_id = blockIdx.x >> 1, num_clusters = gridDim.x >> 1;
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < Cfg::kStages; ++i) {
-      mbar_init(&full_bar[i], 2);    // the two producers (used in the leader only)
-      mbar_init(&empty_bar[i], 1);   // multicast commit
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tfull_bar[i], 1);   // multicast commit
-      mbar_init(&tempty_bar[i], 16); // 8 epilogue warps of each CTA (used in the leader only)
-    }
-    for (int i = 0; i < OB; ++i) {
-      mbar_init(&bufready_bar[i], 1);
-      mbar_init(&outready_bar[i], Cfg::kWarpsPerStep);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 1) tmem_alloc_pair(tmem_slot, Cfg::kTmemCols);
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&p.tmA[0]);
-    tma_prefetch_desc(&p.tmB);
-  }
-  if (warp == 10 && lane == 0) {
-    tma_prefetch_desc(&p.tmOut);
-    if (RES) tma_prefetch_desc(&p.tmRes);
-  }
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_slot);
-  pdl_launch_dependents();
-  pdl_wait();
-
-  int* s_map_mem = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(full_bar) + 256);
-  const int* s_map = ragged_map_setup(p, s_map_mem) ? s_map_mem : nullptr;
-  const int total_pairs = (((s_map ? s_map[p.N] : p.num_m_tiles) + 1) >> 1) * p.num_n_tiles;
+  const TcShared s = tc_prologue<Cfg>(p, warp, &p.tmA[0], RES);
+  const PairWalk walk(p, s.s_map);
+  const bool leader = walk.rank == 0;
   const int kblocks = p.n_taps * p.cblocks + p.cblocks2;
 
   if (warp == 0) {
     // ================================ TMA producer (both CTAs) ================================
     if (elect_one()) {
       uint32_t stage = 0, phase = 0;
-      const uint32_t full0 = mapa_shared(smem_u32(&full_bar[0]), 0);   // the leader's full barriers
+      const uint32_t full0 = mapa_shared(smem_u32(&s.full_bar[0]), 0);   // the leader's full barriers
       int hint = 0;
-      for (int pt = cluster_id; pt < total_pairs; pt += num_clusters) {
-        const PairTile pr = pair_tile(p, s_map, pt, rank, hint);
+      for (int pt = walk.first(); pt < walk.total; pt += walk.step()) {
+        const Tile pr = walk.at(p, pt, hint);
         if (pr.dead) continue;
         const TileCoord t = pr.t;
-        const int n0 = t.n_tile * BN + rank * (BN / 2);
+        const int n0 = t.n_tile * BN + walk.rank * (BN / 2);
         for (int kb = 0; kb < kblocks; ++kb) {
           const CUtensorMap* mA;
           int c0, cw, ch;
@@ -585,11 +636,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kTcThreads, 1)
             mA = &p.tmA[p.map2];
             c0 = (kb - p.n_taps * p.cblocks) * 64, cw = t.w0, ch = t.h0;
           }
-          mbar_wait(&empty_bar[stage], phase ^ 1u, 100 + (int)stage);
-          uint8_t* sA = smem + stage * Cfg::kStageBytes;
+          mbar_wait(&s.empty_bar[stage], phase ^ 1u, 100 + (int)stage);
+          uint8_t* sA = s.stages + stage * Cfg::kStageBytes;
           const uint32_t fb = full0 + stage * 8u;
           if (leader)
-            mbar_expect_tx(&full_bar[stage], 2 * Cfg::kStageBytes);
+            mbar_expect_tx(&s.full_bar[stage], 2 * Cfg::kStageBytes);
           else
             mbar_arrive_cluster(fb);
           tma_load_4d_pair(sA, mA, fb, c0, cw, ch, t.img);
@@ -608,203 +659,56 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kTcThreads, 1)
       constexpr uint32_t idesc = F16 ? umma_idesc_f16(256, BN) : umma_idesc_bf16(256, BN);
       uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
       int hint = 0;
-      for (int pt = cluster_id; pt < total_pairs; pt += num_clusters) {
-        if (pair_tile(p, s_map, pt, rank, hint).dead) continue;
-        mbar_wait(&tempty_bar[acc], acc_phase ^ 1u, 300 + (int)acc);
+      for (int pt = walk.first(); pt < walk.total; pt += walk.step()) {
+        if (walk.at(p, pt, hint).dead) continue;
+        mbar_wait(&s.tempty_bar[acc], acc_phase ^ 1u, 300 + (int)acc);
         tc_fence_after();
-        const uint32_t d_tmem = tmem_base + acc * BN;
+        const uint32_t d_tmem = s.tmem_base + acc * BN;
         for (int kb = 0; kb < kblocks; ++kb) {
-          mbar_wait(&full_bar[stage], phase, 200 + (int)stage);
+          mbar_wait(&s.full_bar[stage], phase, 200 + (int)stage);
           tc_fence_after();
-          const uint32_t a_addr = smem_u32(smem + stage * Cfg::kStageBytes);
+          const uint32_t a_addr = smem_u32(s.stages + stage * Cfg::kStageBytes);
           const uint32_t b_addr = a_addr + kABytes;
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
             umma_bf16_pair(d_tmem, umma_desc_kmajor<128>(a_addr + k * 32), umma_desc_kmajor<128>(b_addr + k * 32), idesc,
                            (uint32_t)((kb | k) != 0));
           }
-          umma_commit_pair(&empty_bar[stage], 3);
+          umma_commit_pair(&s.empty_bar[stage], 3);
           if (++stage == Cfg::kStages) {
             stage = 0;
             phase ^= 1u;
           }
         }
-        umma_commit_pair(&tfull_bar[acc], 3);
+        umma_commit_pair(&s.tfull_bar[acc], 3);
         acc ^= 1u;
         if (acc == 0) acc_phase ^= 1u;
       }
     }
     __syncwarp();
   } else if (warp == 10) {
-    // ================================ output / residual TMA (per CTA, own tile) ================================
-    if (elect_one()) {
-      constexpr int kAhead = RES ? OB - 1 : 0;
-      int ld_pt = cluster_id, st_pt = cluster_id, ld_hint = 0, st_hint = 0, ld_j = 0, st_j = 0;
-      TileCoord ld_t{}, st_t{};
-      auto ld_seek = [&]() {
-        for (; ld_pt < total_pairs; ld_pt += num_clusters) {
-          const PairTile pr = pair_tile(p, s_map, ld_pt, rank, ld_hint);
-          ld_t = pr.t;
-          if (!pr.dead) break;
-        }
-      };
-      auto st_seek = [&]() {
-        for (; st_pt < total_pairs; st_pt += num_clusters) {
-          const PairTile pr = pair_tile(p, s_map, st_pt, rank, st_hint);
-          st_t = pr.t;
-          if (!pr.dead) break;
-        }
-      };
-      ld_seek();
-      st_seek();
-      uint32_t ld_s = 0, st_s = 0;
-      auto issue_load = [&]() {
-        const uint32_t b = ld_s % OB;
-        mbar_expect_tx(&bufready_bar[b], kOutBufBytes);
-        tma_load_4d(obuf + b * kOutBufBytes, &p.tmRes, &bufready_bar[b], ld_t.n_tile * BN + step_group<kSteps>(ld_j) * 64, ld_t.w0,
-                    ld_t.h0, ld_t.img);
-        ++ld_s;
-        if (++ld_j == kSteps) {
-          ld_j = 0;
-          ld_pt += num_clusters;
-          ld_seek();
-        }
-      };
-      if (RES) {
-        for (int i = 0; i < kAhead && ld_pt < total_pairs; ++i) issue_load();
-      }
-      while (st_pt < total_pairs) {
-        if (RES && ld_pt < total_pairs) {
-          tma_store_wait_read<0>();
-          issue_load();
-        }
-        const uint32_t b = st_s % OB;
-        mbar_wait(&outready_bar[b], (st_s / OB) & 1u, 500 + (int)b);
-        tma_store_4d(&p.tmOut, obuf + b * kOutBufBytes, st_t.n_tile * BN + step_group<kSteps>(st_j) * 64, st_t.w0, st_t.h0, st_t.img);
-        tma_store_commit();
-        if (!RES) {
-          tma_store_wait_read<0>();
-          mbar_arrive(&bufready_bar[b]);
-        }
-        ++st_s;
-        if (++st_j == kSteps) {
-          st_j = 0;
-          st_pt += num_clusters;
-          st_seek();
-        }
-      }
-      tma_store_wait_all();
-    }
-    __syncwarp();
+    output_role<BN, OB, RES>(p, s, walk);
   } else {
-    // ================================ epilogue (warps 2..9, per CTA, own 128 TMEM lanes) ================================
-    const int ew = warp - 2;
-    const int q = warp & 3;
-    const int half = ew >> 2;
-    constexpr int kUnits = 8;
-    constexpr int kMySteps = kSteps / 2;
-    const int row = q * 32 + lane;
-    const uint32_t row_off = (uint32_t)row * 128u;
-    const uint32_t rsw = (uint32_t)(row & 7);
-    const uint32_t tempty0 = mapa_shared(smem_u32(&tempty_bar[0]), 0);   // the leader's accumulator-empty barriers
-    uint32_t acc = 0, acc_phase = 0, live_tiles = 0;
-    int hint = 0;
-    for (int pt = cluster_id; pt < total_pairs; pt += num_clusters) {
-      const PairTile pr = pair_tile(p, s_map, pt, rank, hint);
-      const TileCoord t = pr.t;
-      const bool phantom = t.img >= p.N;
-      const int vh = phantom ? 0 : (p.valid_h != nullptr ? __ldg(p.valid_h + t.img) : INT_MAX);
-      const int h = t.h0 + (row >> p.tw_log2), w = t.w0 + (row & (p.tw - 1));
-      if (pr.dead) {
-        if (!phantom && t.h0 < vh + kRaggedHalo && w < p.Wo && h < p.Ho && h < vh + kRaggedHalo) {
-          constexpr int kColsZ = BN / 2;
-          __nv_bfloat16* o = p.out + (((int64_t)t.img * p.Ho + h) * p.Wo + w) * p.Cout + t.n_tile * BN + half * kColsZ;
-          for (int c = 0; c < kColsZ; c += 8) *reinterpret_cast<uint4*>(o + c) = make_uint4(0u, 0u, 0u, 0u);
-        }
-        continue;
-      }
-      const bool live = h < vh;
-      mbar_wait(&tfull_bar[acc], acc_phase, 400 + (int)acc);
-      tc_fence_after();
-#pragma unroll
-      for (int i = 0; i < kMySteps; ++i) {
-        const int j = half + 2 * i;
-        const int grp = step_group<kSteps>(j);
-        const uint32_t s = live_tiles * kSteps + j;
-        const uint32_t b = s % OB;
-        const int col0 = grp * 64;
-        uint32_t a[kUnits * 8];
-        const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * BN + col0;
-#pragma unroll
-        for (int k = 0; k < kUnits / 4; ++k) tmem_ld32(t_addr + 32 * k, reinterpret_cast<uint32_t(&)[32]>(a[32 * k]));
-        const float* bptr = p.bias + t.n_tile * BN + col0;
-        mbar_wait(&bufready_bar[b], RES ? ((s / OB) & 1u) : (((s / OB) & 1u) ^ 1u), 600 + (int)b);
-        tmem_ld_wait();
-        if (i == kMySteps - 1) {
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive_cluster(tempty0 + acc * 8u);
-        }
-        uint8_t* rowp = obuf + b * kOutBufBytes + row_off;
-#pragma unroll
-        for (int u = 0; u < kUnits; ++u) {
-          const float4 b0 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8));
-          const float4 b1 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8 + 4));
-          uint4* sp = reinterpret_cast<uint4*>(rowp + ((((uint32_t)u) ^ rsw) << 4));
-          float v[8] = {__uint_as_float(a[u * 8 + 0]) + b0.x, __uint_as_float(a[u * 8 + 1]) + b0.y,
-                        __uint_as_float(a[u * 8 + 2]) + b0.z, __uint_as_float(a[u * 8 + 3]) + b0.w,
-                        __uint_as_float(a[u * 8 + 4]) + b1.x, __uint_as_float(a[u * 8 + 5]) + b1.y,
-                        __uint_as_float(a[u * 8 + 6]) + b1.z, __uint_as_float(a[u * 8 + 7]) + b1.w};
-          if (RES) {
-            const uint4 r4 = *sp;
-            const uint32_t rv[4] = {r4.x, r4.y, r4.z, r4.w};
-#pragma unroll
-            for (int k = 0; k < 4; ++k) v[2 * k] += lo16(rv[k], F16), v[2 * k + 1] += hi16(rv[k], F16);
-          }
-          if (RELU) {
-#pragma unroll
-            for (int k = 0; k < 8; ++k) v[k] = fmaxf(v[k], 0.f);
-          }
-          uint4 o = make_uint4(pack16x2(v[0], v[1], F16), pack16x2(v[2], v[3], F16), pack16x2(v[4], v[5], F16),
-                               pack16x2(v[6], v[7], F16));
-          if (!live) o = make_uint4(0u, 0u, 0u, 0u);
-          *sp = o;
-        }
-        fence_proxy_async();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&outready_bar[b]);
-      }
-      ++live_tiles;
-      acc ^= 1u;
-      if (acc == 0) acc_phase ^= 1u;
-    }
+    epilogue_role<BN, OB, RES, RELU, F16>(p, s, walk);
   }
-
-  // neither CTA may leave while the other can still touch its shared memory / barriers / TMEM
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == 1) tmem_dealloc_pair(tmem_base, Cfg::kTmemCols);
+  tc_teardown<Cfg>(warp, s.tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// Stem variant with a HALO tile (the default for 128 x 1 tiles; NBC_STEM_HALO=0 switches it off).  conv_tc_kernel<64, 32> fetches
-// the stem's A operand as 7 boxes of 128 rows x 64 bytes per tile -- 896 L2 requests of 1.4 sectors each, and ncu shows
-// the launch bound by that request rate (12 % tensor-pipe activity).  The windows of neighbouring outputs overlap: tap
-// row ky of output wo is the 64 bytes (8 pixels x 4 channels) at padded pixel 2*wo, i.e. 16 bytes after the window of
-// output wo - 1.  16 bytes is exactly the row pitch of a NO-SWIZZLE K-major UMMA core matrix (8 rows x 16 bytes, rows
-// 16 bytes apart): with LBO = 16 B (next 16 bytes of K) and SBO = 128 B (next 8 rows) a descriptor reads the 128
-// overlapping windows of a tile straight out of one contiguous input row.  So a 128 x 1 output tile needs 7 bulk copies
-// of 2 096 bytes (one per tap row) instead of 896 small requests, and the 28 KB of stem weights stay resident in
-// shared memory for the whole kernel.  Epilogue / output path as in conv_tc_kernel<64, ...>.
+// Stem variant with a HALO tile (128 x 1 tiles).  conv_tc_kernel<64, 32> fetches the stem's A operand as 7 boxes of
+// 128 rows x 64 bytes per tile -- 896 L2 requests of 1.4 sectors each, and ncu shows the launch bound by that request
+// rate (12 % tensor-pipe activity).  The windows of neighbouring outputs overlap: tap row ky of output wo is the 64
+// bytes (8 pixels x 4 channels) at padded pixel 2*wo, i.e. 16 bytes after the window of output wo - 1.  16 bytes is
+// exactly the row pitch of a NO-SWIZZLE K-major UMMA core matrix (8 rows x 16 bytes, rows 16 bytes apart): with LBO =
+// 16 B (next 16 bytes of K) and SBO = 128 B (next 8 rows) a descriptor reads the 128 overlapping windows of a tile
+// straight out of one contiguous input row.  So a 128 x 1 output tile needs 7 bulk copies of 2 096 bytes (one per tap
+// row) instead of 896 small requests, and the 28 KB of stem weights stay resident in shared memory for the whole
+// kernel.  Epilogue / output path as in conv_tc_kernel<64, ...>.
 // ------------------------------------------------------------------------------------------------------------
 constexpr int kStemRowBytes = 2112;                 // (2 * 127 + 8) pixels x 8 B = 2 096, rounded up to a multiple of 64
 constexpr int kStemStageBytes = 7 * kStemRowBytes + 64;      // 14 848 = 116 x 128
-constexpr int kStemStages = 6;
-constexpr int kStemOB = 4;
-constexpr int kStemWBytes = 7 * 64 * 64;            // 7 tap rows x 64 output channels x 32 k (64B-swizzled boxes)
-constexpr int kStemSmemBytes = kStemStages * kStemStageBytes + kStemWBytes + kStemOB * kOutBufBytes + 256 + kMapBytes + 1024;
-static_assert(kStemSmemBytes <= kSmemLimit && kStemSmemBytes > 120 * 1024, "stem halo kernel: shared memory budget");
-static_assert(kStemStageBytes % 128 == 0 && (kStemStages * kStemStageBytes) % 1024 == 0, "stem halo kernel: alignment");
+using StemCfg = TcLayout<6, kStemStageBytes, 7 * 64 * 64 /*7 tap rows x 64 output channels x 32 k, 64B-swizzled*/, 64, 4, false>;
+static_assert(StemCfg::kUsedBytes > 120 * 1024, "stem halo kernel: shared memory budget");
 
 __device__ __forceinline__ void bulk_load_1d(void* smem, const void* gmem, uint32_t bytes, uint64_t* bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem)),
@@ -824,72 +728,32 @@ __device__ __forceinline__ uint64_t umma_desc_kmajor_noswizzle(uint32_t smem_add
 
 template <bool RELU, bool F16>
 __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_stem_kernel(const __grid_constant__ ConvTcParams p) {
-  constexpr int BN = 64, OB = kStemOB;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* wres = smem + kStemStages * kStemStageBytes;      // resident weights, 1024-aligned
-  uint8_t* obuf = wres + kStemWBytes;                        // OB staging buffers, 1024-aligned
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(obuf + OB * kOutBufBytes);
-  uint64_t* empty_bar = full_bar + kStemStages;
-  uint64_t* tfull_bar = empty_bar + kStemStages;
-  uint64_t* tempty_bar = tfull_bar + 2;
-  uint64_t* bufready_bar = tempty_bar + 2;
-  uint64_t* outready_bar = bufready_bar + OB;
-  uint64_t* w_bar = outready_bar + OB;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(w_bar + 1);
-
+  using Cfg = StemCfg;
+  constexpr int BN = 64;
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-  const int lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < kStemStages; ++i) {
-      mbar_init(&full_bar[i], 1);
-      mbar_init(&empty_bar[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tfull_bar[i], 1);
-      mbar_init(&tempty_bar[i], 8);
-    }
-    for (int i = 0; i < OB; ++i) {
-      mbar_init(&bufready_bar[i], 1);
-      mbar_init(&outready_bar[i], 8);
-    }
-    mbar_init(w_bar, 1);
-    fence_mbar_init();
-  }
-  if (warp == 1) tmem_alloc(tmem_slot, 2 * BN);
-  if (warp == 0 && lane == 0) tma_prefetch_desc(&p.tmB);
-  if (warp == 10 && lane == 0) tma_prefetch_desc(&p.tmOut);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_slot);
-  pdl_launch_dependents();
-  pdl_wait();
-
-  int* s_map_mem = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(full_bar) + 256);
-  const int* s_map = ragged_map_setup(p, s_map_mem) ? s_map_mem : nullptr;
-  const int total_tiles = s_map ? s_map[p.N] : p.num_m_tiles;      // one N tile: all 64 output channels
+  const TcShared s = tc_prologue<Cfg>(p, warp, nullptr, false);
+  const CtaWalk walk(p, s.s_map);      // one N tile: all 64 output channels
 
   if (warp == 0) {
     // ================================ producer: weights once, then 7 input rows per tile ================================
     if (elect_one()) {
-      mbar_expect_tx(w_bar, kStemWBytes);
-      for (int ky = 0; ky < 7; ++ky) tma_load_2d(wres + ky * 4096, &p.tmB, w_bar, ky * 32, 0);
+      mbar_expect_tx(s.w_bar, Cfg::kWBytes);
+      for (int ky = 0; ky < 7; ++ky) tma_load_2d(s.wres + ky * 4096, &p.tmB, s.w_bar, ky * 32, 0);
       uint32_t stage = 0, phase = 0;
       const int64_t row_bytes = (int64_t)p.stem_wp * 8;
       int hint = 0;
-      for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-        const VTile v = vtile(p, s_map, vt, hint);
+      for (int vt = walk.first(); vt < walk.total; vt += walk.step()) {
+        const Tile v = walk.at(p, vt, hint);
         if (v.dead) continue;
         const TileCoord t = v.t;      // tw = 128, th = 1: h0 = output row, w0 = first output column
         // what is left of the padded row from pixel 2 * w0 on (a multiple of 16 bytes); beyond it lie outputs >= Wo
         const uint32_t len = (uint32_t)min((int64_t)(2 * 127 + 8) * 8, row_bytes - (int64_t)t.w0 * 16);
-        mbar_wait(&empty_bar[stage], phase ^ 1u, 100 + (int)stage);
-        uint8_t* sA = smem + stage * kStemStageBytes;
-        mbar_expect_tx(&full_bar[stage], 7 * len);
+        mbar_wait(&s.empty_bar[stage], phase ^ 1u, 100 + (int)stage);
+        uint8_t* sA = s.stages + stage * Cfg::kStageBytes;
+        mbar_expect_tx(&s.full_bar[stage], 7 * len);
         const uint8_t* src = p.stem_src + ((int64_t)t.img * p.stem_hp + 2 * t.h0) * row_bytes + (int64_t)t.w0 * 16;
-        for (int ky = 0; ky < 7; ++ky) bulk_load_1d(sA + ky * kStemRowBytes, src + ky * row_bytes, len, &full_bar[stage]);
-        if (++stage == kStemStages) {
+        for (int ky = 0; ky < 7; ++ky) bulk_load_1d(sA + ky * kStemRowBytes, src + ky * row_bytes, len, &s.full_bar[stage]);
+        if (++stage == Cfg::kStages) {
           stage = 0;
           phase ^= 1u;
         }
@@ -901,16 +765,16 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_stem_kernel(const __gri
     if (elect_one()) {
       constexpr uint32_t idesc = F16 ? umma_idesc_f16(128, BN) : umma_idesc_bf16(128, BN);
       uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
-      mbar_wait(w_bar, 0, 700);
-      const uint32_t w_addr = smem_u32(wres);
+      mbar_wait(s.w_bar, 0, 700);
+      const uint32_t w_addr = smem_u32(s.wres);
       int hint = 0;
-      for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-        if (vtile(p, s_map, vt, hint).dead) continue;
-        mbar_wait(&tempty_bar[acc], acc_phase ^ 1u, 300 + (int)acc);
-        mbar_wait(&full_bar[stage], phase, 200 + (int)stage);
+      for (int vt = walk.first(); vt < walk.total; vt += walk.step()) {
+        if (walk.at(p, vt, hint).dead) continue;
+        mbar_wait(&s.tempty_bar[acc], acc_phase ^ 1u, 300 + (int)acc);
+        mbar_wait(&s.full_bar[stage], phase, 200 + (int)stage);
         tc_fence_after();
-        const uint32_t d_tmem = tmem_base + acc * BN;
-        const uint32_t a_addr = smem_u32(smem + stage * kStemStageBytes);
+        const uint32_t d_tmem = s.tmem_base + acc * BN;
+        const uint32_t a_addr = smem_u32(s.stages + stage * Cfg::kStageBytes);
 #pragma unroll
         for (int ky = 0; ky < 7; ++ky) {
 #pragma unroll
@@ -919,9 +783,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_stem_kernel(const __gri
                       umma_desc_kmajor<64>(w_addr + ky * 4096 + k * 32), idesc, (uint32_t)((ky | k) != 0));
           }
         }
-        umma_commit(&empty_bar[stage]);
-        umma_commit(&tfull_bar[acc]);
-        if (++stage == kStemStages) {
+        umma_commit(&s.empty_bar[stage]);
+        umma_commit(&s.tfull_bar[acc]);
+        if (++stage == Cfg::kStages) {
           stage = 0;
           phase ^= 1u;
         }
@@ -931,89 +795,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_stem_kernel(const __gri
     }
     __syncwarp();
   } else if (warp == 10) {
-    // ================================ output TMA ================================
-    if (elect_one()) {
-      uint32_t st_s = 0;
-      int hint = 0;
-      for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-        const VTile v = vtile(p, s_map, vt, hint);
-        if (v.dead) continue;
-        const uint32_t b = st_s % OB;
-        mbar_wait(&outready_bar[b], (st_s / OB) & 1u, 500 + (int)b);
-        const TileCoord t = v.t;
-        tma_store_4d(&p.tmOut, obuf + b * kOutBufBytes, 0, t.w0, t.h0, t.img);
-        tma_store_commit();
-        tma_store_wait_read<0>();
-        mbar_arrive(&bufready_bar[b]);
-        ++st_s;
-      }
-      tma_store_wait_all();
-    }
-    __syncwarp();
+    output_role<BN, Cfg::kOB, false>(p, s, walk);
   } else {
-    // ================================ epilogue (warps 2..9): as conv_tc_kernel with BN = 64 ================================
-    const int ew = warp - 2;
-    const int q = warp & 3;
-    const int half = ew >> 2;            // which 32 of the 64 columns
-    const int row = q * 32 + lane;
-    const uint32_t row_off = (uint32_t)row * 128u;
-    const uint32_t rsw = (uint32_t)(row & 7);
-    const int u0 = half * 4;
-    uint32_t acc = 0, acc_phase = 0, live_tiles = 0;
-    int hint = 0;
-    for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-      const TileCoord t = vtile(p, s_map, vt, hint).t;
-      const int vh = p.valid_h != nullptr ? __ldg(p.valid_h + t.img) : INT_MAX;
-      const int h = t.h0, w = t.w0 + row;
-      if (t.h0 >= vh) {
-        if (t.h0 < vh + kRaggedHalo && w < p.Wo && h < p.Ho) {
-          __nv_bfloat16* o = p.out + (((int64_t)t.img * p.Ho + h) * p.Wo + w) * p.Cout + half * 32;
-          for (int c = 0; c < 32; c += 8) *reinterpret_cast<uint4*>(o + c) = make_uint4(0u, 0u, 0u, 0u);
-        }
-        continue;
-      }
-      mbar_wait(&tfull_bar[acc], acc_phase, 400 + (int)acc);
-      tc_fence_after();
-      const uint32_t s = live_tiles;
-      const uint32_t b = s % OB;
-      uint32_t a[32];
-      tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + acc * BN + u0 * 8, a);
-      const float* bptr = p.bias + u0 * 8;
-      mbar_wait(&bufready_bar[b], ((s / OB) & 1u) ^ 1u, 600 + (int)b);
-      tmem_ld_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&tempty_bar[acc]);
-      uint8_t* rowp = obuf + b * kOutBufBytes + row_off;
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const float4 b0 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8));
-        const float4 b1 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8 + 4));
-        float v[8] = {__uint_as_float(a[u * 8 + 0]) + b0.x, __uint_as_float(a[u * 8 + 1]) + b0.y,
-                      __uint_as_float(a[u * 8 + 2]) + b0.z, __uint_as_float(a[u * 8 + 3]) + b0.w,
-                      __uint_as_float(a[u * 8 + 4]) + b1.x, __uint_as_float(a[u * 8 + 5]) + b1.y,
-                      __uint_as_float(a[u * 8 + 6]) + b1.z, __uint_as_float(a[u * 8 + 7]) + b1.w};
-        if (RELU) {
-#pragma unroll
-          for (int k = 0; k < 8; ++k) v[k] = fmaxf(v[k], 0.f);
-        }
-        *reinterpret_cast<uint4*>(rowp + ((((uint32_t)(u0 + u)) ^ rsw) << 4)) =
-            make_uint4(pack16x2(v[0], v[1], F16), pack16x2(v[2], v[3], F16), pack16x2(v[4], v[5], F16), pack16x2(v[6], v[7], F16));
-      }
-      fence_proxy_async();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&outready_bar[b]);
-      ++live_tiles;
-      acc ^= 1u;
-      if (acc == 0) acc_phase ^= 1u;
-    }
+    epilogue_role<BN, Cfg::kOB, false, RELU, F16>(p, s, walk);
   }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, 2 * BN);
+  tc_teardown<Cfg>(warp, s.tmem_base);
 }
-
 
 // ------------------------------------------------------------------------------------------------------------
 // 3x3 HALO kernel for the 64 -> 64 convolutions of layer1 (stride 1, dilation 1, pad 1; 128 x 1 output tiles).
@@ -1027,82 +814,35 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_stem_kernel(const __gri
 // swizzle to the absolute shared-memory address (bits [4,7) ^= bits [7,10)), exactly as the TMA unit did when it wrote
 // the tile; setting base offset = (start >> 7) & 7 gives wrong results.  The nine 8 KB weight slabs stay resident in
 // shared memory for the whole kernel.  Epilogue / output path as in conv_tc_kernel<64, ...>.
-// layer1 conv2: 0.049 -> 0.033 ms per [8,624,1024] pass (480 -> 715 TFLOP/s); NBC_HALO3=0 selects the nine-box path.
+// layer1 conv2: 0.049 -> 0.033 ms per [8,624,1024] pass (480 -> 715 TFLOP/s).
 // ------------------------------------------------------------------------------------------------------------
 constexpr int kHaloW = 130;
-constexpr int kHaloStageBytes = 50176;               // 3 x 130 x 128 B = 49 920, rounded up to 49 x 1024
-constexpr int kHaloStages = 2;
-constexpr int kHaloOB = 3;
-constexpr int kHaloWBytes = 9 * 64 * 128;            // 9 taps x 64 output channels x 64 input channels x 2 B
-constexpr int kHaloSmemBytes = kHaloStages * kHaloStageBytes + kHaloWBytes + kHaloOB * kOutBufBytes + 256 + kMapBytes + 1024;
-static_assert(kHaloSmemBytes <= kSmemLimit && kHaloSmemBytes > 120 * 1024, "3x3 halo kernel: shared memory budget");
-
+// 3 x 130 x 128 B = 49 920 per stage, rounded up to 49 x 1024; 9 taps x 64 output channels x 64 input channels x 2 B of weights
+using Halo3Cfg = TcLayout<2, 50176, 9 * 64 * 128, 64, 3, false>;
+static_assert(Halo3Cfg::kUsedBytes > 120 * 1024, "3x3 halo kernel: shared memory budget");
 
 template <bool RELU, bool F16>
 __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_halo3_kernel(const __grid_constant__ ConvTcParams p) {
-  constexpr int BN = 64, OB = kHaloOB;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* wres = smem + kHaloStages * kHaloStageBytes;      // resident weights, 1024-aligned
-  uint8_t* obuf = wres + kHaloWBytes;                        // OB staging buffers, 1024-aligned
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(obuf + OB * kOutBufBytes);
-  uint64_t* empty_bar = full_bar + kHaloStages;
-  uint64_t* tfull_bar = empty_bar + kHaloStages;
-  uint64_t* tempty_bar = tfull_bar + 2;
-  uint64_t* bufready_bar = tempty_bar + 2;
-  uint64_t* outready_bar = bufready_bar + OB;
-  uint64_t* w_bar = outready_bar + OB;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(w_bar + 1);
-
+  using Cfg = Halo3Cfg;
+  constexpr int BN = 64;
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-  const int lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < kHaloStages; ++i) {
-      mbar_init(&full_bar[i], 1);
-      mbar_init(&empty_bar[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tfull_bar[i], 1);
-      mbar_init(&tempty_bar[i], 8);
-    }
-    for (int i = 0; i < OB; ++i) {
-      mbar_init(&bufready_bar[i], 1);
-      mbar_init(&outready_bar[i], 8);
-    }
-    mbar_init(w_bar, 1);
-    fence_mbar_init();
-  }
-  if (warp == 1) tmem_alloc(tmem_slot, 2 * BN);
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&p.tmA[1]);
-    tma_prefetch_desc(&p.tmB);
-  }
-  if (warp == 10 && lane == 0) tma_prefetch_desc(&p.tmOut);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_slot);
-  pdl_launch_dependents();
-  pdl_wait();
-
-  int* s_map_mem = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(full_bar) + 256);
-  const int* s_map = ragged_map_setup(p, s_map_mem) ? s_map_mem : nullptr;
-  const int total_tiles = s_map ? s_map[p.N] : p.num_m_tiles;      // one N tile: all 64 output channels
+  const TcShared s = tc_prologue<Cfg>(p, warp, &p.tmA[1], false);
+  const CtaWalk walk(p, s.s_map);      // one N tile: all 64 output channels
 
   if (warp == 0) {
     // ================================ producer: weights once, then one halo box per tile ================================
     if (elect_one()) {
-      mbar_expect_tx(w_bar, kHaloWBytes);
-      for (int t = 0; t < 9; ++t) tma_load_2d(wres + t * 8192, &p.tmB, w_bar, t * 64, 0);
+      mbar_expect_tx(s.w_bar, Cfg::kWBytes);
+      for (int t = 0; t < 9; ++t) tma_load_2d(s.wres + t * 8192, &p.tmB, s.w_bar, t * 64, 0);
       uint32_t stage = 0, phase = 0;
       int hint = 0;
-      for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-        const VTile v = vtile(p, s_map, vt, hint);
+      for (int vt = walk.first(); vt < walk.total; vt += walk.step()) {
+        const Tile v = walk.at(p, vt, hint);
         if (v.dead) continue;
-        mbar_wait(&empty_bar[stage], phase ^ 1u, 100 + (int)stage);
-        mbar_expect_tx(&full_bar[stage], 3 * kHaloW * 128);
-        tma_load_4d(smem + stage * kHaloStageBytes, &p.tmA[1], &full_bar[stage], 0, v.t.w0 - 1, v.t.h0 - 1, v.t.img);
-        if (++stage == kHaloStages) {
+        mbar_wait(&s.empty_bar[stage], phase ^ 1u, 100 + (int)stage);
+        mbar_expect_tx(&s.full_bar[stage], 3 * kHaloW * 128);
+        tma_load_4d(s.stages + stage * Cfg::kStageBytes, &p.tmA[1], &s.full_bar[stage], 0, v.t.w0 - 1, v.t.h0 - 1, v.t.img);
+        if (++stage == Cfg::kStages) {
           stage = 0;
           phase ^= 1u;
         }
@@ -1114,16 +854,16 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_halo3_kernel(const __gr
     if (elect_one()) {
       constexpr uint32_t idesc = F16 ? umma_idesc_f16(128, BN) : umma_idesc_bf16(128, BN);
       uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
-      mbar_wait(w_bar, 0, 700);
-      const uint32_t w_addr = smem_u32(wres);
+      mbar_wait(s.w_bar, 0, 700);
+      const uint32_t w_addr = smem_u32(s.wres);
       int hint = 0;
-      for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-        if (vtile(p, s_map, vt, hint).dead) continue;
-        mbar_wait(&tempty_bar[acc], acc_phase ^ 1u, 300 + (int)acc);
-        mbar_wait(&full_bar[stage], phase, 200 + (int)stage);
+      for (int vt = walk.first(); vt < walk.total; vt += walk.step()) {
+        if (walk.at(p, vt, hint).dead) continue;
+        mbar_wait(&s.tempty_bar[acc], acc_phase ^ 1u, 300 + (int)acc);
+        mbar_wait(&s.full_bar[stage], phase, 200 + (int)stage);
         tc_fence_after();
-        const uint32_t d_tmem = tmem_base + acc * BN;
-        const uint32_t a_addr = smem_u32(smem + stage * kHaloStageBytes);
+        const uint32_t d_tmem = s.tmem_base + acc * BN;
+        const uint32_t a_addr = smem_u32(s.stages + stage * Cfg::kStageBytes);
 #pragma unroll
         for (int t = 0; t < 9; ++t) {
           const uint32_t a_tap = a_addr + (uint32_t)((t / 3) * kHaloW + (t % 3)) * 128u;
@@ -1133,9 +873,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_halo3_kernel(const __gr
                       (uint32_t)((t | k) != 0));
           }
         }
-        umma_commit(&empty_bar[stage]);
-        umma_commit(&tfull_bar[acc]);
-        if (++stage == kHaloStages) {
+        umma_commit(&s.empty_bar[stage]);
+        umma_commit(&s.tfull_bar[acc]);
+        if (++stage == Cfg::kStages) {
           stage = 0;
           phase ^= 1u;
         }
@@ -1145,100 +885,16 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_halo3_kernel(const __gr
     }
     __syncwarp();
   } else if (warp == 10) {
-    // ================================ output TMA ================================
-    if (elect_one()) {
-      uint32_t st_s = 0;
-      int hint = 0;
-      for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-        const VTile v = vtile(p, s_map, vt, hint);
-        if (v.dead) continue;
-        const uint32_t b = st_s % OB;
-        mbar_wait(&outready_bar[b], (st_s / OB) & 1u, 500 + (int)b);
-        tma_store_4d(&p.tmOut, obuf + b * kOutBufBytes, 0, v.t.w0, v.t.h0, v.t.img);
-        tma_store_commit();
-        tma_store_wait_read<0>();
-        mbar_arrive(&bufready_bar[b]);
-        ++st_s;
-      }
-      tma_store_wait_all();
-    }
-    __syncwarp();
+    output_role<BN, Cfg::kOB, false>(p, s, walk);
   } else {
-    // ================================ epilogue (warps 2..9): as conv_tc_kernel with BN = 64 ================================
-    const int ew = warp - 2;
-    const int q = warp & 3;
-    const int half = ew >> 2;            // which 32 of the 64 columns
-    const int row = q * 32 + lane;
-    const uint32_t row_off = (uint32_t)row * 128u;
-    const uint32_t rsw = (uint32_t)(row & 7);
-    const int u0 = half * 4;
-    uint32_t acc = 0, acc_phase = 0, live_tiles = 0;
-    int hint = 0;
-    for (int vt = blockIdx.x; vt < total_tiles; vt += gridDim.x) {
-      const TileCoord t = vtile(p, s_map, vt, hint).t;
-      const int vh = p.valid_h != nullptr ? __ldg(p.valid_h + t.img) : INT_MAX;
-      const int h = t.h0, w = t.w0 + row;
-      if (t.h0 >= vh) {
-        if (t.h0 < vh + kRaggedHalo && w < p.Wo && h < p.Ho) {
-          __nv_bfloat16* o = p.out + (((int64_t)t.img * p.Ho + h) * p.Wo + w) * p.Cout + half * 32;
-          for (int c = 0; c < 32; c += 8) *reinterpret_cast<uint4*>(o + c) = make_uint4(0u, 0u, 0u, 0u);
-        }
-        continue;
-      }
-      mbar_wait(&tfull_bar[acc], acc_phase, 400 + (int)acc);
-      tc_fence_after();
-      const uint32_t s = live_tiles;
-      const uint32_t b = s % OB;
-      uint32_t a[32];
-      tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + acc * BN + u0 * 8, a);
-      const float* bptr = p.bias + u0 * 8;
-      mbar_wait(&bufready_bar[b], ((s / OB) & 1u) ^ 1u, 600 + (int)b);
-      tmem_ld_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&tempty_bar[acc]);
-      uint8_t* rowp = obuf + b * kOutBufBytes + row_off;
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const float4 b0 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8));
-        const float4 b1 = __ldg(reinterpret_cast<const float4*>(bptr + u * 8 + 4));
-        float v[8] = {__uint_as_float(a[u * 8 + 0]) + b0.x, __uint_as_float(a[u * 8 + 1]) + b0.y,
-                      __uint_as_float(a[u * 8 + 2]) + b0.z, __uint_as_float(a[u * 8 + 3]) + b0.w,
-                      __uint_as_float(a[u * 8 + 4]) + b1.x, __uint_as_float(a[u * 8 + 5]) + b1.y,
-                      __uint_as_float(a[u * 8 + 6]) + b1.z, __uint_as_float(a[u * 8 + 7]) + b1.w};
-        if (RELU) {
-#pragma unroll
-          for (int k = 0; k < 8; ++k) v[k] = fmaxf(v[k], 0.f);
-        }
-        *reinterpret_cast<uint4*>(rowp + ((((uint32_t)(u0 + u)) ^ rsw) << 4)) =
-            make_uint4(pack16x2(v[0], v[1], F16), pack16x2(v[2], v[3], F16), pack16x2(v[4], v[5], F16), pack16x2(v[6], v[7], F16));
-      }
-      fence_proxy_async();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&outready_bar[b]);
-      ++live_tiles;
-      acc ^= 1u;
-      if (acc == 0) acc_phase ^= 1u;
-    }
+    epilogue_role<BN, Cfg::kOB, false, RELU, F16>(p, s, walk);
   }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, 2 * BN);
+  tc_teardown<Cfg>(warp, s.tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------------------
-// NBC_RAGGED_COMPACT=0 switches the compact tile enumeration of ragged batches off (A/B measurements)
-static int ragged_compact_default() {
-  static const int v = [] {
-    const char* e = getenv("NBC_RAGGED_COMPACT");
-    return (e && *e) ? atoi(e) : 1;
-  }();
-  return v;
-}
-
 static int encode_act_map(CUtensorMap* m, const void* base, uint64_t C, uint64_t Wd, uint64_t Hd, uint64_t Nd,
                           uint64_t strideW, uint64_t strideH, uint64_t strideN, uint32_t boxW, uint32_t boxH,
                           uint32_t boxC = 64) {
@@ -1307,7 +963,7 @@ struct ConvTcLaunch {
   int grid;
   int out_bufs;
   int pair;   // 1: conv_tc_pair_kernel (clusters of 2, cta_group::2 MMA)
-  int stem_halo;   // 1: conv_tc_stem_kernel (halo tile; default where the tile geometry allows)
+  int stem_halo;   // 1: conv_tc_stem_kernel (128 x 1 stem tiles)
   int halo3;       // 1: conv_tc_halo3_kernel (64 -> 64 3x3 out of one halo box per tile)
 };
 
@@ -1315,36 +971,11 @@ struct ConvTcLaunch {
 // where the operand pipeline or the MMA sets the pace -- Cout % 256 == 0 without a residual and K >= 512 (the 1x1
 // reductions out of wide tensors, the 3x3 convs of layer3 / layer4 / the head, conv3 + downsample of layer3 / layer4) --
 // and lose on the residual layers (epilogue / HBM bound), on BN = 128 and on very short K.
-// Environment NBC_CTA2 overrides the rule for experiments: a bit mask of layer classes (1: 1x1 without residual,
-// 2: residual, 4: 3x3, 8: dual source) forced onto pairs whenever Cout % 128 == 0; 0 switches pairs off.
-static int pair_mode() {
-  static int mode = -2;
-  if (mode == -2) {
-    const char* e = getenv("NBC_CTA2");
-    mode = (e && *e) ? atoi(e) : -1;
-  }
-  return mode;
-}
-static int want_pair(int cls, int bn, int kblocks) {
-  const int mode = pair_mode();
-  if (mode >= 0) return (bn >= 128 && (mode & cls)) ? 1 : 0;
-  return (bn == 256 && cls != 2 && kblocks >= 8) ? 1 : 0;
-}
-// SMs the persistent conv kernels occupy: all of them, or NBC_CONV_SMS (an experiment knob: a persistent conv CTA owns
-// its SM, so the kernels of the engine's side streams -- K1, K3, K5 -- only run between conv launches; leaving a few
-// SMs free lets them overlap the network pass at the price of that share of the conv throughput).
-static int conv_sms() {
-  static int n = -1;
-  if (n < 0) {
-    const char* e = getenv("NBC_CONV_SMS");
-    const int all = sm_count();
-    n = (e && *e && atoi(e) >= 2 && atoi(e) < all) ? (atoi(e) & ~1) : all;
-  }
-  return n;
-}
+static int want_pair(bool residual, int bn, int kblocks) { return (!residual && bn == 256 && kblocks >= 8) ? 1 : 0; }
+// the persistent conv kernels occupy every SM (DESIGN §8: leaving some to the side streams never paid)
 static void set_grid(ConvTcLaunch* L) {
   const ConvTcParams& p = L->p;
-  const int sms = conv_sms();
+  const int sms = sm_count();
   if (L->pair) {
     const int pairs = ((p.num_m_tiles + 1) / 2) * p.num_n_tiles;
     L->grid = 2 * (pairs < sms / 2 ? pairs : sms / 2);
@@ -1392,23 +1023,7 @@ static int build_launch(const ConvGeom& g, const void* x, const void* w, const f
   choose_tile(Ho, Wo, &p);
   p.N = g.N, p.Ho = Ho, p.Wo = Wo, p.Cout = g.Cout;
   p.num_m_tiles = g.N * p.tiles_w * p.tiles_h;
-  int bn = (g.Cout % 256 == 0) ? 256 : (g.Cout % 128 == 0 ? 128 : 64);
-  // experiment knob: 128-column tiles on the residual layers (32 KB operand stages: 5 of them next to the 4 staging
-  // buffers instead of 3 -- ncu shows those launches at ~50 % of DRAM, L2 and tensor pipe alike, i.e. latency bound)
-  static const int res_bn = [] {
-    const char* e = getenv("NBC_RES_BN");
-    return (e && *e) ? atoi(e) : 0;
-  }();
-  if (residual != nullptr && res_bn == 128 && g.Cout % 128 == 0) bn = 128;
-  // experiment knob (NBC_SPLIT256=1): the Cout = 256 launches without a residual (layer3 conv1 / conv2) have ONE 256-column
-  // N tile, so their tile count is the number of M tiles -- ~620 pairs for a chunk of 16 scans = 8.4 rounds of the 74 CTA
-  // pairs, 9 paid.  Two 128-column N tiles (still on pairs) double the tile count: 16.9 rounds, 17 paid
-  static const int split256 = [] {
-    const char* e = getenv("NBC_SPLIT256");
-    return (e && *e) ? atoi(e) : 0;
-  }();
-  const bool split = split256 == 1 && residual == nullptr && g.Cout == 256 && g.kh * g.kw * (g.Cin / 64) >= 8;
-  if (split) bn = 128;
+  const int bn = (g.Cout % 256 == 0) ? 256 : (g.Cout % 128 == 0 ? 128 : 64);
   L->block_n = bn;
   L->kblk = 64;
   p.num_n_tiles = g.Cout / bn;
@@ -1458,12 +1073,8 @@ static int build_launch(const ConvGeom& g, const void* x, const void* w, const f
     if (!used[0]) p.tmA[0] = p.tmA[p.tap_map[0]];
   }
   L->stem_halo = 0;
-  // 3x3 halo kernel (layer1's 64 -> 64 convolutions): NBC_HALO3=0 keeps the nine-box path
-  static const int halo3 = [] {
-    const char* e = getenv("NBC_HALO3");
-    return (e && *e) ? atoi(e) : 1;
-  }();
-  L->halo3 = (halo3 == 1 && g.Cin == 64 && g.Cout == 64 && g.kh == 3 && g.kw == 3 && g.stride == 1 && g.dil == 1 && g.pad == 1 &&
+  // 3x3 halo kernel for layer1's 64 -> 64 convolutions; other tiles of that shape take the nine-box path
+  L->halo3 = (g.Cin == 64 && g.Cout == 64 && g.kh == 3 && g.kw == 3 && g.stride == 1 && g.dil == 1 && g.pad == 1 &&
               residual == nullptr && p.tw == 128 && p.th == 1)
                  ? 1
                  : 0;
@@ -1472,7 +1083,7 @@ static int build_launch(const ConvGeom& g, const void* x, const void* w, const f
                             (uint64_t)g.H * g.W * g.Cin * eb, kHaloW, 3);
     if (rc) return rc;
   }
-  L->pair = L->halo3 ? 0 : (split ? 1 : want_pair(residual != nullptr ? 2 : (p.n_taps > 1 ? 4 : 1), bn, p.n_taps * p.cblocks));
+  L->pair = L->halo3 ? 0 : want_pair(residual != nullptr, bn, p.n_taps * p.cblocks);
   int rc = encode_weight_map(&p.tmB, w, (uint64_t)p.n_taps * g.Cin, g.Cout, L->pair ? bn / 2 : bn);
   if (rc) return rc;
   rc = encode_out_maps(&p, g.N, Ho, Wo, g.Cout, y, residual);
@@ -1482,127 +1093,103 @@ static int build_launch(const ConvGeom& g, const void* x, const void* w, const f
   return 0;
 }
 
-// Programmatic dependent launch (environment NBC_PDL=0 switches it off): the prologue of a conv kernel -- barrier init,
-// TMEM allocation, descriptor prefetch -- runs while the previous kernel of the stream drains (see pdl_wait()).
-static bool pdl_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("NBC_PDL");
-    on = (e && *e) ? (atoi(e) != 0) : NBC_PDL_DEFAULT;
+// One launch helper for every conv kernel.  Programmatic dependent launch: the prologue of a conv kernel -- barrier
+// init, TMEM allocation, descriptor prefetch -- runs while the previous kernel of the stream drains (see pdl_wait()).
+// The pair kernel's __cluster_dims__(2, 1, 1) makes its grid a whole number of pairs.
+template <void (*Kernel)(ConvTcParams), int SMEM>
+static int launch_tc(const ConvTcLaunch& L, cudaStream_t stream) {
+  static bool attr_set = false;
+  if (!attr_set) {
+    NBC_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+    attr_set = true;
   }
-  return on != 0;
-}
-static cudaError_t launch_tc(void (*kernel)(const ConvTcParams), const ConvTcLaunch& L, int smem, cudaStream_t stream) {
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3((unsigned)L.grid);
   cfg.blockDim = dim3(kTcThreads);
-  cfg.dynamicSmemBytes = (size_t)smem;
+  cfg.dynamicSmemBytes = (size_t)SMEM;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, L.p);
-}
-
-template <int BN, int KBLK, int OB, bool RES, bool RELU, bool F16>
-static int launch_one(const ConvTcLaunch& L, cudaStream_t stream) {
-  static bool attr_set = false;
-  if (!attr_set) {
-    NBC_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BN, KBLK, OB, RES, RELU, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  TcCfg<BN, KBLK, OB>::kSmemBytes));
-    attr_set = true;
-  }
-  NBC_CUDA(launch_tc(conv_tc_kernel<BN, KBLK, OB, RES, RELU, F16>, L, TcCfg<BN, KBLK, OB>::kSmemBytes, stream));
+  cfg.numAttrs = 1;
+  NBC_CUDA(cudaLaunchKernelEx(&cfg, Kernel, L.p));
   count_launch();
   return 0;
 }
 
-template <int BN, int OB, bool RES, bool RELU, bool F16>
-static int launch_pair_one(const ConvTcLaunch& L, cudaStream_t stream) {
-  static bool attr_set = false;
-  if (!attr_set) {
-    NBC_CUDA(cudaFuncSetAttribute(conv_tc_pair_kernel<BN, OB, RES, RELU, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  TcCfgPair<BN, OB>::kSmemBytes));
-    attr_set = true;
-  }
-  // __cluster_dims__(2, 1, 1) on the kernel: the grid is a whole number of pairs
-  NBC_CUDA(launch_tc(conv_tc_pair_kernel<BN, OB, RES, RELU, F16>, L, TcCfgPair<BN, OB>::kSmemBytes, stream));
-  count_launch();
-  return 0;
+static int no_kernel(const char* family, const ConvTcLaunch& L) {
+  set_error("conv_tc: no %s kernel for block_n=%d out_bufs=%d residual=%d relu=%d f16=%d", family, L.block_n, L.out_bufs,
+            L.p.residual != nullptr ? 1 : 0, L.p.relu, L.p.f16);
+  return NBC_ERR_INVALID;
 }
 
+// Kernel families.  Family::run<OB, RES, RELU, F16> launches the family's kernel for one variant key, or refuses a
+// combination that no selection rule produces: no kernel is compiled for it.
 template <int BN>
-static int launch_pair(const ConvTcLaunch& L, cudaStream_t stream) {
-  const bool res = L.p.residual != nullptr;
-  const int key = (res ? 8 : (L.out_bufs == 4 ? 4 : 0)) | (L.p.relu ? 2 : 0) | (L.p.f16 ? 1 : 0);
+struct CtaKernels {   // conv_tc_kernel with 64-element K blocks: every combination
+  template <int OB, bool RES, bool RELU, bool F16>
+  static int run(const ConvTcLaunch& L, cudaStream_t stream) {
+    return launch_tc<conv_tc_kernel<BN, 64, OB, RES, RELU, F16>, TcCfg<BN, 64, OB>::kSmemBytes>(L, stream);
+  }
+};
+struct StemKernels {   // the per-window stem, conv_tc_kernel<64, 32>: 4 staging buffers, no residual
+  template <int OB, bool RES, bool RELU, bool F16>
+  static int run(const ConvTcLaunch& L, cudaStream_t stream) {
+    if constexpr (OB != 4 || RES)
+      return no_kernel("per-window stem", L);
+    else
+      return launch_tc<conv_tc_kernel<64, 32, 4, false, RELU, F16>, TcCfg<64, 32, 4>::kSmemBytes>(L, stream);
+  }
+};
+struct PairKernels {   // conv_tc_pair_kernel<256>: no residual (want_pair)
+  template <int OB, bool RES, bool RELU, bool F16>
+  static int run(const ConvTcLaunch& L, cudaStream_t stream) {
+    if constexpr (RES)
+      return no_kernel("CTA-pair", L);
+    else
+      return launch_tc<conv_tc_pair_kernel<256, OB, false, RELU, F16>, TcCfgPair<256, OB>::kSmemBytes>(L, stream);
+  }
+};
+// the halo kernels have a fixed staging depth; out_bufs only describes the launch
+struct StemHaloKernels {
+  template <int OB, bool RES, bool RELU, bool F16>
+  static int run(const ConvTcLaunch& L, cudaStream_t stream) {
+    if constexpr (RES)
+      return no_kernel("stem halo", L);
+    else
+      return launch_tc<conv_tc_stem_kernel<RELU, F16>, StemCfg::kSmemBytes>(L, stream);
+  }
+};
+struct Halo3Kernels {
+  template <int OB, bool RES, bool RELU, bool F16>
+  static int run(const ConvTcLaunch& L, cudaStream_t stream) {
+    if constexpr (RES)
+      return no_kernel("3x3 halo", L);
+    else
+      return launch_tc<conv_tc_halo3_kernel<RELU, F16>, Halo3Cfg::kSmemBytes>(L, stream);
+  }
+};
+
+// variant key of a launch: 8 = residual (always with 4 staging buffers), 4 = 4 staging buffers, 2 = ReLU, 1 = fp16
+template <class Family>
+static int launch_variant(const ConvTcLaunch& L, cudaStream_t stream) {
+  const int key = (L.p.residual != nullptr ? 8 : (L.out_bufs == 4 ? 4 : 0)) | (L.p.relu ? 2 : 0) | (L.p.f16 ? 1 : 0);
   switch (key) {
-    case 0: return launch_pair_one<BN, 2, false, false, false>(L, stream);
-    case 1: return launch_pair_one<BN, 2, false, false, true>(L, stream);
-    case 2: return launch_pair_one<BN, 2, false, true, false>(L, stream);
-    case 3: return launch_pair_one<BN, 2, false, true, true>(L, stream);
-    case 4: return launch_pair_one<BN, 4, false, false, false>(L, stream);
-    case 5: return launch_pair_one<BN, 4, false, false, true>(L, stream);
-    case 6: return launch_pair_one<BN, 4, false, true, false>(L, stream);
-    case 7: return launch_pair_one<BN, 4, false, true, true>(L, stream);
-    case 8: return launch_pair_one<BN, 4, true, false, false>(L, stream);
-    case 9: return launch_pair_one<BN, 4, true, false, true>(L, stream);
-    case 10: return launch_pair_one<BN, 4, true, true, false>(L, stream);
-    default: return launch_pair_one<BN, 4, true, true, true>(L, stream);
-  }
-}
-
-template <bool RELU, bool F16>
-static int launch_stem_one(const ConvTcLaunch& L, cudaStream_t stream) {
-  static bool attr_set = false;
-  if (!attr_set) {
-    NBC_CUDA(cudaFuncSetAttribute(conv_tc_stem_kernel<RELU, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStemSmemBytes));
-    attr_set = true;
-  }
-  NBC_CUDA(launch_tc(conv_tc_stem_kernel<RELU, F16>, L, kStemSmemBytes, stream));
-  count_launch();
-  return 0;
-}
-static int launch_stem(const ConvTcLaunch& L, cudaStream_t stream) {
-  if (L.p.relu) return L.p.f16 ? launch_stem_one<true, true>(L, stream) : launch_stem_one<true, false>(L, stream);
-  return L.p.f16 ? launch_stem_one<false, true>(L, stream) : launch_stem_one<false, false>(L, stream);
-}
-
-template <bool RELU, bool F16>
-static int launch_halo3_one(const ConvTcLaunch& L, cudaStream_t stream) {
-  static bool attr_set = false;
-  if (!attr_set) {
-    NBC_CUDA(cudaFuncSetAttribute(conv_tc_halo3_kernel<RELU, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHaloSmemBytes));
-    attr_set = true;
-  }
-  NBC_CUDA(launch_tc(conv_tc_halo3_kernel<RELU, F16>, L, kHaloSmemBytes, stream));
-  count_launch();
-  return 0;
-}
-static int launch_halo3(const ConvTcLaunch& L, cudaStream_t stream) {
-  if (L.p.relu) return L.p.f16 ? launch_halo3_one<true, true>(L, stream) : launch_halo3_one<true, false>(L, stream);
-  return L.p.f16 ? launch_halo3_one<false, true>(L, stream) : launch_halo3_one<false, false>(L, stream);
-}
-
-template <int BN, int KBLK>
-static int launch_bn(const ConvTcLaunch& L, cudaStream_t stream) {
-  const bool res = L.p.residual != nullptr;
-  const int key = (res ? 8 : (L.out_bufs == 4 ? 4 : 0)) | (L.p.relu ? 2 : 0) | (L.p.f16 ? 1 : 0);
-  switch (key) {
-    case 0: return launch_one<BN, KBLK, 2, false, false, false>(L, stream);
-    case 1: return launch_one<BN, KBLK, 2, false, false, true>(L, stream);
-    case 2: return launch_one<BN, KBLK, 2, false, true, false>(L, stream);
-    case 3: return launch_one<BN, KBLK, 2, false, true, true>(L, stream);
-    case 4: return launch_one<BN, KBLK, 4, false, false, false>(L, stream);
-    case 5: return launch_one<BN, KBLK, 4, false, false, true>(L, stream);
-    case 6: return launch_one<BN, KBLK, 4, false, true, false>(L, stream);
-    case 7: return launch_one<BN, KBLK, 4, false, true, true>(L, stream);
-    case 8: return launch_one<BN, KBLK, 4, true, false, false>(L, stream);
-    case 9: return launch_one<BN, KBLK, 4, true, false, true>(L, stream);
-    case 10: return launch_one<BN, KBLK, 4, true, true, false>(L, stream);
-    default: return launch_one<BN, KBLK, 4, true, true, true>(L, stream);
+    case 0: return Family::template run<2, false, false, false>(L, stream);
+    case 1: return Family::template run<2, false, false, true>(L, stream);
+    case 2: return Family::template run<2, false, true, false>(L, stream);
+    case 3: return Family::template run<2, false, true, true>(L, stream);
+    case 4: return Family::template run<4, false, false, false>(L, stream);
+    case 5: return Family::template run<4, false, false, true>(L, stream);
+    case 6: return Family::template run<4, false, true, false>(L, stream);
+    case 7: return Family::template run<4, false, true, true>(L, stream);
+    case 8: return Family::template run<4, true, false, false>(L, stream);
+    case 9: return Family::template run<4, true, false, true>(L, stream);
+    case 10: return Family::template run<4, true, true, false>(L, stream);
+    case 11: return Family::template run<4, true, true, true>(L, stream);
+    default: return no_kernel("conv_tc", L);
   }
 }
 
@@ -1623,7 +1210,6 @@ int conv_tc_prepare_stem(int N, int Ho, int Wo, int Hp, int Wp, const void* padd
   p.n_taps = 7, p.cblocks = 1, p.relu = relu;
   p.bias = bias, p.residual = nullptr, p.out = reinterpret_cast<__nv_bfloat16*>(y);
   p.valid_h = valid_h;
-  p.ragged_compact = ragged_compact_default();
   L->block_n = 64, L->kblk = 32;
   const char* base = reinterpret_cast<const char*>(padded);
   const uint64_t row_bytes = (uint64_t)Wp * 8;
@@ -1640,15 +1226,11 @@ int conv_tc_prepare_stem(int N, int Ho, int Wo, int Hp, int Wp, const void* padd
   L->out_bufs = 4;
   L->pair = 0;
   L->halo3 = 0;
-  // halo kernel (conv_tc_stem_kernel): 128 x 1 tiles only (the production geometry, Wo = 512); verified on B200 in round 2
-  // (stem 0.180 -> 0.105 ms per [8,624,1024] pass) and the default since; NBC_STEM_HALO=0 selects the per-window kernel
-  static const int halo = [] {
-    const char* e = getenv("NBC_STEM_HALO");
-    return (e && *e) ? atoi(e) : 1;
-  }();
+  // halo kernel (conv_tc_stem_kernel): 128 x 1 tiles (the production geometry, Wo = 512; stem 0.180 -> 0.105 ms per
+  // [8,624,1024] pass on B200); other tile shapes take the per-window kernel conv_tc_kernel<64, 32>
   p.stem_src = reinterpret_cast<const uint8_t*>(padded);
   p.stem_hp = Hp, p.stem_wp = Wp;
-  L->stem_halo = (halo == 1 && p.tw == 128 && p.th == 1 && (reinterpret_cast<uintptr_t>(padded) & 15) == 0) ? 1 : 0;
+  L->stem_halo = (p.tw == 128 && p.th == 1 && (reinterpret_cast<uintptr_t>(padded) & 15) == 0) ? 1 : 0;
   set_grid(L);
   return 0;
 }
@@ -1667,7 +1249,6 @@ int conv_tc_prepare(const ConvGeom& g, const void* x, const void* w, const float
   ConvTcLaunch* L = reinterpret_cast<ConvTcLaunch*>(out->storage);
   int rc = build_launch(g, x, w, bias, residual, y, L);
   L->p.valid_h = valid_h;
-  L->p.ragged_compact = ragged_compact_default();
   return rc;
 }
 
@@ -1691,7 +1272,6 @@ int conv_tc_prepare_dual(const ConvGeom& g, const void* x, const ConvGeom& g2, c
   if (rc) return rc;
   ConvTcParams& p = L->p;
   p.valid_h = valid_h;
-  p.ragged_compact = ragged_compact_default();
   const uint64_t eb = 2;
   const char* xb = reinterpret_cast<const char*>(x2);
   p.map2 = 1;        // the main source is a stride-1 convolution: it only uses tmA[0]
@@ -1703,7 +1283,7 @@ int conv_tc_prepare_dual(const ConvGeom& g, const void* x, const ConvGeom& g2, c
     rc = encode_act_map(&p.tmA[1], xb, g2.Cin, (uint64_t)(g2.W + 1) / 2, (uint64_t)(g2.H + 1) / 2, g2.N, 2ull * g2.Cin * eb,
                         2ull * g2.W * g2.Cin * eb, (uint64_t)g2.H * g2.W * g2.Cin * eb, p.tw, p.th);
   if (rc) return rc;
-  L->pair = want_pair(8, L->block_n, p.n_taps * p.cblocks + p.cblocks2);
+  L->pair = want_pair(false, L->block_n, p.n_taps * p.cblocks + p.cblocks2);
   rc = encode_weight_map(&p.tmB, w_cat, (uint64_t)p.n_taps * g.Cin + g2.Cin, g.Cout, L->pair ? L->block_n / 2 : L->block_n);
   if (rc) return rc;
   L->out_bufs = (p.n_taps * p.cblocks + p.cblocks2 <= 8) ? 4 : 2;
@@ -1712,24 +1292,24 @@ int conv_tc_prepare_dual(const ConvGeom& g, const void* x, const ConvGeom& g2, c
 }
 
 int conv_tc_run(const ConvTcPrepared* prep, cudaStream_t stream) {
-  const ConvTcLaunch* L = reinterpret_cast<const ConvTcLaunch*>(prep->storage);
-  if (L->kblk == 32 && L->stem_halo) return launch_stem(*L, stream);
-  if (L->halo3) return launch_halo3(*L, stream);
-  if (L->kblk == 32) return launch_bn<64, 32>(*L, stream);
-  if (L->pair) return L->block_n == 256 ? launch_pair<256>(*L, stream) : launch_pair<128>(*L, stream);
-  switch (L->block_n) {
-    case 256: return launch_bn<256, 64>(*L, stream);
-    case 128: return launch_bn<128, 64>(*L, stream);
-    default: return launch_bn<64, 64>(*L, stream);
+  const ConvTcLaunch& L = *reinterpret_cast<const ConvTcLaunch*>(prep->storage);
+  if (L.stem_halo) return launch_variant<StemHaloKernels>(L, stream);
+  if (L.halo3) return launch_variant<Halo3Kernels>(L, stream);
+  if (L.kblk == 32) return launch_variant<StemKernels>(L, stream);
+  if (L.pair) return L.block_n == 256 ? launch_variant<PairKernels>(L, stream) : no_kernel("CTA-pair", L);
+  switch (L.block_n) {
+    case 256: return launch_variant<CtaKernels<256>>(L, stream);
+    case 128: return launch_variant<CtaKernels<128>>(L, stream);
+    case 64: return launch_variant<CtaKernels<64>>(L, stream);
+    default: return no_kernel("conv_tc_kernel", L);
   }
 }
 
 void conv_tc_describe(const ConvTcPrepared* prep, ConvTcVariant* v) {
   const ConvTcLaunch* L = reinterpret_cast<const ConvTcLaunch*>(prep->storage);
-  v->pair = L->pair, v->halo3 = L->halo3, v->stem_halo = L->kblk == 32 ? L->stem_halo : 0, v->dual = L->p.cblocks2 > 0;
+  v->pair = L->pair, v->halo3 = L->halo3, v->stem_halo = L->stem_halo, v->dual = L->p.cblocks2 > 0;
   v->block_n = L->block_n, v->kblk = L->kblk, v->out_bufs = L->out_bufs;
-  // the same rule as ragged_map_setup
-  v->ragged_map = L->p.valid_h == nullptr ? -1 : (L->p.ragged_compact != 0 && L->p.N <= kMaxRaggedImages ? 1 : 0);
+  v->ragged_map = L->p.valid_h == nullptr ? -1 : (ragged_mapped(L->p) ? 1 : 0);
 }
 
 int conv_tc(const ConvGeom& g, const void* x, const void* w, const float* bias, const void* residual, void* y,

@@ -33,5 +33,4 @@ for _ in range(iters):
 t1.record()
 torch.cuda.synchronize()
 ms = t0.elapsed_time(t1) / iters
-print('forward x%d done, logits %s: %.3f ms per pass, %.3f ms per image (NBC_PDL=%s NBC_CTA2=%s)'
-      % (iters, tuple(out.shape), ms, ms / N, os.environ.get('NBC_PDL'), os.environ.get('NBC_CTA2')))
+print('forward x%d done, logits %s: %.3f ms per pass, %.3f ms per image' % (iters, tuple(out.shape), ms, ms / N))
