@@ -80,6 +80,24 @@ int nbc_preprocess_general_u8(const uint8_t* raw, int H, int W, int64_t pitch, i
 /* trim only, for images that need no resize (max dim <= 1024, models.py:194,200) */
 int nbc_trim_u8(const uint8_t* img, int H, int W, uint8_t* out, int32_t* first_last, void* workspace,
                 size_t workspace_bytes, void* stream);
+/* A CHUNK of n raw images of any sizes, each routed as the Python mirror (Preprocessor.preprocess_array) routes it:
+ * exactly (4 target)^2 -> the 4x kernels (the span applies); larger side above target -> the general-ratio kernel, then
+ * trim; otherwise square -> trim only; otherwise copied unchanged (first = 0, last = H).  descs is a HOST array: `raw` is
+ * the device address of memory row span_row0, and the buffer holds span_rows rows (a span other than (0, H) only for a
+ * 4x scan; NULL with span_rows = 0 for an all-zero one).  Result i (processed width `target`, or W for an image that is
+ * not resized) goes to out + i * out_stride_bytes, its {first,last} to first_last + 2 i; every result equals the
+ * per-image entry's byte for byte.  Each kernel family runs once per chunk. */
+typedef struct nbc_mixed_desc {
+  const uint8_t* raw;
+  int32_t H, W;
+  int64_t pitch;
+  int32_t flags;       /* bit0 = BGR, bit1 = bottom-up */
+  int32_t span_row0, span_rows;
+  int32_t reserved;
+} nbc_mixed_desc;
+size_t nbc_preprocess_mixed_workspace_bytes(const nbc_mixed_desc* descs, int n, int target);
+int nbc_preprocess_mixed_batch_u8(const nbc_mixed_desc* descs, int n, int target, uint8_t* out, int64_t out_stride_bytes,
+                                  int32_t* first_last, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- weights: BatchNorm folding + packing  (models.py:113-139; eval-mode BN of torchvision resnet50) --------
  * w: f32 OIHW [Cout,Cin,kh,kw].  gamma/beta/mean/var may be NULL (no BN: scale 1, shift = conv_bias or 0).

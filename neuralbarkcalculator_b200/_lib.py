@@ -22,6 +22,12 @@ class PlanStep(C.Structure):
                 + [(n, C.c_int64) for n in ('x', 'x2', 'residual', 'y', 'levels')])
 
 
+class MixedDesc(C.Structure):
+    """nbc_mixed_desc: one raw image of a mixed K1 chunk (see include/nbc.h)."""
+    _fields_ = [('raw', C.c_void_p), ('H', C.c_int32), ('W', C.c_int32), ('pitch', C.c_int64), ('flags', C.c_int32),
+                ('span_row0', C.c_int32), ('span_rows', C.c_int32), ('reserved', C.c_int32)]
+
+
 # name -> (restype, argtypes); kept in one table so tests can check it against include/nbc.h
 SIGNATURES = {
     'nbc_version': (c_int, []),
@@ -39,6 +45,9 @@ SIGNATURES = {
     'nbc_preprocess_general_u8': (c_int, [c_void_p, c_int, c_int, c_i64, c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t,
                                   c_void_p]),
     'nbc_trim_u8': (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    'nbc_preprocess_mixed_workspace_bytes': (c_size_t, [C.POINTER(MixedDesc), c_int, c_int]),
+    'nbc_preprocess_mixed_batch_u8': (c_int, [C.POINTER(MixedDesc), c_int, c_int, c_void_p, c_i64, c_void_p, c_void_p, c_size_t,
+                                      c_void_p]),
     'nbc_fold_bn_pack': (c_int, [c_void_p] * 6 + [c_float, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     'nbc_conv_bf16': (c_int, [C.POINTER(ConvDesc), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     'nbc_conv_dual_bf16': (c_int, [C.POINTER(ConvDesc), c_void_p, C.POINTER(ConvDesc), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -12,6 +12,7 @@
 // Pass 2 clamps to the input range and compacts the rows.
 // The BMP pixel array (bottom-up, BGR) is consumed directly: flags bit0 = BGR, bit1 = bottom-up.
 #include <algorithm>
+#include <vector>
 
 #include "common.cuh"
 
@@ -76,17 +77,13 @@ __device__ __forceinline__ void pass1_load(const uint8_t* __restrict__ raw, int 
 // span_lo / span_hi: the memory rows [span_lo, span_hi) are the ones `raw` really holds (multiples of 4); every other row
 // is all zero BY DEFINITION (the host found the scan's dark bands, nbc_host_zero_row_span, and copied only the rows in
 // between) -- such a group of four rows is never dereferenced and contributes min = max = 0, S = 0.
+// The body of one pass-1 block for one scan; resize4x_pass1 (uniform chunk) and mixed_resize4x_pass1 (mixed chunk) only
+// differ in where they find the scan's pointers, span, pitch and flags.
 template <bool kAligned>
-__global__ void __launch_bounds__(256) resize4x_pass1(const __grid_constant__ PreBatch batch, int H, int W, int64_t pitch,
-                                                      int flags, uint8_t* __restrict__ hdrs, size_t hdr_stride,
-                                                      uint8_t* __restrict__ r8s, size_t r8_stride) {
+__device__ __forceinline__ void resize4x_pass1_block(const uint8_t* __restrict__ raw, int span_lo, int span_hi, int H, int W,
+                                                     int64_t pitch, int flags, PreHeader* hdr, int* __restrict__ rowcount,
+                                                     uint8_t* __restrict__ r8) {
   __shared__ __align__(16) uint32_t s_out[8][96];   // per warp: 32 threads x 12 bytes
-  const int z = blockIdx.z;
-  const uint8_t* __restrict__ raw = batch.raw[z];
-  const int span_lo = batch.lo[z], span_hi = batch.hi[z];
-  PreHeader* hdr = reinterpret_cast<PreHeader*>(hdrs + z * hdr_stride);
-  int* __restrict__ rowcount = reinterpret_cast<int*>(hdrs + z * hdr_stride + sizeof(PreHeader));
-  uint8_t* __restrict__ r8 = r8s + z * r8_stride;
   const int Wo = W >> 2;
   const int groups = (Wo + 3) >> 2;  // 4 output pixels per thread
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
@@ -185,6 +182,16 @@ __global__ void __launch_bounds__(256) resize4x_pass1(const __grid_constant__ Pr
   }
 }
 
+template <bool kAligned>
+__global__ void __launch_bounds__(256) resize4x_pass1(const __grid_constant__ PreBatch batch, int H, int W, int64_t pitch,
+                                                      int flags, uint8_t* __restrict__ hdrs, size_t hdr_stride,
+                                                      uint8_t* __restrict__ r8s, size_t r8_stride) {
+  const int z = blockIdx.z;
+  resize4x_pass1_block<kAligned>(batch.raw[z], batch.lo[z], batch.hi[z], H, W, pitch, flags,
+                                 reinterpret_cast<PreHeader*>(hdrs + z * hdr_stride),
+                                 reinterpret_cast<int*>(hdrs + z * hdr_stride + sizeof(PreHeader)), r8s + z * r8_stride);
+}
+
 // rows of a u8 image that needs no resize: nondark <=> any channel non-zero (sum/255 > 1e-3)
 __global__ void __launch_bounds__(256) rowcount_u8(const uint8_t* __restrict__ img, int H, int W,
                                                     int* __restrict__ rowcount) {
@@ -203,12 +210,9 @@ __global__ void __launch_bounds__(256) rowcount_u8(const uint8_t* __restrict__ i
 // last = H - argmax(keep[::-1]); nothing kept -> (0, H).  all_nondark: min(in) >= 1 makes every pixel non-dark.
 // One block per scan: block z reads the row counts / header `ws_stride` bytes after those of block z - 1 (0 for a single
 // scan) and writes first_last + 2 z.
-__global__ void __launch_bounds__(1024) trim_rows_kernel(const int* __restrict__ rowcount, const PreHeader* hdr,
-                                                         int Ho, int Wo, int square, int32_t* first_last, size_t ws_stride = 0) {
+__device__ __forceinline__ void trim_rows_block(const int* __restrict__ rowcount, const PreHeader* hdr, int Ho, int Wo, int square,
+                                                int32_t* first_last) {
   __shared__ int s_first, s_last_from_end;
-  rowcount = reinterpret_cast<const int*>(reinterpret_cast<const char*>(rowcount) + blockIdx.x * ws_stride);
-  if (hdr) hdr = reinterpret_cast<const PreHeader*>(reinterpret_cast<const char*>(hdr) + blockIdx.x * ws_stride);
-  first_last += 2 * blockIdx.x;
   if (threadIdx.x == 0) s_first = INT_MAX, s_last_from_end = INT_MAX;
   __syncthreads();
   const bool all_nondark = hdr && (255 - hdr->inv_min) >= 1;
@@ -230,6 +234,13 @@ __global__ void __launch_bounds__(1024) trim_rows_kernel(const int* __restrict__
     first_last[0] = first;
     first_last[1] = last;
   }
+}
+
+__global__ void __launch_bounds__(1024) trim_rows_kernel(const int* __restrict__ rowcount, const PreHeader* hdr,
+                                                         int Ho, int Wo, int square, int32_t* first_last, size_t ws_stride = 0) {
+  rowcount = reinterpret_cast<const int*>(reinterpret_cast<const char*>(rowcount) + blockIdx.x * ws_stride);
+  if (hdr) hdr = reinterpret_cast<const PreHeader*>(reinterpret_cast<const char*>(hdr) + blockIdx.x * ws_stride);
+  trim_rows_block(rowcount, hdr, Ho, Wo, square, first_last + 2 * blockIdx.x);
 }
 
 __global__ void __launch_bounds__(256) resize4x_pass2(const uint8_t* __restrict__ hdrs, size_t hdr_stride,
@@ -281,7 +292,7 @@ static size_t pre_header_bytes(int Ho) { return align_up(sizeof(PreHeader) + (si
 // oracle's order (no FMA contraction), so that the bytes match the restatement.  Not a bandwidth kernel: one thread per
 // output pixel gathers 4 x 4 x 3 input bytes; the 4x path above stays the one for the scanner's 4096^2 images.
 // ------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) minmax_u8(const uint8_t* __restrict__ raw, int H, int W, int64_t pitch, PreHeader* hdr) {
+__device__ __forceinline__ void minmax_block(const uint8_t* __restrict__ raw, int H, int W, int64_t pitch, PreHeader* hdr) {
   int mn = 255, mx = 0;
   const int64_t rowb = (int64_t)W * 3;
   for (int r = blockIdx.x; r < H; r += gridDim.x) {
@@ -300,6 +311,10 @@ __global__ void __launch_bounds__(256) minmax_u8(const uint8_t* __restrict__ raw
     atomicMax(&hdr->inv_min, 255 - mn);
     atomicMax(&hdr->max, mx);
   }
+}
+
+__global__ void __launch_bounds__(256) minmax_u8(const uint8_t* __restrict__ raw, int H, int W, int64_t pitch, PreHeader* hdr) {
+  minmax_block(raw, H, W, pitch, hdr);
 }
 
 struct CubicTaps {
@@ -331,9 +346,9 @@ __device__ __forceinline__ double cubic_f64(double f0, double f1, double f2, dou
   return __dadd_rn(f1, __dmul_rn(__dmul_rn(0.5, x), c));
 }
 
-__global__ void __launch_bounds__(256) resize_general_kernel(const uint8_t* __restrict__ raw, int H, int W, int64_t pitch,
-                                                             int flags, int Ho, int Wo, const PreHeader* __restrict__ hdr,
-                                                             uint8_t* __restrict__ r8, int* __restrict__ rowcount) {
+__device__ __forceinline__ void resize_general_block(const uint8_t* __restrict__ raw, int H, int W, int64_t pitch, int flags,
+                                                     int Ho, int Wo, const PreHeader* __restrict__ hdr, uint8_t* __restrict__ r8,
+                                                     int* __restrict__ rowcount) {
   const int ho = blockIdx.y;
   const int wo = blockIdx.x * blockDim.x + threadIdx.x;
   int nondark = 0;
@@ -363,6 +378,122 @@ __global__ void __launch_bounds__(256) resize_general_kernel(const uint8_t* __re
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) nondark += __shfl_xor_sync(0xffffffffu, nondark, o);
   if ((threadIdx.x & 31) == 0 && nondark) atomicAdd(&rowcount[ho], nondark);
+}
+
+__global__ void __launch_bounds__(256) resize_general_kernel(const uint8_t* __restrict__ raw, int H, int W, int64_t pitch,
+                                                             int flags, int Ho, int Wo, const PreHeader* __restrict__ hdr,
+                                                             uint8_t* __restrict__ r8, int* __restrict__ rowcount) {
+  resize_general_block(raw, H, W, pitch, flags, Ho, Wo, hdr, r8, rowcount);
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Mixed chunk: raw images of any size in one call (nbc_preprocess_mixed_batch_u8), each routed as Preprocessor.preprocess_array
+// routes it.  The per-image geometry lives in a device table at the start of the workspace; every kernel family runs once
+// for the chunk with blockIdx.z = the z-th image of its kind (the table's per-kind index lists), and each image has its own
+// header (global min / max, row counts), intermediate and {first,last}.  The blocks run the same device code as the
+// per-image entries, so every image's bytes equal theirs.
+// ------------------------------------------------------------------------------------------------------------
+enum MixedKind { kMixed4x = 0, kMixedGeneral = 1, kMixedTrim = 2, kMixedCopy = 3 };
+
+struct MixedImage {
+  const uint8_t* raw;   // memory row r of the pixel array is at raw + r * pitch (rows outside [lo, hi) are never read)
+  int64_t pitch;
+  int H, W, flags, kind;
+  int lo, hi;           // memory rows the buffer really holds (the zero-band span of a 4x scan; [0, H) otherwise)
+  int Ho, Wo;           // processed size before the trim
+};
+
+struct MixedTable {
+  const MixedImage* img;
+  const int* list[4];   // per kind: the images of that kind, in chunk order
+  uint8_t* hdrs;        // per image: PreHeader + row counts
+  size_t hdr_stride;
+  uint8_t* r8s;         // per image: the untrimmed processed image, Ho x Wo x 3
+  size_t r8_stride;
+};
+
+template <bool kAligned>
+__global__ void __launch_bounds__(256) mixed_resize4x_pass1(const __grid_constant__ MixedTable t, int H, int W) {
+  const int i = t.list[kMixed4x][blockIdx.z];
+  const MixedImage& m = t.img[i];
+  uint8_t* hdr = t.hdrs + i * t.hdr_stride;
+  resize4x_pass1_block<kAligned>(m.raw, m.lo, m.hi, H, W, m.pitch, m.flags, reinterpret_cast<PreHeader*>(hdr),
+                                 reinterpret_cast<int*>(hdr + sizeof(PreHeader)), t.r8s + i * t.r8_stride);
+}
+
+__global__ void __launch_bounds__(256) mixed_minmax(const __grid_constant__ MixedTable t) {
+  const int i = t.list[kMixedGeneral][blockIdx.z];
+  const MixedImage& m = t.img[i];
+  minmax_block(m.raw, m.H, m.W, m.pitch, reinterpret_cast<PreHeader*>(t.hdrs + i * t.hdr_stride));
+}
+
+__global__ void __launch_bounds__(256) mixed_resize_general(const __grid_constant__ MixedTable t) {
+  const int i = t.list[kMixedGeneral][blockIdx.z];
+  const MixedImage& m = t.img[i];
+  uint8_t* hdr = t.hdrs + i * t.hdr_stride;
+  resize_general_block(m.raw, m.H, m.W, m.pitch, m.flags, m.Ho, m.Wo, reinterpret_cast<const PreHeader*>(hdr),
+                       t.r8s + i * t.r8_stride, reinterpret_cast<int*>(hdr + sizeof(PreHeader)));
+}
+
+// images that need no resize: one block per row turns the raw row (pitch, BGR, bottom-up) into RGB top-down in the
+// intermediate and, for those that are trimmed, counts its non-dark pixels as rowcount_u8 does (any channel non-zero)
+__global__ void __launch_bounds__(256) mixed_small_rows(const __grid_constant__ MixedTable t, int kind) {
+  const int i = t.list[kind][blockIdx.z];
+  const MixedImage& m = t.img[i];
+  const int h = blockIdx.x;
+  if (h >= m.H) return;
+  const uint8_t* src = m.raw + ((m.flags & 2) ? (int64_t)(m.H - 1 - h) : (int64_t)h) * m.pitch;
+  uint8_t* dst = t.r8s + i * t.r8_stride + (int64_t)h * m.W * 3;
+  const bool bgr = m.flags & 1;
+  int cnt = 0;
+  for (int w = threadIdx.x; w < m.W; w += blockDim.x) {
+    const uint8_t c0 = src[w * 3], c1 = src[w * 3 + 1], c2 = src[w * 3 + 2];
+    dst[w * 3] = bgr ? c2 : c0, dst[w * 3 + 1] = c1, dst[w * 3 + 2] = bgr ? c0 : c2;
+    cnt += ((int)c0 + c1 + c2) >= 1 ? 1 : 0;
+  }
+  if (kind != kMixedTrim) return;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+  if ((threadIdx.x & 31) == 0 && cnt) atomicAdd(reinterpret_cast<int*>(t.hdrs + i * t.hdr_stride + sizeof(PreHeader)) + h, cnt);
+}
+
+// {first,last} of every image (block z = image z): trim_black on the square results, [0, H) for the untouched ones.
+// Resized images pass their header, as the per-image entries do (min(in) >= 1 makes every pixel non-dark).
+__global__ void __launch_bounds__(1024) mixed_trim_rows(const __grid_constant__ MixedTable t, int32_t* first_last) {
+  const int i = blockIdx.x;
+  const MixedImage& m = t.img[i];
+  const uint8_t* hdr = t.hdrs + i * t.hdr_stride;
+  const bool resized = m.kind == kMixed4x || m.kind == kMixedGeneral;
+  trim_rows_block(reinterpret_cast<const int*>(hdr + sizeof(PreHeader)), resized ? reinterpret_cast<const PreHeader*>(hdr) : nullptr,
+                  m.Ho, m.Wo, m.kind != kMixedCopy ? 1 : 0, first_last + 2 * i);
+}
+
+// rows [first, last) of every image to out + z * out_stride; the 4x intermediate is saturated to [0, 255] and is clamped to
+// the input range here (resize4x_pass2), the others are final already (copy_rows_u8)
+__global__ void __launch_bounds__(256) mixed_store(const __grid_constant__ MixedTable t, const int32_t* __restrict__ first_last,
+                                                   uint8_t* __restrict__ out_all, int64_t out_stride) {
+  const int i = blockIdx.y;
+  const MixedImage& m = t.img[i];
+  const PreHeader* hdr = reinterpret_cast<const PreHeader*>(t.hdrs + i * t.hdr_stride);
+  const bool clamp = m.kind == kMixed4x;
+  const uint32_t lo = clamp ? (uint32_t)(255 - hdr->inv_min) : 0u, hi = clamp ? (uint32_t)hdr->max : 255u;
+  const uint32_t lo4 = lo * 0x01010101u, hi4 = hi * 0x01010101u;
+  const int first = first_last[2 * i], last = first_last[2 * i + 1];
+  const int64_t total = (int64_t)(last - first) * m.Wo * 3;
+  const uint8_t* src = t.r8s + i * t.r8_stride + (int64_t)first * m.Wo * 3;
+  uint8_t* __restrict__ out = out_all + i * out_stride;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x * 16;
+  const bool vec = ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
+  for (int64_t j = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 16; j < total; j += stride) {
+    if (vec && j + 16 <= total) {
+      uint4 v = __ldg(reinterpret_cast<const uint4*>(src + j));
+      v.x = __vminu4(__vmaxu4(v.x, lo4), hi4), v.y = __vminu4(__vmaxu4(v.y, lo4), hi4);
+      v.z = __vminu4(__vmaxu4(v.z, lo4), hi4), v.w = __vminu4(__vmaxu4(v.w, lo4), hi4);
+      *reinterpret_cast<uint4*>(out + j) = v;
+    } else {
+      for (int64_t k = j; k < min(j + 16, total); ++k) out[k] = (uint8_t)min(max((uint32_t)src[k], lo), hi);
+    }
+  }
 }
 
 }  // namespace nbc
@@ -505,6 +636,106 @@ extern "C" int nbc_preprocess_general_u8(const uint8_t* raw, int H, int W, int64
   trim_rows_kernel<<<1, 1024, 0, stream>>>(rowcount, hdr, Ho, Wo, 1, first_last);
   NBC_CHECK_LAUNCH();
   copy_rows_u8<<<4 * 148, 256, 0, stream>>>(r8, Wo, first_last, out);
+  NBC_CHECK_LAUNCH();
+  return 0;
+}
+
+// ---- mixed chunk ---------------------------------------------------------------------------------------------
+static size_t mixed_table_bytes(int n) { return align_up((size_t)n * sizeof(MixedImage) + 4 * (size_t)n * sizeof(int), 256); }
+static size_t mixed_hdr_stride(int target) { return pre_header_bytes(target); }
+static size_t mixed_r8_stride(int target) { return align_up((size_t)target * target * 3, 256); }
+
+extern "C" size_t nbc_preprocess_mixed_workspace_bytes(const nbc_mixed_desc* descs, int n, int target) {
+  (void)descs;
+  if (n <= 0 || target <= 0) return 0;
+  return mixed_table_bytes(n) + (size_t)n * (mixed_hdr_stride(target) + mixed_r8_stride(target));
+}
+
+extern "C" int nbc_preprocess_mixed_batch_u8(const nbc_mixed_desc* descs, int n, int target, uint8_t* out, int64_t out_stride_bytes,
+                                             int32_t* first_last, void* workspace, size_t workspace_bytes, void* stream_) {
+  const char* who = "nbc_preprocess_mixed_batch_u8";
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  NBC_REQUIRE(descs && out && first_last && workspace, "%s: null pointer", who);
+  NBC_REQUIRE(n > 0 && n <= 4096 && target > 0 && target < (1 << 14), "%s: bad image count %d or target %d", who, n, target);
+  const size_t need = nbc_preprocess_mixed_workspace_bytes(descs, n, target);
+  if (workspace_bytes < need) {
+    set_error("%s: workspace %zu < %zu", who, workspace_bytes, need);
+    return NBC_ERR_WORKSPACE;
+  }
+  // the table: images, then the four per-kind index lists; routed as Preprocessor.preprocess_array (models.py:194-201)
+  std::vector<uint8_t> host(mixed_table_bytes(n), 0);
+  MixedImage* img = reinterpret_cast<MixedImage*>(host.data());
+  int* lists = reinterpret_cast<int*>(host.data() + (size_t)n * sizeof(MixedImage));
+  int count[4] = {0, 0, 0, 0}, small_rows = 0, general_rows = 0;
+  bool aligned = true;
+  std::vector<int> order[4];
+  for (int i = 0; i < n; ++i) {
+    const nbc_mixed_desc& d = descs[i];
+    NBC_REQUIRE(d.H > 0 && d.W > 0 && d.H < (1 << 20) && d.W < (1 << 20) && d.pitch >= (int64_t)d.W * 3 && d.flags >= 0 && d.flags <= 3,
+                "%s: image %d: bad geometry %dx%d, pitch %lld, flags %d", who, i, d.H, d.W, (long long)d.pitch, d.flags);
+    MixedImage& m = img[i];
+    const bool resize = (d.H > d.W ? d.H : d.W) > target;
+    m.kind = !resize ? (d.H == d.W ? kMixedTrim : kMixedCopy) : (d.H == 4 * target && d.W == 4 * target ? kMixed4x : kMixedGeneral);
+    if (m.kind == kMixed4x) {
+      NBC_REQUIRE((d.raw || d.span_rows == 0) && d.span_row0 >= 0 && d.span_rows >= 0 && d.span_row0 % 4 == 0 && d.span_rows % 4 == 0 &&
+                      d.span_row0 + d.span_rows <= d.H,
+                  "%s: image %d: the span [%d, +%d) must be made of whole groups of 4 rows inside the image", who, i, d.span_row0,
+                  d.span_rows);
+    } else {
+      NBC_REQUIRE(d.raw && d.span_row0 == 0 && d.span_rows == d.H,
+                  "%s: image %d (%dx%d): only a 4 * target square scan may hold a part of its rows", who, i, d.H, d.W);
+    }
+    // the kernels address memory row r at raw + r * pitch and never touch a row outside the span
+    m.raw = d.raw ? d.raw - (int64_t)d.span_row0 * d.pitch : reinterpret_cast<const uint8_t*>(workspace);
+    m.pitch = d.pitch, m.H = d.H, m.W = d.W, m.flags = d.flags;
+    m.lo = d.span_row0, m.hi = d.span_row0 + d.span_rows;
+    m.Ho = resize ? target : d.H, m.Wo = resize ? target : d.W;
+    NBC_REQUIRE(out_stride_bytes >= (int64_t)m.Ho * m.Wo * 3, "%s: out stride %lld smaller than the %dx%d result of image %d", who,
+                (long long)out_stride_bytes, m.Ho, m.Wo, i);
+    if (m.kind == kMixed4x) aligned = aligned && d.pitch % 16 == 0 && reinterpret_cast<uintptr_t>(m.raw) % 16 == 0;
+    if (m.kind == kMixedTrim || m.kind == kMixedCopy) small_rows = d.H > small_rows ? d.H : small_rows;
+    if (m.kind == kMixedGeneral) general_rows = d.H > general_rows ? d.H : general_rows;
+    order[m.kind].push_back(i);
+  }
+  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
+  MixedTable t;
+  t.img = reinterpret_cast<const MixedImage*>(ws);
+  for (int k = 0, off = 0; k < 4; ++k) {
+    count[k] = (int)order[k].size();
+    std::copy(order[k].begin(), order[k].end(), lists + off);
+    t.list[k] = reinterpret_cast<const int*>(ws + (size_t)n * sizeof(MixedImage)) + off;
+    off += count[k];
+  }
+  t.hdr_stride = mixed_hdr_stride(target), t.r8_stride = mixed_r8_stride(target);
+  t.hdrs = ws + mixed_table_bytes(n);
+  t.r8s = t.hdrs + (size_t)n * t.hdr_stride;
+  // pageable source: the copy is staged before cudaMemcpyAsync returns, so `host` may go out of scope
+  NBC_CUDA(cudaMemcpyAsync(ws, host.data(), host.size(), cudaMemcpyHostToDevice, stream));
+  NBC_CUDA(cudaMemsetAsync(t.hdrs, 0, (size_t)n * t.hdr_stride, stream));
+  if (count[kMixed4x]) {
+    const dim3 grid(ceil_div((target + 3) / 4, 256), target, count[kMixed4x]);
+    if (aligned)
+      mixed_resize4x_pass1<true><<<grid, 256, 0, stream>>>(t, 4 * target, 4 * target);
+    else
+      mixed_resize4x_pass1<false><<<grid, 256, 0, stream>>>(t, 4 * target, 4 * target);
+    NBC_CHECK_LAUNCH();
+  }
+  if (count[kMixedGeneral]) {
+    mixed_minmax<<<dim3(general_rows < 4 * 148 ? general_rows : 4 * 148, 1, count[kMixedGeneral]), 256, 0, stream>>>(t);
+    NBC_CHECK_LAUNCH();
+    mixed_resize_general<<<dim3(ceil_div(target, 256), target, count[kMixedGeneral]), 256, 0, stream>>>(t);
+    NBC_CHECK_LAUNCH();
+  }
+  for (int kind : {kMixedTrim, kMixedCopy}) {
+    if (!count[kind]) continue;
+    mixed_small_rows<<<dim3(small_rows, 1, count[kind]), 256, 0, stream>>>(t, kind);
+    NBC_CHECK_LAUNCH();
+  }
+  mixed_trim_rows<<<n, 1024, 0, stream>>>(t, first_last);
+  NBC_CHECK_LAUNCH();
+  const int64_t total16 = ceil_div64((int64_t)target * target * 3, 16);
+  const int blocks = (int)(ceil_div64(total16, 256) < 4 * 148 ? ceil_div64(total16, 256) : 4 * 148);
+  mixed_store<<<dim3(blocks, n), 256, 0, stream>>>(t, first_last, out, out_stride_bytes);
   NBC_CHECK_LAUNCH();
   return 0;
 }

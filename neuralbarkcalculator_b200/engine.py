@@ -14,7 +14,11 @@ Dark bands stay on the host: the rows of a scan above and below the bark that ar
 resize to exact zeros, so ``submit_host`` finds them with a host scan (``nbc_host_zero_row_span``, a few worker threads,
 GIL released), copies only the rows in between -- still one ``cudaMemcpyAsync`` per scan -- and K1 treats the rest as
 zeros (``nbc_preprocess_4x_span_u8``).  Bit-identical to copying the whole scan (global min / max clip included);
-``NBC_ZERO_SPAN=0`` switches it off."""
+``NBC_ZERO_SPAN=0`` switches it off.
+
+``submit_mixed`` / ``collect_mixed`` take raw images of any sizes and layouts (the folder pipeline's mixed route): K1 routes
+each image as ``Preprocessor.preprocess_array`` does (``nbc_preprocess_mixed_batch_u8``), and a batch runs as chunks of one
+canvas width."""
 import ctypes as C
 import os
 from concurrent.futures import ThreadPoolExecutor
@@ -81,6 +85,8 @@ class PredictEngine:
         self._chunks = 0          # chunks issued so far (logits double buffer)
         self._issued = 0          # host scans staged so far (staging ring)
         self._copy_stream = None
+        self._stage = None
+        self._mixed_stage, self._mixed_bytes, self._mixed_issued = None, 0, 0
 
     # -- buffers ------------------------------------------------------------------------------------------------
     def _slot(self, n):
@@ -107,17 +113,23 @@ class PredictEngine:
         self._pre_stream = torch.cuda.Stream(dev)       # K1 (resize + trim)
         self._out_stream = torch.cuda.Stream(dev)       # D2H of masks and counts
         self._post_stream = torch.cuda.Stream(dev)      # K3 + K5 of a chunk, behind the network pass of the next one
-        self._stage = [torch.empty(S * S * 3, dtype=torch.uint8, device=dev) for _ in range(self.depth)]
-        self._staged = [torch.cuda.Event() for _ in range(self.depth)]
-        self._freed = [torch.cuda.Event() for _ in range(self.depth)]
         lib = ops._lib.load()
-        self._pre_ws = torch.empty(self.chunk * lib.nbc_preprocess_workspace_bytes(S, S), dtype=torch.uint8, device=dev)
         self._ccl_ws = torch.empty(lib.nbc_ccl_workspace_bytes(self.chunk, Hc, Wo), dtype=torch.uint8, device=dev)
         hl = (((Hc - 1) // 2 + 1 - 1) // 2 + 1 - 1) // 2 + 1
         wl = (((Wo - 1) // 2 + 1 - 1) // 2 + 1 - 1) // 2 + 1
         self._logits = [torch.empty((self.chunk, 3, hl, wl), dtype=torch.float32, device=dev) for _ in range(2)]
         self._logits_free = [None, None]
         return True
+
+    def _standard_buffers(self):
+        """Staging ring (``depth`` raw scans of raw_size^2 x 3 bytes) and K1 workspace of the uniform host path."""
+        if self._stage is not None:
+            return
+        S, dev = self.raw_size, self.device
+        self._stage = [torch.empty(S * S * 3, dtype=torch.uint8, device=dev) for _ in range(self.depth)]
+        self._staged = [torch.cuda.Event() for _ in range(self.depth)]
+        self._freed = [torch.cuda.Event() for _ in range(self.depth)]
+        self._pre_ws = torch.empty(self.chunk * ops._lib.load().nbc_preprocess_workspace_bytes(S, S), dtype=torch.uint8, device=dev)
 
     def _preprocess_into(self, slot, i, raw, bgr, bottom_up, span=None):
         """K1 on the current stream.  span = (row0, rows): ``raw`` holds only those memory rows of the scan, the others are
@@ -166,27 +178,36 @@ class PredictEngine:
             self._scan_pool = ThreadPoolExecutor(int(os.environ.get('NBC_SCAN_THREADS', 4)), thread_name_prefix='nbc-scan')
         return [self._scan_pool.submit(self._scan, get_raw(i)).result for i in range(n)]
 
-    def _segment_chunk(self, slot, a, b, exclude_nodes):
+    def _segment_chunk(self, slot, a, b, exclude_nodes, proc=None, masks=None):
         """Images a..b-1 as ONE ragged batch: network, K3 and K5 read the per-image heights on the device.  The network
         runs on the main stream; K3 (upsample+argmax) and K5 (region removal + counts) follow on the post stream (two
-        logits buffers).  Returns the event that marks the chunk's masks and counts as final."""
+        logits buffers).  proc / masks: the chunk's canvases when they are narrower than the slot's (mixed path).
+        Returns the event that marks the chunk's masks and counts as final."""
+        proc = slot.proc[a:b] if proc is None else proc
+        masks = slot.masks[a:b] if masks is None else masks
         plan = self.model.native_plan()
         main = torch.cuda.current_stream(self.device)
         k = self._chunks & 1
         self._chunks += 1
         if self._logits_free[k] is not None:
             main.wait_event(self._logits_free[k])        # K3 of two chunks ago has consumed this logits buffer
-        logits = plan.forward_ragged(slot.proc[a:b], heights=slot.heights[a:b], out=self._logits[k][:b - a])
+        Hc, W = masks.shape[1], masks.shape[2]
+        lg = self._logits[k]
+        if W == self.out_w:
+            lg = lg[:b - a]
+        else:        # a narrower canvas: its logits, ceil(W / 8) wide, in the front of the same buffer
+            lg = lg.view(-1)[:(b - a) * 3 * lg.shape[2] * ((W + 7) // 8)].view(b - a, 3, lg.shape[2], (W + 7) // 8)
+        logits = plan.forward_ragged(proc, heights=slot.heights[a:b], out=lg)
         net_done = torch.cuda.Event()
         net_done.record(main)
         done = torch.cuda.Event()
         with torch.cuda.stream(self._post_stream):
             self._post_stream.wait_event(net_done)
-            ops.upsample_argmax_ragged(logits, slot.heights[a:b], (self.raw_size // 4, self.out_w), out=slot.masks[a:b])
+            ops.upsample_argmax_ragged(logits, slot.heights[a:b], (Hc, W), out=masks)
             free = torch.cuda.Event()
             free.record(self._post_stream)
             self._logits_free[k] = free
-            ops.remove_small_zones_ragged(slot.masks[a:b], slot.heights[a:b], self.threshold, exclude_nodes,
+            ops.remove_small_zones_ragged(masks, slot.heights[a:b], self.threshold, exclude_nodes,
                                           workspace=self._ccl_ws, counts=slot.counts[a:b])
             done.record(self._post_stream)
         return done
@@ -204,6 +225,7 @@ class PredictEngine:
         chunk, depth = self.chunk, self.depth
         with torch.cuda.device(dev):
             first = self._streams()
+            self._standard_buffers()
             slot = self._slot(n)
             main = torch.cuda.current_stream(dev)
             if first or on_device:
@@ -310,3 +332,151 @@ class PredictEngine:
     def run_host(self, raws_host, masks_host=None, bgr=True, bottom_up=True, exclude_nodes=False):
         """Synchronous end-to-end call: submit_host + collect."""
         return self.collect(self.submit_host(raws_host, masks_host, bgr, bottom_up, exclude_nodes))
+
+    # -- heterogeneous raw images from pinned host memory -------------------------------------------------------------
+    def reserve_mixed(self, nbytes):
+        """Size the staging ring of ``submit_mixed`` for raw images of up to ``nbytes`` bytes (``depth`` buffers).  The
+        folder pipeline reserves the largest raw image of its run once, before the first submit; a later, larger image
+        reallocates after a device synchronise."""
+        if nbytes <= self._mixed_bytes:
+            return
+        with torch.cuda.device(self.device):
+            if self._mixed_stage is not None:
+                torch.cuda.synchronize(self.device)
+            self._mixed_stage = None
+            self._mixed_stage = [torch.empty(nbytes, dtype=torch.uint8, device=self.device) for _ in range(self.depth)]
+            self._mixed_staged = [torch.cuda.Event() for _ in range(self.depth)]
+            self._mixed_freed = [torch.cuda.Event() for _ in range(self.depth)]
+            self._mixed_bytes, self._mixed_issued = nbytes, 0
+
+    def _mixed_chunks(self, widths):
+        """Slot order and chunks of a mixed batch: the images processed to the full canvas width first, then the narrower
+        ones grouped by width (a ragged pass needs one width).  -> (order: slot position -> caller index, [(a, b, width)])"""
+        T = self.out_w
+        order = sorted(range(len(widths)), key=lambda i: (widths[i] != T, widths[i]))
+        chunks, a = [], 0
+        while a < len(order):
+            w = widths[order[a]]
+            b = a + 1
+            while b < len(order) and b - a < self.chunk and widths[order[b]] == w:
+                b += 1
+            chunks.append((a, b, w))
+            a = b
+        return order, chunks
+
+    def submit_mixed(self, raws_host, geoms, masks_host=None, exclude_nodes=False, want_processed=False, only_preprocess=False,
+                     spans=None):
+        """``submit_host`` for raw images of any sizes and layouts.  geoms[i] = (H, W, pitch, bgr, bottom_up) of the pixel
+        array in the pinned u8 CPU tensor raws_host[i]; spans[i] = (row0, rows): only those memory rows are copied (a
+        (4 * out_w)^2 scan's rows between its all-zero bands, see the module docstring; (0, H) otherwise, the default).
+        K1 routes each image as ``Preprocessor.preprocess_array`` does (``nbc_preprocess_mixed_batch_u8``).  Images
+        processed to the full width share chunks; narrower ones (images that need no resize) form chunks of one width.
+        ``collect_mixed`` waits for the ticket; masks_host[i] (pinned, out_w^2 bytes) receives image i's mask in its
+        first rows[i] * widths[i] bytes."""
+        n = len(raws_host)
+        T = self.out_w
+        widths = [ops.processed_size(g[0], g[1], T)[1] for g in geoms]
+        spans = [(0, g[0]) for g in geoms] if spans is None else list(spans)
+        order, chunks = self._mixed_chunks(widths)
+        dev, depth = self.device, self.depth
+        Hc = self.raw_size // 4
+        lib = ops._lib.load()
+        self.reserve_mixed(max(rows * g[2] for g, (_, rows) in zip(geoms, spans)))
+        with torch.cuda.device(dev):
+            first = self._streams()
+            if getattr(self, '_mixed_ws', None) is None:
+                self._mixed_ws = torch.empty(lib.nbc_preprocess_mixed_workspace_bytes(None, self.chunk, T), dtype=torch.uint8,
+                                             device=dev)
+            slot = self._slot(n)
+            main = torch.cuda.current_stream(dev)
+            if first:
+                start = torch.cuda.Event()
+                start.record(main)
+                for st in (self._copy_stream, self._pre_stream, self._out_stream, self._post_stream):
+                    st.wait_event(start)
+            if slot.done is not None:
+                self._pre_stream.wait_event(slot.done)
+            if want_processed and slot.proc_host is None:
+                slot.proc_host = torch.empty(slot.proc.shape, dtype=torch.uint8).pin_memory()
+            proc_flat, masks_flat = slot.proc.view(-1), slot.masks.view(-1)
+            views = []        # per chunk: (proc canvas, mask canvas, flat byte offset of the proc canvas)
+            for (a, b, w) in chunks:
+                off = a * Hc * T * 3
+                proc = proc_flat[off:off + (b - a) * Hc * w * 3].view(b - a, Hc, w, 3)
+                masks = masks_flat[a * Hc * T:a * Hc * T + (b - a) * Hc * w].view(b - a, Hc, w)
+                views.append((proc, masks, off))
+                items, used = [], []
+                for p in range(a, b):
+                    i = order[p]
+                    H, W, pitch, bgr, bottom_up = geoms[i]
+                    row0, rows = spans[i]
+                    k = self._mixed_issued % depth
+                    with torch.cuda.stream(self._copy_stream):
+                        if self._mixed_issued >= depth:
+                            self._copy_stream.wait_event(self._mixed_freed[k])
+                        if rows:      # one cudaMemcpyAsync per image
+                            self._mixed_stage[k][:rows * pitch].copy_(raws_host[i][row0 * pitch:(row0 + rows) * pitch],
+                                                                      non_blocking=True)
+                    self.h2d_bytes += rows * pitch
+                    items.append((self._mixed_stage[k].data_ptr() if rows else None, H, W, pitch, bgr, bottom_up, (row0, rows)))
+                    used.append(k)
+                    self._mixed_issued += 1
+                self._mixed_staged[used[-1]].record(self._copy_stream)
+                self._pre_stream.wait_event(self._mixed_staged[used[-1]])
+                descs = ops.mixed_descs(items)
+                pre_done = torch.cuda.Event()
+                with torch.cuda.stream(self._pre_stream):
+                    ops._lib.check(lib.nbc_preprocess_mixed_batch_u8(descs, b - a, T, C.c_void_p(proc.data_ptr()), Hc * w * 3,
+                                                                     C.c_void_p(slot.fl[a].data_ptr()), C.c_void_p(self._mixed_ws.data_ptr()),
+                                                                     self._mixed_ws.numel(),
+                                                                     C.c_void_p(self._pre_stream.cuda_stream)),
+                                   'nbc_preprocess_mixed_batch_u8')
+                    for k in used:
+                        self._mixed_freed[k].record(self._pre_stream)
+                    ops.heights_from_first_last(slot.fl[a:b], out=slot.heights[a:b])
+                    pre_done.record(self._pre_stream)
+                if want_processed:
+                    with torch.cuda.stream(self._out_stream):
+                        self._out_stream.wait_event(pre_done)
+                        slot.proc_host.view(-1)[off:off + proc.numel()].copy_(proc.view(-1), non_blocking=True)
+                if only_preprocess:
+                    continue
+                main.wait_event(pre_done)
+                ev = self._segment_chunk(slot, a, b, exclude_nodes, proc=proc, masks=masks)
+                if masks_host is not None:
+                    with torch.cuda.stream(self._out_stream):
+                        self._out_stream.wait_event(ev)
+                        for p in range(a, b):
+                            masks_host[order[p]][:Hc * w].copy_(masks[p - a].view(-1), non_blocking=True)
+            with torch.cuda.stream(self._out_stream):
+                self._out_stream.wait_stream(self._post_stream)
+                self._out_stream.wait_stream(self._pre_stream)
+                slot.fl_host[:n].copy_(slot.fl[:n], non_blocking=True)
+                slot.counts_host[:n].copy_(slot.counts[:n], non_blocking=True)
+                slot.done = torch.cuda.Event()
+                slot.done.record(self._out_stream)
+        slot.pending = True
+        ticket = Ticket(slot, n, masks_host)
+        ticket.order, ticket.widths = order, widths
+        ticket.proc_offsets = [0] * n       # caller index -> flat byte offset of its processed image in slot.proc_host
+        for (a, b, w), (_, _, off) in zip(chunks, views):
+            for p in range(a, b):
+                ticket.proc_offsets[order[p]] = off + (p - a) * Hc * w * 3
+        return ticket
+
+    def collect_mixed(self, ticket):
+        """-> (rows, widths, counts numpy [n,3], masks_host) in the caller's order; image i's processed image is
+        ``processed(ticket, i, rows[i])``."""
+        rows, counts, masks_host = self.collect(ticket)
+        n = ticket.n
+        rows_c, counts_c = [0] * n, counts.copy()
+        for p, i in enumerate(ticket.order):
+            rows_c[i] = rows[p]
+            counts_c[i] = counts[p]
+        return rows_c, list(ticket.widths), counts_c, masks_host
+
+    @staticmethod
+    def processed(ticket, i, rows):
+        """Image i of a collected ``submit_mixed(want_processed=True)`` ticket: a u8 view [rows, width, 3] of pinned memory."""
+        w, off = ticket.widths[i], ticket.proc_offsets[i]
+        return ticket.slot.proc_host.view(-1)[off:off + rows * w * 3].view(rows, w, 3)

@@ -129,6 +129,44 @@ def preprocess_general(raw, H, W, target=1024, pitch=None, bgr=False, bottom_up=
     return out, fl
 
 
+def processed_size(H, W, target=1024):
+    """(rows, cols) of a raw H x W image after the resize and before the trim, as Preprocessor.preprocess_array routes it
+    (models.py:194-201): target x target when the larger side exceeds target, unchanged otherwise."""
+    return (target, target) if max(H, W) > target else (H, W)
+
+
+def mixed_descs(items):
+    """ctypes array of nbc_mixed_desc from (device address, H, W, pitch, bgr, bottom_up, (span_row0, span_rows))."""
+    arr = (_lib.MixedDesc * len(items))()
+    for d, (ptr, H, W, pitch, bgr, bottom_up, span) in zip(arr, items):
+        d.raw, d.H, d.W, d.pitch = ptr or None, H, W, pitch
+        d.flags = (1 if bgr else 0) | (2 if bottom_up else 0)
+        d.span_row0, d.span_rows = span
+    return arr
+
+
+def preprocess_mixed_batch(raws, geoms, target=1024, spans=None):
+    """K1 for a chunk of raw images of any sizes in one call (nbc_preprocess_mixed_batch_u8), each routed as
+    ``Preprocessor.preprocess_array`` routes it.  raws: u8 CUDA tensors; geoms: (H, W, pitch, bgr, bottom_up) per image;
+    spans: optional (row0, rows) per image (only a (4 target)^2 scan may hold a part of its rows).  Returns (canvas u8
+    [n, Hmax * Wmax * 3] -- image i is ``canvas[i, :(last-first) * w_i * 3].view(last-first, w_i, 3)`` with w_i its
+    processed width --, first_last int32 [n, 2])."""
+    lib = _lib.load()
+    n = len(raws)
+    raws = [_contig(r, torch.uint8, 'raw') for r in raws]
+    dev = raws[0].device
+    spans = [(0, g[0]) for g in geoms] if spans is None else list(spans)
+    descs = mixed_descs([(r.data_ptr() if r.numel() else None,) + tuple(g) + (sp,) for r, g, sp in zip(raws, geoms, spans)])
+    stride = max(h * w for h, w in (processed_size(g[0], g[1], target) for g in geoms)) * 3
+    with torch.cuda.device(dev):
+        ws = torch.empty(lib.nbc_preprocess_mixed_workspace_bytes(descs, n, target), dtype=torch.uint8, device=dev)
+        out = torch.empty((n, stride), dtype=torch.uint8, device=dev)
+        fl = torch.empty((n, 2), dtype=torch.int32, device=dev)
+        _lib.check(lib.nbc_preprocess_mixed_batch_u8(descs, n, target, _ptr(out), stride, _ptr(fl), _ptr(ws), ws.numel(),
+                                                     _stream(dev)), 'nbc_preprocess_mixed_batch_u8')
+    return out, fl
+
+
 def trim_u8(img):
     """img: u8 CUDA [H, W, 3] that needs no resize -> (out flat, first_last).  (models.py:157-166, 200-201)"""
     lib = _lib.load()

@@ -10,8 +10,15 @@ NeuralBarkCalculator.predict, models.py:173-203 and 230-364).
 The files are the reference's: same names, same CSV layout, and the pixels of the oracle's restatement of the reference --
 processed images equal to the reference's except, possibly, one LSB on exact rounding ties (the float -> u8 rounding of
 scikit-image 0.15's save path is unpinned, see oracle/preprocess.py), class maps within the floating-point bar of
-DESIGN.md 5.  Only the PNG compression level is a knob (``png_compress_level``, pixels are unaffected).  Works for the standard input -- uncompressed 24-bit 4096x4096 BMP;
-``supported()`` says whether a folder qualifies, otherwise predict.py takes the per-image path of models.py."""
+DESIGN.md 5.  Only the PNG compression level is a knob (``png_compress_level``, pixels are unaffected).
+
+Two routes, one streaming pass each.  A folder of standard scans (uncompressed 24-bit 4096x4096 BMPs of one row order,
+``supported()``) takes the uniform route: the readers copy BMP pixel arrays, K1 is the 4x kernel for every scan.  Any
+other folder takes the mixed route, which accepts every input the per-image route of models.py accepts: the readers copy
+the pixel array of any 24-bit BMP and decode everything else with ``dataset.pil_loader`` (the per-image route's decoder),
+``PredictEngine.submit_mixed`` routes each image as ``Preprocessor.preprocess_array`` does (4x, general-ratio resize,
+trim only, or unchanged) and images narrower than the canvas run in ragged chunks of their own width.  Both routes write
+the per-image route's files: same names, formats, pixels and CSV rows (in dataset order)."""
 import csv
 import mmap
 import os
@@ -24,7 +31,7 @@ from os.path import join
 import numpy as np
 import torch
 from ._png import write_png
-from .dataset import make_dataset
+from .dataset import make_dataset, pil_loader
 from . import figure, ops
 from .engine import PredictEngine
 
@@ -127,6 +134,65 @@ def supported(items):
     return len(geo) > 0 and all(g is not None for g in geo) and len({g[1] for g in geo}) == 1
 
 
+def raw_geometry(path):
+    """How a reader gets an input's pixels, for the mixed route: (bmp data offset or None, H, W, pitch, bgr, bottom_up).
+    An uncompressed 24-bit BMP (any size, either row order) is read as its pixel array, as ``Preprocessor`` reads it
+    (``dataset.read_bmp_pixels``); any other file is decoded by ``dataset.pil_loader`` into RGB top-down rows."""
+    if path.lower().endswith('.bmp'):
+        try:
+            with open(path, 'rb') as f:
+                head = f.read(54)
+            size = os.path.getsize(path)
+        except OSError:
+            head, size = b'', 0
+        if len(head) == 54 and head[:2] == b'BM':
+            off = struct.unpack_from('<I', head, 10)[0]
+            hdr_size, w, h, planes, bpp, comp = struct.unpack_from('<IiiHHI', head, 14)
+            pitch = (w * 3 + 3) & ~3
+            if hdr_size >= 40 and bpp == 24 and comp == 0 and planes == 1 and w > 0 and h != 0 and size >= off + pitch * abs(h):
+                return off, abs(h), w, pitch, True, h > 0
+    from PIL import Image
+    with Image.open(path) as im:
+        w, h = im.size
+    return None, h, w, w * 3, False, False
+
+
+def read_raw(path, geo, buf, zero_span, target):
+    """Pixels of one input of the mixed route into the pinned buffer ``buf`` -> (row0, rows) to copy to the device.  A
+    (4 target)^2 image is reduced to the rows between its all-zero bands when ``zero_span`` (``read_scan`` for the BMP,
+    the same host scan after decoding otherwise); any other image is copied whole."""
+    off, H, W, pitch, _, _ = geo
+    scan = zero_span and H == W == 4 * target
+    if off is not None and scan and H == RAW:
+        return read_scan(path, off, buf, True)
+    view = buf.numpy()
+    if off is not None:
+        with open(path, 'rb', buffering=0) as f:
+            f.seek(off)
+            mv, got = memoryview(view), 0
+            while got < H * pitch:
+                n = f.readinto(mv[got:H * pitch])
+                if not n:
+                    raise IOError('short read: ' + path)
+                got += n
+    else:
+        img = pil_loader(path)
+        if img.shape != (H, W, 3):
+            raise IOError('%s decodes to %s, its header says %dx%d' % (path, img.shape, H, W))
+        np.copyto(view[:H * pitch].reshape(H, W, 3), img)
+    return ops.host_zero_row_span(buf, H, pitch, W * 3) if scan else (0, H)
+
+
+def save_image(path, arr, png_level, lut=None):
+    """One output file as the per-image route writes it: a PNG with the library's encoder, any other extension through
+    PIL in the format the extension names (models.py:203, 356)."""
+    if path.lower().endswith('.png'):
+        write_png(path, arr, png_level, lut=lut)
+    else:
+        from PIL import Image
+        Image.fromarray(arr if lut is None else lut[arr]).save(path)
+
+
 def read_scan(path, off, buf, zero_span=True):
     """Pixel array of a RAW x RAW 24-bit BMP (file offset ``off``) into the pinned buffer ``buf`` -> (row0, rows), the
     memory rows between the scan's all-zero dark bands (whole groups of 4; engine.py).  With ``zero_span`` the file is
@@ -163,6 +229,8 @@ def read_scan(path, off, buf, zero_span=True):
     return ops.host_zero_row_span(buf, RAW, pitch) if zero_span else (0, RAW)
 
 
+
+
 class FolderPipeline:
     def __init__(self, calculator, batch=16, io_threads=None, png_compress_level=None):
         if png_compress_level is None:      # 0 = stored (fastest, 1.9 MB per processed image), 1 = fast deflate (default)
@@ -178,21 +246,88 @@ class FolderPipeline:
 
     def run(self, root_path, excludes_nodes, only_preprocess=False, shard=None):
         """shard=(start, end): process only that slice of the dataset order and return its CSV rows WITHOUT writing
-        final_stats.csv (data-parallel runs: one process per GPU, rank 0 merges the rows -- distributed.merge_rows)."""
+        final_stats.csv (data-parallel runs: one process per GPU, rank 0 merges the rows -- distributed.merge_rows).
+        A folder of standard scans (``supported``) takes the uniform route: 4x K1 on every scan, one canvas width.  Any
+        other folder takes the mixed route: every input the per-image route accepts, each resized / trimmed as
+        ``Preprocessor.preprocess_array`` does, in the same streaming pass."""
         t_start = time.perf_counter()
         timing = {'read_s': 0.0, 'save_s': 0.0}      # summed over the IO threads
         items = make_dataset(root_path)
         if len(items) == 0:
             raise RuntimeError("Found 0 files in subfolders of: " + root_path)
+        standard = supported(items)
         if shard is not None:
             items = items[shard[0]:shard[1]]
             if len(items) == 0:
                 self.last_timing = {'images': 0}
                 return []
-        geo = [bmp_geometry(p) for p, _, _, _ in items]
-        bottom_up = geo[0][1]
+        rows_csv = [None] * len(items)
+        out_proc = join(root_path, 'processed', 'samples')
+        out_dual = join(root_path, 'results', 'outputs')
+        out_comb = join(root_path, 'results', 'combined_images')
+        engine = self.engine
+        Wo = RAW // 4
+        if standard:
+            geo = [bmp_geometry(p) for p, _, _, _ in items]
+            bottom_up = geo[0][1]
+            nbytes = RAW * RAW * 3
+
+            def read(i, buf):
+                # the reader finds the scan's all-zero dark bands while it reads: they never enter the pinned buffer, let
+                # alone cross PCIe (engine.py)
+                return read_scan(items[i][0], geo[i][0], buf, engine.zero_span)
+
+            def submit(idx, bufs, spans, masks):
+                return engine.submit_host(bufs, masks, bgr=True, bottom_up=bottom_up, exclude_nodes=excludes_nodes,
+                                          want_processed=True, only_preprocess=only_preprocess, spans=spans)
+
+            def results(ticket):
+                rows, counts, masks = engine.collect(ticket)
+                proc_host = ticket.slot.proc_host
+                for k, h in enumerate(rows):
+                    yield proc_host[k, :h], None if only_preprocess else masks[k][:h * Wo].numpy().reshape(h, Wo), counts[k]
+
+            save_file = write_png
+        else:
+            geo = [raw_geometry(p) for p, _, _, _ in items]
+            nbytes = max(g[1] * g[3] for g in geo)
+            engine.reserve_mixed(nbytes)
+
+            def read(i, buf):
+                return read_raw(items[i][0], geo[i], buf, engine.zero_span, Wo)
+
+            def submit(idx, bufs, spans, masks):
+                return engine.submit_mixed(bufs, [geo[i][1:] for i in idx], masks, exclude_nodes=excludes_nodes,
+                                           want_processed=True, only_preprocess=only_preprocess, spans=spans)
+
+            def results(ticket):
+                rows, widths, counts, masks = engine.collect_mixed(ticket)
+                for k, (h, w) in enumerate(zip(rows, widths)):
+                    yield (engine.processed(ticket, k, h), None if only_preprocess else masks[k][:h * w].numpy().reshape(h, w),
+                           counts[k])
+
+            save_file = save_image
+        timing['setup_s'] = time.perf_counter() - t_start
+        self._stream(items, nbytes, read, submit, results, save_file, rows_csv, timing, only_preprocess,
+                     (out_proc, out_dual, out_comb))
+        timing['total_s'] = time.perf_counter() - t_start
+        timing['images'] = len(items)
+        self.last_timing = timing
+        if only_preprocess:
+            return None
+        if shard is not None:
+            return rows_csv
+        results_csv = [CSV_HEADER] + rows_csv
+        with open(join(root_path, 'results', 'final_stats.csv'), 'w') as f:   # as models.py:360-364 (tab-delimited)
+            csv.writer(f, delimiter='\t').writerows(results_csv)
+        return results_csv
+
+    def _stream(self, items, nbytes, read, submit, results, save_file, rows_csv, timing, only_preprocess, out_dirs):
+        """The streaming pass: reader threads -> batches of B items submitted to the engine (two in flight) -> writer
+        threads.  read(i, buf) -> span; submit(idx, bufs, spans, masks) -> ticket; results(ticket) yields (processed u8
+        [h, w, 3], mask u8 [h, w] or None, counts) per item of the batch; save_file(path, arr, level, lut=None)."""
+        out_proc, out_dual, out_comb = out_dirs
         B = self.batch
-        nbytes = RAW * RAW * 3
         # Pinned staging buffers: 3 batches' worth (2 in flight + 1 being read).  The MAIN thread hands them out as tokens
         # in item order -- a reader can therefore never hold a buffer that an earlier item is still waiting for (a free-for-
         # all pool deadlocks: later items overtake a parked reader and exhaust it) -- while the page-locking itself (about
@@ -203,20 +338,12 @@ class FolderPipeline:
         spans = [None] * n_tokens
         mask_sets = [[torch.empty((RAW // 4) * (RAW // 4), dtype=torch.uint8).pin_memory() for _ in range(min(B, len(items)))]
                      for _ in range(2)]
-        rows_csv = [None] * len(items)
-        out_proc = join(root_path, 'processed', 'samples')
-        out_dual = join(root_path, 'results', 'outputs')
-        out_comb = join(root_path, 'results', 'combined_images')
-        Wo = RAW // 4
-        timing['setup_s'] = time.perf_counter() - t_start
 
         def load(i, tok):
             if pinned[tok] is None:
                 pinned[tok] = torch.empty(nbytes, dtype=torch.uint8).pin_memory()
             t0 = time.perf_counter()
-            # the reader finds the scan's all-zero dark bands while it reads: they never enter the pinned buffer, let alone
-            # cross PCIe (engine.py)
-            spans[tok] = read_scan(items[i][0], geo[i][0], pinned[tok], self.engine.zero_span)
+            spans[tok] = read(i, pinned[tok])
             timing['read_s'] += time.perf_counter() - t0
             return tok
 
@@ -224,9 +351,9 @@ class FolderPipeline:
             t0 = time.perf_counter()
             _, _, fname, wood = items[i]
             fname = fname.replace('.bmp', '.png')           # models.py:185
-            write_png(join(out_proc, wood, fname), proc, self.png_level)
+            save_file(join(out_proc, wood, fname), proc, self.png_level)
             if mask is not None:
-                write_png(join(out_dual, wood, fname), mask, self.png_level, lut=_DUAL_LUT)
+                save_file(join(out_dual, wood, fname), mask, self.png_level, lut=_DUAL_LUT)
                 rows_csv[i] = [fname, wood] + self.calc._stats_strings(counts, mask.size)
                 if self.combined:
                     write_combined(join(out_comb, wood, fname), proc, mask, rows_csv[i][2:], fname, self.calc.mean, self.calc.std,
@@ -246,13 +373,9 @@ class FolderPipeline:
 
             def finish(entry):
                 ticket, idx, toks = entry
-                rows, counts, masks = self.engine.collect(ticket)
-                proc_host = ticket.slot.proc_host
-                for k, i in enumerate(idx):
-                    h = rows[k]
-                    proc = proc_host[k, :h].numpy().copy()
-                    mask = None if only_preprocess else masks[k][:h * Wo].numpy().reshape(h, Wo).copy()
-                    saves.append(writers.submit(save, i, proc, mask, None if only_preprocess else counts[k].tolist()))
+                for i, (proc, mask, counts) in zip(idx, results(ticket)):
+                    saves.append(writers.submit(save, i, proc.numpy().copy(), None if mask is None else mask.copy(),
+                                                None if only_preprocess else counts.tolist()))
                 tokens.extend(toks)      # the H2D copies of this batch are done: its staging buffers are free again
                 feed()
 
@@ -260,9 +383,8 @@ class FolderPipeline:
             for a in range(0, len(items), B):
                 idx = list(range(a, min(a + B, len(items))))
                 toks = [loads[i].result() for i in idx]
-                ticket = self.engine.submit_host([pinned[t] for t in toks], None if only_preprocess else mask_sets[(a // B) & 1][:len(idx)],
-                                                 bgr=True, bottom_up=bottom_up, exclude_nodes=excludes_nodes, want_processed=True,
-                                                 only_preprocess=only_preprocess, spans=[spans[t] for t in toks])
+                ticket = submit(idx, [pinned[t] for t in toks], [spans[t] for t in toks],
+                                None if only_preprocess else mask_sets[(a // B) & 1][:len(idx)])
                 pending.append((ticket, idx, toks))
                 if len(pending) == 2:
                     finish(pending.pop(0))
@@ -276,14 +398,3 @@ class FolderPipeline:
                     f.cancel()
             readers.shutdown(wait=True)
             writers.shutdown(wait=True)
-        timing['total_s'] = time.perf_counter() - t_start
-        timing['images'] = len(items)
-        self.last_timing = timing
-        if only_preprocess:
-            return None
-        if shard is not None:
-            return rows_csv
-        results_csv = [CSV_HEADER] + rows_csv
-        with open(join(root_path, 'results', 'final_stats.csv'), 'w') as f:   # as models.py:360-364 (tab-delimited)
-            csv.writer(f, delimiter='\t').writerows(results_csv)
-        return results_csv

@@ -7,7 +7,7 @@ Same arguments, same ``processed/`` and ``results/`` layout, weights from ``./be
 import argparse
 import os
 
-from .models import NeuralBarkCalculator, Preprocessor
+from .models import NeuralBarkCalculator
 
 ALL_WOOD_TYPES = ['epinette_gelee', 'epinette_non_gelee', 'sapin']
 
@@ -24,9 +24,10 @@ def generate_folders(root_path, only_preprocess):
 
 
 def main(args, state_dict=None):
-    """predict.py:51-58.  Folders of standard scans (4096x4096 24-bit BMP) go through the streaming FolderPipeline --
-    preprocessing and prediction fused into one pass with batched GPU work and threaded file IO; anything else takes the
-    per-image path of models.py.  Both write the same files.
+    """predict.py:51-58.  Every folder goes through the streaming FolderPipeline -- preprocessing and prediction fused
+    into one pass with batched GPU work and threaded file IO.  Folders of standard scans (4096x4096 24-bit BMP) take its
+    uniform route, any other folder its mixed route; both write the files the per-image path of models.py
+    (``Preprocessor`` + ``NeuralBarkCalculator.predict``) writes.
 
     Under ``torchrun`` (one process per GPU) every rank takes a contiguous shard of the dataset order on cuda:LOCAL_RANK --
     images are independent, there is no collective on the data path -- and rank 0 merges the CSV rows back into dataset
@@ -49,30 +50,23 @@ def main(args, state_dict=None):
         import torch.distributed as dist
         dist.barrier()
     items = make_dataset(args.root_path)
-    if pipeline.supported(items):
-        model = NeuralBarkCalculator(None if state_dict is not None else './best_model.pt', device, state_dict=state_dict,
-                                     load_weights=not args.only_preprocess)
-        if os.environ.get('NBC_TIMING'):
-            print('[nbc] folders + model construction: %.3f s' % (time.perf_counter() - t0))
-        pipe = pipeline.FolderPipeline(model)
-        shard = ndist.shard_bounds(len(items), rank, world) if world > 1 else None
-        out = pipe.run(args.root_path, args.exclude_nodes, args.only_preprocess, shard=shard)
-        if world > 1 and not args.only_preprocess:
-            rows = ndist.merge_rows(out, shard[0], len(items))
-            out = None
-            if rank == 0:
-                out = [pipeline.CSV_HEADER] + rows
-                with open(os.path.join(args.root_path, 'results', 'final_stats.csv'), 'w') as f:   # models.py:360-364
-                    csv.writer(f, delimiter='\t').writerows(out)
-        if os.environ.get('NBC_TIMING'):
-            print('[nbc] folder pipeline timing: %s' % pipe.last_timing)
-        return out
-    if world > 1:
-        raise RuntimeError('multi-GPU predict needs the standard input (4096x4096 24-bit BMP scans)')
-    processed = Preprocessor(device=device).preprocess_images(args.root_path)
-    if not args.only_preprocess:
-        model = NeuralBarkCalculator('./best_model.pt', device, state_dict=state_dict)
-        return model.predict(args.root_path, args.exclude_nodes, processed=processed)
+    model = NeuralBarkCalculator(None if state_dict is not None else './best_model.pt', device, state_dict=state_dict,
+                                 load_weights=not args.only_preprocess)
+    if os.environ.get('NBC_TIMING'):
+        print('[nbc] folders + model construction: %.3f s' % (time.perf_counter() - t0))
+    pipe = pipeline.FolderPipeline(model)
+    shard = ndist.shard_bounds(len(items), rank, world) if world > 1 else None
+    out = pipe.run(args.root_path, args.exclude_nodes, args.only_preprocess, shard=shard)
+    if world > 1 and not args.only_preprocess:
+        rows = ndist.merge_rows(out, shard[0], len(items))
+        out = None
+        if rank == 0:
+            out = [pipeline.CSV_HEADER] + rows
+            with open(os.path.join(args.root_path, 'results', 'final_stats.csv'), 'w') as f:   # models.py:360-364
+                csv.writer(f, delimiter='\t').writerows(out)
+    if os.environ.get('NBC_TIMING'):
+        print('[nbc] folder pipeline timing: %s' % pipe.last_timing)
+    return out
 
 
 def parse_args(argv=None):
