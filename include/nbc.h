@@ -203,6 +203,25 @@ int nbc_argmax3_u8(const float* logits, int N, int H, int W, uint8_t* out, void*
 int nbc_confusion_matrix(const uint8_t* pred, const void* target, int target_is_i64, int64_t n_pixels, uint64_t* cm9,
                          void* stream);
 
+/* ---- N3: batched evaluation of a ragged chunk  (__main__.py:293-437, the post-training per-image dump) -------------
+ * logits: the low-resolution logits canvas of nbc_plan_forward_ragged, f32 [N,3,hc,w] with hc, w = ceil(Hc/8),
+ * ceil(W/8); heights int32 [N] on the device (image n has rows [0, heights[n]) of the Hc x W canvas); labels u8 classes
+ * [N,Hc,W]; weights3 f32[3] (may be NULL without the weighted CE); losses: bitmask, 1 = weighted CE, 2 = Lovasz.
+ * Per image n, each bit-identical to the per-image ops on that image alone (nbc_upsample_bicubic of its logits, then):
+ *   loss_wce[n]     f32, nbc_wce_fwd_bwd (utils.py:151-165); 0 without bit 1
+ *   loss_lovasz[n]  f32, nbc_lovasz_softmax_fwd_bwd (lovasz_losses.py:162-218); 0 without bit 2
+ *   cm_raw[n][9]    u64, nbc_confusion_matrix of nbc_argmax3_u8 (the iou / miou of lovasz_losses.py:54-77)
+ *   cm_rsz[n][9]    u64, the same after nbc_remove_small_zones (threshold 150, no node rewrite; PixelWiseF1,
+ *                   utils.py:201-235)
+ *   counts[n][3]    int32, nbc_remove_small_zones' class counts of that mask (models.py:323-332)
+ * heights are read back to the host first (N x 4 bytes, which waits for the stream).  N < 1, a height outside [1, Hc],
+ * 3 N Hc W >= 2^31 (the sort's item count and its 31-bit pixel payload) and a workspace smaller than
+ * nbc_eval_workspace_bytes(N, Hc, W) are refused before anything is launched. */
+size_t nbc_eval_workspace_bytes(int N, int Hc, int W);
+int nbc_eval_ragged(const float* logits, int N, int Hc, int W, const int32_t* heights, const uint8_t* labels,
+                    const float* weights3, int losses, float* loss_wce, float* loss_lovasz, uint64_t* cm_raw, uint64_t* cm_rsz,
+                    int32_t* counts, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- N4: training-time augmentation of a batch  (__main__.py:153-176 get_loader_for_crop_batch; dataset.py:171-193) --
  * images u8 [M,Hs,Ws,3] and their dual label images u8 [M,Hs,Ws] (0/127/255) resident on the device; for each of the B
  * output samples the caller draws the parameters: source index, crop offset (x0, y0) in the pad_resize'd (reflect-padded

@@ -75,6 +75,9 @@ SIGNATURES = {
                                    c_size_t, c_void_p]),
     'nbc_argmax3_u8': (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     'nbc_confusion_matrix': (c_int, [c_void_p, c_void_p, c_int, c_i64, c_void_p, c_void_p]),
+    'nbc_eval_workspace_bytes': (c_size_t, [c_int, c_int, c_int]),
+    'nbc_eval_ragged': (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
+                        c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     'nbc_augment_batch': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p,
                           c_void_p]),
     'nbc_augment_ragged': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int,

@@ -160,10 +160,12 @@ class DeviceDataset:
         return self._tables[key]
 
 
-def load_dataset(root, device='cuda:0'):
+def load_dataset(root, device='cuda:0', items=None):
     """``samples/<wood>/*`` and ``duals/<wood>/*`` of a labelled folder in ``dataset.make_dataset`` order, decoded on the
-    host (RGB and L) and copied once to ``device``.  Every sample needs its dual image."""
-    items = make_dataset(root)
+    host (RGB and L) and copied once to ``device``.  Every sample needs its dual image.  ``items`` (optional): indices
+    into that order; only those items are loaded, in the order given."""
+    entries = make_dataset(root)
+    items = entries if items is None else [entries[int(i)] for i in items]
     if not items:
         raise RuntimeError('load_dataset: no images under %s/samples' % root)
     missing = [f for _, t, f, _ in items if not t]

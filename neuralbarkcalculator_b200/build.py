@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libnbc.so')
 SOURCES = ['api.cu', 'preprocess.cu', 'stem.cu', 'conv_tc.cu', 'conv_mma.cu', 'head.cu', 'ccl.cu', 'wce.cu', 'plan.cu',
-           'train_kernels.cu', 'train_kernels2.cu', 'train_plan.cu', 'wgrad_tc.cu', 'lovasz.cu', 'augment.cu', 'png_host.cu', 'host_scan.cu']
+           'train_kernels.cu', 'train_kernels2.cu', 'train_plan.cu', 'wgrad_tc.cu', 'lovasz.cu', 'eval.cu', 'augment.cu', 'png_host.cu', 'host_scan.cu']
 FLAGS = ['-O3', '-std=c++17', '-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-Xcompiler', '-fPIC',
          '--expt-relaxed-constexpr']
 

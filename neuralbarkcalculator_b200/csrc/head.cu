@@ -7,7 +7,7 @@
 //    f32 with explicit IEEE operations (no fma contraction) in the order of oracle/model.py
 //    ``upsample_bicubic_restated`` so the result is bit-identical to that restatement.
 #include "common.cuh"
-#include "cubic.cuh"
+#include "k3.cuh"
 
 namespace nbc {
 
@@ -85,22 +85,6 @@ __global__ void __launch_bounds__(256) head1x1_kernel(const __nv_bfloat16* __res
   }
 }
 
-__device__ __forceinline__ float cubic_sample(const float* __restrict__ plane, int w, const int (&iy)[4],
-                                              const float (&wy)[4], const int (&ix)[4], const float (&wx)[4]) {
-  float out = 0.f;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const float* r = plane + (int64_t)iy[i] * w;
-    float inner = __fmul_rn(__ldg(r + ix[0]), wx[0]);
-    inner = __fadd_rn(inner, __fmul_rn(__ldg(r + ix[1]), wx[1]));
-    inner = __fadd_rn(inner, __fmul_rn(__ldg(r + ix[2]), wx[2]));
-    inner = __fadd_rn(inner, __fmul_rn(__ldg(r + ix[3]), wx[3]));
-    const float term = __fmul_rn(inner, wy[i]);
-    out = (i == 0) ? term : __fadd_rn(out, term);
-  }
-  return out;
-}
-
 template <bool kArgmax>
 __global__ void __launch_bounds__(256) upsample_kernel(const float* __restrict__ logits, int N, int C, int h, int w,
                                                        int H, int W, float scale_y, float scale_x,
@@ -129,80 +113,6 @@ __global__ void __launch_bounds__(256) upsample_kernel(const float* __restrict__
   }
 }
 
-// Ragged batch: image n has H_n valid rows in a canvas of Hc rows; its logits occupy ceil(H_n/8) rows of the hc-row
-// logits canvas -- per-image in / out heights (scale = h_n / H_n), otherwise the arithmetic of upsample_kernel<true>.
-// K3 with the x pass SHARED by the output rows of a group.  An output pixel is a 4 x 4 cubic sample of each class plane:
-// the inner (x) sums depend on (source row, X) only, and kRows = 8 consecutive output rows of an 8x upsample touch at
-// most 6 distinct source rows -- so a thread (one X) computes the <= 6 x 3 inner sums once, keeps them in its own column
-// of shared memory (no synchronisation: a thread only reads what it wrote) and finishes its 8 outputs from them: 9
-// global loads per output pixel instead of 48.  Exactly the arithmetic of cubic_sample (same operations, same order), so
-// the mask is bit-identical; a group that would need more than kSrc source rows (upscaling by less than ~2x) takes the
-// per-pixel path.  heights == nullptr: dense batch (every image H rows, h logits rows).
-constexpr int kK3Rows = 8, kK3Src = 6;
-__global__ void __launch_bounds__(256) upsample_argmax_rows_kernel(const float* __restrict__ logits, int hc, int w, int Hc, int W,
-                                                                   int h_dense, float scale_x, const int* __restrict__ heights,
-                                                                   uint8_t* __restrict__ mask) {
-  __shared__ float s_inner[3][kK3Src][256];
-  const int X = blockIdx.x * blockDim.x + threadIdx.x;
-  const int Y0 = blockIdx.y * kK3Rows;
-  const int n = blockIdx.z;
-  const int H = heights != nullptr ? min(max(__ldg(heights + n), 1), Hc) : Hc;
-  if (X >= W || Y0 >= H) return;
-  const int h = heights != nullptr ? ((((H - 1) / 2 + 1) - 1) / 2 + 1 - 1) / 2 + 1 : h_dense;
-  const float scale_y = __fdiv_rn((float)h, (float)H);
-  const int rows = min(kK3Rows, H - Y0);
-  int ix[4];
-  float wx[4];
-  cubic_taps(X, scale_x, w, ix, wx);
-  int iy[4];
-  float wy[4];
-  cubic_taps(Y0, scale_y, h, iy, wy);
-  const int r_min = iy[0];
-  cubic_taps(Y0 + rows - 1, scale_y, h, iy, wy);
-  const int nsrc = iy[3] - r_min + 1;      // tap rows are non-decreasing in Y and in k
-  const int64_t plane = (int64_t)hc * w;
-  const float* base = logits + (int64_t)n * 3 * plane;
-  uint8_t* out = mask + ((int64_t)n * Hc + Y0) * W + X;
-  if (nsrc > kK3Src) {
-    for (int y = 0; y < rows; ++y) {
-      cubic_taps(Y0 + y, scale_y, h, iy, wy);
-      float best = 0.f;
-      int arg = 0;
-#pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        const float v = cubic_sample(base + c * plane, w, iy, wy, ix, wx);
-        if (c == 0 || v > best) best = v, arg = c;
-      }
-      out[(int64_t)y * W] = (uint8_t)arg;
-    }
-    return;
-  }
-#pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    for (int r = 0; r < nsrc; ++r) {
-      const float* rp = base + c * plane + (int64_t)(r_min + r) * w;
-      float inner = __fmul_rn(__ldg(rp + ix[0]), wx[0]);
-      inner = __fadd_rn(inner, __fmul_rn(__ldg(rp + ix[1]), wx[1]));
-      inner = __fadd_rn(inner, __fmul_rn(__ldg(rp + ix[2]), wx[2]));
-      inner = __fadd_rn(inner, __fmul_rn(__ldg(rp + ix[3]), wx[3]));
-      s_inner[c][r][threadIdx.x] = inner;
-    }
-  }
-  for (int y = 0; y < rows; ++y) {
-    cubic_taps(Y0 + y, scale_y, h, iy, wy);
-    float best = 0.f;
-    int arg = 0;
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-      float v = __fmul_rn(s_inner[c][iy[0] - r_min][threadIdx.x], wy[0]);
-#pragma unroll
-      for (int k = 1; k < 4; ++k) v = __fadd_rn(v, __fmul_rn(s_inner[c][iy[k] - r_min][threadIdx.x], wy[k]));
-      if (c == 0 || v > best) best = v, arg = c;
-    }
-    out[(int64_t)y * W] = (uint8_t)arg;
-  }
-}
-
 __global__ void heights_kernel(const int* __restrict__ first_last, int N, int* __restrict__ heights) {
   const int n = blockIdx.x * blockDim.x + threadIdx.x;
   if (n < N) heights[n] = first_last[2 * n + 1] - first_last[2 * n];
@@ -225,7 +135,8 @@ extern "C" int nbc_upsample_argmax_ragged(const float* logits, int N, int hc, in
   NBC_REQUIRE(N > 0 && hc > 0 && w > 0 && Hc > 0 && W > 0 && Hc <= 65535 && N <= 65535, "nbc_upsample_argmax_ragged: bad shape");
   dim3 grid(ceil_div(W, 256), ceil_div(Hc, kK3Rows), N);
   upsample_argmax_rows_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(logits, hc, w, Hc, W, 0,
-                                                                                         (float)w / (float)W, heights, mask);
+                                                                                         (float)w / (float)W, heights, mask,
+                                                                                         K3Mask());
   NBC_CHECK_LAUNCH();
   return 0;
 }
@@ -266,7 +177,7 @@ static int upsample_common(const float* logits, int N, int C, int h, int w, int 
   dim3 grid(ceil_div(W, 256), H, N);
   if (mask && C == 3)
     upsample_argmax_rows_kernel<<<dim3(ceil_div(W, 256), ceil_div(H, kK3Rows), N), 256, 0, stream>>>(logits, h, w, H, W, h, sx, nullptr,
-                                                                                                    mask);
+                                                                                                    mask, K3Mask());
   else if (mask)
     upsample_kernel<true><<<grid, 256, 0, stream>>>(logits, N, C, h, w, H, W, sy, sx, mask, nullptr);
   else

@@ -18,25 +18,9 @@
 #include <cub/cub.cuh>
 #include <thrust/iterator/transform_iterator.h>
 
-#include "common.cuh"
+#include "loss.cuh"
 
 namespace nbc {
-
-constexpr int kLvThreads = 256;
-
-struct LovaszHeader {
-  int gts[3];        // pixels per label
-  int pad;
-  float loss[3];     // per-class loss (only meaningful where gts > 0)
-  float pad2;
-};
-
-__device__ __forceinline__ void softmax3(float a, float b, float c, float (&p)[3]) {
-  const float m = fmaxf(a, fmaxf(b, c));
-  const float ea = expf(a - m), eb = expf(b - m), ec = expf(c - m);
-  const float s = ea + eb + ec;
-  p[0] = ea / s, p[1] = eb / s, p[2] = ec / s;
-}
 
 template <typename T>
 __global__ void __launch_bounds__(kLvThreads) lovasz_errors_kernel(const float* __restrict__ logits, const T* __restrict__ target,
@@ -53,7 +37,7 @@ __global__ void __launch_bounds__(kLvThreads) lovasz_errors_kernel(const float* 
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
       const bool fg = (t == c);
-      keys[(int64_t)c * P + i] = fabsf((fg ? 1.f : 0.f) - p[c]);
+      keys[(int64_t)c * P + i] = lovasz_error(p[c], fg);
       vals[(int64_t)c * P + i] = (uint32_t)i | (fg ? 0x80000000u : 0u);
     }
   }
@@ -64,10 +48,6 @@ __global__ void __launch_bounds__(kLvThreads) lovasz_errors_kernel(const float* 
     if (lane == 0 && k) atomicAdd(&hdr->gts[c], k);
   }
 }
-
-struct FgOf {
-  __host__ __device__ __forceinline__ uint32_t operator()(const uint32_t& v) const { return v >> 31; }
-};
 
 // rank i of class c: Lovasz gradient, loss partial, scatter to the pixel
 __global__ void __launch_bounds__(kLvThreads) lovasz_grad_kernel(const float* __restrict__ e_sorted, const uint32_t* __restrict__ v_sorted,
@@ -82,51 +62,23 @@ __global__ void __launch_bounds__(kLvThreads) lovasz_grad_kernel(const float* __
     const uint32_t v = v_sorted[i];
     const uint32_t fg = v >> 31;
     const uint32_t cf = cum[i];
-    const float gts = (float)G;
-    // exactly the reference's f32 expression: 1. - intersection / union
-    const float inter = gts - (float)cf;
-    const float uni = gts + (float)((uint32_t)(i + 1) - cf);
-    float g = 1.f - inter / uni;
-    if (i > 0) {
-      const uint32_t cfp = cf - fg;
-      const float inter_p = gts - (float)cfp;
-      const float uni_p = gts + (float)((uint32_t)i - cfp);
-      g = g - (1.f - inter_p / uni_p);
-    }
+    const float g = lovasz_rank_grad(G, i, cf, fg);
     contrib = e_sorted[i] * g;
     ge[v & 0x7FFFFFFFu] = g;
   }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) contrib += __shfl_xor_sync(0xffffffffu, contrib, o);
-  if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = contrib;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float s = 0.f;
-    for (int w = 0; w < kLvThreads / 32; ++w) s += s_part[w];
-    partial[blockIdx.x] = s;
-  }
+  const float s = lovasz_block_sum(contrib, s_part);
+  if (threadIdx.x == 0) partial[blockIdx.x] = s;
 }
 
 // sums the block partials of one class in double (one block), fixed order
 __global__ void __launch_bounds__(256) lovasz_class_sum(const float* __restrict__ partial, int nblocks, int c, LovaszHeader* hdr) {
   __shared__ double s[256];
-  double a = 0.0;
-  for (int i = threadIdx.x; i < nblocks; i += 256) a += (double)partial[i];
-  s[threadIdx.x] = a;
-  __syncthreads();
-  for (int o = 128; o > 0; o >>= 1) {
-    if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) hdr->loss[c] = (float)s[0];
+  const float sum = lovasz_partials_sum(partial, nblocks, s);
+  if (threadIdx.x == 0) hdr->loss[c] = sum;
 }
 
 __global__ void lovasz_finish(const LovaszHeader* __restrict__ hdr, float* __restrict__ loss_out) {
-  int np = 0;
-  float acc = 0.f;
-  for (int c = 0; c < 3; ++c)
-    if (hdr->gts[c] > 0) acc += hdr->loss[c], ++np;     // mean() of lovasz_losses.py:258-276: acc / n, 0 when empty
-  *loss_out = np > 0 ? acc / (float)np : 0.f;
+  *loss_out = lovasz_present_mean(hdr->gts, hdr->loss);
 }
 
 // out[i] = scale_a * a[i] + scale_b * b[i]   (MixedLoss: CE / 4 + Lovasz, utils.py:185-192)

@@ -5,7 +5,7 @@
 // The reference runs five separate full-tensor torch ops; here each pixel's three logits are read once
 // (planar f32 [N,3,H,W], coalesced per class plane) and the three gradients written once: 25 B/pixel in f32.
 // The loss is reduced deterministically: per-block partial sums in double, then one block sums them in order.
-#include "common.cuh"
+#include "loss.cuh"
 
 namespace nbc {
 
@@ -21,17 +21,8 @@ __global__ void __launch_bounds__(256) wce_kernel(const float* __restrict__ logi
     const float* lp = logits + n * 3 * HW + pix;
     const float l0 = __ldg(lp), l1 = __ldg(lp + HW), l2 = __ldg(lp + 2 * HW);
     const int t = (int)target[i];
-    int am = 0;
-    float mx = l0;
-    if (l1 > mx) mx = l1, am = 1;
-    if (l2 > mx) mx = l2, am = 2;
-    const float e0 = expf(l0 - mx), e1 = expf(l1 - mx), e2 = expf(l2 - mx);
-    const float s = e0 + e1 + e2;
-    const float lse = mx + logf(s);
-    const float lt = (t == 0) ? l0 : (t == 1 ? l1 : l2);
-    const int mc = max(am, t);
-    const float w = (mc == 0) ? w0 : (mc == 1 ? w1 : w2);
-    local += (double)((lse - lt) * w);
+    float e0, e1, e2, s, w;
+    local += (double)wce_term(l0, l1, l2, t, w0, w1, w2, e0, e1, e2, s, w);
     if (grad) {
       const float k = w * inv_total, inv_s = 1.f / s;
       float* gp = grad + n * 3 * HW + pix;
@@ -41,26 +32,13 @@ __global__ void __launch_bounds__(256) wce_kernel(const float* __restrict__ logi
     }
   }
   __shared__ double s_part[8];
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) local += __shfl_xor_sync(0xffffffffu, local, o);
-  if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = local;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double s = 0.0;
-    for (int k = 0; k < 8; ++k) s += s_part[k];
-    partial[blockIdx.x] = s;
-  }
+  const double s = wce_block_sum(local, s_part);
+  if (threadIdx.x == 0) partial[blockIdx.x] = s;
 }
 
 __global__ void wce_finish(const double* __restrict__ partial, int n, double inv_total, float* __restrict__ loss) {
-  if (threadIdx.x == 0 && blockIdx.x == 0) {
-    double s = 0.0;
-    for (int i = 0; i < n; ++i) s += partial[i];
-    *loss = (float)(s * inv_total);
-  }
+  if (threadIdx.x == 0 && blockIdx.x == 0) *loss = wce_partials_mean(partial, n, inv_total);
 }
-
-constexpr int kWceBlocks = 148 * 8;
 
 }  // namespace nbc
 

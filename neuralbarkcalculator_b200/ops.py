@@ -508,6 +508,46 @@ def confusion_matrix(pred_u8, target):
     return cm.view(3, 3)
 
 
+EVAL_WCE, EVAL_LOVASZ = 1, 2
+
+
+def eval_ragged(logits, heights, labels, weights=None, losses=EVAL_WCE | EVAL_LOVASZ, workspace=None):
+    """N3: the per-image evaluation of a ragged chunk in one call.  logits f32 [N,3,ceil(Hc/8),ceil(W/8)] as
+    ``Plan.forward_ragged`` leaves them, heights int32 [N], labels u8 classes [N,Hc,W], weights f32[3] (needed with
+    ``EVAL_WCE``), ``losses`` a bitmask of EVAL_WCE / EVAL_LOVASZ.  Returns a dict of device tensors: loss_wce f32 [N],
+    loss_lovasz f32 [N], cm_raw int64 [N,3,3] (argmax), cm_rsz int64 [N,3,3] (after region removal) and counts int32
+    [N,3], each equal to the per-image ops on that image alone (see include/nbc.h)."""
+    lib = _lib.load()
+    logits = _contig(logits, torch.float32, 'logits')
+    heights = _contig(heights, torch.int32, 'heights')
+    labels = _contig(labels, torch.uint8, 'labels')
+    if labels.dim() != 3:
+        raise RuntimeError('eval_ragged: labels must be u8 [N,Hc,W]')
+    N, Hc, W = labels.shape
+    hc = ((((Hc - 1) // 2 + 1) - 1) // 2 + 1 - 1) // 2 + 1
+    w = ((((W - 1) // 2 + 1) - 1) // 2 + 1 - 1) // 2 + 1
+    if tuple(logits.shape) != (N, 3, hc, w) or tuple(heights.shape) != (N,):
+        raise RuntimeError('eval_ragged: expected logits [%d,3,%d,%d] and heights [%d] for labels %s'
+                           % (N, hc, w, N, tuple(labels.shape)))
+    if weights is not None:
+        weights = _contig(weights, torch.float32, 'weights')
+    dev = logits.device
+    with torch.cuda.device(dev):
+        need = lib.nbc_eval_workspace_bytes(N, Hc, W)
+        if workspace is None or workspace.numel() < need:
+            workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+        out = {'loss_wce': torch.empty(N, dtype=torch.float32, device=dev),
+               'loss_lovasz': torch.empty(N, dtype=torch.float32, device=dev),
+               'cm_raw': torch.empty((N, 3, 3), dtype=torch.int64, device=dev),
+               'cm_rsz': torch.empty((N, 3, 3), dtype=torch.int64, device=dev),
+               'counts': torch.empty((N, 3), dtype=torch.int32, device=dev)}
+        _lib.check(lib.nbc_eval_ragged(_ptr(logits), N, Hc, W, _ptr(heights), _ptr(labels), _ptr(weights), int(losses),
+                                       _ptr(out['loss_wce']), _ptr(out['loss_lovasz']), _ptr(out['cm_raw']),
+                                       _ptr(out['cm_rsz']), _ptr(out['counts']), _ptr(workspace), workspace.numel(),
+                                       _stream(dev)), 'nbc_eval_ragged')
+    return out
+
+
 # ---- the network plan ---------------------------------------------------------------------------------------------
 class Plan:
     """Owns an nbc_plan (BN-folded bf16 weights on the device) built from the 326 state_dict tensors."""
