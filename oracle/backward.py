@@ -2,7 +2,7 @@
 
 Each helper takes the operands a kernel consumed and returns what it should have produced, so a test can check one
 backward kernel from the kernel's own stored inputs (teacher forcing).  Tensors are NCHW; everything is computed in
-float64.  Each helper is checked against torch autograd in tests/test_oracle.py."""
+float64, on the device of the operands.  Each helper is checked against torch autograd in tests/test_oracle.py."""
 import numpy as np
 import torch
 import torch.nn.functional as F
@@ -56,8 +56,8 @@ def maxpool_backward(dy, x, last=False):
     N, C, H, W = x.shape
     Ho, Wo = (H - 1) // 2 + 1, (W - 1) // 2 + 1
     xp = F.pad(x.double(), (1, 1, 1, 1), value=float('-inf'))
-    best = torch.full((N, C, Ho, Wo), float('-inf'), dtype=torch.float64)
-    pos = torch.zeros((N, C, Ho, Wo), dtype=torch.int64)
+    best = torch.full((N, C, Ho, Wo), float('-inf'), dtype=torch.float64, device=x.device)
+    pos = torch.zeros((N, C, Ho, Wo), dtype=torch.int64, device=x.device)
     for k in range(9):
         ky, kx = divmod(k, 3)
         v = xp[:, :, ky:ky + 2 * Ho - 1:2, kx:kx + 2 * Wo - 1:2]
@@ -70,29 +70,30 @@ def maxpool_backward(dy, x, last=False):
     return dxp[:, :, 1:H + 1, 1:W + 1]
 
 
-def bicubic_matrix(in_size, out_size, clamp=True):
+def bicubic_matrix(in_size, out_size, clamp=True, device=None):
     """Dense [out, in] interpolation matrix of F.interpolate(mode='bicubic', align_corners=False) along one axis, from
-    the float32 tap weights the kernels use.  ``clamp=False`` drops the taps outside the input instead of clamping them
-    to the edge (a negative control)."""
+    the float32 tap weights the kernels use, on ``device`` (default: the CPU).  ``clamp=False`` drops the taps outside
+    the input instead of clamping them to the edge (a negative control)."""
     idx, w = bicubic_weights_f32(in_size, out_size, clamp=clamp)
     m = np.zeros((out_size, in_size))
     for d in range(out_size):
         for k in range(4):
             if 0 <= idx[d, k] < in_size:
                 m[d, idx[d, k]] += float(w[d, k])
-    return torch.from_numpy(m)
+    return torch.from_numpy(m).to(device)
 
 
 def upsample_bicubic(low, size):
     """up = Wy . low . Wx^T per plane: [N,C,h,w] -> [N,C,H,W]."""
-    wy, wx = bicubic_matrix(low.shape[-2], size[0]), bicubic_matrix(low.shape[-1], size[1])
+    wy = bicubic_matrix(low.shape[-2], size[0], device=low.device)
+    wx = bicubic_matrix(low.shape[-1], size[1], device=low.device)
     return torch.einsum('Yi,ncij,Xj->ncYX', wy, low.double(), wx)
 
 
 def upsample_adjoint(dup, low_size, clamp=True):
     """Adjoint of ``upsample_bicubic``: dlow = Wy^T . dup . Wx per plane, [N,C,H,W] -> [N,C,h,w]."""
-    wy = bicubic_matrix(low_size[0], dup.shape[-2], clamp=clamp)
-    wx = bicubic_matrix(low_size[1], dup.shape[-1], clamp=clamp)
+    wy = bicubic_matrix(low_size[0], dup.shape[-2], clamp=clamp, device=dup.device)
+    wx = bicubic_matrix(low_size[1], dup.shape[-1], clamp=clamp, device=dup.device)
     return torch.einsum('Yi,ncYX,Xj->ncij', wy, dup.double(), wx)
 
 

@@ -56,6 +56,32 @@ def lovasz_softmax_with_grad(logits, labels):
     return loss.detach(), p.grad
 
 
+def lovasz_softmax_f64(logits, labels):
+    """``lovasz_softmax`` in float64 throughout (softmax, Jaccard), on the device of the operands, with the errors
+    sorted STABLY in descending order.  The value does not depend on how tied errors are ordered (a group of equal
+    errors adds e * the Jaccard step over the whole group), so this is the reference's value without its rounding.
+    Returns (loss, A) with A the same mean of sums over magnitudes, for error bars."""
+    probas = F.softmax(logits.double(), dim=1)
+    C = probas.shape[1]
+    probas = probas.permute(0, 2, 3, 1).reshape(-1, C)
+    labels = labels.reshape(-1)
+    per_class, mag = [], []
+    for c in range(C):
+        fg = (labels == c).double()
+        gts = fg.sum()
+        if gts == 0:
+            continue
+        errors, perm = torch.sort((fg - probas[:, c]).abs(), dim=0, descending=True, stable=True)
+        fg_sorted = fg[perm]
+        jaccard = 1. - (gts - fg_sorted.cumsum(0)) / (gts + (1 - fg_sorted).cumsum(0))
+        grad = torch.diff(jaccard, prepend=jaccard.new_zeros(1))
+        per_class.append(torch.dot(errors, grad))
+        mag.append(torch.dot(errors, grad.abs()))
+    if not per_class:
+        return torch.zeros((), dtype=torch.float64), torch.zeros((), dtype=torch.float64)
+    return sum(per_class) / len(per_class), sum(mag) / len(mag)
+
+
 def mixed_loss(logits, labels, weights):
     """utils.py:185-192: CustomWeightedCrossEntropy / 4 + LovaszSoftmax."""
     return losses.custom_weighted_cross_entropy(logits, labels, weights) / 4 + lovasz_softmax(logits, labels)

@@ -28,6 +28,7 @@ import torch.nn.functional as F
 from oracle import backward as ob
 from oracle import model as omodel
 from oracle import synth
+from oracle.teacher import Bars, bf16_bar, check_head, f32_bar, plan_units, run_step, stored_inputs
 
 pytestmark = pytest.mark.gpu
 
@@ -43,106 +44,18 @@ GEOMETRIES = {
 }
 
 
-def _plan_units():
-    """The native plan's units in its order (state_dict order, 0 = stem, last = head conv) and its bottleneck blocks."""
-    units = [dict(conv='backbone.conv1', bn='backbone.bn1', s=2, p=3, d=1, relu=True)]
-    blocks, dil = [], 1
-    for li, (nb, stride, dilate) in enumerate(((3, 1, False), (4, 2, False), (6, 1, True), (3, 1, True)), start=1):
-        for b in range(nb):
-            pre = 'backbone.layer%d.%d.' % (li, b)
-            s_ = stride if (b == 0 and not dilate) else 1
-            prev = dil
-            if b == 0 and dilate:
-                dil *= 2
-            d2 = prev if b == 0 else dil
-            B = dict(c1=len(units), c2=len(units) + 1, c3=len(units) + 2, ds=None)
-            units += [dict(conv=pre + 'conv1', bn=pre + 'bn1', s=1, p=0, d=1, relu=True),
-                      dict(conv=pre + 'conv2', bn=pre + 'bn2', s=s_, p=d2, d=d2, relu=True),
-                      dict(conv=pre + 'conv3', bn=pre + 'bn3', s=1, p=0, d=1, relu=True)]   # ReLU after the residual add
-            if b == 0:
-                B['ds'] = len(units)
-                units.append(dict(conv=pre + 'downsample.0', bn=pre + 'downsample.1', s=s_, p=0, d=1, relu=False))
-            blocks.append(B)
-    units.append(dict(conv='classifier.0', bn='classifier.1', s=1, p=1, d=1, relu=True))
-    return units, blocks, len(units) - 1
-
-
-def bf16_bar(S, ref):
-    return 2.0 ** -7 * S + 2e-3 * ref.abs().max()
-
-
-def f32_bar(A):
-    return 2.0 ** -14 * A + 2.0 ** -20 * A.max()
-
-
-class Bars:
-    """Worst err / tol per check class.  Failures are collected, not raised at the first one, so that one run on the
-    GPU reports every check that fails."""
-
-    def __init__(self):
-        self.worst, self.failures, self.controls = {}, [], {}
-
-    def check(self, cls, what, got, ref, tol):
-        got, ref = got.double(), ref.double()
-        assert got.shape == ref.shape, (what, got.shape, ref.shape)
-        err = (got - ref).abs()
-        ratio = err / (tol + 1e-300)
-        r = float(ratio.max())
-        if cls not in self.worst or r > self.worst[cls][0]:
-            self.worst[cls] = (r, what)
-        if not r <= 1.0:
-            i = int(ratio.argmax())
-            idx = np.unravel_index(i, ratio.shape)
-            self.failures.append('%s / %s: err/tol %.3g at %s (got %.6g ref %.6g tol %.3g), %d of %d elements out' % (
-                cls, what, r, tuple(int(v) for v in idx), float(got.flatten()[i]), float(ref.flatten()[i]),
-                float(tol.flatten()[i]) if tol.dim() else float(tol), int((ratio > 1).sum()), ratio.numel()))
-
-    def exact(self, cls, what, got, ref):
-        bad = int((got != ref).sum())
-        self.worst[cls] = (max(self.worst.get(cls, (0, ''))[0], bad), 'elements that differ')
-        if bad:
-            self.failures.append('%s / %s: %d of %d elements differ' % (cls, what, bad, got.numel()))
-
-    @staticmethod
-    def within(got, ref, tol):
-        return bool(((got.double() - ref.double()).abs() <= tol).all())
-
-    def control(self, name, rejected):
-        self.controls[name] = self.controls.get(name, False) or bool(rejected)
-
-    def report(self, tag):
-        for cls, (r, what) in sorted(self.worst.items()):
-            print('[%s] worst err/tol %-26s %.4f  (%s)' % (tag, cls, r, what))
-        for name, rej in sorted(self.controls.items()):
-            print('[%s] negative control %-28s %s' % (tag, name, 'rejected' if rej else 'NOT REJECTED'))
-        for f in self.failures[:40]:
-            print('[%s] FAIL %s' % (tag, f))
-        assert not self.failures, '%d checks failed; first: %s' % (len(self.failures), self.failures[0])
-        assert all(self.controls.values()), self.controls
-
-
 def _step(cuda_device, sd, N, H, W, impl, dropout_p, seed):
     """One forward_backward with capture on (after the same step with capture off, which must compute the same)."""
-    from neuralbarkcalculator_b200 import _lib
     from neuralbarkcalculator_b200.train import Trainer
     x = torch.cat([omodel.normalise_u8(synth.texture_u8(H, W, 11 + i)) for i in range(N)])   # f32 NCHW input
     tgt = np.stack([synth.class_mask(H, W, 111 + i) for i in range(N)])
     tr = Trainer(sd, N, H, W, device='cuda:0', dropout=dropout_p, class_weights=torch.ones(3))
-    _lib.check(tr.lib.nbc_train_set_wgrad_impl(C.c_void_p(tr.handle), impl), 'nbc_train_set_wgrad_impl')
-    xi, ti = x.to(cuda_device), torch.from_numpy(tgt).to(cuda_device)
-    n_units = tr.lib.nbc_train_num_units(C.c_void_p(tr.handle))
-    loss_off = float(tr.forward_backward(xi, ti, seed=seed, update_stats=False))
-    zy_off = [tr.debug_tensor(k, u).clone() for u in range(n_units) for k in (0, 1)]
-    tr.enable_capture()
-    loss = float(tr.forward_backward(xi, ti, seed=seed))
-    torch.cuda.synchronize()
-    assert loss == loss_off, (loss, loss_off)
-    assert all(torch.equal(a, tr.debug_tensor(k, u)) for a, (u, k) in zip(zy_off, [(u, k) for u in range(n_units) for k in (0, 1)]))
+    run_step(tr, x.to(cuda_device), torch.from_numpy(tgt).to(cuda_device), seed, impl)
     return tr, x
 
 
 def _check_step(tr, sd, x, dropout_p, seed, bars):
-    units, blocks, head = _plan_units()
+    units, blocks, head = plan_units()
     assert len(units) == tr.lib.nbc_train_num_units(C.c_void_p(tr.handle))
     N = x.shape[0]
     dims = (0, 2, 3)
@@ -157,13 +70,7 @@ def _check_step(tr, sd, x, dropout_p, seed, bars):
         return sd[units[u]['conv'] + '.weight'].to(torch.bfloat16).double()
 
     # stored input of every unit: the bf16 staging image, the maxpool output (a max of bf16 values is exact) or a y
-    src, cur = {0: 'image'}, 'pool'
-    for B in blocks:
-        src[B['c1']], src[B['c2']], src[B['c3']] = cur, B['c1'], B['c2']
-        if B['ds'] is not None:
-            src[B['ds']] = cur
-        cur = B['c3']
-    src[head] = cur
+    src = stored_inputs(blocks, head)
 
     def x_of(u):
         s = src[u]
@@ -235,38 +142,7 @@ def _check_step(tr, sd, x, dropout_p, seed, bars):
     bars.check('dgrad', 'classifier.0', t(6, blocks[-1]['c3']), ref, bf16_bar(ref.abs(), ref))
 
     # ---- head: bicubic adjoint, classifier backward (through the dropout mask), low-res logits
-    dfull = tr.debug_tensor(4).cpu().double()
-    dlow = tr.debug_tensor(5).cpu().double()
-    low = tr.debug_tensor(2).cpu().double()
-    h8, w8 = dlow.shape[-2:]
-    wy, wx = ob.bicubic_matrix(h8, dfull.shape[-2]).abs(), ob.bicubic_matrix(w8, dfull.shape[-1]).abs()
-    A = torch.einsum('Yi,ncYX,Xj->ncij', wy, dfull.abs(), wx)
-    bars.check('dlow (upsample adjoint)', 'dlow', dlow, ob.upsample_adjoint(dfull, (h8, w8)), f32_bar(A))
-    bars.control('adjoint without clamping',
-                 not bars.within(dlow, ob.upsample_adjoint(dfull, (h8, w8), clamp=False), f32_bar(A)))
-
-    Wc = sd['classifier.4.weight'].view(3, -1).double()
-    bc = sd['classifier.4.bias'].double()
-    yh = t(1, head)
-    keep = torch.ones_like(yh, dtype=torch.bool)
-    xc = yh
-    if dropout_p > 0:
-        keep = torch.from_numpy(ob.dropout_keep(seed, yh.numel(), dropout_p)).view(N, h8, w8, -1).permute(0, 3, 1, 2)
-        scale = torch.tensor(np.float32(1) / (np.float32(1) - np.float32(dropout_p)))
-        xc = torch.where(keep, (yh.float() * scale).to(torch.bfloat16).float(), torch.zeros(())).double()
-        kept = float(keep.double().mean())
-        print('dropout p=%.2f: kept fraction %.4f' % (dropout_p, kept))
-        assert abs(kept - (1 - dropout_p)) < 0.01
-    A = torch.einsum('ck,nkhw->nchw', Wc.abs(), xc.abs()) + bc.abs().view(1, 3, 1, 1)
-    bars.check('low logits', 'classifier.4 forward', low, torch.einsum('ck,nkhw->nchw', Wc, xc) + bc.view(1, 3, 1, 1), f32_bar(A))
-    g = torch.einsum('nchw,ck->nkhw', dlow, Wc)
-    if dropout_p > 0:
-        g = torch.where(keep, g * float(scale), torch.zeros(()).double())
-        bars.exact('dropped dy(head) == 0', 'classifier.1 dy', t(6, head)[~keep], torch.zeros(int((~keep).sum())).double())
-    bars.check('head dy', 'classifier.1 dy', t(6, head), g, bf16_bar(g.abs(), g))
-    bars.check('classifier dW db', 'classifier.4.weight', grads['classifier.4.weight'].view(3, -1),
-               torch.einsum('nchw,nkhw->ck', dlow, xc), f32_bar(torch.einsum('nchw,nkhw->ck', dlow.abs(), xc.abs())))
-    bars.check('classifier dW db', 'classifier.4.bias', grads['classifier.4.bias'], dlow.sum(dims), f32_bar(dlow.abs().sum(dims)))
+    check_head(tr, sd, t(1, head), t(6, head), dropout_p, seed, bars)
 
 
 @pytest.mark.parametrize('impl', [0, 1], ids=['wgrad_tc', 'wgrad_mma'])

@@ -315,3 +315,18 @@ def test_backward_oracle_dropout_hash():
                                                            0xF88BB8A8724C81EC]
     k1, k2 = ob.dropout_keep(7, 200000, 0.8), ob.dropout_keep(8, 200000, 0.8)
     assert abs(k1.mean() - 0.2) < 0.005 and (k1 != k2).mean() > 0.2
+
+
+def test_lovasz_oracle_float64_stable(golden_dir):
+    """The float64 restatement with a stable sort gives the reference's value up to its float32 rounding, and does not
+    depend on how tied errors are ordered (pixels permuted, so equal errors meet in another order)."""
+    from oracle import lovasz as olovasz
+    g = np.load(os.path.join(golden_dir, 'lovasz_small.npz'))
+    logits, target = torch.from_numpy(g['logits']), torch.from_numpy(g['target']).long()
+    loss, A = olovasz.lovasz_softmax_f64(logits, target)
+    assert loss.dtype == torch.float64 and abs(float(loss) - float(g['loss'])) < 1e-6 and float(A) >= float(loss) - 1e-12
+    q = (logits * 4).round() / 4           # many exactly tied errors
+    a = olovasz.lovasz_softmax_f64(q, target)[0]
+    perm = torch.randperm(q.shape[-1], generator=torch.Generator().manual_seed(0))
+    b = olovasz.lovasz_softmax_f64(q[..., perm], target[..., perm])[0]
+    assert abs(float(a) - float(b)) < 1e-12 and abs(float(a) - float(olovasz.lovasz_softmax(q, target))) < 1e-6
