@@ -311,7 +311,8 @@ int nbc_plan_step_info(const nbc_plan* plan, int i, nbc_plan_step* out);
  * gives per-layer gradients in state_dict layout (stats = NULL).
  * nbc_train_forward_backward: input_kind 0 = u8 NHWC images (normalised inside), 1 = f32 NCHW; target u8 [N,H,W];
  * BatchNorm uses batch statistics and updates `stats` (momentum 0.1) unless stats is NULL; dropout_p applies to the
- * head (mask = hash(seed, index)); loss = mean weighted CE (device scalar); grads are overwritten.
+ * head (mask = hash(seed, index)); loss = mean weighted CE (device scalar); grads are overwritten, or added to after
+ * nbc_train_set_accumulate(plan, 1) (gradient accumulation over micro-batches: the caller zeroes `grads` first).
  * Data-parallel training: all-reduce `grads` (sum) across ranks, then nbc_train_adam with grad_scale = 1/world.
  * nbc_train_adam follows torch.optim.Adam (L2 weight decay added to the gradient, bias correction by `step` >= 1). */
 typedef struct nbc_train_plan nbc_train_plan;
@@ -351,6 +352,9 @@ int nbc_train_set_wgrad_impl(nbc_train_plan* plan, int impl);
 /* loss of the step: 0 = CustomWeightedCrossEntropy (utils.py:151-165, default), 1 = LovaszSoftmax (__main__.py:239),
  * 2 = MixedLoss = CE / 4 + Lovasz (utils.py:185-192) */
 int nbc_train_set_loss(nbc_train_plan* plan, int kind);
+/* 1: nbc_train_forward_backward adds its gradients to `grads` instead of overwriting them (no memset; every gradient
+ * write is an atomic add); each segment event then marks the segment's running sum as final.  0 = overwrite (default). */
+int nbc_train_set_accumulate(nbc_train_plan* plan, int on);
 int nbc_train_adam(float* params, const float* grads, float* adam_m, float* adam_v, int64_t n, float lr, float beta1,
                    float beta2, float eps, float weight_decay, int step, float grad_scale, void* stream);
 

@@ -115,6 +115,7 @@ SIGNATURES = {
     'nbc_train_set_capture': (c_int, [c_void_p, c_void_p, c_size_t]),
     'nbc_train_set_wgrad_impl': (c_int, [c_void_p, c_int]),
     'nbc_train_set_loss': (c_int, [c_void_p, c_int]),
+    'nbc_train_set_accumulate': (c_int, [c_void_p, c_int]),
     'nbc_train_adam': (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_i64, c_float, c_float, c_float, c_float, c_float,
                        c_int, c_float, c_void_p]),
 }

@@ -53,6 +53,7 @@ struct nbc_train_plan {
   void* prepared_ws = nullptr;
   int wgrad_impl = 0;   // 0 = tcgen05 (wgrad_tc.cu), 1 = mma.sync / CUDA-core cross-check kernels
   int loss_kind = 0;    // 0 = weighted CE, 1 = Lovasz-Softmax, 2 = CE / 4 + Lovasz
+  int accumulate = 0;   // 1: the step adds to `grads` (every gradient writer is an atomic / red add) instead of zeroing it
   size_t lov_off = 0, dfull2_off = 0, loss2_off = 0;
   // gradient-ready events, one per SEGMENT of the flat gradient buffer in the order the backward finishes them:
   // segment 0 = head conv + classifier, then the bottleneck blocks last to first, then the stem (created lazily)
@@ -390,7 +391,7 @@ extern "C" int nbc_train_forward_backward(nbc_train_plan* p, float* params, floa
   const int N = p->N, H = p->H, W = p->W;
   int rc = prepare(p, ws);
   if (rc) return rc;
-  NBC_CUDA(cudaMemsetAsync(grads, 0, p->n_params * sizeof(float), stream));
+  if (!p->accumulate) NBC_CUDA(cudaMemsetAsync(grads, 0, p->n_params * sizeof(float), stream));
   NBC_CUDA(cudaMemsetAsync(ws + p->zeros_off, 0, 2048 * 4, stream));
 
   // ---- weights of this step: bf16 copies for the forward and the data-gradient convolutions
@@ -532,6 +533,11 @@ extern "C" int nbc_train_set_wgrad_impl(nbc_train_plan* p, int impl) {
 extern "C" int nbc_train_set_loss(nbc_train_plan* p, int kind) {
   NBC_REQUIRE(p && kind >= 0 && kind <= 2, "nbc_train_set_loss: kind must be 0 (weighted CE), 1 (Lovasz) or 2 (mixed)");
   p->loss_kind = kind;
+  return 0;
+}
+extern "C" int nbc_train_set_accumulate(nbc_train_plan* p, int on) {
+  NBC_REQUIRE(p && (on == 0 || on == 1), "nbc_train_set_accumulate: on must be 0 (overwrite) or 1 (add)");
+  p->accumulate = on;
   return 0;
 }
 extern "C" int nbc_train_num_units(const nbc_train_plan* p) { return p ? (int)p->units.size() : 0; }

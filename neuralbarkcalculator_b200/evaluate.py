@@ -120,8 +120,42 @@ def evaluate_plan(plan, ds, indices, loss='lovasz', class_weights=None, chunk=8)
         host = {k: torch.cat([o[k] for o in outs]).cpu().numpy() for k in outs[0]}
     rows = [image_row(i, loss, host['loss_wce'][j], host['loss_lovasz'][j], host['cm_raw'][j], host['cm_rsz'][j],
                       host['counts'][j]) for j, i in enumerate(order)]
+    return summary(rows)
+
+
+def summary(rows):
+    """{'loss', 'miou', 'f1', 'rows'}: the means over ``rows`` in their order (the order fixes the float sums)."""
     return {'loss': float(np.mean([r['loss'] for r in rows])), 'miou': float(np.mean([r['miou'] for r in rows])),
             'f1': np.mean([r['f1'] for r in rows], axis=0), 'rows': rows}
+
+
+def width_order(ds, indices):
+    """``indices`` in the row order of ``evaluate_plan``: widths ascending, each width in the order given."""
+    return [i for _, part in _width_chunks(ds, [int(i) for i in indices], max(len(indices), 1)) for i in part]
+
+
+def evaluate_sharded(plan, ds, indices, loss='lovasz', class_weights=None, chunk=8):
+    """``evaluate_plan`` spread over the ranks of the torch.distributed process group: ``indices`` are put in
+    ``evaluate_plan``'s row order, each rank evaluates a contiguous shard of that order (``distributed.shard_bounds``;
+    a shard may be empty, the rank still joins the gather) and every rank gets all rows back.  Rows are per-image exact,
+    so every rank returns what ``evaluate_plan`` returns in one process for the same network, bit for bit.  Every rank
+    must call it with the same ``indices``; without a group of more than one process it is ``evaluate_plan``."""
+    import torch.distributed as dist
+    from .distributed import shard_bounds
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
+        return evaluate_plan(plan, ds, indices, loss, class_weights, chunk)
+    if loss not in LOSSES:      # checked on every rank before the shards part: a rank must not leave the gather
+        raise ValueError("loss must be 'weighted_ce', 'lovasz' or 'mixed'")
+    if len(indices) == 0:
+        raise RuntimeError('evaluate: no images')
+    if int(chunk) < 1:
+        raise ValueError('evaluate: chunk must be at least 1')
+    order = width_order(ds, indices)
+    start, end = shard_bounds(len(order), dist.get_rank(), dist.get_world_size())
+    mine = evaluate_plan(plan, ds, order[start:end], loss, class_weights, chunk)['rows'] if end > start else []
+    gathered = [None] * dist.get_world_size()
+    dist.all_gather_object(gathered, mine)
+    return summary([r for part in gathered for r in part])
 
 
 def evaluate(state_dict, ds, indices, loss='lovasz', class_weights=None, precision=DEFAULT_PRECISION, chunk=8):

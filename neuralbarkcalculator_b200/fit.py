@@ -2,7 +2,9 @@
 reference's ``__main__.py:199-291``, which runs it through Poutyne).
 
     python -m neuralbarkcalculator_b200.fit ROOT --init SD.pt|random [--out best_model.pt] [--epochs 30] [--crop 512]
-        [--batch 5] [--loss lovasz] [--lr 5e-4] [--weight-decay 2e-3] [--dropout 0.8] [--seed 0] [--device cuda:0]
+        [--batch 5] [--accumulate 1] [--loss lovasz] [--lr 5e-4] [--weight-decay 2e-3] [--dropout 0.8] [--seed 0]
+        [--device cuda:0]
+    torchrun --nproc_per_node W -m neuralbarkcalculator_b200.fit ROOT ...      (data parallel, one GPU per rank)
 
 ROOT holds ``samples/<wood>/*`` and ``duals/<wood>/*`` (processed images and their dual label images, any height up to
 ``--target``).  The dataset is loaded once onto the GPU; ``utils.get_splits`` makes the 80 / 10 / 10 split per wood type
@@ -18,8 +20,25 @@ The reference's values are used where SURVEY records them (Adam lr 5e-4, weight 
 batch 5, 30 epochs, Lovasz loss).  It does not record the parameters of its ``ReduceLROnPlateau`` and ``EarlyStopping``:
 the plateau rule takes torch's defaults (factor 0.1, patience 10), and early stopping waits 20 epochs, twice the plateau
 patience, so that the learning rate is lowered before training gives up.  Normalisation is predict's
-(``NeuralBarkCalculator.DEFAULT_MEAN / DEFAULT_STD``): the checkpoint carries none.  One GPU; ``--init random`` starts
-from torchvision's initialisation (ImageNet weights would need a download)."""
+(``NeuralBarkCalculator.DEFAULT_MEAN / DEFAULT_STD``): the checkpoint carries none.  ``--init random`` starts from
+torchvision's initialisation (ImageNet weights would need a download).
+
+Data parallel and gradient accumulation.  ``--batch`` is the micro-batch, the size the network step runs at; under
+``torchrun`` with W ranks (rank r on cuda:LOCAL_RANK, NCCL) and ``--accumulate K`` one optimizer step covers the global
+batch G = W * K * batch.  Every rank loads the whole folder and draws the same epoch batches of G and the same
+augmentation parameters of each (same seeds: no communication); micro-batch j is the slice [j * batch, (j + 1) * batch)
+of both, and rank r runs micro-batches r * K .. r * K + K - 1, accumulating their gradients, before one all-reduce and one
+Adam step on the mean.  Micro-batch j's dropout seed depends on j and the step only (``train.dropout_seed``), so a W-GPU
+run is the same training as a one-GPU run with ``--accumulate`` W * K, draw for draw, except for the BatchNorm running
+statistics: each rank updates its own once per micro-batch, and at the end of each epoch they are averaged over the
+ranks (one small all-reduce), where the one-GPU run updates one set once per micro-batch in sequence.  As in torch DDP
+without SyncBatchNorm, the BatchNorm batch statistics and the Lovasz sort see the micro-batch, not the global batch,
+and ``--lr`` is not rescaled with G.  W = 1 and K = 1 make exactly the draws and calls of a one-GPU run.  The epoch's
+training loss is the mean over all micro-batches of all ranks (one all-reduce per epoch).  Validation is sharded over
+the ranks (``evaluate.evaluate_sharded``) and gives every rank the figures of a one-GPU evaluation bit for bit, so the
+plateau and early-stopping decisions agree; rank 0 alone writes ``--log`` and ``--out``.  Every rank keeps the best
+state_dict in host memory and evaluates the test split from it, sharded.  On stdout, rank 0 reports each epoch's
+optimizer steps, training-loop and validation seconds, and every rank its dataset load time."""
 import argparse
 import math
 import os
@@ -97,54 +116,97 @@ def initial_state_dict(init, dropout):
     return torch.load(init, map_location='cpu')
 
 
+def rank_micro_batches(batches, rng, rank, accumulate, batch, n_sources, crop, target):
+    """This rank's share of each global batch of the epoch.  ``batches``: int64 [steps, G] sources from
+    ``utils.weighted_epoch_batches``; per row, the augmentation parameters of all G samples are drawn from ``rng``
+    (every rank makes the same draws), and the row's micro-batches j = rank * accumulate .. (rank + 1) * accumulate - 1
+    are yielded as [(j, params[j * batch:(j + 1) * batch])]."""
+    from . import augment
+    for row in batches:
+        params = augment.draw_params(rng, len(row), n_sources, crop, target, sources=row.numpy())
+        yield [(j, params[j * batch:(j + 1) * batch]) for j in range(rank * accumulate, (rank + 1) * accumulate)]
+
+
 def main(args):
     import torch
-    from . import augment, utils
-    from .evaluate import evaluate
+    from . import augment, distributed as ndist, utils
+    from .evaluate import evaluate_sharded, make_plan
     from .train import Trainer
+    rank, local_rank, world = ndist.env_world()
+    device = args.device
+    if world > 1:
+        import torch.distributed as dist
+        device = 'cuda:%d' % local_rank
+        torch.cuda.set_device(local_rank)
+        ndist.init_from_env('cuda')
+        ndist.bind_to_gpu_numa(local_rank)
     torch.manual_seed(args.seed)
     np.random.seed(args.seed)            # get_splits shuffles with numpy's global generator, as the reference
     target = (args.target, args.target)
-    ds = augment.load_dataset(args.root, args.device)
+    t0 = time.perf_counter()
+    ds = augment.load_dataset(args.root, device)       # every rank: any rank may be handed any source
+    print('fit: rank %d loaded %d images in %.3f s' % (rank, len(ds), time.perf_counter() - t0), flush=True)
     train_split, valid_split, test_split, train_weights = utils.get_splits(ds.split_items(), label_pixels=ds.label_pixels)
     if len(valid_split) == 0:
         raise RuntimeError('fit: the validation split is empty (a wood type needs at least 10 images for one)')
-    trainer = Trainer(initial_state_dict(args.init, args.dropout), args.batch, args.crop, args.crop, device=args.device,
+    trainer = Trainer(initial_state_dict(args.init, args.dropout), args.batch, args.crop, args.crop, device=device,
                       lr=args.lr, weight_decay=args.weight_decay, dropout=args.dropout, loss=args.loss, seed=args.seed)
     generator = torch.Generator().manual_seed(args.seed)
     rng = np.random.default_rng(args.seed)
     plateau = Plateau(args.lr, factor=args.plateau_factor, patience=args.plateau_patience)
     stopper = EarlyStopping(args.early_stop_patience)
-    with open(args.log, 'w') as f:
-        f.write('\t'.join(LOG_HEADER) + '\n')
-    best_miou = -math.inf
+    if rank == 0:
+        with open(args.log, 'w') as f:
+            f.write('\t'.join(LOG_HEADER) + '\n')
+    global_batch = world * args.accumulate * args.batch
+    best_miou, best_sd = -math.inf, None
     for epoch in range(1, args.epochs + 1):
         t0 = time.perf_counter()
         lr = trainer.lr
-        batches = utils.weighted_epoch_batches(train_split, train_weights, args.batch, generator=generator)
+        batches = utils.weighted_epoch_batches(train_split, train_weights, global_batch, generator=generator)
         if len(batches) == 0:
-            raise RuntimeError('fit: the training split gives no full batch of %d' % args.batch)
+            raise RuntimeError('fit: the training split gives no full global batch of %d' % global_batch)
         with torch.cuda.device(trainer.device):
             total = torch.zeros((), dtype=torch.float32, device=trainer.device)
-            for row in batches:
-                params = augment.draw_params(rng, args.batch, len(ds), args.crop, target, sources=row.numpy())
-                images, classes = augment.augment_ragged(ds, params, args.crop, target)
-                total += trainer.step(images, classes)
-            train_loss = float(total) / len(batches)
-        val = trainer.evaluate(ds, valid_split)
-        _log(args.log, [epoch, repr(lr), repr(train_loss), repr(val['loss']), repr(val['miou'])]
-             + [repr(float(v)) for v in val['f1']] + ['%.3f' % (time.perf_counter() - t0)])
+            for micro in rank_micro_batches(batches, rng, rank, args.accumulate, args.batch, len(ds), args.crop, target):
+                for i, (j, params) in enumerate(micro):
+                    images, classes = augment.augment_ragged(ds, params, args.crop, target)
+                    total += trainer.forward_backward(images, classes, seed=trainer.dropout_seed(j), accumulate=i > 0)
+                trainer.optimizer_step()
+            if world > 1:
+                dist.all_reduce(total)
+                dist.all_reduce(trainer.stats)          # BatchNorm running statistics: the mean over the ranks
+                trainer.stats.div_(world)
+            train_loss = float(total) / (len(batches) * world * args.accumulate)
+        t_train = time.perf_counter() - t0
+        with torch.cuda.device(trainer.device):
+            sd = trainer.state_dict()
+            val = evaluate_sharded(make_plan(sd, trainer.device), ds, valid_split, loss=args.loss,
+                                   class_weights=trainer.class_weights)
+        if rank == 0:
+            _log(args.log, [epoch, repr(lr), repr(train_loss), repr(val['loss']), repr(val['miou'])]
+                 + [repr(float(v)) for v in val['f1']] + ['%.3f' % (time.perf_counter() - t0)])
+            print('fit: epoch %d: %d steps of %d samples, training %.3f s, validation %.3f s'
+                  % (epoch, len(batches), global_batch, t_train, time.perf_counter() - t0 - t_train), flush=True)
         if val['miou'] > best_miou:
             best_miou = val['miou']
-            torch.save({k: v.cpu() for k, v in trainer.state_dict().items()}, args.out)
+            best_sd = {k: v.cpu() for k, v in sd.items()}
+            if rank == 0:
+                torch.save(best_sd, args.out)
+        del sd
         trainer.lr = plateau.step(val['loss'])
         if stopper.step(val['loss']):
             break
     if len(test_split):
         t0 = time.perf_counter()
-        test = evaluate(torch.load(args.out, map_location='cpu'), ds, test_split, loss=args.loss)
-        _log(args.log, ['test', '', '', repr(test['loss']), repr(test['miou'])] + [repr(float(v)) for v in test['f1']]
-             + ['%.3f' % (time.perf_counter() - t0)])
+        with torch.cuda.device(trainer.device):
+            test = evaluate_sharded(make_plan(best_sd, trainer.device), ds, test_split, loss=args.loss)
+        if rank == 0:
+            _log(args.log, ['test', '', '', repr(test['loss']), repr(test['miou'])] + [repr(float(v)) for v in test['f1']]
+                 + ['%.3f' % (time.perf_counter() - t0)])
+    if world > 1:
+        dist.barrier()
+        dist.destroy_process_group()
     return best_miou
 
 
@@ -156,7 +218,9 @@ def parse_args(argv=None):
     parser.add_argument('--log', default='log.tsv', help='one tab-separated row per epoch, then the test row')
     parser.add_argument('--epochs', type=int, default=30)
     parser.add_argument('--crop', type=int, default=512)
-    parser.add_argument('--batch', type=int, default=5)
+    parser.add_argument('--batch', type=int, default=5, help='micro-batch: the size one network step runs at')
+    parser.add_argument('--accumulate', type=int, default=1,
+                        help='micro-batches per rank summed into one optimizer step (global batch = ranks x this x --batch)')
     parser.add_argument('--target', type=int, default=1024, help='pad_resize size of every image')
     parser.add_argument('--loss', default='lovasz', choices=['lovasz', 'weighted_ce', 'mixed'])
     parser.add_argument('--lr', type=float, default=5e-4)
@@ -166,12 +230,14 @@ def parse_args(argv=None):
     parser.add_argument('--plateau-patience', type=int, default=10)
     parser.add_argument('--early-stop-patience', type=int, default=20)
     parser.add_argument('--seed', type=int, default=0)
-    parser.add_argument('--device', default='cuda:0', help='CUDA device (cuda, cuda:N)')
+    parser.add_argument('--device', default='cuda:0', help='CUDA device (cuda, cuda:N); under torchrun cuda:LOCAL_RANK')
     args = parser.parse_args(argv)
     if not args.device.startswith('cuda'):
         parser.error('--device %s: only CUDA devices are supported (no CPU path)' % args.device)
     if args.epochs < 1 or args.batch < 1 or args.crop < 1 or args.crop > args.target:
         parser.error('--epochs and --batch must be positive and --crop within [1, --target]')
+    if args.accumulate < 1:
+        parser.error('--accumulate must be at least 1')
     return args
 
 

@@ -13,7 +13,9 @@ the bottleneck blocks last to first, then the stem) is final, consecutive segmen
 Measured on 8 B200 (profiles/r02c_bench_train_g8*.json): 1 336 img/s with the single all-reduce (97.4 % of 8 x one GPU),
 1 318 with 7 overlapped buckets -- an NCCL kernel that starts in the middle of the backward takes SMs away from the
 persistent convolution kernels, which need all 148, and that costs more than the exposed half millisecond; hence the
-default.  No torch autograd, no torch ops on the data path."""
+default.  Gradient accumulation: ``forward_backward(..., accumulate=True)`` adds a micro-batch's gradients to the
+buffer, so a global batch of ``world * k`` micro-batches costs k backward passes per rank and ONE exchange; Adam then
+applies 1 / (world * k).  No torch autograd, no torch ops on the data path."""
 import ctypes as C
 import os
 
@@ -33,6 +35,13 @@ def gradient_segments(lib, handle):
         _lib.check(lib.nbc_train_segment(h, i, C.byref(off), C.byref(cnt)), 'nbc_train_segment')
         out.append((off.value, cnt.value))
     return out
+
+
+def dropout_seed(base_seed, micro_batch, step):
+    """Dropout seed of global micro-batch ``micro_batch`` of optimizer step ``step``: micro-batch i of rank r, with k
+    micro-batches per rank, is j = r * k + i, so a global micro-batch draws the same mask whatever (world, k) runs it
+    (with k = 1, j is the rank)."""
+    return (int(base_seed) << 40) + (int(micro_batch) << 28) + int(step)
 
 
 def merge_segments(segments, min_bytes):
@@ -63,6 +72,8 @@ class Trainer:
         self.std3 = (C.c_float * 3)(*std)
         self.step_count = 0
         self.base_seed = int(seed)
+        self.micro_batches = 0          # forward_backward calls summed in self.grads since the last optimizer_step
+        self._accumulating = False      # the plan's nbc_train_set_accumulate state
         env = os.environ.get('NBC_TRAIN_BUCKETS')
         if env is not None and env != '':      # 0: single all-reduce; 1: 16 MB buckets; any other number: that many MB
             bucket_mb = 0.0 if env == '0' else (16.0 if env == '1' else float(env))
@@ -180,9 +191,11 @@ class Trainer:
                             precision=DEFAULT_PRECISION if precision is None else precision, chunk=chunk)
 
     # -- the step ------------------------------------------------------------------------------------------------------
-    def forward_backward(self, images, targets, seed=0, dropout=None, update_stats=True):
+    def forward_backward(self, images, targets, seed=0, dropout=None, update_stats=True, accumulate=False):
         """images: u8 NHWC [N,H,W,3] (normalised inside) or f32 NCHW [N,3,H,W]; targets: u8 [N,H,W].
-        Returns the loss (0-dim CUDA tensor); gradients are left in ``self.grads``."""
+        Returns the loss (0-dim CUDA tensor); gradients are left in ``self.grads``: overwritten, or with ``accumulate``
+        added to what the buffer holds (the first micro-batch of a step overwrites, the next ones accumulate; the next
+        ``optimizer_step`` divides by the number of micro-batches summed)."""
         p = self.dropout if dropout is None else dropout
         if images.dtype == torch.uint8:
             kind, shape = 0, (self.N, self.H, self.W, 3)
@@ -195,7 +208,11 @@ class Trainer:
         if not targets.is_cuda or targets.dtype != torch.uint8 or tuple(targets.shape) != (self.N, self.H, self.W):
             raise RuntimeError('targets must be a CUDA u8 tensor [N,H,W]')
         images, targets = images.contiguous(), targets.contiguous()
+        accumulate = bool(accumulate)
         with torch.cuda.device(self.device):
+            if accumulate != self._accumulating:
+                _lib.check(self.lib.nbc_train_set_accumulate(C.c_void_p(self.handle), int(accumulate)), 'nbc_train_set_accumulate')
+                self._accumulating = accumulate
             off = (-self.ws.data_ptr()) % 1024
             _lib.check(self.lib.nbc_train_forward_backward(
                 C.c_void_p(self.handle), C.c_void_p(self.params.data_ptr()),
@@ -204,6 +221,7 @@ class Trainer:
                 C.c_void_p(self.class_weights.data_ptr()), C.c_float(p), C.c_uint64(seed), C.c_void_p(self.loss.data_ptr()),
                 C.c_void_p(self.ws.data_ptr() + off), C.c_size_t(self.ws.numel() - off),
                 C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), 'nbc_train_forward_backward')
+        self.micro_batches = self.micro_batches + 1 if accumulate else 1
         if update_stats:
             for k in self.num_batches_tracked:
                 self.num_batches_tracked[k] += 1
@@ -218,7 +236,7 @@ class Trainer:
         return self._buckets
 
     def all_reduce_gradients(self):
-        """SUM the gradients over the data-parallel group (Adam applies 1/world).  Bucketed: every bucket's all-reduce is
+        """SUM the gradients over the data-parallel group (Adam applies 1 / (world * micro-batches)).  Bucketed: every bucket's all-reduce is
         enqueued on a side stream behind the event the backward records when that part of the buffer is final, so the
         exchange of the last layers runs under the backward of the first ones.  Returns the number of collectives."""
         import torch.distributed as dist
@@ -242,25 +260,29 @@ class Trainer:
         return len(works)
 
     def optimizer_step(self):
-        """All-reduce the gradients over the data-parallel group (if any), then one fused Adam pass."""
+        """All-reduce the gradients over the data-parallel group (if any), then one fused Adam pass on their mean over
+        the world's micro-batches since the last step."""
         import torch.distributed as dist
         world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
+        micro = max(self.micro_batches, 1)
         self.all_reduce_gradients()
         self.step_count += 1
+        self.micro_batches = 0
         with torch.cuda.device(self.device):
             _lib.check(self.lib.nbc_train_adam(C.c_void_p(self.params.data_ptr()), C.c_void_p(self.grads.data_ptr()),
                                                C.c_void_p(self.adam_m.data_ptr()), C.c_void_p(self.adam_v.data_ptr()),
                                                self.params.numel(), C.c_float(self.lr), C.c_float(self.betas[0]),
                                                C.c_float(self.betas[1]), C.c_float(self.eps), C.c_float(self.wd), self.step_count,
-                                               C.c_float(1.0 / world),
+                                               C.c_float(1.0 / (world * micro)),
                                                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), 'nbc_train_adam')
 
-    def dropout_seed(self):
-        """A different dropout mask per step, per data-parallel rank and per run seed (every rank drawing the same mask
-        would correlate the replicas' gradients)."""
-        import torch.distributed as dist
-        rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
-        return (self.base_seed << 40) + (rank << 28) + self.step_count
+    def dropout_seed(self, micro_batch=None):
+        """A different dropout mask per step, per global micro-batch and per run seed (every rank drawing the same mask
+        would correlate the replicas' gradients).  ``micro_batch`` defaults to the rank (one micro-batch per rank)."""
+        if micro_batch is None:
+            import torch.distributed as dist
+            micro_batch = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
+        return dropout_seed(self.base_seed, micro_batch, self.step_count)
 
     def step(self, images, targets, seed=None):
         loss = self.forward_backward(images, targets, seed=self.dropout_seed() if seed is None else seed)
