@@ -355,6 +355,19 @@ int nbc_train_set_loss(nbc_train_plan* plan, int kind);
 /* 1: nbc_train_forward_backward adds its gradients to `grads` instead of overwriting them (no memset; every gradient
  * write is an atomic add); each segment event then marks the segment's running sum as final.  0 = overwrite (default). */
 int nbc_train_set_accumulate(nbc_train_plan* plan, int on);
+/* Fine-tuning with a frozen backbone.  stages: 0 = nothing frozen (default), 1 = the stem (conv1 + bn1), 2..5 = the
+ * stem through layer1..layer4; any other value is refused.  A frozen unit is torchvision's FrozenBatchNorm2d after its
+ * conv: each nbc_train_forward_backward folds its BatchNorm (gamma, beta from `params`, running mean / var from `stats`,
+ * eps 1e-5) into bf16 weights and an f32 bias and runs it as one convolution with bias, residual and ReLU in the
+ * epilogue (so `stats` may not be NULL while stages > 0).  Its running statistics are never written, and neither is its
+ * part of `grads`: the memset and every gradient writer cover only the trainable suffix, and the backward ends at the
+ * first trainable block (whose conv1 and downsample, or the head conv at stages = 5, compute no data gradient).  The
+ * gradient segments of frozen blocks and of a frozen stem report count 0, and nbc_train_wait_segment on them returns at
+ * once.  nbc_train_debug_offset gives only y (what 1) for a frozen unit; z, dy and dz are refused (-1).
+ * nbc_train_trainable_offsets: the first trainable float of the params / grads / Adam buffers and of `stats` (units are
+ * laid out in order, so the trainable part of each buffer is a suffix); both 0 when nothing is frozen. */
+int nbc_train_set_frozen(nbc_train_plan* plan, int stages);
+int nbc_train_trainable_offsets(const nbc_train_plan* plan, int64_t* param_off, int64_t* stats_off);
 int nbc_train_adam(float* params, const float* grads, float* adam_m, float* adam_v, int64_t n, float lr, float beta1,
                    float beta2, float eps, float weight_decay, int step, float grad_scale, void* stream);
 

@@ -116,6 +116,8 @@ SIGNATURES = {
     'nbc_train_set_wgrad_impl': (c_int, [c_void_p, c_int]),
     'nbc_train_set_loss': (c_int, [c_void_p, c_int]),
     'nbc_train_set_accumulate': (c_int, [c_void_p, c_int]),
+    'nbc_train_set_frozen': (c_int, [c_void_p, c_int]),
+    'nbc_train_trainable_offsets': (c_int, [c_void_p, c_void_p, c_void_p]),
     'nbc_train_adam': (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_i64, c_float, c_float, c_float, c_float, c_float,
                        c_int, c_float, c_void_p]),
 }

@@ -27,6 +27,7 @@ struct Unit {
   size_t dgrad_out_off, dgrad_res_off;
   size_t cap_off;              // bytes, in the capture buffer: dy, then dz (each N*Ho*Wo*Cout bf16)
   bool dgrad_has_res = false, need_dgrad = true;
+  bool frozen = false;         // nbc_train_set_frozen: eval-mode BN folded into the conv, no backward
   ConvTcPrepared fwd, dgrad;
 };
 
@@ -54,6 +55,9 @@ struct nbc_train_plan {
   int wgrad_impl = 0;   // 0 = tcgen05 (wgrad_tc.cu), 1 = mma.sync / CUDA-core cross-check kernels
   int loss_kind = 0;    // 0 = weighted CE, 1 = Lovasz-Softmax, 2 = CE / 4 + Lovasz
   int accumulate = 0;   // 1: the step adds to `grads` (every gradient writer is an atomic / red add) instead of zeroing it
+  // nbc_train_set_frozen: units [0, first_unit) and blocks [0, first_block) are frozen; both 0 = nothing frozen
+  int frozen = 0, first_unit = 0, first_block = 0;
+  size_t fold_off = 0;  // bytes, workspace: the frozen stem's folded f32 weights [64][7][7][3] before the w224 pack
   size_t lov_off = 0, dfull2_off = 0, loss2_off = 0;
   // gradient-ready events, one per SEGMENT of the flat gradient buffer in the order the backward finishes them:
   // segment 0 = head conv + classifier, then the bottleneck blocks last to first, then the stem (created lazily)
@@ -176,6 +180,7 @@ extern "C" nbc_train_plan* nbc_train_create(int N, int H, int W) {
   p->lov_off = off, off += al(nbc_lovasz_workspace_bytes(N, H, W));
   p->dfull2_off = off, off += al((size_t)N * 3 * H * W * 4);
   p->loss2_off = off, off += al(16);
+  p->fold_off = off, off += al(64 * 147 * 4);
   p->ws_bytes = off;
   p->capture_bytes = cap;
 
@@ -211,6 +216,14 @@ extern "C" nbc_train_plan* nbc_train_create(int N, int H, int W) {
 extern "C" void nbc_train_destroy(nbc_train_plan* p) { delete p; }
 
 // ---- gradient segments (for overlapping the data-parallel all-reduce with the backward) ------------------------------
+// segment i belongs to frozen units (nbc_train_set_frozen): the backward neither writes it nor records its event
+static bool segment_frozen(const nbc_train_plan* p, int i) {
+  const int nb = (int)p->blocks.size();
+  if (i == 0) return false;
+  if (i <= nb) return nb - i < p->first_block;
+  return p->frozen > 0;
+}
+
 extern "C" int nbc_train_num_segments(const nbc_train_plan* p) { return p ? (int)p->blocks.size() + 2 : 0; }
 
 extern "C" int nbc_train_segment(const nbc_train_plan* p, int i, int64_t* offset, int64_t* count) {
@@ -226,6 +239,7 @@ extern "C" int nbc_train_segment(const nbc_train_plan* p, int i, int64_t* offset
   } else {
     lo = 0, hi = p->units[p->blocks[0].c1].w_off;      // the stem
   }
+  if (segment_frozen(p, i)) hi = lo;
   *offset = (int64_t)lo, *count = (int64_t)(hi - lo);
   return 0;
 }
@@ -241,6 +255,7 @@ static int record_segment(nbc_train_plan* p, int i, cudaStream_t stream) {
 
 extern "C" int nbc_train_wait_segment(nbc_train_plan* p, int i, void* stream) {
   NBC_REQUIRE(p && i >= 0 && i < (int)p->blocks.size() + 2, "nbc_train_wait_segment: bad argument");
+  if (segment_frozen(p, i)) return 0;
   NBC_REQUIRE(!p->seg_events.empty(), "nbc_train_wait_segment: no backward has been enqueued yet");
   NBC_CUDA(cudaStreamWaitEvent(reinterpret_cast<cudaStream_t>(stream), p->seg_events[i], 0));
   return 0;
@@ -293,16 +308,39 @@ extern "C" int nbc_train_exchange(nbc_train_plan* p, void* const* tensors, int n
 namespace nbc {
 
 // tensor maps depend on the workspace address: (re)build the conv launches when it changes
+// the folded bias of a frozen unit lives in its (otherwise unused) BatchNorm scratch
+static float* fold_bias(char* ws, const Unit& u) { return reinterpret_cast<float*>(ws + u.st_off); }
+
+// frozen unit: y = act(conv(x, folded w) + folded bias (+ residual)) in one launch, straight into y
+static int prepare_frozen(nbc_train_plan* p, char* ws, Unit& u, const void* residual) {
+  ConvGeom g{p->N, u.Hin, u.Win, u.Cin, u.Cout, u.k, u.k, u.stride, u.pad, u.dil, u.relu, 0};
+  return conv_tc_prepare(g, ws + u.x_off, ws + u.wf_off, fold_bias(ws, u), residual, ws + u.y_off, &u.fwd);
+}
+
 static int prepare(nbc_train_plan* p, char* ws) {
   if (p->prepared_ws == ws) return 0;
   const float* zeros = reinterpret_cast<const float*>(ws + p->zeros_off);
   const int N = p->N;
   Unit& s = p->units[0];
-  int rc = conv_tc_prepare_stem(N, s.Ho, s.Wo, 2 * s.Ho + 5, 2 * s.Wo + 6, ws + p->padded_off, ws + s.wf_off, zeros, ws + s.z_off,
-                                &s.fwd, nullptr, 0, /*relu=*/0);   // BN sits between the conv and the ReLU here
+  int rc = s.frozen ? conv_tc_prepare_stem(N, s.Ho, s.Wo, 2 * s.Ho + 5, 2 * s.Wo + 6, ws + p->padded_off, ws + s.wf_off,
+                                           fold_bias(ws, s), ws + s.y_off, &s.fwd, nullptr, 0, /*relu=*/1)
+                    : conv_tc_prepare_stem(N, s.Ho, s.Wo, 2 * s.Ho + 5, 2 * s.Wo + 6, ws + p->padded_off, ws + s.wf_off, zeros,
+                                           ws + s.z_off, &s.fwd, nullptr, 0, /*relu=*/0);   // BN sits between the conv and the ReLU
   if (rc) return rc;
+  for (int b = 0; b < p->first_block; ++b) {
+    const TBlock& B = p->blocks[b];
+    const void* skip = ws + p->units[B.c1].x_off;
+    if ((rc = prepare_frozen(p, ws, p->units[B.c1], nullptr))) return rc;
+    if ((rc = prepare_frozen(p, ws, p->units[B.c2], nullptr))) return rc;
+    if (B.ds >= 0) {
+      if ((rc = prepare_frozen(p, ws, p->units[B.ds], nullptr))) return rc;
+      skip = ws + p->units[B.ds].y_off;
+    }
+    if ((rc = prepare_frozen(p, ws, p->units[B.c3], skip))) return rc;
+  }
   for (size_t i = 1; i < p->units.size(); ++i) {
     Unit& u = p->units[i];
+    if (u.frozen) continue;
     ConvGeom g{N, u.Hin, u.Win, u.Cin, u.Cout, u.k, u.k, u.stride, u.pad, u.dil, 0, 0};
     rc = conv_tc_prepare(g, ws + u.x_off, ws + u.wf_off, zeros, nullptr, ws + u.z_off, &u.fwd);
     if (rc) return rc;
@@ -336,7 +374,7 @@ struct Ctx {
 
 static int unit_forward(const Ctx& c, Unit& u, const void* residual, int relu) {
   int rc = conv_tc_run(&u.fwd, c.stream);
-  if (rc) return rc;
+  if (rc || u.frozen) return rc;   // a frozen unit's launch already wrote y (bias, residual and ReLU in its epilogue)
   const int64_t M = (int64_t)c.p->N * u.Ho * u.Wo;
   return bn_forward_train(c.ws + u.z_off, M, u.Cout, c.params + u.g_off, c.params + u.b_off, 1e-5f, 0.1f,
                           c.stats ? c.stats + u.rs_off : nullptr, c.stats ? c.stats + u.rs_off + u.Cout : nullptr, c.st(u, 0),
@@ -382,6 +420,7 @@ extern "C" int nbc_train_forward_backward(nbc_train_plan* p, float* params, floa
   NBC_REQUIRE(p && params && grads && input && target && weights3 && loss && workspace, "nbc_train_forward_backward: null pointer");
   NBC_REQUIRE(dropout_p >= 0.f && dropout_p < 1.f, "nbc_train_forward_backward: dropout_p must be in [0,1)");
   NBC_REQUIRE(reinterpret_cast<uintptr_t>(workspace) % 1024 == 0, "nbc_train_forward_backward: workspace must be 1024-byte aligned");
+  NBC_REQUIRE(stats || p->frozen == 0, "nbc_train_forward_backward: frozen stages need `stats` (their running statistics)");
   if (workspace_bytes < p->ws_bytes) {
     set_error("nbc_train_forward_backward: workspace %zu < %zu", workspace_bytes, p->ws_bytes);
     return NBC_ERR_WORKSPACE;
@@ -391,12 +430,22 @@ extern "C" int nbc_train_forward_backward(nbc_train_plan* p, float* params, floa
   const int N = p->N, H = p->H, W = p->W;
   int rc = prepare(p, ws);
   if (rc) return rc;
-  if (!p->accumulate) NBC_CUDA(cudaMemsetAsync(grads, 0, p->n_params * sizeof(float), stream));
+  const size_t g0 = p->units[p->first_unit].w_off;   // the frozen prefix of `grads` is never written
+  if (!p->accumulate) NBC_CUDA(cudaMemsetAsync(grads + g0, 0, (p->n_params - g0) * sizeof(float), stream));
   NBC_CUDA(cudaMemsetAsync(ws + p->zeros_off, 0, 2048 * 4, stream));
 
   // ---- weights of this step: bf16 copies for the forward and the data-gradient convolutions
   for (Unit& u : p->units) {
-    if (u.Cin == 3) {
+    if (u.frozen) {
+      // eval-mode BatchNorm folded into the conv; the flat [Cout][kh][kw][Cin] row of each output channel is scaled
+      // as a whole (fold_pack with Cin = kh = 1, kw = k*k*Cin), so the packed layout is the trainable forward's
+      const float* rs = stats + u.rs_off;
+      const int row = u.k * u.k * u.Cin;
+      float* f32 = reinterpret_cast<float*>(ws + p->fold_off);
+      rc = fold_pack(params + u.w_off, params + u.g_off, params + u.b_off, rs, rs + u.Cout, nullptr, 1e-5f, u.Cout, 1, 1, row, 1,
+                     u.Cin == 3 ? nullptr : ws + u.wf_off, u.Cin == 3 ? f32 : nullptr, fold_bias(ws, u), stream);
+      if (!rc && u.Cin == 3) rc = nbc_stem_pack_weights(f32, 0, ws + u.wf_off, stream);
+    } else if (u.Cin == 3) {
       rc = nbc_stem_pack_weights(params + u.w_off, 0, ws + u.wf_off, stream);
     } else {
       rc = cast_pack(params + u.w_off, (int64_t)u.Cout * u.k * u.k * u.Cin, ws + u.wf_off, stream);
@@ -411,7 +460,8 @@ extern "C" int nbc_train_forward_backward(nbc_train_plan* p, float* params, floa
   if (rc) return rc;
   rc = unit_forward(c, stem, nullptr, 1);
   if (rc) return rc;
-  rc = maxpool_forward_idx(ws + stem.y_off, N, p->H2, p->W2, 64, ws + p->pool_off, ws + p->pidx_off, stream);
+  rc = stem.frozen ? maxpool_ragged(ws + stem.y_off, N, p->H2, p->W2, 64, ws + p->pool_off, nullptr, stream)
+                   : maxpool_forward_idx(ws + stem.y_off, N, p->H2, p->W2, 64, ws + p->pool_off, ws + p->pidx_off, stream);
   if (rc) return rc;
   for (TBlock& B : p->blocks) {
     Unit &u1 = p->units[B.c1], &u2 = p->units[B.c2], &u3 = p->units[B.c3];
@@ -470,7 +520,7 @@ extern "C" int nbc_train_forward_backward(nbc_train_plan* p, float* params, floa
   if ((rc = unit_backward(c, head, ws + p->d2_off, 1, nullptr))) return rc;
   if ((rc = record_segment(p, 0, stream))) return rc;
   const int nb = (int)p->blocks.size();
-  for (int b = nb - 1; b >= 0; --b) {
+  for (int b = nb - 1; b >= p->first_block; --b) {   // the backward ends at the first trainable block
     TBlock& B = p->blocks[b];
     Unit &u1 = p->units[B.c1], &u2 = p->units[B.c2], &u3 = p->units[B.c3];
     // y3 = relu(bn3(z3) + skip): masked gradient g3 feeds both the main path and the skip path (kept in gskip)
@@ -484,6 +534,7 @@ extern "C" int nbc_train_forward_backward(nbc_train_plan* p, float* params, floa
     if ((rc = unit_backward(c, u1, ws + p->d1_off, 1, nullptr))) return rc;
     if ((rc = record_segment(p, nb - b, stream))) return rc;
   }
+  if (p->frozen > 0) return 0;
   // maxpool and stem
   const size_t g_pool = p->blocks[0].gout_off;
   if ((rc = maxpool_backward(ws + g_pool, ws + p->pidx_off, N, p->H2, p->W2, 64, ws + p->gskip_off, stream))) return rc;
@@ -501,6 +552,7 @@ extern "C" int64_t nbc_train_debug_offset(const nbc_train_plan* p, int what, int
   if (what == 0 || what == 1 || what == 6 || what == 7) {
     if (index < 0 || index >= (int)p->units.size()) return -1;
     const Unit& u = p->units[index];
+    if (u.frozen && what != 1) return -1;   // a frozen unit has only its y
     dims_out[0] = p->N, dims_out[1] = u.Ho, dims_out[2] = u.Wo, dims_out[3] = u.Cout;
     if (what >= 6) return (int64_t)(u.cap_off + (what == 7 ? al((size_t)p->N * u.Ho * u.Wo * u.Cout * 2) : 0));
     return (int64_t)(what == 0 ? u.z_off : u.y_off);
@@ -538,6 +590,35 @@ extern "C" int nbc_train_set_loss(nbc_train_plan* p, int kind) {
 extern "C" int nbc_train_set_accumulate(nbc_train_plan* p, int on) {
   NBC_REQUIRE(p && (on == 0 || on == 1), "nbc_train_set_accumulate: on must be 0 (overwrite) or 1 (add)");
   p->accumulate = on;
+  return 0;
+}
+extern "C" int nbc_train_set_frozen(nbc_train_plan* p, int stages) {
+  NBC_REQUIRE(p, "nbc_train_set_frozen: null plan");
+  if (stages < 0 || stages > 5) {
+    set_error("nbc_train_set_frozen: stages must be 0 (none), 1 (stem) or 2..5 (stem through layer1..layer4), got %d", stages);
+    return NBC_ERR_INVALID;
+  }
+  const int first_block[6] = {0, 0, 3, 7, 13, 16};   // layers of 3, 4, 6 and 3 bottlenecks
+  p->frozen = stages, p->first_block = first_block[stages];
+  p->first_unit = stages == 0 ? 0 : (stages == 5 ? p->head_unit : p->blocks[p->first_block].c1);
+  for (size_t i = 0; i < p->units.size(); ++i) {
+    p->units[i].frozen = (int)i < p->first_unit;
+    p->units[i].need_dgrad = i > 0 && (int)i >= p->first_unit;
+  }
+  // the first trainable unit(s) read a frozen activation: no data gradient is wanted there
+  if (stages > 0 && stages < 5) {
+    p->units[p->blocks[p->first_block].c1].need_dgrad = false;
+    p->units[p->blocks[p->first_block].ds].need_dgrad = false;
+  } else if (stages == 5) {
+    p->units[p->head_unit].need_dgrad = false;
+  }
+  p->prepared_ws = nullptr;   // the launches change
+  return 0;
+}
+extern "C" int nbc_train_trainable_offsets(const nbc_train_plan* p, int64_t* param_off, int64_t* stats_off) {
+  NBC_REQUIRE(p && param_off && stats_off, "nbc_train_trainable_offsets: null pointer");
+  *param_off = (int64_t)p->units[p->first_unit].w_off;
+  *stats_off = (int64_t)p->units[p->first_unit].rs_off;
   return 0;
 }
 extern "C" int nbc_train_num_units(const nbc_train_plan* p) { return p ? (int)p->units.size() : 0; }

@@ -2,8 +2,8 @@
 reference's ``__main__.py:199-291``, which runs it through Poutyne).
 
     python -m neuralbarkcalculator_b200.fit ROOT --init SD.pt|random [--out best_model.pt] [--epochs 30] [--crop 512]
-        [--batch 5] [--accumulate 1] [--loss lovasz] [--lr 5e-4] [--weight-decay 2e-3] [--dropout 0.8] [--seed 0]
-        [--device cuda:0]
+        [--batch 5] [--accumulate 1] [--freeze none] [--loss lovasz] [--lr 5e-4] [--weight-decay 2e-3] [--dropout 0.8]
+        [--seed 0] [--device cuda:0]
     torchrun --nproc_per_node W -m neuralbarkcalculator_b200.fit ROOT ...      (data parallel, one GPU per rank)
 
 ROOT holds ``samples/<wood>/*`` and ``duals/<wood>/*`` (processed images and their dual label images, any height up to
@@ -38,13 +38,23 @@ training loss is the mean over all micro-batches of all ranks (one all-reduce pe
 the ranks (``evaluate.evaluate_sharded``) and gives every rank the figures of a one-GPU evaluation bit for bit, so the
 plateau and early-stopping decisions agree; rank 0 alone writes ``--log`` and ``--out``.  Every rank keeps the best
 state_dict in host memory and evaluates the test split from it, sharded.  On stdout, rank 0 reports each epoch's
-optimizer steps, training-loop and validation seconds, and every rank its dataset load time."""
+optimizer steps, training-loop and validation seconds, and every rank its dataset load time.
+
+Fine-tuning a checkpoint.  ``--freeze stem|layer1|layer2|layer3|layer4`` freezes the backbone from the stem through
+that stage (``--init`` must then be a checkpoint, not ``random``).  The frozen units run as eval-mode BatchNorm with
+the checkpoint's running statistics (torchvision's FrozenBatchNorm2d, with ``requires_grad_(False)`` on their weights):
+their weights, running statistics and ``num_batches_tracked`` stay exactly as loaded, Adam and its weight decay never
+touch them, the backward stops at the first trainable block, and the epoch-end average of the running statistics over
+the ranks covers only the trainable units.  Dropout, the loss and the sampling are unchanged; the checkpoint is the same
+326-key state_dict.  Rank 0 prints the number of trainable parameters."""
 import argparse
 import math
 import os
 import time
 
 import numpy as np
+
+from .train import FREEZE
 
 
 class Plateau:
@@ -116,6 +126,15 @@ def initial_state_dict(init, dropout):
     return torch.load(init, map_location='cpu')
 
 
+def average_running_stats(stats, stats_off, world):
+    """BatchNorm running statistics averaged over the ranks, in place, for the trainable units only (``stats_off`` on):
+    a mean of identical values is not always exact ((x + x + x) / 3), and frozen statistics must stay bit-identical."""
+    import torch.distributed as dist
+    trainable = stats[stats_off:]
+    dist.all_reduce(trainable)
+    trainable.div_(world)
+
+
 def rank_micro_batches(batches, rng, rank, accumulate, batch, n_sources, crop, target):
     """This rank's share of each global batch of the epoch.  ``batches``: int64 [steps, G] sources from
     ``utils.weighted_epoch_batches``; per row, the augmentation parameters of all G samples are drawn from ``rng``
@@ -150,7 +169,11 @@ def main(args):
     if len(valid_split) == 0:
         raise RuntimeError('fit: the validation split is empty (a wood type needs at least 10 images for one)')
     trainer = Trainer(initial_state_dict(args.init, args.dropout), args.batch, args.crop, args.crop, device=device,
-                      lr=args.lr, weight_decay=args.weight_decay, dropout=args.dropout, loss=args.loss, seed=args.seed)
+                      lr=args.lr, weight_decay=args.weight_decay, dropout=args.dropout, loss=args.loss, seed=args.seed,
+                      freeze=args.freeze)
+    if rank == 0:
+        print('fit: --freeze %s: %d of %d parameters trainable' % (
+            args.freeze, trainer.params.numel() - trainer.param_off, trainer.params.numel()), flush=True)
     generator = torch.Generator().manual_seed(args.seed)
     rng = np.random.default_rng(args.seed)
     plateau = Plateau(args.lr, factor=args.plateau_factor, patience=args.plateau_patience)
@@ -175,8 +198,7 @@ def main(args):
                 trainer.optimizer_step()
             if world > 1:
                 dist.all_reduce(total)
-                dist.all_reduce(trainer.stats)          # BatchNorm running statistics: the mean over the ranks
-                trainer.stats.div_(world)
+                average_running_stats(trainer.stats, trainer.stats_off, world)
             train_loss = float(total) / (len(batches) * world * args.accumulate)
         t_train = time.perf_counter() - t0
         with torch.cuda.device(trainer.device):
@@ -221,6 +243,8 @@ def parse_args(argv=None):
     parser.add_argument('--batch', type=int, default=5, help='micro-batch: the size one network step runs at')
     parser.add_argument('--accumulate', type=int, default=1,
                         help='micro-batches per rank summed into one optimizer step (global batch = ranks x this x --batch)')
+    parser.add_argument('--freeze', default='none', choices=list(FREEZE),
+                        help='freeze the backbone from the stem through this stage (eval-mode BatchNorm; needs --init SD.pt)')
     parser.add_argument('--target', type=int, default=1024, help='pad_resize size of every image')
     parser.add_argument('--loss', default='lovasz', choices=['lovasz', 'weighted_ce', 'mixed'])
     parser.add_argument('--lr', type=float, default=5e-4)
@@ -238,6 +262,9 @@ def parse_args(argv=None):
         parser.error('--epochs and --batch must be positive and --crop within [1, --target]')
     if args.accumulate < 1:
         parser.error('--accumulate must be at least 1')
+    if args.freeze != 'none' and args.init == 'random':
+        parser.error('--freeze %s needs --init SD.pt: freezing randomly initialised layers is almost certainly a mistake'
+                     % args.freeze)
     return args
 
 

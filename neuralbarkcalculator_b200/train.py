@@ -15,7 +15,11 @@ Measured on 8 B200 (profiles/r02c_bench_train_g8*.json): 1 336 img/s with the si
 persistent convolution kernels, which need all 148, and that costs more than the exposed half millisecond; hence the
 default.  Gradient accumulation: ``forward_backward(..., accumulate=True)`` adds a micro-batch's gradients to the
 buffer, so a global batch of ``world * k`` micro-batches costs k backward passes per rank and ONE exchange; Adam then
-applies 1 / (world * k).  No torch autograd, no torch ops on the data path."""
+applies 1 / (world * k).  Fine-tuning: ``freeze='stem'|'layer1'|..|'layer4'`` freezes the stem through that stage
+(``nbc_train_set_frozen``): those units run as eval-mode BatchNorm folded into their convolutions (torchvision's
+FrozenBatchNorm2d), their parameters, running statistics and ``num_batches_tracked`` never change, and the backward,
+the gradient exchange and Adam cover only the trainable suffix of the flat buffers.  No torch autograd, no torch ops on
+the data path."""
 import ctypes as C
 import os
 
@@ -35,6 +39,15 @@ def gradient_segments(lib, handle):
         _lib.check(lib.nbc_train_segment(h, i, C.byref(off), C.byref(cnt)), 'nbc_train_segment')
         out.append((off.value, cnt.value))
     return out
+
+
+FREEZE = ('none', 'stem', 'layer1', 'layer2', 'layer3', 'layer4')    # index = nbc_train_set_frozen's stages
+
+
+def frozen_prefixes(freeze):
+    """state_dict key prefixes of the units ``freeze`` freezes (the stem, then whole layers)."""
+    stages = FREEZE.index(freeze)
+    return tuple((['backbone.conv1.', 'backbone.bn1.'] if stages else []) + ['backbone.layer%d.' % i for i in range(1, stages)])
 
 
 def dropout_seed(base_seed, micro_batch, step):
@@ -62,7 +75,7 @@ def merge_segments(segments, min_bytes):
 class Trainer:
     def __init__(self, state_dict, N, H, W, device='cuda:0', lr=5e-4, weight_decay=2e-3, betas=(0.9, 0.999), eps=1e-8,
                  dropout=0.8, class_weights=None, mean=(0.7399, 0.6139, 0.4401), std=(0.1068, 0.1272, 0.1271),
-                 loss='weighted_ce', bucket_mb=0.0, seed=0):
+                 loss='weighted_ce', bucket_mb=0.0, seed=0, freeze='none'):
         self.lib = _lib.load()
         self.device = torch.device(device)
         _lib.require_device(self.device.index if self.device.index is not None else torch.cuda.current_device())
@@ -83,6 +96,9 @@ class Trainer:
         self.keys = list(state_dict.keys())
         if len(self.keys) != 326:
             raise RuntimeError('Trainer expects the 326-key fcn_resnet50 state_dict')
+        if freeze not in FREEZE:
+            raise ValueError('freeze must be one of %s' % ', '.join(FREEZE))
+        self.freeze = freeze
         with torch.cuda.device(self.device):
             self.handle = self.lib.nbc_train_create(N, H, W)
             if not self.handle:
@@ -93,6 +109,10 @@ class Trainer:
                 raise ValueError("loss must be 'weighted_ce', 'lovasz' or 'mixed'")
             _lib.check(self.lib.nbc_train_set_loss(h, kinds[loss]), 'nbc_train_set_loss')
             self.loss_kind = loss
+            _lib.check(self.lib.nbc_train_set_frozen(h, FREEZE.index(freeze)), 'nbc_train_set_frozen')
+            poff, soff = C.c_int64(0), C.c_int64(0)
+            _lib.check(self.lib.nbc_train_trainable_offsets(h, C.byref(poff), C.byref(soff)), 'nbc_train_trainable_offsets')
+            self.param_off, self.stats_off = poff.value, soff.value     # first trainable float of params / stats
             n = self.lib.nbc_train_param_count(h)
             self.params = torch.zeros(n, dtype=torch.float32, device=self.device)
             self.grads = torch.zeros(n, dtype=torch.float32, device=self.device)
@@ -105,6 +125,8 @@ class Trainer:
             self.class_weights = w.to(device=self.device, dtype=torch.float32).contiguous()
             self._exchange(self._device_tensors(state_dict), self.params, self.stats, 0)
         self.num_batches_tracked = {k: int(v) for k, v in state_dict.items() if k.endswith('num_batches_tracked')}
+        frozen = frozen_prefixes(freeze)
+        self._counted = [k for k in self.num_batches_tracked if not k.startswith(frozen)]   # frozen BNs do not count
         self.capture = None
 
     def __del__(self):
@@ -195,7 +217,8 @@ class Trainer:
         """images: u8 NHWC [N,H,W,3] (normalised inside) or f32 NCHW [N,3,H,W]; targets: u8 [N,H,W].
         Returns the loss (0-dim CUDA tensor); gradients are left in ``self.grads``: overwritten, or with ``accumulate``
         added to what the buffer holds (the first micro-batch of a step overwrites, the next ones accumulate; the next
-        ``optimizer_step`` divides by the number of micro-batches summed)."""
+        ``optimizer_step`` divides by the number of micro-batches summed).  ``update_stats=False`` leaves the running
+        statistics as they are (frozen units still read theirs)."""
         p = self.dropout if dropout is None else dropout
         if images.dtype == torch.uint8:
             kind, shape = 0, (self.N, self.H, self.W, 3)
@@ -214,25 +237,30 @@ class Trainer:
                 _lib.check(self.lib.nbc_train_set_accumulate(C.c_void_p(self.handle), int(accumulate)), 'nbc_train_set_accumulate')
                 self._accumulating = accumulate
             off = (-self.ws.data_ptr()) % 1024
+            stats = self.stats if update_stats else (self.stats.clone() if self.stats_off else None)
             _lib.check(self.lib.nbc_train_forward_backward(
                 C.c_void_p(self.handle), C.c_void_p(self.params.data_ptr()),
-                C.c_void_p(self.stats.data_ptr()) if update_stats else C.c_void_p(0), C.c_void_p(self.grads.data_ptr()),
+                C.c_void_p(stats.data_ptr() if stats is not None else 0), C.c_void_p(self.grads.data_ptr()),
                 C.c_void_p(images.data_ptr()), kind, self.mean3, self.std3, C.c_void_p(targets.data_ptr()),
                 C.c_void_p(self.class_weights.data_ptr()), C.c_float(p), C.c_uint64(seed), C.c_void_p(self.loss.data_ptr()),
                 C.c_void_p(self.ws.data_ptr() + off), C.c_size_t(self.ws.numel() - off),
                 C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), 'nbc_train_forward_backward')
         self.micro_batches = self.micro_batches + 1 if accumulate else 1
         if update_stats:
-            for k in self.num_batches_tracked:
+            for k in self._counted:
                 self.num_batches_tracked[k] += 1
         return self.loss
 
     def gradient_buckets(self):
         """[(last segment of the bucket, offset, count)] in the order the backward completes them: consecutive gradient
-        segments (``nbc_train_segment``) merged until a bucket holds at least ``bucket_mb`` MB."""
+        segments (``nbc_train_segment``) merged until a bucket holds at least ``bucket_mb`` MB.  The empty segments of
+        frozen units come last, so dropping them keeps every other segment's index."""
         if self._buckets is None:
-            self._buckets = merge_segments(gradient_segments(self.lib, self.handle), self.bucket_mb * 1e6)
-            assert sum(c for _, _, c in self._buckets) == self.grads.numel()
+            segments = gradient_segments(self.lib, self.handle)
+            trainable = [s for s in segments if s[1] > 0]
+            assert segments[:len(trainable)] == trainable
+            self._buckets = merge_segments(trainable, self.bucket_mb * 1e6)
+            assert sum(c for _, _, c in self._buckets) == self.grads.numel() - self.param_off
         return self._buckets
 
     def all_reduce_gradients(self):
@@ -244,7 +272,7 @@ class Trainer:
         if world == 1:
             return 0
         if self.bucket_mb <= 0:
-            dist.all_reduce(self.grads, op=dist.ReduceOp.SUM)
+            dist.all_reduce(self.grads[self.param_off:], op=dist.ReduceOp.SUM)
             return 1
         if self._comm_stream is None:
             self._comm_stream = torch.cuda.Stream(self.device)
@@ -261,17 +289,19 @@ class Trainer:
 
     def optimizer_step(self):
         """All-reduce the gradients over the data-parallel group (if any), then one fused Adam pass on their mean over
-        the world's micro-batches since the last step."""
+        the world's micro-batches since the last step, over the trainable suffix only (weight decay never touches a
+        frozen weight)."""
         import torch.distributed as dist
         world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
         micro = max(self.micro_batches, 1)
         self.all_reduce_gradients()
         self.step_count += 1
         self.micro_batches = 0
+        o = self.param_off * 4      # bytes
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.nbc_train_adam(C.c_void_p(self.params.data_ptr()), C.c_void_p(self.grads.data_ptr()),
-                                               C.c_void_p(self.adam_m.data_ptr()), C.c_void_p(self.adam_v.data_ptr()),
-                                               self.params.numel(), C.c_float(self.lr), C.c_float(self.betas[0]),
+            _lib.check(self.lib.nbc_train_adam(C.c_void_p(self.params.data_ptr() + o), C.c_void_p(self.grads.data_ptr() + o),
+                                               C.c_void_p(self.adam_m.data_ptr() + o), C.c_void_p(self.adam_v.data_ptr() + o),
+                                               self.params.numel() - self.param_off, C.c_float(self.lr), C.c_float(self.betas[0]),
                                                C.c_float(self.betas[1]), C.c_float(self.eps), C.c_float(self.wd), self.step_count,
                                                C.c_float(1.0 / (world * micro)),
                                                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), 'nbc_train_adam')
