@@ -129,8 +129,18 @@ int nbc_conv_dual_bf16(const nbc_conv_desc* desc, const void* x, const nbc_conv_
 
 /* Weight gradient of the same layer (training path, __main__.py:231-269 backward of every nn.Conv2d):
  * dw[Cout][kh][kw][Cin] (f32) += sum over output pixels of dz[N,Ho,Wo,Cout]^T * x[N,H,W,Cin] (both bf16 NHWC);
- * accumulates into dw (zero it first).  desc.impl: 0 = auto, 1 = tcgen05 (MN-major operands), 2 = mma.sync. */
+ * accumulates into dw (zero it first).  desc.impl: 0 = auto, 1 = tcgen05 (MN-major operands), 2 = mma.sync.
+ * The tcgen05 kernel here has no scratch, so one CTA per weight tile sums every pixel (no split over the pixels): each
+ * element of dw has one writer and the result is bit-reproducible.  The mma.sync kernel adds with f32 atomics and is
+ * not (its order depends on timing).
+ * nbc_conv_wgrad_bf16_ws: the tcgen05 kernel with the pixels split over the SMs (one wave, as the training plan runs
+ * it); the f32 partial tiles of the splits go to `workspace` (>= nbc_conv_wgrad_workspace_bytes(desc), 16-byte
+ * aligned; 0 bytes when the shape runs one split, and then workspace may be NULL) and a second launch adds them in a
+ * fixed order, dw = dw + sum over splits.  Bit-reproducible for a given shape and SM count.  desc.impl is ignored. */
 int nbc_conv_wgrad_bf16(const nbc_conv_desc* desc, const void* dz, const void* x, float* dw, void* stream);
+size_t nbc_conv_wgrad_workspace_bytes(const nbc_conv_desc* desc);
+int nbc_conv_wgrad_bf16_ws(const nbc_conv_desc* desc, const void* dz, const void* x, float* dw, void* workspace,
+                           size_t workspace_bytes, void* stream);
 
 /* ---- stem: ToTensor + Normalize + conv1 7x7/2 + bn1 + relu, then maxpool 3x3/2
  *      (dataset.py:181-190, models.py:233-237, torchvision resnet50 stem) ---------------------------------------
@@ -308,11 +318,16 @@ int nbc_plan_step_info(const nbc_plan* plan, int i, nbc_plan_step* out);
  *   stats                            : f32[nbc_train_stats_count]   (BatchNorm running mean / var)
  * nbc_train_exchange converts between the 326 state_dict tensors (torchvision order, OIHW) and the flat buffers:
  * direction 0 loads tensors -> (params, stats), 1 stores (params, stats) -> tensors.  Storing the gradient buffer
- * gives per-layer gradients in state_dict layout (stats = NULL).
+ * gives per-layer gradients in state_dict layout (stats = NULL); with stats = NULL either direction leaves the running
+ * statistics alone, so the Adam moments load and store the same way.  Both directions are pure copies (bit-exact).
  * nbc_train_forward_backward: input_kind 0 = u8 NHWC images (normalised inside), 1 = f32 NCHW; target u8 [N,H,W];
  * BatchNorm uses batch statistics and updates `stats` (momentum 0.1) unless stats is NULL; dropout_p applies to the
  * head (mask = hash(seed, index)); loss = mean weighted CE (device scalar); grads are overwritten, or added to after
  * nbc_train_set_accumulate(plan, 1) (gradient accumulation over micro-batches: the caller zeroes `grads` first).
+ * Reproducible: with the default tcgen05 weight-gradient kernels every gradient element has one writer that adds
+ * a fixed-order sum (split-K partials and the classifier's per-block partials are reduced from the workspace, which
+ * nbc_train_workspace_bytes includes), so the same inputs give bit-identical grads, stats, loss and, through
+ * nbc_train_adam, params -- on the same GPU model and SM count with the same library build.
  * Data-parallel training: all-reduce `grads` (sum) across ranks, then nbc_train_adam with grad_scale = 1/world.
  * nbc_train_adam follows torch.optim.Adam (L2 weight decay added to the gradient, bias correction by `step` >= 1). */
 typedef struct nbc_train_plan nbc_train_plan;
@@ -347,13 +362,14 @@ int64_t nbc_train_debug_offset(const nbc_train_plan* plan, int what, int index, 
 size_t nbc_train_capture_bytes(const nbc_train_plan* plan);
 int nbc_train_set_capture(nbc_train_plan* plan, void* buf, size_t bytes);
 int nbc_train_num_units(const nbc_train_plan* plan);
-/* weight-gradient kernels used by the plan: 0 = tcgen05 (default), 1 = mma.sync / CUDA-core cross-check kernels */
+/* weight-gradient kernels used by the plan: 0 = tcgen05 (default, deterministic), 1 = mma.sync / CUDA-core cross-check
+ * kernels (f32 atomics: not deterministic, the last bits of two runs differ) */
 int nbc_train_set_wgrad_impl(nbc_train_plan* plan, int impl);
 /* loss of the step: 0 = CustomWeightedCrossEntropy (utils.py:151-165, default), 1 = LovaszSoftmax (__main__.py:239),
  * 2 = MixedLoss = CE / 4 + Lovasz (utils.py:185-192) */
 int nbc_train_set_loss(nbc_train_plan* plan, int kind);
 /* 1: nbc_train_forward_backward adds its gradients to `grads` instead of overwriting them (no memset; every gradient
- * write is an atomic add); each segment event then marks the segment's running sum as final.  0 = overwrite (default). */
+ * writer adds, grads[i] = grads[i] + this step's sum); each segment event then marks the segment's running sum as final.  0 = overwrite (default). */
 int nbc_train_set_accumulate(nbc_train_plan* plan, int on);
 /* Fine-tuning with a frozen backbone.  stages: 0 = nothing frozen (default), 1 = the stem (conv1 + bn1), 2..5 = the
  * stem through layer1..layer4; any other value is refused.  A frozen unit is torchvision's FrozenBatchNorm2d after its

@@ -52,6 +52,8 @@ SIGNATURES = {
     'nbc_conv_bf16': (c_int, [C.POINTER(ConvDesc), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     'nbc_conv_dual_bf16': (c_int, [C.POINTER(ConvDesc), c_void_p, C.POINTER(ConvDesc), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     'nbc_conv_wgrad_bf16': (c_int, [C.POINTER(ConvDesc), c_void_p, c_void_p, c_void_p, c_void_p]),
+    'nbc_conv_wgrad_workspace_bytes': (c_size_t, [C.POINTER(ConvDesc)]),
+    'nbc_conv_wgrad_bf16_ws': (c_int, [C.POINTER(ConvDesc), c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     'nbc_stem_u8': (c_int, [c_void_p, c_int, c_int, c_int, C.POINTER(c_float), C.POINTER(c_float), c_void_p, c_void_p, c_void_p, c_void_p]),
     'nbc_stem_f32': (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     'nbc_stem_tc_workspace_bytes': (c_size_t, [c_int, c_int, c_int]),

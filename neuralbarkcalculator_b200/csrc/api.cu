@@ -158,10 +158,27 @@ extern "C" int nbc_conv_wgrad_bf16(const nbc_conv_desc* d, const void* dz, const
   ConvGeom g{d->N, d->H, d->W, d->Cin, d->Cout, d->kh, d->kw, d->stride, d->pad, d->dil, 0, 0};
   NBC_REQUIRE(g.N > 0 && g.H > 0 && g.W > 0 && g.Ho() > 0 && g.Wo() > 0, "nbc_conv_wgrad_bf16: bad shape");
   const bool tc_ok = wgrad_tc_supported(g);
-  if (d->impl == 1 || (d->impl == 0 && tc_ok)) return wgrad_tc(g, dz, x, dw, stream);
+  if (d->impl == 1 || (d->impl == 0 && tc_ok)) return wgrad_tc(g, dz, x, dw, nullptr, 0, stream);
   if (d->impl == 2 || d->impl == 0) return wgrad_mma(g, dz, x, dw, stream);
   set_error("nbc_conv_wgrad_bf16: unknown impl %d", d->impl);
   return NBC_ERR_INVALID;
+}
+
+extern "C" size_t nbc_conv_wgrad_workspace_bytes(const nbc_conv_desc* d) {
+  if (!d) return 0;
+  const ConvGeom g{d->N, d->H, d->W, d->Cin, d->Cout, d->kh, d->kw, d->stride, d->pad, d->dil, 0, 0};
+  if (g.N <= 0 || g.H <= 0 || g.W <= 0 || g.Ho() <= 0 || g.Wo() <= 0) return 0;
+  return wgrad_tc_scratch_bytes(g);
+}
+
+extern "C" int nbc_conv_wgrad_bf16_ws(const nbc_conv_desc* d, const void* dz, const void* x, float* dw, void* workspace,
+                                      size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  NBC_REQUIRE(d && dz && x && dw, "nbc_conv_wgrad_bf16_ws: null pointer");
+  NBC_REQUIRE(!d->f16, "nbc_conv_wgrad_bf16_ws: the training path is bf16 only");
+  ConvGeom g{d->N, d->H, d->W, d->Cin, d->Cout, d->kh, d->kw, d->stride, d->pad, d->dil, 0, 0};
+  NBC_REQUIRE(g.N > 0 && g.H > 0 && g.W > 0 && g.Ho() > 0 && g.Wo() > 0, "nbc_conv_wgrad_bf16_ws: bad shape");
+  return wgrad_tc(g, dz, x, dw, workspace, workspace_bytes, stream);
 }
 
 extern "C" int nbc_conv_dual_bf16(const nbc_conv_desc* d, const void* x, const nbc_conv_desc* d2, const void* x2, const void* w_cat,

@@ -21,10 +21,17 @@ int dgrad_pack(const float* w_ohwi, int Cout, int Cin, int kh, int kw, void* out
 int oihw_ohwi(const float* src, int Cout, int Cin, int kh, int kw, float* dst, int reverse, cudaStream_t stream);
 // dW[Cout][kh][kw][Cin] (f32, accumulated with atomics) += dz^T * x over all output pixels
 int wgrad_mma(const ConvGeom& g, const void* dz, const void* x, float* dw, cudaStream_t stream);
-// the same on the tcgen05 tensor cores (wgrad_tc.cu); Cin % 64 == 0, Cout % 64 == 0, stride 1 or 2
+// the same on the tcgen05 tensor cores (wgrad_tc.cu); Cin % 64 == 0, Cout % 64 == 0, stride 1 or 2.  Deterministic:
+// with scratch (>= wgrad_tc_scratch_bytes, 16-byte aligned) the pixels are split over the SMs and the split partials
+// are added in a fixed order by a second launch; with scratch == null one CTA per tile sums all pixels.  Either way
+// every element of dw has one writer, dw += sum.
 bool wgrad_tc_supported(const ConvGeom& g);
-int wgrad_tc(const ConvGeom& g, const void* dz, const void* x, float* dw, cudaStream_t stream);
-int stem_wgrad_tc(const void* dz, const void* padded, int N, int Ho, int Wo, float* dw, cudaStream_t stream);
+size_t wgrad_tc_scratch_bytes(const ConvGeom& g);
+int wgrad_tc(const ConvGeom& g, const void* dz, const void* x, float* dw, void* scratch, size_t scratch_bytes,
+             cudaStream_t stream);
+size_t stem_wgrad_tc_scratch_bytes(int N, int Ho, int Wo);
+int stem_wgrad_tc(const void* dz, const void* padded, int N, int Ho, int Wo, float* dw, void* scratch, size_t scratch_bytes,
+                  cudaStream_t stream);
 
 // 3x3/2 max pooling that records the position of the first maximum (idx: one byte per output element), and its backward
 int maxpool_forward_idx(const void* x, int N, int H, int W, int C, void* y, void* idx, cudaStream_t stream);
@@ -32,8 +39,10 @@ int maxpool_backward(const void* dy, const void* idx, int N, int H, int W, int C
 // stem: dW f32 [64][7][7][3] += dz^T * padded image (the bf16 staging buffer [N][2Ho+5][2Wo+6][4] of the stem)
 int stem_wgrad(const void* dz, const void* padded, int N, int Ho, int Wo, float* dw, cudaStream_t stream);
 int dropout_apply(const void* x, int64_t n, float p, uint64_t seed, void* y, cudaStream_t stream);
+// classifier backward; dW / db get the per-block partials (partial: cls_partial_bytes) added in a fixed order
+size_t cls_partial_bytes(int C);
 int cls_backward(const float* dlow, const void* x, const float* w, int N, int64_t P, int C, float drop_p, uint64_t seed,
-                 void* dx, float* dw, float* db, cudaStream_t stream);
+                 void* dx, float* dw, float* db, void* partial, cudaStream_t stream);
 size_t upsample_bwd_workspace_bytes(int N, int C, int h, int w, int H, int W);
 int upsample_backward(const float* dup, int N, int C, int h, int w, int H, int W, float* dlow, void* workspace,
                       cudaStream_t stream);

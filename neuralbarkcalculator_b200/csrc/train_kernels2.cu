@@ -186,15 +186,20 @@ int dropout_apply(const void* x, int64_t n, float p, uint64_t seed, void* y, cud
 // ------------------------------------------------------------------------------------------------ classifier backward
 // dlow f32 [N][3][P];  x bf16 [N*P][C] (after dropout);  w f32 [3][C]
 // dx[p][k] = sum_c dlow[c][p] * w[c][k]  (then through the dropout mask);  dW[c][k] += sum_p dlow[c][p] x[p][k]; db[c] += sum_p
+// Each block stores its pixel slab's dW and db to partial[block][3C + 3]; cls_finalize_kernel adds the blocks in a fixed
+// order, so the gradient does not depend on the order the blocks finish.
+constexpr int kClsBlocks = 148 * 4;
+size_t cls_partial_bytes(int C) { return (size_t)kClsBlocks * (3 * C + 3) * sizeof(float); }
+
 __global__ void __launch_bounds__(256) cls_bwd_kernel(const float* __restrict__ dlow, const __nv_bfloat16* __restrict__ x,
                                                       const float* __restrict__ w, int N, int64_t P, int C, float drop_p,
-                                                      uint64_t seed, __nv_bfloat16* __restrict__ dx, float* __restrict__ dw,
-                                                      float* __restrict__ db) {
+                                                      uint64_t seed, __nv_bfloat16* __restrict__ dx, float* __restrict__ partial) {
   // thread owns channels k = tid, tid + 256, ...; block owns a slab of pixels
   const int64_t M = (int64_t)N * P;
   const int64_t per_block = ceil_div64(M, gridDim.x);
   const int64_t m0 = (int64_t)blockIdx.x * per_block, m1 = min(M, m0 + per_block);
   const float scale = 1.f / (1.f - drop_p);
+  float* part = partial + (int64_t)blockIdx.x * (3 * C + 3);
   for (int k = threadIdx.x; k < C; k += blockDim.x) {
     const float w0 = w[k], w1 = w[C + k], w2 = w[2 * C + k];
     float a0 = 0.f, a1 = 0.f, a2 = 0.f;
@@ -208,7 +213,7 @@ __global__ void __launch_bounds__(256) cls_bwd_kernel(const float* __restrict__ 
       if (drop_p > 0.f) g = hash_uniform(seed, (uint64_t)(m * C + k)) >= drop_p ? g * scale : 0.f;
       dx[m * C + k] = __float2bfloat16_rn(g);
     }
-    atomicAdd(dw + k, a0), atomicAdd(dw + C + k, a1), atomicAdd(dw + 2 * C + k, a2);
+    part[k] = a0, part[C + k] = a1, part[2 * C + k] = a2;
   }
   if (threadIdx.x < 3) {
     float s = 0.f;
@@ -216,13 +221,31 @@ __global__ void __launch_bounds__(256) cls_bwd_kernel(const float* __restrict__ 
       const int64_t n = m / P, pix = m - n * P;
       s += dlow[n * 3 * P + threadIdx.x * P + pix];
     }
-    atomicAdd(db + threadIdx.x, s);
+    part[3 * C + threadIdx.x] = s;
+  }
+}
+// one warp per output: lane l adds blocks l, l + 32, ... in order, then a fixed butterfly over the lanes; one writer
+__global__ void __launch_bounds__(256) cls_finalize_kernel(const float* __restrict__ partial, int C, int blocks, float* __restrict__ dw,
+                                                           float* __restrict__ db) {
+  const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  const int n = 3 * C + 3;
+  if (i >= n) return;
+  float s = 0.f;
+  for (int b = lane; b < blocks; b += 32) s += partial[(int64_t)b * n + i];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if (lane == 0) {
+    float* d = i < 3 * C ? dw + i : db + (i - 3 * C);
+    *d += s;
   }
 }
 int cls_backward(const float* dlow, const void* x, const float* w, int N, int64_t P, int C, float drop_p, uint64_t seed,
-                 void* dx, float* dw, float* db, cudaStream_t stream) {
-  cls_bwd_kernel<<<148 * 4, 256, 0, stream>>>(dlow, reinterpret_cast<const __nv_bfloat16*>(x), w, N, P, C, drop_p, seed,
-                                              reinterpret_cast<__nv_bfloat16*>(dx), dw, db);
+                 void* dx, float* dw, float* db, void* partial, cudaStream_t stream) {
+  float* part = reinterpret_cast<float*>(partial);
+  cls_bwd_kernel<<<kClsBlocks, 256, 0, stream>>>(dlow, reinterpret_cast<const __nv_bfloat16*>(x), w, N, P, C, drop_p, seed,
+                                                 reinterpret_cast<__nv_bfloat16*>(dx), part);
+  NBC_CHECK_LAUNCH();
+  cls_finalize_kernel<<<ceil_div((3 * C + 3) * 32, 256), 256, 0, stream>>>(part, C, kClsBlocks, dw, db);
   NBC_CHECK_LAUNCH();
   return 0;
 }

@@ -59,6 +59,9 @@ struct nbc_train_plan {
   int frozen = 0, first_unit = 0, first_block = 0;
   size_t fold_off = 0;  // bytes, workspace: the frozen stem's folded f32 weights [64][7][7][3] before the w224 pack
   size_t lov_off = 0, dfull2_off = 0, loss2_off = 0;
+  // scratch of the deterministic weight-gradient reductions: the split partials of one wgrad_tc launch (reused by
+  // the next, which the stream orders behind its reduction) and the classifier's per-block partials
+  size_t wgpart_off = 0, wgpart_bytes = 0, clspart_off = 0;
   // gradient-ready events, one per SEGMENT of the flat gradient buffer in the order the backward finishes them:
   // segment 0 = head conv + classifier, then the bottleneck blocks last to first, then the stem (created lazily)
   std::vector<cudaEvent_t> seg_events;
@@ -181,6 +184,13 @@ extern "C" nbc_train_plan* nbc_train_create(int N, int H, int W) {
   p->dfull2_off = off, off += al((size_t)N * 3 * H * W * 4);
   p->loss2_off = off, off += al(16);
   p->fold_off = off, off += al(64 * 147 * 4);
+  for (const Unit& u : p->units) {
+    const ConvGeom g{N, u.Hin, u.Win, u.Cin, u.Cout, u.k, u.k, u.stride, u.pad, u.dil, 0, 0};
+    const size_t b = u.Cin == 3 ? stem_wgrad_tc_scratch_bytes(N, u.Ho, u.Wo) : wgrad_tc_scratch_bytes(g);
+    if (b > p->wgpart_bytes) p->wgpart_bytes = b;
+  }
+  p->wgpart_off = off, off += al(p->wgpart_bytes);
+  p->clspart_off = off, off += al(cls_partial_bytes(512));
   p->ws_bytes = off;
   p->capture_bytes = cap;
 
@@ -395,12 +405,15 @@ static int unit_backward(const Ctx& c, Unit& u, const void* dy, int relu, void* 
     NBC_CUDA(cudaMemcpyAsync(cap, dy, bytes, cudaMemcpyDeviceToDevice, c.stream));
     NBC_CUDA(cudaMemcpyAsync(cap + al(bytes), dz, bytes, cudaMemcpyDeviceToDevice, c.stream));
   }
+  void* scratch = c.ws + p->wgpart_off;
   if (u.Cin == 3)
-    return c.p->wgrad_impl == 1 ? stem_wgrad(dz, c.ws + p->padded_off, p->N, u.Ho, u.Wo, c.grads + u.w_off, c.stream)
-                                : stem_wgrad_tc(dz, c.ws + p->padded_off, p->N, u.Ho, u.Wo, c.grads + u.w_off, c.stream);
+    return c.p->wgrad_impl == 1
+               ? stem_wgrad(dz, c.ws + p->padded_off, p->N, u.Ho, u.Wo, c.grads + u.w_off, c.stream)
+               : stem_wgrad_tc(dz, c.ws + p->padded_off, p->N, u.Ho, u.Wo, c.grads + u.w_off, scratch, p->wgpart_bytes, c.stream);
   ConvGeom g{p->N, u.Hin, u.Win, u.Cin, u.Cout, u.k, u.k, u.stride, u.pad, u.dil, 0, 0};
-  rc = (c.p->wgrad_impl == 1 || !wgrad_tc_supported(g)) ? wgrad_mma(g, dz, c.ws + u.x_off, c.grads + u.w_off, c.stream)
-                                                         : wgrad_tc(g, dz, c.ws + u.x_off, c.grads + u.w_off, c.stream);
+  rc = (c.p->wgrad_impl == 1 || !wgrad_tc_supported(g))
+           ? wgrad_mma(g, dz, c.ws + u.x_off, c.grads + u.w_off, c.stream)
+           : wgrad_tc(g, dz, c.ws + u.x_off, c.grads + u.w_off, scratch, p->wgpart_bytes, c.stream);
   if (rc) return rc;
   if (!u.need_dgrad) return 0;
   if (u.stride == 2) {
@@ -515,7 +528,7 @@ extern "C" int nbc_train_forward_backward(nbc_train_plan* p, float* params, floa
   if ((rc = upsample_backward(dfull, N, 3, p->H8, p->W8, H, W, dlow, ws + p->upws_off, stream))) return rc;
   // classifier: gradient w.r.t. the head activations (through the dropout mask) goes to d2
   if ((rc = cls_backward(dlow, cls_in, params + p->cls_w_off, N, P8, 512, dropout_p, seed, ws + p->d2_off,
-                         grads + p->cls_w_off, grads + p->cls_b_off, stream)))
+                         grads + p->cls_w_off, grads + p->cls_b_off, ws + p->clspart_off, stream)))
     return rc;
   if ((rc = unit_backward(c, head, ws + p->d2_off, 1, nullptr))) return rc;
   if ((rc = record_segment(p, 0, stream))) return rc;

@@ -11,7 +11,10 @@
 //   * one CTA = one (co tile of 128, ci tile of BN, tap, pixel range): split-K over the pixels fills the 148 SMs
 //   * K block = 64 pixels (a tw x th rectangle of the output); x is read through the same shifted / parity-lattice
 //     tensor maps as the forward operand (zero fill outside the image = the conv padding)
-//   * f32 accumulator in TMEM; epilogue = red.global.add.v4.f32 into the f32 gradient buffer
+//   * f32 accumulator in TMEM.  Epilogue: with one split, dw += acc (this CTA is the element's only writer); with
+//     several, plain 16-byte stores of the partial tile to its scratch slot [item][split][128][BN], and
+//     wgrad_reduce_kernel then adds the splits in a fixed order, dw = dw + sum_s partial[s], one writer per element.
+//     The result depends on the shape and the SM count only, never on the order in which the CTAs finish.
 // Warp roles: 0 = TMA producer, 1 = MMA issuer + TMEM owner, 2..5 = epilogue.
 #include <algorithm>
 
@@ -25,6 +28,7 @@ struct WgradTcParams {
   CUtensorMap tmDz;     // dz [N][Ho][Wo][Cout], box {64, tw, th, 1}
   CUtensorMap tmX[4];   // x  [N][H][W][Cin] (stride 1) or its four parity lattices (stride 2), box {64, tw, th, 1}
   float* dw;            // [Cout][taps][Cin]
+  float* partial;       // splits > 1: scratch [grid][128][BN], slot blockIdx.x = item * splits + split; else null
   int Cout, Cin, taps;
   int tw_log2, th, tw, tiles_w, tiles_h;
   int num_pix_tiles;    // N * tiles_h * tiles_w
@@ -68,10 +72,6 @@ __device__ __forceinline__ uint64_t umma_desc_mnmajor(uint32_t smem_addr, uint32
 // kind::f16 instruction descriptor with both operands MN-major (bits 15 / 16)
 __host__ __device__ constexpr uint32_t umma_idesc_bf16_mn(int M, int N) {
   return umma_idesc_bf16(M, N) | (1u << 15) | (1u << 16);
-}
-
-__device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
-  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
 template <int BN>
@@ -182,25 +182,35 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
       const int co = co_tile * 128 + q * 32 + lane;
       mbar_wait(tfull_bar, 0, 400);
       tc_fence_after();
+      const bool row_ok = co < p.Cout;
+      float* prow = p.partial ? p.partial + ((int64_t)blockIdx.x * 128 + q * 32 + lane) * BN : nullptr;
       float* drow = p.dw + ((int64_t)co * p.taps + tap) * p.Cin + ci_tile * BN;
 #pragma unroll 1
       for (int c = 0; c < BN; c += 32) {
         uint32_t r[32];
         tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + c, r);
         tmem_ld_wait();
-        if (co < p.Cout) {
-          if (Cfg::kStem) {
-            // column = kx * 4 + c of tap row ky = tap; the stem gradient is f32 [64][7][7][3]
-            float* d = p.dw + ((int64_t)co * 49 + tap * 7) * 3;
+        if (!row_ok) continue;
+        if (prow != nullptr) {
 #pragma unroll
-            for (int kx = 0; kx < 7; ++kx)
+          for (int i = 0; i < 32; i += 4)
+            *reinterpret_cast<float4*>(prow + c + i) =
+                make_float4(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), __uint_as_float(r[i + 2]), __uint_as_float(r[i + 3]));
+        } else if (Cfg::kStem) {
+          // column = kx * 4 + c of tap row ky = tap; the stem gradient is f32 [64][7][7][3]
+          float* d = p.dw + ((int64_t)co * 49 + tap * 7) * 3;
 #pragma unroll
-              for (int ch = 0; ch < 3; ++ch) atomicAdd(d + kx * 3 + ch, __uint_as_float(r[kx * 4 + ch]));
-          } else {
+          for (int kx = 0; kx < 7; ++kx)
 #pragma unroll
-            for (int i = 0; i < 32; i += 4)
-              red_add_v4(drow + c + i, __uint_as_float(r[i]), __uint_as_float(r[i + 1]), __uint_as_float(r[i + 2]),
-                         __uint_as_float(r[i + 3]));
+            for (int ch = 0; ch < 3; ++ch) d[kx * 3 + ch] += __uint_as_float(r[kx * 4 + ch]);
+        } else {
+#pragma unroll
+          for (int i = 0; i < 32; i += 4) {
+            float4* d = reinterpret_cast<float4*>(drow + c + i);
+            float4 v = *d;
+            v.x += __uint_as_float(r[i]), v.y += __uint_as_float(r[i + 1]), v.z += __uint_as_float(r[i + 2]),
+                v.w += __uint_as_float(r[i + 3]);
+            *d = v;
           }
         }
       }
@@ -222,27 +232,77 @@ bool wgrad_tc_supported(const ConvGeom& g) {
 
 static int floordiv2(int a) { return (a >= 0) ? a / 2 : -((-a + 1) / 2); }
 
-template <int BN>
-static int launch_wgrad(const WgradTcParams& p, int grid, cudaStream_t stream) {
-  static bool attr_set = false;
-  if (!attr_set) {
-    NBC_CUDA(cudaFuncSetAttribute(wgrad_tc_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, WgCfg<BN>::kSmemBytes));
-    attr_set = true;
+// Fixed-order sum of the split partials into dw.  A block covers 32 elements (float4 columns of a tile row, or single
+// stem taps) x 8 groups of splits: group g adds splits [g * per, (g + 1) * per) in index order, then the group sums are
+// added in group order and dw = dw + sum is stored by one thread.  The order is a function of `splits` alone.
+struct WgReduceParams {
+  const float* partial;
+  float* dw;
+  int64_t n;            // elements: float4 columns of the partial tiles, or stem gradient entries
+  int splits, BN, taps, ci_tiles, Cout, Cin;
+};
+constexpr int kRedLanes = 32, kRedGroups = 8;
+
+__device__ __forceinline__ float4 add4(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
+
+template <bool kStem>
+__global__ void __launch_bounds__(kRedLanes * kRedGroups) wgrad_reduce_kernel(const WgReduceParams r) {
+  __shared__ float4 part[kRedGroups][kRedLanes];
+  const int lane = threadIdx.x, grp = threadIdx.y;
+  const int64_t e = (int64_t)blockIdx.x * kRedLanes + lane;
+  bool valid = e < r.n;
+  int64_t src = 0;   // floats: the element in split 0
+  float* dst = nullptr;
+  if (valid) {
+    if (kStem) {
+      // e = (tap * 64 + co) * 21 + kx * 3 + ch; partial column kx * 4 + ch of row co in slot tap * splits + s
+      const int j = (int)(e % 21);
+      const int t = (int)(e / 21), co = t % 64, tap = t / 64;
+      src = ((int64_t)tap * r.splits * 128 + co) * 32 + (j / 3) * 4 + j % 3;
+      dst = r.dw + (co * 49 + tap * 7) * 3 + j;
+    } else {
+      const int vpr = r.BN / 4;
+      const int c4 = (int)(e % vpr);
+      const int64_t t = e / vpr;
+      const int row = (int)(t % 128);
+      const int64_t item = t / 128;
+      const int tap = (int)(item % r.taps), ci_tile = (int)((item / r.taps) % r.ci_tiles), co_tile = (int)(item / r.taps / r.ci_tiles);
+      const int co = co_tile * 128 + row;
+      valid = co < r.Cout;
+      src = (item * r.splits * 128 + row) * r.BN + c4 * 4;
+      dst = r.dw + ((int64_t)co * r.taps + tap) * r.Cin + ci_tile * r.BN + c4 * 4;
+    }
   }
-  wgrad_tc_kernel<BN><<<grid, kWgThreads, WgCfg<BN>::kSmemBytes, stream>>>(p);
-  NBC_CHECK_LAUNCH();
-  return 0;
+  const int64_t slot = (int64_t)128 * r.BN;
+  const int per = ceil_div(r.splits, kRedGroups);
+  const int s0 = grp * per, s1 = min(r.splits, s0 + per);
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (valid && s0 < s1) {
+    if (kStem) {
+      float a = r.partial[src + s0 * slot];
+      for (int s = s0 + 1; s < s1; ++s) a += r.partial[src + s * slot];
+      acc.x = a;
+    } else {
+      acc = *reinterpret_cast<const float4*>(r.partial + src + s0 * slot);
+#pragma unroll 4
+      for (int s = s0 + 1; s < s1; ++s) acc = add4(acc, *reinterpret_cast<const float4*>(r.partial + src + s * slot));
+    }
+  }
+  part[grp][lane] = acc;
+  __syncthreads();
+  if (grp != 0 || !valid) return;
+  float4 sum = part[0][lane];
+  for (int g = 1; g * per < r.splits; ++g) sum = add4(sum, part[g][lane]);
+  if (kStem) {
+    *dst += sum.x;
+  } else {
+    float4* d = reinterpret_cast<float4*>(dst);
+    *d = add4(*d, sum);
+  }
 }
 
-int wgrad_tc(const ConvGeom& g, const void* dz, const void* x, float* dw, cudaStream_t stream) {
-  if (!wgrad_tc_supported(g)) {
-    set_error("wgrad_tc: unsupported shape Cin=%d Cout=%d k=%dx%d stride=%d", g.Cin, g.Cout, g.kh, g.kw, g.stride);
-    return NBC_ERR_INVALID;
-  }
-  NBC_REQUIRE((reinterpret_cast<uintptr_t>(dw) & 15) == 0, "wgrad_tc: dw must be 16-byte aligned");
-  WgradTcParams p;
-  memset(&p, 0, sizeof(p));
-  const int Ho = g.Ho(), Wo = g.Wo();
+// output tiling (64-pixel rectangles) and the split-K of the pixel tiles; shapes only, no pointers
+static void wg_tiling(WgradTcParams& p, int N, int Ho, int Wo) {
   // 64-pixel output rectangle: fewest tiles, widest on ties
   int best_tw = 64, best_tiles = INT32_MAX;
   for (int tw = 64; tw >= 8; tw >>= 1) {
@@ -250,14 +310,102 @@ int wgrad_tc(const ConvGeom& g, const void* dz, const void* x, float* dw, cudaSt
     if (tiles < best_tiles) best_tiles = tiles, best_tw = tw;
   }
   p.tw = best_tw, p.th = 64 / best_tw;
+  p.tw_log2 = 0;
   while ((1 << p.tw_log2) < p.tw) ++p.tw_log2;
   p.tiles_w = ceil_div(Wo, p.tw), p.tiles_h = ceil_div(Ho, p.th);
-  p.num_pix_tiles = g.N * p.tiles_w * p.tiles_h;
-  p.Cout = g.Cout, p.Cin = g.Cin, p.taps = g.kh * g.kw;
-  p.dw = dw;
+  p.num_pix_tiles = N * p.tiles_w * p.tiles_h;
+}
+// each split with at least 16 K blocks; splits recomputed so that none is empty
+static void wg_split(WgradTcParams& p, int splits) {
+  const int max_splits = ceil_div(p.num_pix_tiles, 16);
+  if (splits > max_splits) splits = max_splits;
+  if (splits < 1) splits = 1;
+  p.tiles_per_split = ceil_div(p.num_pix_tiles, splits);
+  p.splits = ceil_div(p.num_pix_tiles, p.tiles_per_split);
+}
+static int wg_bn(const ConvGeom& g) {
   const int bn = (g.Cin % 256 == 0) ? 256 : (g.Cin % 128 == 0 ? 128 : 64);
-  p.ci_tiles = g.Cin / bn;
+  return bn;
+}
+// one wave: as many splits as fit the SMs once.  More, smaller splits balance better but every split adds a full tile
+// of f32 partials to reduce (with the former atomics, 4x oversubscription cost 6 % of the training step)
+static void wg_geometry(WgradTcParams& p, const ConvGeom& g) {
+  wg_tiling(p, g.N, g.Ho(), g.Wo());
+  p.Cout = g.Cout, p.Cin = g.Cin, p.taps = g.kh * g.kw;
+  p.ci_tiles = g.Cin / wg_bn(g);
   p.co_tiles = ceil_div(g.Cout, 128);
+  const int base_items = p.co_tiles * p.ci_tiles * p.taps;
+  int splits = std::max(1, sm_count() / base_items);
+  wg_split(p, splits);
+}
+static void wg_stem_geometry(WgradTcParams& p, int N, int Ho, int Wo) {
+  wg_tiling(p, N, Ho, Wo);
+  p.Cout = 64, p.Cin = 32, p.taps = 7;
+  p.ci_tiles = 1, p.co_tiles = 1;
+  int splits = ceil_div(sm_count() * 2, 7);
+  wg_split(p, splits);
+}
+static size_t wg_scratch_bytes(const WgradTcParams& p, int bn) {
+  return p.splits > 1 ? (size_t)p.co_tiles * p.ci_tiles * p.taps * p.splits * 128 * bn * sizeof(float) : 0;
+}
+
+size_t wgrad_tc_scratch_bytes(const ConvGeom& g) {
+  if (!wgrad_tc_supported(g)) return 0;
+  WgradTcParams p;
+  memset(&p, 0, sizeof(p));
+  wg_geometry(p, g);
+  return wg_scratch_bytes(p, wg_bn(g));
+}
+size_t stem_wgrad_tc_scratch_bytes(int N, int Ho, int Wo) {
+  WgradTcParams p;
+  memset(&p, 0, sizeof(p));
+  wg_stem_geometry(p, N, Ho, Wo);
+  return wg_scratch_bytes(p, 32);
+}
+
+// scratch == null: one split (dw += acc in the epilogue).  Otherwise the shape's split-K, then the reduction.
+template <int BN>
+static int launch_wgrad(WgradTcParams& p, void* scratch, size_t scratch_bytes, cudaStream_t stream) {
+  static bool attr_set = false;
+  if (!attr_set) {
+    NBC_CUDA(cudaFuncSetAttribute(wgrad_tc_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, WgCfg<BN>::kSmemBytes));
+    attr_set = true;
+  }
+  if (scratch == nullptr) wg_split(p, 1);
+  const size_t need = wg_scratch_bytes(p, BN);
+  if (need > scratch_bytes) {
+    set_error("wgrad_tc: scratch %zu < %zu bytes", scratch_bytes, need);
+    return NBC_ERR_WORKSPACE;
+  }
+  p.partial = need > 0 ? reinterpret_cast<float*>(scratch) : nullptr;
+  const int grid = p.co_tiles * p.ci_tiles * p.taps * p.splits;
+  wgrad_tc_kernel<BN><<<grid, kWgThreads, WgCfg<BN>::kSmemBytes, stream>>>(p);
+  NBC_CHECK_LAUNCH();
+  if (p.partial == nullptr) return 0;
+  WgReduceParams r;
+  r.partial = p.partial, r.dw = p.dw;
+  r.splits = p.splits, r.BN = BN, r.taps = p.taps, r.ci_tiles = p.ci_tiles, r.Cout = p.Cout, r.Cin = p.Cin;
+  constexpr bool kStem = WgCfg<BN>::kStem;
+  r.n = kStem ? (int64_t)7 * 64 * 21 : (int64_t)p.co_tiles * p.ci_tiles * p.taps * 128 * (BN / 4);
+  wgrad_reduce_kernel<kStem><<<(unsigned)ceil_div64(r.n, kRedLanes), dim3(kRedLanes, kRedGroups), 0, stream>>>(r);
+  NBC_CHECK_LAUNCH();
+  return 0;
+}
+
+int wgrad_tc(const ConvGeom& g, const void* dz, const void* x, float* dw, void* scratch, size_t scratch_bytes,
+             cudaStream_t stream) {
+  if (!wgrad_tc_supported(g)) {
+    set_error("wgrad_tc: unsupported shape Cin=%d Cout=%d k=%dx%d stride=%d", g.Cin, g.Cout, g.kh, g.kw, g.stride);
+    return NBC_ERR_INVALID;
+  }
+  NBC_REQUIRE((reinterpret_cast<uintptr_t>(dw) & 15) == 0, "wgrad_tc: dw must be 16-byte aligned");
+  NBC_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 15) == 0, "wgrad_tc: scratch must be 16-byte aligned");
+  WgradTcParams p;
+  memset(&p, 0, sizeof(p));
+  wg_geometry(p, g);
+  const int Ho = g.Ho(), Wo = g.Wo();
+  p.dw = dw;
+  const int bn = wg_bn(g);
 
   const uint64_t eb = 2;
   int rc = conv_encode_act_map(&p.tmDz, dz, (uint64_t)g.Cout, (uint64_t)Wo, (uint64_t)Ho, (uint64_t)g.N, (uint64_t)g.Cout * eb,
@@ -297,40 +445,21 @@ int wgrad_tc(const ConvGeom& g, const void* dz, const void* x, float* dw, cudaSt
         if (rc) return rc;
       }
   }
-  // split-K over the pixel tiles, each split with at least 16 K blocks
-  const int base_items = p.co_tiles * p.ci_tiles * p.taps;
-  // one wave: as many splits as fit the SMs once.  More, smaller splits balance better but every split adds a full tile
-  // of f32 atomics to the same gradient block (4x oversubscription cost 6 % of the training step)
-  int splits = std::max(1, sm_count() / base_items);
-  const int max_splits = ceil_div(p.num_pix_tiles, 16);
-  if (splits > max_splits) splits = max_splits;
-  if (splits < 1) splits = 1;
-  p.tiles_per_split = ceil_div(p.num_pix_tiles, splits);
-  p.splits = ceil_div(p.num_pix_tiles, p.tiles_per_split);
-  const int grid = base_items * p.splits;
   switch (bn) {
-    case 256: return launch_wgrad<256>(p, grid, stream);
-    case 128: return launch_wgrad<128>(p, grid, stream);
-    default: return launch_wgrad<64>(p, grid, stream);
+    case 256: return launch_wgrad<256>(p, scratch, scratch_bytes, stream);
+    case 128: return launch_wgrad<128>(p, scratch, scratch_bytes, stream);
+    default: return launch_wgrad<64>(p, scratch, scratch_bytes, stream);
   }
 }
 
 // stem: dW f32 [64][7][7][3] += dz^T * padded image (the bf16 staging buffer [N][Hp = 2Ho+5][Wp = 2Wo+6][4] of stem.cu)
-int stem_wgrad_tc(const void* dz, const void* padded, int N, int Ho, int Wo, float* dw, cudaStream_t stream) {
+int stem_wgrad_tc(const void* dz, const void* padded, int N, int Ho, int Wo, float* dw, void* scratch, size_t scratch_bytes,
+                  cudaStream_t stream) {
+  NBC_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 15) == 0, "stem_wgrad_tc: scratch must be 16-byte aligned");
   WgradTcParams p;
   memset(&p, 0, sizeof(p));
-  int best_tw = 64, best_tiles = INT32_MAX;
-  for (int tw = 64; tw >= 8; tw >>= 1) {
-    const int tiles = ceil_div(Wo, tw) * ceil_div(Ho, 64 / tw);
-    if (tiles < best_tiles) best_tiles = tiles, best_tw = tw;
-  }
-  p.tw = best_tw, p.th = 64 / best_tw;
-  while ((1 << p.tw_log2) < p.tw) ++p.tw_log2;
-  p.tiles_w = ceil_div(Wo, p.tw), p.tiles_h = ceil_div(Ho, p.th);
-  p.num_pix_tiles = N * p.tiles_w * p.tiles_h;
-  p.Cout = 64, p.Cin = 32, p.taps = 7;
+  wg_stem_geometry(p, N, Ho, Wo);
   p.dw = dw;
-  p.ci_tiles = 1, p.co_tiles = 1;
   const int Hp = 2 * Ho + 5, Wp = 2 * Wo + 6;
   int rc = conv_encode_act_map(&p.tmDz, dz, 64, (uint64_t)Wo, (uint64_t)Ho, (uint64_t)N, 128, (uint64_t)Wo * 128,
                                (uint64_t)Ho * Wo * 128, p.tw, p.th);
@@ -343,13 +472,7 @@ int stem_wgrad_tc(const void* dz, const void* padded, int N, int Ho, int Wo, flo
     if (rc) return rc;
   }
   for (int ky = 0; ky < 7; ++ky) p.tap_map[ky] = (int8_t)(ky & 1), p.tap_dh[ky] = (int16_t)(ky >> 1), p.tap_dw[ky] = 0;
-  int splits = ceil_div(sm_count() * 2, 7);
-  const int max_splits = ceil_div(p.num_pix_tiles, 16);
-  if (splits > max_splits) splits = max_splits;
-  if (splits < 1) splits = 1;
-  p.tiles_per_split = ceil_div(p.num_pix_tiles, splits);
-  p.splits = ceil_div(p.num_pix_tiles, p.tiles_per_split);
-  return launch_wgrad<32>(p, 7 * p.splits, stream);
+  return launch_wgrad<32>(p, scratch, scratch_bytes, stream);
 }
 
 }  // namespace nbc

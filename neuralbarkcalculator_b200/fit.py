@@ -3,7 +3,7 @@ reference's ``__main__.py:199-291``, which runs it through Poutyne).
 
     python -m neuralbarkcalculator_b200.fit ROOT --init SD.pt|random [--out best_model.pt] [--epochs 30] [--crop 512]
         [--batch 5] [--accumulate 1] [--freeze none] [--loss lovasz] [--lr 5e-4] [--weight-decay 2e-3] [--dropout 0.8]
-        [--seed 0] [--device cuda:0]
+        [--seed 0] [--device cuda:0] [--state run.state [--resume]]
     torchrun --nproc_per_node W -m neuralbarkcalculator_b200.fit ROOT ...      (data parallel, one GPU per rank)
 
 ROOT holds ``samples/<wood>/*`` and ``duals/<wood>/*`` (processed images and their dual label images, any height up to
@@ -46,7 +46,25 @@ the checkpoint's running statistics (torchvision's FrozenBatchNorm2d, with ``req
 their weights, running statistics and ``num_batches_tracked`` stay exactly as loaded, Adam and its weight decay never
 touch them, the backward stops at the first trainable block, and the epoch-end average of the running statistics over
 the ranks covers only the trainable units.  Dropout, the loss and the sampling are unchanged; the checkpoint is the same
-326-key state_dict.  Rank 0 prints the number of trainable parameters."""
+326-key state_dict.  Rank 0 prints the number of trainable parameters.
+
+Resuming an interrupted run.  With ``--state FILE``, rank 0 writes FILE at the end of every epoch, after the log row and
+the checkpoint: a format version, the run-defining arguments (the folder's items with their wood types and sizes,
+--crop --batch --accumulate, the world size, --freeze --target --loss --lr --weight-decay --dropout --plateau-*
+--early-stop-patience --seed), the epoch just finished, ``Trainer.training_state()`` (weights and running statistics,
+Adam moments, step count, learning rate, ``num_batches_tracked``), the plateau and early-stopping counters, the best
+val_miou and its state_dict, the log rows so far, the epoch-sampling ``torch.Generator`` and the augmentation
+``numpy`` generator states, and whether the run stopped early.  The file is written to a temporary file in the same
+directory, flushed, fsynced and renamed over FILE, so a kill during the write leaves the previous state intact.  At an
+epoch boundary every rank holds the same state (same all-reduced gradients, same Adam step, averaged running
+statistics); fit checks this with a digest of each rank's buffers before each write and stops if they differ.
+``--resume`` continues from FILE: it refuses, naming each field, if a run-defining argument or the folder differs
+(``--epochs``, ``--log``, ``--out``, ``--device`` and ``--init`` may change; a larger ``--epochs`` continues a finished
+run), recomputes the splits as at the start, restores all of the above, rewrites ``--log`` as the header plus the saved
+epochs' rows and ``--out`` from the saved best state_dict, and continues with the next epoch.  A run that had stopped
+early only re-runs the test evaluation.  The weight-gradient reductions are deterministic, so a resumed run writes
+exactly the log (but for ``seconds``), checkpoint and state of the run that was never interrupted (same GPU model,
+world size and library build)."""
 import argparse
 import math
 import os
@@ -89,6 +107,14 @@ class Plateau:
         return self.lr
 
 
+    def state_dict(self):
+        return {'lr': self.lr, 'best': self.best, 'num_bad_epochs': self.num_bad_epochs, 'cooldown_counter': self.cooldown_counter}
+
+    def load_state_dict(self, d):
+        self.lr, self.best = float(d['lr']), float(d['best'])
+        self.num_bad_epochs, self.cooldown_counter = int(d['num_bad_epochs']), int(d['cooldown_counter'])
+
+
 class EarlyStopping:
     """Poutyne's ``EarlyStopping(mode='min', min_delta=0)``: stop once the metric has not decreased for ``patience``
     epochs in a row."""
@@ -107,6 +133,12 @@ class EarlyStopping:
         self.wait += 1
         return self.wait >= self.patience
 
+    def state_dict(self):
+        return {'best': self.best, 'wait': self.wait}
+
+    def load_state_dict(self, d):
+        self.best, self.wait = float(d['best']), int(d['wait'])
+
 
 LOG_HEADER = ['epoch', 'lr', 'loss', 'val_loss', 'val_miou', 'val_f1_0', 'val_f1_1', 'val_f1_2', 'seconds']
 
@@ -114,6 +146,74 @@ LOG_HEADER = ['epoch', 'lr', 'loss', 'val_loss', 'val_miou', 'val_f1_0', 'val_f1
 def _log(path, fields):
     with open(path, 'a') as f:
         f.write('\t'.join(str(v) for v in fields) + '\n')
+
+
+STATE_VERSION = 1
+# run-defining fields of the state file and how a refusal names them
+RUN_FIELDS = {'version': 'the state format version', 'items': 'the folder (item names, wood types, sizes)',
+              'world': 'the world size', 'crop': '--crop', 'batch': '--batch', 'accumulate': '--accumulate',
+              'freeze': '--freeze', 'target': '--target', 'loss': '--loss', 'lr': '--lr', 'weight_decay': '--weight-decay',
+              'dropout': '--dropout', 'plateau_factor': '--plateau-factor', 'plateau_patience': '--plateau-patience',
+              'early_stop_patience': '--early-stop-patience', 'seed': '--seed'}
+
+
+def run_config(args, items, world):
+    """The arguments a resumed run must share with the run that wrote the state.  ``items``: [(name, wood type,
+    height, width)] of the folder in dataset order."""
+    cfg = {k: getattr(args, k) for k in RUN_FIELDS if hasattr(args, k)}
+    cfg.update(version=STATE_VERSION, items=[(str(n), str(w), int(h), int(wd)) for n, w, h, wd in items], world=int(world))
+    return cfg
+
+
+def check_resume(saved, current):
+    """Raise naming every run-defining field in which ``current`` differs from ``saved``."""
+    bad = [k for k in RUN_FIELDS if saved.get(k) != current.get(k)]
+    if bad:
+        def show(v):
+            return '%d items' % len(v) if isinstance(v, list) else repr(v)
+        raise RuntimeError('fit --resume: the state was written by a different run; it differs in ' + '; '.join(
+            '%s (saved %s, now %s)' % (RUN_FIELDS[k], show(saved.get(k)), show(current.get(k))) for k in bad))
+
+
+def write_state(path, state):
+    """torch.save ``state`` to ``path`` atomically: a temporary file in the same directory, flushed and fsynced, then
+    renamed over ``path``.  An exception or a kill before the rename leaves the previous file as it was."""
+    import torch
+    d = os.path.dirname(os.path.abspath(path))
+    tmp = os.path.join(d, '.%s.tmp%d' % (os.path.basename(path), os.getpid()))
+    try:
+        with open(tmp, 'wb') as f:
+            torch.save(state, f)
+            f.flush()
+            os.fsync(f.fileno())
+        os.replace(tmp, path)
+    finally:
+        if os.path.exists(tmp):
+            os.remove(tmp)
+
+
+def read_state(path):
+    import torch
+    if not os.path.isfile(path):
+        raise RuntimeError('fit --resume: no state file %s' % path)
+    return torch.load(path, map_location='cpu', weights_only=False)
+
+
+def rewrite_log(path, rows):
+    """--log as the header plus ``rows`` (the saved epochs): drops whatever a killed run appended after its last
+    state, and the test row of a finished run."""
+    with open(path, 'w') as f:
+        f.write('\t'.join(LOG_HEADER) + '\n')
+        for r in rows:
+            f.write('\t'.join(str(v) for v in r) + '\n')
+
+
+def state_digest(trainer):
+    """int64 sums of the bit patterns of the weights, statistics and Adam moments: equal on every rank when the
+    ranks hold the same training state."""
+    import torch
+    bufs = (trainer.params, trainer.stats, trainer.adam_m, trainer.adam_v)
+    return torch.stack([b.view(torch.int32).to(torch.int64).sum() for b in bufs])
 
 
 def initial_state_dict(init, dropout):
@@ -146,6 +246,10 @@ def rank_micro_batches(batches, rng, rank, accumulate, batch, n_sources, crop, t
         yield [(j, params[j * batch:(j + 1) * batch]) for j in range(rank * accumulate, (rank + 1) * accumulate)]
 
 
+def _items(ds):
+    return [(f, w, int(h), int(wd)) for f, w, (h, wd) in zip(ds.fnames, ds.wood_types, ds.sizes)]
+
+
 def main(args):
     import torch
     from . import augment, distributed as ndist, utils
@@ -168,7 +272,11 @@ def main(args):
     train_split, valid_split, test_split, train_weights = utils.get_splits(ds.split_items(), label_pixels=ds.label_pixels)
     if len(valid_split) == 0:
         raise RuntimeError('fit: the validation split is empty (a wood type needs at least 10 images for one)')
-    trainer = Trainer(initial_state_dict(args.init, args.dropout), args.batch, args.crop, args.crop, device=device,
+    saved = read_state(args.state) if args.resume else None
+    if saved is not None:
+        check_resume(saved['config'], run_config(args, _items(ds), world))
+    init_sd = saved['trainer']['model'] if saved is not None else initial_state_dict(args.init, args.dropout)
+    trainer = Trainer(init_sd, args.batch, args.crop, args.crop, device=device,
                       lr=args.lr, weight_decay=args.weight_decay, dropout=args.dropout, loss=args.loss, seed=args.seed,
                       freeze=args.freeze)
     if rank == 0:
@@ -178,12 +286,28 @@ def main(args):
     rng = np.random.default_rng(args.seed)
     plateau = Plateau(args.lr, factor=args.plateau_factor, patience=args.plateau_patience)
     stopper = EarlyStopping(args.early_stop_patience)
-    if rank == 0:
-        with open(args.log, 'w') as f:
-            f.write('\t'.join(LOG_HEADER) + '\n')
     global_batch = world * args.accumulate * args.batch
-    best_miou, best_sd = -math.inf, None
-    for epoch in range(1, args.epochs + 1):
+    best_miou, best_sd, log_rows, first_epoch, stopped = -math.inf, None, [], 1, False
+    if saved is not None:
+        trainer.load_training_state(saved['trainer'])
+        plateau.load_state_dict(saved['plateau'])
+        stopper.load_state_dict(saved['early_stopping'])
+        generator.set_state(saved['generator'])
+        rng.bit_generator.state = saved['rng']
+        best_miou, best_sd, log_rows = saved['best_miou'], saved['best_model'], saved['log']
+        first_epoch, stopped = saved['epoch'] + 1, saved['stopped']
+        if rank == 0:
+            if best_sd is not None:
+                torch.save(best_sd, args.out)
+            print('fit: resuming from %s after epoch %d%s' % (args.state, saved['epoch'],
+                  ' (the run had stopped early: only the test evaluation runs)' if stopped else ''), flush=True)
+        del saved
+    if rank == 0:
+        rewrite_log(args.log, log_rows)
+    reported = False
+    for epoch in range(first_epoch, args.epochs + 1):
+        if stopped:
+            break
         t0 = time.perf_counter()
         lr = trainer.lr
         batches = utils.weighted_epoch_batches(train_split, train_weights, global_batch, generator=generator)
@@ -205,9 +329,11 @@ def main(args):
             sd = trainer.state_dict()
             val = evaluate_sharded(make_plan(sd, trainer.device), ds, valid_split, loss=args.loss,
                                    class_weights=trainer.class_weights)
+        row = ([epoch, repr(lr), repr(train_loss), repr(val['loss']), repr(val['miou'])] + [repr(float(v)) for v in val['f1']]
+               + ['%.3f' % (time.perf_counter() - t0)])
+        log_rows.append(row)
         if rank == 0:
-            _log(args.log, [epoch, repr(lr), repr(train_loss), repr(val['loss']), repr(val['miou'])]
-                 + [repr(float(v)) for v in val['f1']] + ['%.3f' % (time.perf_counter() - t0)])
+            _log(args.log, row)
             print('fit: epoch %d: %d steps of %d samples, training %.3f s, validation %.3f s'
                   % (epoch, len(batches), global_batch, t_train, time.perf_counter() - t0 - t_train), flush=True)
         if val['miou'] > best_miou:
@@ -217,7 +343,28 @@ def main(args):
                 torch.save(best_sd, args.out)
         del sd
         trainer.lr = plateau.step(val['loss'])
-        if stopper.step(val['loss']):
+        stopped = stopper.step(val['loss'])
+        if args.state:
+            if world > 1:
+                with torch.cuda.device(trainer.device):
+                    digest = state_digest(trainer)
+                    lo, hi = digest.clone(), digest.clone()
+                    dist.all_reduce(lo, op=dist.ReduceOp.MIN)
+                    dist.all_reduce(hi, op=dist.ReduceOp.MAX)
+                    if not torch.equal(lo, hi):
+                        raise RuntimeError('fit: the ranks hold different training states after epoch %d' % epoch)
+            if rank == 0:
+                t1 = time.perf_counter()
+                write_state(args.state, {
+                    'config': run_config(args, _items(ds), world), 'epoch': epoch, 'trainer': trainer.training_state(),
+                    'plateau': plateau.state_dict(), 'early_stopping': stopper.state_dict(), 'best_miou': best_miou,
+                    'best_model': best_sd, 'log': log_rows, 'generator': generator.get_state(),
+                    'rng': rng.bit_generator.state, 'stopped': stopped})
+                if not reported:
+                    print('fit: state %s: %.1f MB, written in %.3f s' % (
+                        args.state, os.path.getsize(args.state) / 1e6, time.perf_counter() - t1), flush=True)
+                    reported = True
+        if stopped:
             break
     if len(test_split):
         t0 = time.perf_counter()
@@ -255,6 +402,8 @@ def parse_args(argv=None):
     parser.add_argument('--early-stop-patience', type=int, default=20)
     parser.add_argument('--seed', type=int, default=0)
     parser.add_argument('--device', default='cuda:0', help='CUDA device (cuda, cuda:N); under torchrun cuda:LOCAL_RANK')
+    parser.add_argument('--state', default=None, help='training state written at the end of every epoch (for --resume)')
+    parser.add_argument('--resume', action='store_true', help='continue the run whose --state file is given')
     args = parser.parse_args(argv)
     if not args.device.startswith('cuda'):
         parser.error('--device %s: only CUDA devices are supported (no CPU path)' % args.device)
@@ -262,7 +411,9 @@ def parse_args(argv=None):
         parser.error('--epochs and --batch must be positive and --crop within [1, --target]')
     if args.accumulate < 1:
         parser.error('--accumulate must be at least 1')
-    if args.freeze != 'none' and args.init == 'random':
+    if args.resume and not args.state:
+        parser.error('--resume needs --state FILE')
+    if args.freeze != 'none' and args.init == 'random' and not args.resume:
         parser.error('--freeze %s needs --init SD.pt: freezing randomly initialised layers is almost certainly a mistake'
                      % args.freeze)
     return args

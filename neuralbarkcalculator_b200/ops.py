@@ -246,9 +246,12 @@ def conv_dual_bf16(x, w, x2, w2, bias, stride2=1, relu=True):
     return y
 
 
-def conv_wgrad_bf16(dz, x, kh, kw, stride=1, pad=0, dil=1, impl=0, out=None):
+def conv_wgrad_bf16(dz, x, kh, kw, stride=1, pad=0, dil=1, impl=0, out=None, split=True):
     """Weight gradient of conv_bf16: dz bf16 NHWC [N,Ho,Wo,Cout], x bf16 NHWC [N,H,W,Cin] -> f32 [Cout,kh,kw,Cin]
-    (accumulated into ``out`` when given).  impl 0 auto, 1 tcgen05, 2 mma.sync."""
+    (accumulated into ``out`` when given).  impl 0 auto, 1 tcgen05, 2 mma.sync.  The tcgen05 kernel runs as the
+    training plan runs it: the pixels split over the SMs, the partials in a scratch buffer allocated here and added in a
+    fixed order (``nbc_conv_wgrad_bf16_ws``); ``split=False`` makes one CTA per weight tile sum every pixel
+    (``nbc_conv_wgrad_bf16`` without scratch).  Both are bit-reproducible; the mma.sync kernel is not."""
     lib = _lib.load()
     dz = _contig(dz, torch.bfloat16, 'dz')
     x = _contig(x, torch.bfloat16, 'x')
@@ -264,7 +267,13 @@ def conv_wgrad_bf16(dz, x, kh, kw, stride=1, pad=0, dil=1, impl=0, out=None):
         else:
             out = _contig(out, torch.float32, 'out')
         d = _lib.ConvDesc(N, H, W, Cin, Cout, kh, kw, stride, pad, dil, 0, impl, 0)
-        _lib.check(lib.nbc_conv_wgrad_bf16(C.byref(d), _ptr(dz), _ptr(x), _ptr(out), _stream(x.device)), 'nbc_conv_wgrad_bf16')
+        n = lib.nbc_conv_wgrad_workspace_bytes(C.byref(d)) if split and impl != 2 else 0    # 0: no split (or no tcgen05)
+        if n > 0:
+            ws = torch.empty(n, dtype=torch.uint8, device=x.device)
+            _lib.check(lib.nbc_conv_wgrad_bf16_ws(C.byref(d), _ptr(dz), _ptr(x), _ptr(out), _ptr(ws), n, _stream(x.device)),
+                       'nbc_conv_wgrad_bf16_ws')
+        else:
+            _lib.check(lib.nbc_conv_wgrad_bf16(C.byref(d), _ptr(dz), _ptr(x), _ptr(out), _stream(x.device)), 'nbc_conv_wgrad_bf16')
     return out
 
 

@@ -172,6 +172,47 @@ class Trainer:
                 sd[k].fill_(self.num_batches_tracked.get(k, 0))
         return sd
 
+    def _moments(self, flat):
+        """An Adam moment buffer in state_dict layout (a pure permutation of the flat buffer: bit-exact both ways)."""
+        with torch.cuda.device(self.device):
+            sd = self._template()
+            self._exchange([sd[k] for k in self.keys], flat, None, 1)
+        return {k: v for k, v in sd.items() if 'running' not in k and 'num_batches' not in k}
+
+    def training_state(self):
+        """Everything the next optimizer steps depend on, in state_dict layout (independent of the plan's internal
+        buffer layout): ``model`` (the 326-key state_dict), ``adam_m`` / ``adam_v`` (per parameter key; a frozen unit's
+        moments are zero), ``step_count``, ``lr`` and ``num_batches_tracked``.  Tensors are on the CPU."""
+        if self.micro_batches:
+            raise RuntimeError('training_state: %d micro-batches are accumulated but not applied; take it after '
+                               'optimizer_step' % self.micro_batches)
+        cpu = lambda d: {k: v.cpu() for k, v in d.items()}
+        return {'model': cpu(self.state_dict()), 'adam_m': cpu(self._moments(self.adam_m)),
+                'adam_v': cpu(self._moments(self.adam_v)), 'step_count': int(self.step_count), 'lr': float(self.lr),
+                'num_batches_tracked': dict(self.num_batches_tracked)}
+
+    def load_training_state(self, state):
+        """Restore ``training_state()``: afterwards ``params``, ``stats``, ``adam_m`` and ``adam_v`` are bit-identical to
+        the trainer that produced it, and so are the following steps (same inputs, same seeds)."""
+        if sorted(state['model']) != sorted(self.keys):
+            raise RuntimeError('load_training_state: the model is not the 326-key fcn_resnet50 state_dict')
+        moment_keys = [k for k in self.keys if 'running' not in k and 'num_batches' not in k]
+        for name in ('adam_m', 'adam_v'):
+            if sorted(state[name]) != sorted(moment_keys):
+                raise RuntimeError('load_training_state: %s does not hold the %d parameter keys' % (name, len(moment_keys)))
+        with torch.cuda.device(self.device):
+            self._exchange(self._device_tensors(state['model']), self.params, self.stats, 0)
+            for name, flat in (('adam_m', self.adam_m), ('adam_v', self.adam_v)):
+                sd = dict(state['model'])
+                sd.update(state[name])
+                flat.zero_()
+                self._exchange(self._device_tensors(sd), flat, None, 0)
+                flat[:self.param_off].zero_()      # frozen units carry no moments
+        self.step_count = int(state['step_count'])
+        self.lr = float(state['lr'])
+        self.num_batches_tracked = {k: int(v) for k, v in state['num_batches_tracked'].items()}
+        self.micro_batches = 0
+
     def gradients(self):
         """Gradients of the last forward_backward in state_dict layout (OIHW conv weights; BN weight / bias; classifier)."""
         with torch.cuda.device(self.device):
