@@ -174,6 +174,25 @@ int nbc_upsample_bicubic(const float* logits, int N, int C, int h, int w, int H,
  * occupy ceil(heights[n]/8) rows of the [N,3,hc,w] logits canvas.  Rows beyond the valid height are not written. */
 int nbc_upsample_argmax_ragged(const float* logits, int N, int hc, int w, int Hc, int W, const int32_t* heights,
                                uint8_t* mask, void* stream);
+/* ---- flip test-time augmentation  (models.py:38-41, 270 over a set of mirrored views) ----------------------------
+ * nbc_flip_ragged_u8: dst u8 [N,Hc,W,3] = src with image n mirrored within its own rows [0, heights[n]) (flags & 2) and
+ * the W columns (flags & 1); rows heights[n]..Hc-1 of dst are written as zeros.  Bit-identical to torch.flip of each
+ * image.  flags 0..3 (0 copies); dst may not be src.  The network then runs unchanged on dst (nbc_plan_forward_ragged).
+ * The view set: logits / flips are HOST arrays of V = 1, 2 or 4 entries -- view v's low-resolution logits canvas
+ * [N,3,hc,w] (the network's output for the batch mirrored with flips[v], flags 0..3) -- anything else is refused.
+ * Per output pixel (Y, X) of image n, L_v = K3's f32 bicubic value of view v at the mirrored pixel
+ * (flips[v] & 2 ? H_n-1-Y : Y, flips[v] & 1 ? W-1-X : X) (same taps, weights and operation order), and
+ *   mean = (((L_0 + L_1) + L_2) + L_3) * (1/V)       f32, round-to-nearest, in view order; V = 1: L_0 unscaled
+ * nbc_upsample_argmax_views_ragged: mask u8 [N,Hc,W] = argmax_c mean (ties -> lowest class), rows [0, heights[n]) only.
+ * nbc_upsample_bicubic_views_ragged: out f32 [N,3,Hc,W] = mean, rows [0, heights[n]) only.
+ * nbc_eval_ragged_views: nbc_eval_ragged with the view set in place of its logits canvas: the same outputs, each computed
+ * from the mean logits, and the same workspace (nbc_eval_workspace_bytes).
+ * None of them allocates. */
+int nbc_flip_ragged_u8(const uint8_t* src, uint8_t* dst, int N, int Hc, int W, const int32_t* heights, int flags, void* stream);
+int nbc_upsample_argmax_views_ragged(const float* const* logits, const int32_t* flips, int V, int N, int hc, int w, int Hc, int W,
+                                     const int32_t* heights, uint8_t* mask, void* stream);
+int nbc_upsample_bicubic_views_ragged(const float* const* logits, const int32_t* flips, int V, int N, int hc, int w, int Hc,
+                                      int W, const int32_t* heights, float* out, void* stream);
 /* heights[n] = last - first from the {first,last}[N] pairs written by nbc_preprocess_4x_u8 (device -> device) */
 int nbc_heights_from_first_last(const int32_t* first_last, int N, int32_t* heights, void* stream);
 
@@ -231,6 +250,11 @@ size_t nbc_eval_workspace_bytes(int N, int Hc, int W);
 int nbc_eval_ragged(const float* logits, int N, int Hc, int W, const int32_t* heights, const uint8_t* labels,
                     const float* weights3, int losses, float* loss_wce, float* loss_lovasz, uint64_t* cm_raw, uint64_t* cm_rsz,
                     int32_t* counts, void* workspace, size_t workspace_bytes, void* stream);
+
+int nbc_eval_ragged_views(const float* const* logits, const int32_t* flips, int V, int N, int Hc, int W, const int32_t* heights,
+                          const uint8_t* labels, const float* weights3, int losses, float* loss_wce, float* loss_lovasz,
+                          uint64_t* cm_raw, uint64_t* cm_rsz, int32_t* counts, void* workspace, size_t workspace_bytes,
+                          void* stream);
 
 /* ---- N4: training-time augmentation of a batch  (__main__.py:153-176 get_loader_for_crop_batch; dataset.py:171-193) --
  * images u8 [M,Hs,Ws,3] and their dual label images u8 [M,Hs,Ws] (0/127/255) resident on the device; for each of the B

@@ -65,6 +65,11 @@ SIGNATURES = {
     'nbc_upsample_argmax': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     'nbc_upsample_bicubic': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     'nbc_upsample_argmax_ragged': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    'nbc_flip_ragged_u8': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p]),
+    'nbc_upsample_argmax_views_ragged': (c_int, [C.POINTER(c_void_p), C.POINTER(C.c_int32), c_int, c_int, c_int, c_int, c_int, c_int,
+                                         c_void_p, c_void_p, c_void_p]),
+    'nbc_upsample_bicubic_views_ragged': (c_int, [C.POINTER(c_void_p), C.POINTER(C.c_int32), c_int, c_int, c_int, c_int, c_int, c_int,
+                                          c_void_p, c_void_p, c_void_p]),
     'nbc_heights_from_first_last': (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     'nbc_ccl_workspace_bytes': (c_size_t, [c_int, c_int, c_int]),
     'nbc_remove_small_zones': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
@@ -80,6 +85,8 @@ SIGNATURES = {
     'nbc_eval_workspace_bytes': (c_size_t, [c_int, c_int, c_int]),
     'nbc_eval_ragged': (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
                         c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    'nbc_eval_ragged_views': (c_int, [C.POINTER(c_void_p), C.POINTER(C.c_int32), c_int, c_int, c_int, c_int, c_void_p, c_void_p,
+                              c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     'nbc_augment_batch': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p,
                           c_void_p]),
     'nbc_augment_ragged': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int,

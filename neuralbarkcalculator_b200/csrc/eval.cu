@@ -29,6 +29,7 @@ namespace nbc {
 constexpr int kEvalThreshold = 150;   // utils.py:135-148, PixelWiseF1's region removal
 
 struct EvalSink {
+  static constexpr bool kMask = true;
   const uint8_t* __restrict__ labels;   // [N,Hc,W]
   const int* __restrict__ off;          // [N+1] first compact pixel of each image
   const float* __restrict__ weights;    // [3] class weights of the weighted CE
@@ -240,11 +241,12 @@ extern "C" size_t nbc_eval_workspace_bytes(int N, int Hc, int W) {
   return eval_layout(N, Hc, W).total;
 }
 
-extern "C" int nbc_eval_ragged(const float* logits, int N, int Hc, int W, const int32_t* heights, const uint8_t* labels,
-                               const float* weights3, int losses, float* loss_wce, float* loss_lovasz, uint64_t* cm_raw,
-                               uint64_t* cm_rsz, int32_t* counts, void* workspace, size_t workspace_bytes, void* stream_) {
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  NBC_REQUIRE(logits && heights && labels && loss_wce && loss_lovasz && cm_raw && cm_rsz && counts && workspace,
+namespace nbc {
+// nbc_eval_ragged on a view set (K3Views, V = 1, 2 or 4, checked by the caller): K3's sink sees the mean of the views
+static int eval_ragged_views(const K3Views& views, int V, int N, int Hc, int W, const int32_t* heights, const uint8_t* labels,
+                             const float* weights3, int losses, float* loss_wce, float* loss_lovasz, uint64_t* cm_raw,
+                             uint64_t* cm_rsz, int32_t* counts, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  NBC_REQUIRE(heights && labels && loss_wce && loss_lovasz && cm_raw && cm_rsz && counts && workspace,
               "nbc_eval_ragged: null pointer");
   NBC_REQUIRE(N >= 1, "nbc_eval_ragged: N must be at least 1 (got %d)", N);
   NBC_REQUIRE(eval_shape_ok(N, Hc, W),
@@ -287,8 +289,7 @@ extern "C" int nbc_eval_ragged(const float* logits, int N, int Hc, int W, const 
   EvalSink sink;
   sink.labels = labels, sink.off = off, sink.weights = weights3, sink.losses = losses, sink.Hc = Hc, sink.W = W;
   sink.wce = wce, sink.keys = keys_in, sink.vals = vals_in, sink.cm = cm0;
-  upsample_argmax_rows_kernel<EvalSink><<<dim3(ceil_div(W, 256), ceil_div(Hc, kK3Rows), N), 256, 0, stream>>>(
-      logits, hc, w, Hc, W, 0, (float)w / (float)W, heights, mask, sink);
+  launch_k3(V, views, N, hc, w, Hc, W, 0, heights, mask, sink, stream);
   NBC_CHECK_LAUNCH();
 
   int total = 0;
@@ -321,4 +322,24 @@ extern "C" int nbc_eval_ragged(const float* logits, int N, int Hc, int W, const 
                                                                                                  off, cm1);
   NBC_CHECK_LAUNCH();
   return 0;
+}
+}  // namespace nbc
+
+extern "C" int nbc_eval_ragged(const float* logits, int N, int Hc, int W, const int32_t* heights, const uint8_t* labels,
+                               const float* weights3, int losses, float* loss_wce, float* loss_lovasz, uint64_t* cm_raw,
+                               uint64_t* cm_rsz, int32_t* counts, void* workspace, size_t workspace_bytes, void* stream) {
+  NBC_REQUIRE(logits, "nbc_eval_ragged: null pointer");
+  return eval_ragged_views(k3_one(logits), 1, N, Hc, W, heights, labels, weights3, losses, loss_wce, loss_lovasz, cm_raw, cm_rsz,
+                           counts, workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int nbc_eval_ragged_views(const float* const* logits, const int32_t* flips, int V, int N, int Hc, int W,
+                                     const int32_t* heights, const uint8_t* labels, const float* weights3, int losses,
+                                     float* loss_wce, float* loss_lovasz, uint64_t* cm_raw, uint64_t* cm_rsz, int32_t* counts,
+                                     void* workspace, size_t workspace_bytes, void* stream) {
+  K3Views views;
+  const int rc = k3_views_args(logits, flips, V, views, "nbc_eval_ragged_views");
+  if (rc != 0) return rc;
+  return eval_ragged_views(views, V, N, Hc, W, heights, labels, weights3, losses, loss_wce, loss_lovasz, cm_raw, cm_rsz, counts,
+                           workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
 }

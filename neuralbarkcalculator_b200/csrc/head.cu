@@ -133,10 +133,83 @@ extern "C" int nbc_upsample_argmax_ragged(const float* logits, int N, int hc, in
                                           uint8_t* mask, void* stream) {
   NBC_REQUIRE(logits && heights && mask, "nbc_upsample_argmax_ragged: null pointer");
   NBC_REQUIRE(N > 0 && hc > 0 && w > 0 && Hc > 0 && W > 0 && Hc <= 65535 && N <= 65535, "nbc_upsample_argmax_ragged: bad shape");
-  dim3 grid(ceil_div(W, 256), ceil_div(Hc, kK3Rows), N);
-  upsample_argmax_rows_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(logits, hc, w, Hc, W, 0,
-                                                                                         (float)w / (float)W, heights, mask,
-                                                                                         K3Mask());
+  launch_k3(1, k3_one(logits), N, hc, w, Hc, W, 0, heights, mask, K3Mask(), reinterpret_cast<cudaStream_t>(stream));
+  NBC_CHECK_LAUNCH();
+  return 0;
+}
+
+namespace nbc {
+// The full-resolution logits sink of the view set: f32 [N,3,Hc,W], rows [0, H_n) of image n.
+struct K3Logits {
+  static constexpr bool kMask = false;
+  struct Acc {};
+  float* __restrict__ out;
+  int Hc, W;
+  __device__ __forceinline__ void pixel(Acc&, int n, int, int Y, int X, const float (&v)[3], int) const {
+    const int64_t plane = (int64_t)Hc * W, at = (int64_t)n * 3 * plane + (int64_t)Y * W + X;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) out[at + c * plane] = v[c];
+  }
+  __device__ __forceinline__ void flush(Acc&, int) const {}
+};
+
+// dst image n = src image n mirrored within its rows [0, H_n) (flags & 2) and the W columns (flags & 1); rows H_n..Hc-1
+// of dst are zero.  One block per (canvas row, image); bytes of a row are independent, so threads stride over them.
+__global__ void __launch_bounds__(256) flip_ragged_kernel(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst, int Hc, int W,
+                                                          const int* __restrict__ heights, int flags) {
+  const int y = blockIdx.x, n = blockIdx.y;
+  const int H = min(max(__ldg(heights + n), 1), Hc);
+  const int64_t row = 3ll * W;
+  uint8_t* d = dst + ((int64_t)n * Hc + y) * row;
+  if (y >= H) {
+    for (int i = threadIdx.x; i < (int)row; i += blockDim.x) d[i] = 0;
+    return;
+  }
+  const uint8_t* s = src + ((int64_t)n * Hc + ((flags & 2) ? H - 1 - y : y)) * row;
+  for (int i = threadIdx.x; i < (int)row; i += blockDim.x) {
+    const int x = i / 3, ch = i - 3 * x;
+    d[i] = __ldg(s + ((flags & 1) ? 3 * (W - 1 - x) + ch : i));
+  }
+}
+
+}  // namespace nbc
+
+extern "C" int nbc_flip_ragged_u8(const uint8_t* src, uint8_t* dst, int N, int Hc, int W, const int32_t* heights, int flags,
+                                  void* stream) {
+  NBC_REQUIRE(src && dst && heights, "nbc_flip_ragged_u8: null pointer");
+  NBC_REQUIRE(src != dst, "nbc_flip_ragged_u8: src and dst must not be the same canvas");
+  NBC_REQUIRE(N > 0 && Hc > 0 && W > 0 && N <= 65535 && 3ll * W < (1ll << 31), "nbc_flip_ragged_u8: bad shape N=%d Hc=%d W=%d",
+              N, Hc, W);
+  NBC_REQUIRE(flags >= 0 && flags <= 3, "nbc_flip_ragged_u8: flags is 1 (columns), 2 (rows) or 3 (both), got %d", flags);
+  flip_ragged_kernel<<<dim3(Hc, N), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(src, dst, Hc, W, heights, flags);
+  NBC_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int nbc_upsample_argmax_views_ragged(const float* const* logits, const int32_t* flips, int V, int N, int hc, int w, int Hc,
+                                                int W, const int32_t* heights, uint8_t* mask, void* stream) {
+  K3Views views;
+  const int rc = k3_views_args(logits, flips, V, views, "nbc_upsample_argmax_views_ragged");
+  if (rc != 0) return rc;
+  NBC_REQUIRE(heights && mask, "nbc_upsample_argmax_views_ragged: null pointer");
+  NBC_REQUIRE(N > 0 && hc > 0 && w > 0 && Hc > 0 && W > 0 && Hc <= 65535 * kK3Rows && N <= 65535,
+              "nbc_upsample_argmax_views_ragged: bad shape");
+  launch_k3(V, views, N, hc, w, Hc, W, 0, heights, mask, K3Mask(), reinterpret_cast<cudaStream_t>(stream));
+  NBC_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int nbc_upsample_bicubic_views_ragged(const float* const* logits, const int32_t* flips, int V, int N, int hc, int w,
+                                                 int Hc, int W, const int32_t* heights, float* out, void* stream) {
+  K3Views views;
+  const int rc = k3_views_args(logits, flips, V, views, "nbc_upsample_bicubic_views_ragged");
+  if (rc != 0) return rc;
+  NBC_REQUIRE(heights && out, "nbc_upsample_bicubic_views_ragged: null pointer");
+  NBC_REQUIRE(N > 0 && hc > 0 && w > 0 && Hc > 0 && W > 0 && Hc <= 65535 * kK3Rows && N <= 65535,
+              "nbc_upsample_bicubic_views_ragged: bad shape");
+  K3Logits sink;
+  sink.out = out, sink.Hc = Hc, sink.W = W;
+  launch_k3(V, views, N, hc, w, Hc, W, 0, heights, nullptr, sink, reinterpret_cast<cudaStream_t>(stream));
   NBC_CHECK_LAUNCH();
   return 0;
 }
@@ -176,8 +249,7 @@ static int upsample_common(const float* logits, int N, int C, int h, int w, int 
   const float sy = (float)h / (float)H, sx = (float)w / (float)W;  // IEEE f32 division, as torch
   dim3 grid(ceil_div(W, 256), H, N);
   if (mask && C == 3)
-    upsample_argmax_rows_kernel<<<dim3(ceil_div(W, 256), ceil_div(H, kK3Rows), N), 256, 0, stream>>>(logits, h, w, H, W, h, sx, nullptr,
-                                                                                                    mask, K3Mask());
+    launch_k3(1, k3_one(logits), N, h, w, H, W, h, nullptr, mask, K3Mask(), stream);
   else if (mask)
     upsample_kernel<true><<<grid, 256, 0, stream>>>(logits, N, C, h, w, H, W, sy, sx, mask, nullptr);
   else

@@ -63,14 +63,16 @@ class Ticket:
 
 class PredictEngine:
     """chunk: images per ragged batch (one network launch sequence per chunk); default DEFAULT_CHUNK, or the
-    environment variable NBC_CHUNK."""
+    environment variable NBC_CHUNK.  tta: flip test-time augmentation, 'none', 'h' or 'hv' (``ops.tta_views``): a chunk
+    runs the network once per view and K3 averages the views' logits."""
 
-    def __init__(self, model, device='cuda:0', threshold=150, raw_size=4096, chunk=None, depth=None):
+    def __init__(self, model, device='cuda:0', threshold=150, raw_size=4096, chunk=None, depth=None, tta='none'):
         if chunk is None:
             chunk = int(os.environ.get('NBC_CHUNK', DEFAULT_CHUNK))
         if depth is None:      # staging buffers (NBC_STAGE_DEPTH counts chunks)
             depth = int(os.environ.get('NBC_STAGE_DEPTH', DEFAULT_STAGE_DEPTH)) * chunk
         self.model = model
+        self.tta_flags = ops.tta_views(tta)[1]
         self.device = torch.device(device)
         self.threshold = threshold
         self.raw_size = raw_size
@@ -117,8 +119,12 @@ class PredictEngine:
         self._ccl_ws = torch.empty(lib.nbc_ccl_workspace_bytes(self.chunk, Hc, Wo), dtype=torch.uint8, device=dev)
         hl = (((Hc - 1) // 2 + 1 - 1) // 2 + 1 - 1) // 2 + 1
         wl = (((Wo - 1) // 2 + 1 - 1) // 2 + 1 - 1) // 2 + 1
-        self._logits = [torch.empty((self.chunk, 3, hl, wl), dtype=torch.float32, device=dev) for _ in range(2)]
+        # per logits buffer (two, alternating over chunks) one canvas per view; the mirrored copies of a chunk's images share
+        # one scratch canvas (the views' network passes run one after another on the main stream)
+        V = len(self.tta_flags)
+        self._logits = [[torch.empty((self.chunk, 3, hl, wl), dtype=torch.float32, device=dev) for _ in range(V)] for _ in range(2)]
         self._logits_free = [None, None]
+        self._flipped = torch.empty((self.chunk, Hc, Wo, 3), dtype=torch.uint8, device=dev) if V > 1 else None
         return True
 
     def _standard_buffers(self):
@@ -182,7 +188,8 @@ class PredictEngine:
         """Images a..b-1 as ONE ragged batch: network, K3 and K5 read the per-image heights on the device.  The network
         runs on the main stream; K3 (upsample+argmax) and K5 (region removal + counts) follow on the post stream (two
         logits buffers).  proc / masks: the chunk's canvases when they are narrower than the slot's (mixed path).
-        Returns the event that marks the chunk's masks and counts as final."""
+        With several views the main stream runs flip + network per view (the identity view reads proc itself) and K3
+        averages them.  Returns the event that marks the chunk's masks and counts as final."""
         proc = slot.proc[a:b] if proc is None else proc
         masks = slot.masks[a:b] if masks is None else masks
         plan = self.model.native_plan()
@@ -192,22 +199,30 @@ class PredictEngine:
         if self._logits_free[k] is not None:
             main.wait_event(self._logits_free[k])        # K3 of two chunks ago has consumed this logits buffer
         Hc, W = masks.shape[1], masks.shape[2]
-        lg = self._logits[k]
-        if W == self.out_w:
-            lg = lg[:b - a]
-        else:        # a narrower canvas: its logits, ceil(W / 8) wide, in the front of the same buffer
-            lg = lg.view(-1)[:(b - a) * 3 * lg.shape[2] * ((W + 7) // 8)].view(b - a, 3, lg.shape[2], (W + 7) // 8)
-        logits = plan.forward_ragged(proc, heights=slot.heights[a:b], out=lg)
+        heights = slot.heights[a:b]
+        logits = []
+        for lg, flags in zip(self._logits[k], self.tta_flags):
+            if W == self.out_w:
+                lg = lg[:b - a]
+            else:        # a narrower canvas: its logits, ceil(W / 8) wide, in the front of the same buffer
+                lg = lg.view(-1)[:(b - a) * 3 * lg.shape[2] * ((W + 7) // 8)].view(b - a, 3, lg.shape[2], (W + 7) // 8)
+            src = proc
+            if flags:
+                src = ops.flip_ragged(proc, heights, flags, out=self._flipped.view(-1)[:proc.numel()].view(proc.shape))
+            logits.append(plan.forward_ragged(src, heights=heights, out=lg))
         net_done = torch.cuda.Event()
         net_done.record(main)
         done = torch.cuda.Event()
         with torch.cuda.stream(self._post_stream):
             self._post_stream.wait_event(net_done)
-            ops.upsample_argmax_ragged(logits, slot.heights[a:b], (Hc, W), out=masks)
+            if len(logits) == 1:
+                ops.upsample_argmax_ragged(logits[0], heights, (Hc, W), out=masks)
+            else:
+                ops.upsample_argmax_views_ragged(logits, self.tta_flags, heights, (Hc, W), out=masks)
             free = torch.cuda.Event()
             free.record(self._post_stream)
             self._logits_free[k] = free
-            ops.remove_small_zones_ragged(masks, slot.heights[a:b], self.threshold, exclude_nodes,
+            ops.remove_small_zones_ragged(masks, heights, self.threshold, exclude_nodes,
                                           workspace=self._ccl_ws, counts=slot.counts[a:b])
             done.record(self._post_stream)
         return done

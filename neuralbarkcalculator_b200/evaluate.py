@@ -15,11 +15,15 @@ forward of that image alone) and one ``ops.eval_ragged`` call, which gives every
 region-removal counts exactly as the per-image ops would (bicubic upsample, loss forward, argmax, confusion matrix,
 region removal); everything is read back once at the end.
 
+With ``tta`` ('h' or 'hv', ``ops.tta_views``) a chunk runs one ``ops.flip_ragged`` per mirrored view and one network pass
+per view, and ``ops.eval_ragged_views`` scores the views' mean logits (each view flipped back after the bicubic upsample):
+the same figures for the test-time-augmented prediction ``predict --tta`` writes.
+
 As a command, it scores a checkpoint on a labelled folder and writes one row per image (see ``main``):
 
     python -m neuralbarkcalculator_b200.evaluate ROOT --model best_model.pt [--split all|train|valid|test] [--seed 0]
         [--loss lovasz|weighted_ce|mixed] [--exclude_nodes] [--chunk 8] [--block 256] [--out evaluation.tsv]
-        [--device cuda:0]"""
+        [--device cuda:0] [--tta none|h|hv]"""
 import argparse
 import os
 
@@ -87,11 +91,13 @@ def image_row(index, loss, ce, lov, cm_raw, cm_rsz, counts):
             'cm_rsz': cm_rsz, 'counts': counts}
 
 
-def evaluate_plan(plan, ds, indices, loss='lovasz', class_weights=None, chunk=8):
+def evaluate_plan(plan, ds, indices, loss='lovasz', class_weights=None, chunk=8, tta='none'):
     """``evaluate`` with a plan made beforehand: one ``forward_ragged`` and one ``ops.eval_ragged`` per chunk of up to
     ``chunk`` equally wide images, one read-back at the end.  Rows are grouped by width, as ``image_logits`` yields them;
     besides 'index', 'loss', 'miou' and 'f1' each row has 'iou' (the three per-class IoU behind 'miou'), 'cm_rsz' (the
-    3x3 confusion matrix after region removal, behind 'f1') and 'counts' (the class counts of that mask)."""
+    3x3 confusion matrix after region removal, behind 'f1') and 'counts' (the class counts of that mask).  tta 'h' / 'hv':
+    one flip and one ``forward_ragged`` per view, then one ``ops.eval_ragged_views`` per chunk."""
+    flags = ops.tta_views(tta)[1]
     if loss not in LOSSES:
         raise ValueError("loss must be 'weighted_ce', 'lovasz' or 'mixed'")
     if len(indices) == 0:
@@ -110,12 +116,15 @@ def evaluate_plan(plan, ds, indices, loss='lovasz', class_weights=None, chunk=8)
             heights = torch.tensor(hs, dtype=torch.int32, device=dev)
             canvas = ds.images.index_select(0, sel)[:, :max(hs), :w].contiguous()
             labels = ds.classes.index_select(0, sel)[:, :max(hs), :w].contiguous()
-            low = plan.forward_ragged(canvas, heights=heights)
+            lows = [plan.forward_ragged(canvas if f == 0 else ops.flip_ragged(canvas, heights, f), heights=heights) for f in flags]
             need = ops._lib.load().nbc_eval_workspace_bytes(len(part), max(hs), w)
             if ws is None or ws.numel() < need:
                 ws = None
                 ws = torch.empty(need, dtype=torch.uint8, device=dev)
-            outs.append(ops.eval_ragged(low, heights, labels, wts, bits, workspace=ws))
+            if len(lows) == 1:
+                outs.append(ops.eval_ragged(lows[0], heights, labels, wts, bits, workspace=ws))
+            else:
+                outs.append(ops.eval_ragged_views(lows, flags, heights, labels, wts, bits, workspace=ws))
             order.extend(part)
         host = {k: torch.cat([o[k] for o in outs]).cpu().numpy() for k in outs[0]}
     rows = [image_row(i, loss, host['loss_wce'][j], host['loss_lovasz'][j], host['cm_raw'][j], host['cm_rsz'][j],
@@ -134,7 +143,7 @@ def width_order(ds, indices):
     return [i for _, part in _width_chunks(ds, [int(i) for i in indices], max(len(indices), 1)) for i in part]
 
 
-def evaluate_sharded(plan, ds, indices, loss='lovasz', class_weights=None, chunk=8):
+def evaluate_sharded(plan, ds, indices, loss='lovasz', class_weights=None, chunk=8, tta='none'):
     """``evaluate_plan`` spread over the ranks of the torch.distributed process group: ``indices`` are put in
     ``evaluate_plan``'s row order, each rank evaluates a contiguous shard of that order (``distributed.shard_bounds``;
     a shard may be empty, the rank still joins the gather) and every rank gets all rows back.  Rows are per-image exact,
@@ -142,23 +151,25 @@ def evaluate_sharded(plan, ds, indices, loss='lovasz', class_weights=None, chunk
     must call it with the same ``indices``; without a group of more than one process it is ``evaluate_plan``."""
     import torch.distributed as dist
     from .distributed import shard_bounds
+    views = {} if tta == 'none' else {'tta': tta}      # fit's validation makes the call without it
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
-        return evaluate_plan(plan, ds, indices, loss, class_weights, chunk)
+        return evaluate_plan(plan, ds, indices, loss, class_weights, chunk, **views)
     if loss not in LOSSES:      # checked on every rank before the shards part: a rank must not leave the gather
         raise ValueError("loss must be 'weighted_ce', 'lovasz' or 'mixed'")
+    ops.tta_views(tta)
     if len(indices) == 0:
         raise RuntimeError('evaluate: no images')
     if int(chunk) < 1:
         raise ValueError('evaluate: chunk must be at least 1')
     order = width_order(ds, indices)
     start, end = shard_bounds(len(order), dist.get_rank(), dist.get_world_size())
-    mine = evaluate_plan(plan, ds, order[start:end], loss, class_weights, chunk)['rows'] if end > start else []
+    mine = evaluate_plan(plan, ds, order[start:end], loss, class_weights, chunk, **views)['rows'] if end > start else []
     gathered = [None] * dist.get_world_size()
     dist.all_gather_object(gathered, mine)
     return summary([r for part in gathered for r in part])
 
 
-def evaluate(state_dict, ds, indices, loss='lovasz', class_weights=None, precision=DEFAULT_PRECISION, chunk=8):
+def evaluate(state_dict, ds, indices, loss='lovasz', class_weights=None, precision=DEFAULT_PRECISION, chunk=8, tta='none'):
     """Validation of ``state_dict`` on the items ``indices`` of ``ds`` (see the module docstring for the definition).
     Returns {'loss', 'miou', 'f1' (3 values): means over the images, 'rows': one dict per image with the same keys and
     'index'} (rows grouped by width; ``evaluate_plan`` lists the further keys of a row)."""
@@ -168,7 +179,7 @@ def evaluate(state_dict, ds, indices, loss='lovasz', class_weights=None, precisi
         raise RuntimeError('evaluate: no images')
     with torch.cuda.device(ds.device):
         plan = make_plan(state_dict, ds.device, precision)
-    return evaluate_plan(plan, ds, indices, loss, class_weights, chunk)
+    return evaluate_plan(plan, ds, indices, loss, class_weights, chunk, tta)
 
 
 # ---- the command -------------------------------------------------------------------------------------------------
@@ -277,7 +288,7 @@ def main(args):
             for b in range(0, len(mine), args.block):
                 sub = mine[b:b + args.block]
                 ds = load_dataset(args.root, device, items=sub)
-                res = evaluate_plan(plan, ds, range(len(sub)), args.loss, chunk=args.chunk)
+                res = evaluate_plan(plan, ds, range(len(sub)), args.loss, chunk=args.chunk, tta=getattr(args, 'tta', 'none'))
                 by = {r['index']: r for r in res['rows']}
                 for j, i in enumerate(sub):
                     _, _, fname, wood = items[i]
@@ -309,6 +320,8 @@ def parse_args(argv=None):
     parser.add_argument('--block', type=int, default=256, help='images loaded onto the GPU at a time')
     parser.add_argument('--out', default='evaluation.tsv')
     parser.add_argument('--device', default='cuda:0', help='CUDA device (cuda, cuda:N)')
+    parser.add_argument('--tta', default='none', choices=list(ops.TTA_MODES),
+                        help="flip test-time augmentation, as predict --tta: none, h or hv")
     args = parser.parse_args(argv)
     if not args.device.startswith('cuda'):
         parser.error('--device %s: only CUDA devices are supported (no CPU path)' % args.device)

@@ -214,14 +214,19 @@ class NeuralBarkCalculator():
     ``results/final_stats.csv`` for every processed image, plus ``results/combined_images/<wood>/*.png`` as NBC_COMBINED says
     (figure.py: the native two-panel stand-in by default, the reference's matplotlib figure of models.py:280-347 with
     NBC_COMBINED=figure when matplotlib is installed, nothing with NBC_COMBINED=0) -- the same files the streaming
-    FolderPipeline writes."""
+    FolderPipeline writes.
+
+    tta: flip test-time augmentation, 'none' (default), 'h' or 'hv' (``ops.tta_views``): the network runs on each mirrored
+    view of the image and the mask is the argmax of the views' mean logits, each flipped back after the bicubic upsample."""
 
     DEFAULT_MEAN = [0.7399, 0.6139, 0.4401]
     DEFAULT_STD = [0.1068, 0.1272, 0.1271]
     DEFAULT_MM_PER_PIXEL = 3.6 * 3.6
 
     def __init__(self, model_path, device, mean=DEFAULT_MEAN, std=DEFAULT_STD, target_size=1024,
-                 mm_per_pix=DEFAULT_MM_PER_PIXEL, state_dict=None, precision=DEFAULT_PRECISION, load_weights=True):
+                 mm_per_pix=DEFAULT_MM_PER_PIXEL, state_dict=None, precision=DEFAULT_PRECISION, load_weights=True, tta='none'):
+        self.tta_flags = ops.tta_views(tta)[1]
+        self.tta = tta
         self.device = torch.device(device)
         if self.device.type != 'cuda':
             raise RuntimeError("device '%s': this build runs on CUDA (B200) only -- no CPU path" % device)
@@ -252,9 +257,28 @@ class NeuralBarkCalculator():
 
     def predict_array(self, image_u8, excludes_nodes=False):
         """u8 CUDA [H,W,3] processed image -> (u8 mask [H,W] CUDA, counts int32[3] CUDA)."""
-        mask = self.model.predict_mask_u8(image_u8.unsqueeze(0))
+        if self.tta == 'none':
+            mask = self.model.predict_mask_u8(image_u8.unsqueeze(0))
+        else:
+            mask = self.tta_mask(image_u8)
         mask, counts = ops.remove_small_zones_u8(mask, 150, exclude_nodes=excludes_nodes)
         return mask[0], counts[0]
+
+    def tta_mask(self, image_u8):
+        """The mask of ``self.tta``'s view set for one processed image (u8 CUDA [H,W,3]) -> u8 [1,H,W]: the views run as
+        a ragged batch of one image -- flip, network, then the multi-view K3 over all views.  The canvas has at least the
+        16 rows the network takes; rows below the image are zero and take no part."""
+        H, W = image_u8.shape[0], image_u8.shape[1]
+        Hc = max(H, 16)
+        canvas = torch.zeros((1, Hc, W, 3), dtype=torch.uint8, device=image_u8.device)
+        canvas[0, :H] = image_u8
+        heights = torch.tensor([H], dtype=torch.int32, device=image_u8.device)
+        self.model._check_eval()
+        plan = self.model.native_plan()
+        lows = [plan.forward_ragged(canvas if f == 0 else ops.flip_ragged(canvas, heights, f), heights=heights)
+                for f in self.tta_flags]
+        mask = ops.upsample_argmax_views_ragged(lows, self.tta_flags, heights, (Hc, W))
+        return mask[:, :H].contiguous()
 
     def predict(self, root_path, excludes_nodes, processed=None, io_threads=8):
         output_path = join(root_path, 'results')

@@ -393,6 +393,87 @@ def upsample_argmax_ragged(logits, heights, canvas_hw, out=None):
     return out
 
 
+# ---- flip test-time augmentation ------------------------------------------------------------------------------------
+TTA_MODES = ('none', 'h', 'hv')
+_TTA_VIEWS = {'none': (['id'], [0]), 'h': (['id', 'h'], [0, 1]), 'hv': (['id', 'h', 'v', 'hv'], [0, 1, 2, 3])}
+
+
+def tta_views(mode):
+    """The view set of ``--tta mode`` in summation order: (names, flip flags), flag 1 mirrors the columns, 2 the rows of
+    each image's own height.  'none' -> (['id'], [0]); 'h' -> (['id', 'h'], [0, 1]); 'hv' -> (['id', 'h', 'v', 'hv'],
+    [0, 1, 2, 3])."""
+    if mode not in _TTA_VIEWS:
+        raise ValueError("tta must be one of %s (got %r)" % (', '.join(TTA_MODES), mode))
+    names, flags = _TTA_VIEWS[mode]
+    return list(names), list(flags)
+
+
+def flip_ragged(canvas, heights, flags, out=None):
+    """canvas u8 [N,Hc,W,3], heights int32 [N] (CUDA) -> a new canvas with image n mirrored within its rows [0, heights[n])
+    (flags & 2) and its columns (flags & 1), rows below zero (nbc_flip_ragged_u8)."""
+    lib = _lib.load()
+    canvas = _contig(canvas, torch.uint8, 'canvas')
+    heights = _contig(heights, torch.int32, 'heights')
+    if canvas.dim() != 4 or canvas.shape[3] != 3 or tuple(heights.shape) != (canvas.shape[0],):
+        raise RuntimeError('flip_ragged: canvas u8 [N,Hc,W,3] and heights [N] expected')
+    N, Hc, W, _ = canvas.shape
+    with torch.cuda.device(canvas.device):
+        if out is None:
+            out = torch.empty_like(canvas)
+        elif not (out.dtype == torch.uint8 and out.is_contiguous() and out.shape == canvas.shape):
+            raise RuntimeError('flip_ragged: out must be a contiguous u8 tensor of the canvas shape')
+        _lib.check(lib.nbc_flip_ragged_u8(_ptr(canvas), _ptr(out), N, Hc, W, _ptr(heights), int(flags), _stream(canvas.device)),
+                   'nbc_flip_ragged_u8')
+    return out
+
+
+def _view_set(logits, flips, name):
+    """Checked view set: (contiguous f32 canvases, ctypes pointer array, ctypes flag array, (N, hc, w))."""
+    logits = [_contig(t, torch.float32, name) for t in logits]
+    flips = [int(f) for f in flips]
+    if len(logits) != len(flips) or len(logits) not in (1, 2, 4):
+        raise RuntimeError('%s: 1, 2 or 4 views, one flip flag each (got %d canvases, %d flags)' % (name, len(logits), len(flips)))
+    shape = tuple(logits[0].shape)
+    if len(shape) != 4 or shape[1] != 3 or any(tuple(t.shape) != shape for t in logits):
+        raise RuntimeError('%s: every view is an f32 [N,3,hc,w] canvas of one shape' % name)
+    ptrs = (C.c_void_p * len(logits))(*[t.data_ptr() for t in logits])
+    fl = (C.c_int32 * len(flips))(*flips)
+    return logits, ptrs, fl, (shape[0], shape[2], shape[3])
+
+
+def upsample_argmax_views_ragged(logits, flips, heights, canvas_hw, out=None):
+    """Multi-view K3: logits = list of f32 [N,3,hc,w] canvases (the network's output for the batch mirrored with
+    flips[v]), heights int32 [N] -> u8 mask canvas [N,Hc,W] = argmax of the views' mean bicubic logits, each view un-flipped
+    (nbc_upsample_argmax_views_ragged)."""
+    lib = _lib.load()
+    logits, ptrs, fl, (N, hc, w) = _view_set(logits, flips, 'upsample_argmax_views_ragged')
+    heights = _contig(heights, torch.int32, 'heights')
+    Hc, W = canvas_hw
+    dev = logits[0].device
+    with torch.cuda.device(dev):
+        if out is None:
+            out = torch.zeros((N, Hc, W), dtype=torch.uint8, device=dev)
+        _lib.check(lib.nbc_upsample_argmax_views_ragged(ptrs, fl, len(logits), N, hc, w, Hc, W, _ptr(heights), _ptr(out),
+                                                        _stream(dev)), 'nbc_upsample_argmax_views_ragged')
+    return out
+
+
+def upsample_bicubic_views_ragged(logits, flips, heights, canvas_hw, out=None):
+    """The mean logits of ``upsample_argmax_views_ragged`` at full resolution: f32 [N,3,Hc,W], rows [0, heights[n]) of
+    image n written (nbc_upsample_bicubic_views_ragged)."""
+    lib = _lib.load()
+    logits, ptrs, fl, (N, hc, w) = _view_set(logits, flips, 'upsample_bicubic_views_ragged')
+    heights = _contig(heights, torch.int32, 'heights')
+    Hc, W = canvas_hw
+    dev = logits[0].device
+    with torch.cuda.device(dev):
+        if out is None:
+            out = torch.zeros((N, 3, Hc, W), dtype=torch.float32, device=dev)
+        _lib.check(lib.nbc_upsample_bicubic_views_ragged(ptrs, fl, len(logits), N, hc, w, Hc, W, _ptr(heights), _ptr(out),
+                                                         _stream(dev)), 'nbc_upsample_bicubic_views_ragged')
+    return out
+
+
 def heights_from_first_last(first_last, out=None):
     lib = _lib.load()
     first_last = _contig(first_last, torch.int32, 'first_last')
@@ -526,8 +607,20 @@ def eval_ragged(logits, heights, labels, weights=None, losses=EVAL_WCE | EVAL_LO
     ``EVAL_WCE``), ``losses`` a bitmask of EVAL_WCE / EVAL_LOVASZ.  Returns a dict of device tensors: loss_wce f32 [N],
     loss_lovasz f32 [N], cm_raw int64 [N,3,3] (argmax), cm_rsz int64 [N,3,3] (after region removal) and counts int32
     [N,3], each equal to the per-image ops on that image alone (see include/nbc.h)."""
+    return _eval([logits], [0], heights, labels, weights, losses, workspace, views=False)
+
+
+def eval_ragged_views(logits, flips, heights, labels, weights=None, losses=EVAL_WCE | EVAL_LOVASZ, workspace=None):
+    """``eval_ragged`` on a view set (nbc_eval_ragged_views): logits is a list of 1, 2 or 4 canvases, view v the network's
+    output for the chunk mirrored with flips[v] (``flip_ragged``); every output is computed from the views' mean bicubic
+    logits, as ``upsample_bicubic_views_ragged`` gives them."""
+    return _eval(logits, flips, heights, labels, weights, losses, workspace, views=True)
+
+
+def _eval(logits, flips, heights, labels, weights, losses, workspace, views):
+    """nbc_eval_ragged (views=False: the one canvas logits[0]) or nbc_eval_ragged_views."""
     lib = _lib.load()
-    logits = _contig(logits, torch.float32, 'logits')
+    logits, ptrs, fl, _ = _view_set(logits, flips, 'eval_ragged')
     heights = _contig(heights, torch.int32, 'heights')
     labels = _contig(labels, torch.uint8, 'labels')
     if labels.dim() != 3:
@@ -535,12 +628,12 @@ def eval_ragged(logits, heights, labels, weights=None, losses=EVAL_WCE | EVAL_LO
     N, Hc, W = labels.shape
     hc = ((((Hc - 1) // 2 + 1) - 1) // 2 + 1 - 1) // 2 + 1
     w = ((((W - 1) // 2 + 1) - 1) // 2 + 1 - 1) // 2 + 1
-    if tuple(logits.shape) != (N, 3, hc, w) or tuple(heights.shape) != (N,):
+    if tuple(logits[0].shape) != (N, 3, hc, w) or tuple(heights.shape) != (N,):
         raise RuntimeError('eval_ragged: expected logits [%d,3,%d,%d] and heights [%d] for labels %s'
                            % (N, hc, w, N, tuple(labels.shape)))
     if weights is not None:
         weights = _contig(weights, torch.float32, 'weights')
-    dev = logits.device
+    dev = logits[0].device
     with torch.cuda.device(dev):
         need = lib.nbc_eval_workspace_bytes(N, Hc, W)
         if workspace is None or workspace.numel() < need:
@@ -550,10 +643,12 @@ def eval_ragged(logits, heights, labels, weights=None, losses=EVAL_WCE | EVAL_LO
                'cm_raw': torch.empty((N, 3, 3), dtype=torch.int64, device=dev),
                'cm_rsz': torch.empty((N, 3, 3), dtype=torch.int64, device=dev),
                'counts': torch.empty((N, 3), dtype=torch.int32, device=dev)}
-        _lib.check(lib.nbc_eval_ragged(_ptr(logits), N, Hc, W, _ptr(heights), _ptr(labels), _ptr(weights), int(losses),
-                                       _ptr(out['loss_wce']), _ptr(out['loss_lovasz']), _ptr(out['cm_raw']),
-                                       _ptr(out['cm_rsz']), _ptr(out['counts']), _ptr(workspace), workspace.numel(),
-                                       _stream(dev)), 'nbc_eval_ragged')
+        rest = (N, Hc, W, _ptr(heights), _ptr(labels), _ptr(weights), int(losses), _ptr(out['loss_wce']), _ptr(out['loss_lovasz']),
+                _ptr(out['cm_raw']), _ptr(out['cm_rsz']), _ptr(out['counts']), _ptr(workspace), workspace.numel(), _stream(dev))
+        if not views:
+            _lib.check(lib.nbc_eval_ragged(_ptr(logits[0]), *rest), 'nbc_eval_ragged')
+        else:
+            _lib.check(lib.nbc_eval_ragged_views(ptrs, fl, len(logits), *rest), 'nbc_eval_ragged_views')
     return out
 
 

@@ -242,7 +242,7 @@ class FolderPipeline:
         self.batch = batch
         self.io_threads = io_threads or max(4, min(32, (os.cpu_count() or 8)))
         self.png_level = png_compress_level
-        self.engine = PredictEngine(calculator.model, calculator.device, raw_size=RAW)
+        self.engine = PredictEngine(calculator.model, calculator.device, raw_size=RAW, tta=calculator.tta)
 
     def run(self, root_path, excludes_nodes, only_preprocess=False, shard=None):
         """shard=(start, end): process only that slice of the dataset order and return its CSV rows WITHOUT writing

@@ -1,13 +1,17 @@
 """``predict.py`` of the reference (predict.py:1-81) on the B200 path.
 
     python -m neuralbarkcalculator_b200.predict ROOT_DIR [--device cuda:0] [--exclude_nodes] [--only_preprocess]
+        [--tta none|h|hv]
 
-Same arguments, same ``processed/`` and ``results/`` layout, weights from ``./best_model.pt``.  ``--device`` accepts
+Same arguments, same ``processed/`` and ``results/`` layout, weights from ``./best_model.pt``.  ``--tta`` adds flip
+test-time augmentation (``h``: the image and its column mirror, ``hv``: also the row mirrors; the class map is the argmax
+of the views' mean logits); without it every file is the one the plain network gives.  ``--device`` accepts
 ``cuda`` / ``cuda:N``; ``cpu`` is rejected (this build has no CPU path -- use the reference for that)."""
 import argparse
 import os
 
 from .models import NeuralBarkCalculator
+from .ops import TTA_MODES
 
 ALL_WOOD_TYPES = ['epinette_gelee', 'epinette_non_gelee', 'sapin']
 
@@ -51,7 +55,7 @@ def main(args, state_dict=None):
         dist.barrier()
     items = make_dataset(args.root_path)
     model = NeuralBarkCalculator(None if state_dict is not None else './best_model.pt', device, state_dict=state_dict,
-                                 load_weights=not args.only_preprocess)
+                                 load_weights=not args.only_preprocess, tta=getattr(args, 'tta', 'none'))
     if os.environ.get('NBC_TIMING'):
         print('[nbc] folders + model construction: %.3f s' % (time.perf_counter() - t0))
     pipe = pipeline.FolderPipeline(model)
@@ -75,9 +79,13 @@ def parse_args(argv=None):
     parser.add_argument('--device', type=str, default='cuda:0', help='Which CUDA device to run on (cuda, cuda:N).')
     parser.add_argument('--exclude_nodes', action='store_true', default=False)
     parser.add_argument('--only_preprocess', action='store_true', default=False)
+    parser.add_argument('--tta', default='none', choices=list(TTA_MODES),
+                        help='flip test-time augmentation: none, h (image + column mirror) or hv (+ row mirrors)')
     args = parser.parse_args(argv)
     if not args.device.startswith('cuda'):
         parser.error("--device %s: only CUDA devices are supported by this build (no CPU path)" % args.device)
+    if args.only_preprocess and args.tta != 'none':
+        parser.error('--tta %s: --only_preprocess runs no network' % args.tta)
     return args
 
 
